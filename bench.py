@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 sort (BASELINE.json metric: Gpairs/s, key+payload sorted).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c3|c4] [--dump-outputs DIR]
 
 A "step" is one complete sort of one batch of synthetic records.
   N = 1 : --config c2 (default) = BASELINE.json configs[1]: uint64 key + uint64 payload, 1e9 uniform records, ascending
@@ -65,6 +65,8 @@ def parse_args():
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--cpu-sample", type=int, default=0, help="records of the CPU baseline sample (default: per config)")
     ap.add_argument("--opt", action="append", default=[], help="library option name=value (development / ablations)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the arrays the last step sorted as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -235,6 +237,53 @@ def run_reference_arm(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+# ---------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path returned, so that two builds can be compared output for output
+# ---------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 20  # records per dump: at most 5 float64 columns of them, 40 MB
+
+
+def dump_outputs(out_dir: str, cfg: str, work, m: int, world: int, rank: int):
+    """Writes records at fixed positions of the sorted output work[*][:m] as float32 / float64 .npy files.
+
+    The positions are one seeded random record per stratum of m / DUMP_SAMPLE records (every record when m is
+    smaller) and are written too, as positions.npy.  Values are exact: 32-bit and narrower integers become
+    float64, and every 64-bit integer column is split into the unsigned 32-bit halves <name>_hi / <name>_lo of its
+    bit pattern.  The sort is not stable, so payloads of equal keys may legitimately come in another order."""
+    import torch
+    s = min(m, DUMP_SAMPLE // world)
+    if s == m:
+        pos = np.arange(m, dtype=np.int64)
+    else:
+        lo = np.arange(s, dtype=np.int64) * m // s
+        hi = np.arange(1, s + 1, dtype=np.int64) * m // s
+        pos = lo + (np.random.default_rng(SEED).random(s) * (hi - lo)).astype(np.int64)
+    idx = torch.from_numpy(pos).to(work[0].device)
+
+    def take(t):
+        t = t[:m]
+        return (t.view(torch.int64) if t.dtype == torch.uint64 else t)[idx].cpu().numpy()
+
+    if cfg == "c2":
+        cols = {"keys": take(work[0]), "payload": take(work[1])}
+    elif cfg == "c3":
+        cols = {"keys": take(work[0]), "payload_i32": take(work[1]), "payload_f64": take(work[2]),
+                "payload_u16": take(work[3]).view(np.uint16)}
+    else:
+        cols = {"keys": take(work[0][:, 0]), "payload_f64": take(work[0][:, 1]).view(np.float64)}
+    cols["positions"] = pos
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    for name, a in cols.items():
+        if a.dtype.kind in "iu" and a.dtype.itemsize == 8 and name != "positions":
+            u = a.view(np.uint64)
+            np.save(out / f"{prefix}{name}_hi.npy", (u >> np.uint64(32)).astype(np.float64))
+            np.save(out / f"{prefix}{name}_lo.npy", (u & np.uint64(0xFFFFFFFF)).astype(np.float64))
+        else:
+            np.save(out / f"{prefix}{name}.npy", a if a.dtype.kind == "f" else a.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -473,6 +522,8 @@ def main():
     launches = S.launch_count() - launches0
     S.set_option("profile", 0)
     stats = S.last_stats()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cfg, work, out_n[0], world, rank)
 
     total_ms = sum(step_ms)
     if multi:

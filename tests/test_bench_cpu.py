@@ -55,6 +55,38 @@ def test_reference_arm_prints_its_json_line(cfg):
     assert abs(line["ms_per_step"] * 1e-3 * line["value"] * 1e9 - (1 << 16)) < 1
 
 
+@pytest.mark.parametrize("cfg", ["c2", "c3", "c4"])
+def test_dump_outputs_are_exact_float_samples(cfg, tmp_path, monkeypatch):
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    work = bench.device_records(cfg, None, 0, 5000, "cpu")
+    for m, want in ((5000, 1000), (700, 700)):  # a sample of a larger output, all of a smaller one
+        out = tmp_path / str(m)
+        bench.dump_outputs(str(out), cfg, work, m, 1, 0)
+        got = {p.stem: np.load(p) for p in out.glob("*.npy")}
+        assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+        pos = got["positions"].astype(np.int64)
+        assert len(pos) == want and np.all(np.diff(pos) > 0) and pos[0] >= 0 and pos[-1] < m
+
+        def u64(name):
+            return (got[name + "_hi"].astype(np.uint64) << np.uint64(32)) | got[name + "_lo"].astype(np.uint64)
+
+        if cfg == "c2":
+            assert np.array_equal(u64("keys"), work[0].view(torch.int64).numpy().view(np.uint64)[pos])
+            assert np.array_equal(u64("payload"), work[1].view(torch.int64).numpy().view(np.uint64)[pos])
+        elif cfg == "c3":
+            assert got["keys"].tobytes() == work[0].numpy()[pos].tobytes()
+            assert np.array_equal(got["payload_i32"], work[1].numpy()[pos])
+            assert np.array_equal(got["payload_f64"], work[2].numpy()[pos])
+            assert np.array_equal(got["payload_u16"], work[3].numpy().view(np.uint16)[pos])
+        else:
+            rec = work[0].numpy()
+            assert np.array_equal(u64("keys").view(np.int64), rec[pos, 0])
+            assert np.array_equal(got["payload_f64"], rec[pos, 1].view(np.float64))
+    # the positions are a fixed function of (m, sample size)
+    bench.dump_outputs(str(tmp_path / "again"), cfg, work, 5000, 1, 0)
+    assert np.array_equal(np.load(tmp_path / "again" / "positions.npy"), np.load(tmp_path / "5000" / "positions.npy"))
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     import os
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
