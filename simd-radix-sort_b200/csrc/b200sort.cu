@@ -15,8 +15,10 @@
 #include <cstdio>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -60,7 +62,7 @@ static std::atomic<int64_t> opt_mgpu_chunk_min_log2{24};  // ... when a rank hol
 static std::atomic<int64_t> opt_host_plan_min_log2{24};  // hybrid sorts of at least 2^this records read the plan back
 
 // optional per-kernel timing (option "profile"): CUDA events around every launch of the last sort
-enum ProfKind { PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5 };
+enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5 };
 struct ProfEntry { int kind; cudaEvent_t e0, e1; int dev; };
 static std::atomic<int64_t> opt_profile{0};
 static thread_local std::vector<ProfEntry> g_prof;
@@ -75,15 +77,15 @@ static cudaEvent_t prof_event(int dev) {
   if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
   cudaEvent_t e; cudaEventCreate(&e); return e;
 }
-struct ProfScope {
+struct ProfScope {  // (kind PK_NONE: records nothing)
   bool on; ProfEntry pe; cudaStream_t st;
-  ProfScope(int kind, cudaStream_t s) : on(opt_profile.load() != 0), st(s), kind_(kind) {
+  ProfScope(int kind, cudaStream_t s) : on(kind != PK_NONE && opt_profile.load() != 0), st(s), kind_(kind) {
     if (on) { pe.dev = 0; cudaGetDevice(&pe.dev); pe.kind = kind; pe.e0 = prof_event(pe.dev); pe.e1 = prof_event(pe.dev); cudaEventRecord(pe.e0, st); }
   }
   ~ProfScope() {
     if (on) { cudaEventRecord(pe.e1, st); g_prof.push_back(pe); }
     static const bool dbg = getenv("B200SORT_DEBUG_SYNC") != nullptr;  // development: wait for every kernel, say which one
-    if (dbg) {
+    if (dbg && kind_ != PK_NONE) {
       static const char *names[] = {"hist", "scan", "sweep", "copyback", "segfix", "other"};
       fprintf(stderr, "[b200sort] %s launched ...", names[kind_ < 6 ? kind_ : 5]);
       const cudaError_t e = cudaStreamSynchronize(st);
@@ -92,6 +94,29 @@ struct ProfScope {
   }
   int kind_ = 5;
 };
+
+// Every kernel of the library is launched here: on stream st, counted (b200sort_launch_count), and timed for
+// b200sort_last_profile under profile kind `kind` (PK_NONE: not timed).  Returns the launch's error.
+template <typename... P, typename... A>
+static cudaError_t launch(int kind, void (*k)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A &&...args) {
+  {
+    ProfScope ps(kind, st);
+    k<<<grid, block, smem, st>>>(std::forward<A>(args)...);
+  }
+  g_launches++;
+  return cudaGetLastError();
+}
+
+// f(std::integral_constant<int, KB>{}) for the key width kb (1, 2, 4 or 8 bytes): one instantiation per width
+template <typename F>
+static auto with_kb(int kb, F &&f) {
+  switch (kb) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    default: return f(std::integral_constant<int, 8>{});
+  }
+}
 
 static int fail(int code, const char *fmt, ...) {
   char buf[512];
@@ -212,9 +237,7 @@ static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_t
     e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return e;
   }
-  ProfScope ps(PK_SWEEP, st);
   (void)sm_count;
-  // (grid_cap: the partition pass of the overlapped exchange runs with fewer, looping CTAs)
   // L2 prefetch of the tile's part of the first column after the keys (16-byte aligned on both sides)
   a2.prefetch_cols = 0;
   {
@@ -228,9 +251,8 @@ static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_t
       }
     }
   }
-  k<<<(unsigned)(grid_cap > 0 ? std::min<int64_t>(n_tiles, grid_cap) : n_tiles), tc.threads, smem, st>>>(a2);
-  g_launches++;
-  return cudaGetLastError();
+  // (grid_cap: the partition pass of the overlapped exchange runs with fewer, looping CTAs)
+  return launch(PK_SWEEP, k, (unsigned)(grid_cap > 0 ? std::min<int64_t>(n_tiles, grid_cap) : n_tiles), tc.threads, smem, st, a2);
 }
 
 constexpr int HIST_THREADS = 256;  // key-only sweeps: 256 threads x NLD x 16 B per tile, 4 CTAs per SM
@@ -238,18 +260,10 @@ constexpr int hist_nld(int kb) { return kb == 1 ? 2 : (kb >= 4 ? 8 : 4); }  // a
 
 template <int KB, int NLD>
 static cudaError_t launch_hist_t(const HistArgs &a, int grid, bool use_match, int probe, cudaStream_t st) {
-  ProfScope ps(PK_HIST, st);
-  if (probe == 2) {
-    minmax_kernel<KB, HIST_THREADS, NLD><<<grid, HIST_THREADS, 0, st>>>(a);
-  } else if (probe) {
-    if (use_match) probe_kernel<KB, HIST_THREADS, NLD, true><<<grid, HIST_THREADS, 0, st>>>(a);
-    else probe_kernel<KB, HIST_THREADS, NLD, false><<<grid, HIST_THREADS, 0, st>>>(a);
-  } else {
-    if (use_match) hist_kernel<KB, HIST_THREADS, NLD, true><<<grid, HIST_THREADS, 0, st>>>(a);
-    else hist_kernel<KB, HIST_THREADS, NLD, false><<<grid, HIST_THREADS, 0, st>>>(a);
-  }
-  g_launches++;
-  return cudaGetLastError();
+  auto *k = probe == 2 ? minmax_kernel<KB, HIST_THREADS, NLD>
+            : probe    ? (use_match ? probe_kernel<KB, HIST_THREADS, NLD, true> : probe_kernel<KB, HIST_THREADS, NLD, false>)
+                       : (use_match ? hist_kernel<KB, HIST_THREADS, NLD, true> : hist_kernel<KB, HIST_THREADS, NLD, false>);
+  return launch(PK_HIST, k, grid, HIST_THREADS, 0, st, a);
 }
 
 // keys per tile of the key-only sweeps over this key array
@@ -266,14 +280,12 @@ cudaError_t launch_hist(int kb, const HistArgs &a, int sm_count, int probe, cuda
   const int64_t tiles = (a.n + tile_keys - 1) / tile_keys;
   const int grid = (int)std::min<int64_t>(tiles, (int64_t)sm_count * 8);
   const bool m = opt_hist_match.load() != 0;
-  switch (kb) {
-    case 1: return launch_hist_t<1, hist_nld(1)>(a, grid, m, probe, st);
-    case 2: return launch_hist_t<2, hist_nld(2)>(a, grid, m, probe, st);
-    case 4: return launch_hist_t<4, hist_nld(4)>(a, grid, m, probe, st);
-    default:
-      return tile_keys == (int64_t)HIST_THREADS * 4 * 2 ? launch_hist_t<8, 4>(a, grid, m, probe, st)
-                                                        : launch_hist_t<8, hist_nld(8)>(a, grid, m, probe, st);
-  }
+  return with_kb(kb, [&](auto K) {
+    constexpr int KB = decltype(K)::value;
+    if constexpr (KB == 8)
+      if (tile_keys == (int64_t)HIST_THREADS * 4 * 2) return launch_hist_t<8, 4>(a, grid, m, probe, st);
+    return launch_hist_t<KB, hist_nld(KB)>(a, grid, m, probe, st);
+  });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -283,7 +295,8 @@ struct DevInfo { int sm_count = 0; size_t smem_optin = 0; bool ok = false; };
 static std::mutex g_mu;
 static std::map<int, DevInfo> g_dev;
 struct CacheEntry { void *ptr = nullptr; size_t bytes = 0; uint64_t gen = 0; };  // gen: bumped by every (re)allocation
-static std::map<int, CacheEntry> g_cache;
+enum CacheKind { CACHE_WORKSPACE = 0, CACHE_STAGE = 1 };  // the sort's workspace, the staging of host arrays
+static std::map<int, CacheEntry> g_cache[2];              // [kind][device]
 
 // The library-owned caches (workspace, host staging) are one allocation per device.  Sorts that use them are
 // serialised: a per-device (recursive) mutex covers the launching of a sort, and the stream of the next sort
@@ -327,9 +340,10 @@ static int dev_info(int dev, DevInfo *out) {
   return 0;
 }
 
-static int cached_workspace(int dev, size_t bytes, void **out) {
+// the cached buffer of this kind on the current device `dev`, grown to at least `bytes`
+static int cached_buffer(CacheKind kind, int dev, size_t bytes, void **out) {
   std::lock_guard<std::mutex> lk(g_mu);
-  CacheEntry &c = g_cache[dev];
+  CacheEntry &c = g_cache[kind][dev];
   if (c.bytes < bytes) {
     if (c.ptr) {
       CUDA_TRY(cudaDeviceSynchronize());
@@ -341,7 +355,8 @@ static int cached_workspace(int dev, size_t bytes, void **out) {
     cudaError_t e = cudaMalloc(&p, bytes);
     if (e != cudaSuccess) {
       cudaGetLastError();
-      return fail(B200SORT_ENOMEM, "cudaMalloc of %zu workspace bytes failed: %s", bytes, cudaGetErrorString(e));
+      return fail(B200SORT_ENOMEM, "cudaMalloc of %zu %s bytes failed: %s", bytes, kind == CACHE_STAGE ? "staging" : "workspace",
+                  cudaGetErrorString(e));
     }
     c.ptr = p;
     c.bytes = bytes;
@@ -351,14 +366,9 @@ static int cached_workspace(int dev, size_t bytes, void **out) {
   return 0;
 }
 
-static size_t cached_workspace_bytes(int dev) {
+static CacheEntry cache_entry(CacheKind kind, int dev) {
   std::lock_guard<std::mutex> lk(g_mu);
-  return g_cache[dev].bytes;
-}
-
-static uint64_t cached_workspace_gen(int dev) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return g_cache[dev].gen;
+  return g_cache[kind][dev];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -415,11 +425,23 @@ static void make_layout(const std::vector<StreamDesc> &streams, int64_t n, int t
   L->total = align_up(off, 256);
 }
 
-static uint32_t chunk_for(const void *p, uint32_t elem) {
-  // largest power of two <= 16 dividing both the address and the element size
-  uint32_t c = 16;
-  while (c > 1 && ((elem % c) != 0 || ((uintptr_t)p % c) != 0)) c >>= 1;
-  return c;
+// The arrays as the streams the scatter kernel moves: each one in chunks of the largest power of two <= max_chunk
+// (and <= 16) dividing both its address and its element size.  Returns the staging buffer's element size: the
+// largest chunk, at least the key.
+static uint32_t make_stream_set(const std::vector<StreamDesc> &streams, int kb, uint32_t max_chunk, StreamSet *ss) {
+  uint32_t stage_bytes = (uint32_t)kb;
+  *ss = StreamSet{};
+  ss->n_streams = (int)streams.size();
+  for (size_t s = 0; s < streams.size(); s++) {
+    uint32_t c = 16;
+    while (c > 1 && ((streams[s].elem_bytes % c) != 0 || ((uintptr_t)streams[s].ptr % c) != 0)) c >>= 1;
+    c = std::min(c, max_chunk);
+    ss->streams[s].chunk_bytes = c;
+    ss->streams[s].chunks_per_elem = streams[s].elem_bytes / c;
+    ss->streams[s].buf[0] = (unsigned char *)streams[s].ptr;
+    stage_bytes = std::max(stage_bytes, c);
+  }
+  return stage_bytes;
 }
 
 // Sort arrays that are all in device memory.  streams[0] carries the key at offset 0.
@@ -432,8 +454,7 @@ struct DevSortOpts {
                                 // there (landing -> shadow -> caller -> ...), so that an even number of passes
                                 // ends in the caller's arrays without a copy
   int force_algo = 0;           // 1 / 2: use this algorithm whatever option "algo" says (the hybrid path's fall-back)
-  // Multi-GPU sort with the exchange overlapped (mgpu.cuh): the plan is fixed by the caller (hybrid: digit
-  // positions forced_cut .. 7 of the key shifted left by forced_lshift are swept, no range reduction), the
+  // Multi-GPU sort with the exchange overlapped (mgpu.cuh): the plan is fixed by the caller (forced_plan), the
   // control block has been cleared by the caller, and the FIRST executed pass has already been run by the
   // caller (landing arrays -> shadow arrays, its successor's digit counted into the exact histograms).
   bool forced = false;
@@ -452,235 +473,231 @@ static cudaEvent_t plan_event_of(int dev) {
   if (e == nullptr && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) e = nullptr;
   return e;
 }
+
+// The plan of the overlapped multi-GPU exchange's local sort: the hybrid sweep of digit positions cut .. kb-1 of
+// the key shifted left by lshift, in LSD order, without range reduction; the first of them is run by the caller.
+static Plan forced_plan(int kb, uint32_t cut, uint32_t lshift) {
+  Plan p{};
+  uint32_t sel = 0, prev = 0;
+  bool any_prev = false;
+  for (int d = 0; d < kb; d++) {
+    p.skip[d] = (uint32_t)d < cut ? 1u : 0u;
+    p.src_sel[d] = sel;
+    if (!p.skip[d]) {
+      sel ^= 1u;
+      p.n_exec++;
+      if (!any_prev) p.first_exec_p1 = (uint32_t)d + 1; else p.next_exec_p1[prev] = (uint32_t)d + 1;
+      prev = (uint32_t)d;
+      any_prev = true;
+    }
+  }
+  p.final_sel = sel;
+  p.cut_digit = cut;
+  p.lshift = lshift;
+  p.hist_done = 1;
+  return p;
+}
+
 static int sort_device(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
-                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo = DevSortOpts()) {
-  const int start_sel = xo.start_sel;
-  const int64_t layout_n = xo.layout_n;
-  const int hint_lead_bits = xo.hint_lead_bits;
+                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo = DevSortOpts());
+
+// One sort of device arrays, phase by phase: one histogram sweep over all digit positions, the bucket-offset scan
+// (+ pass plan), one scatter pass per digit position, the segment finish, the copy-back.
+struct DevSort {
+  const int key_type;
+  const bool ascending;
+  const int64_t n;
+  const std::vector<StreamDesc> &streams;
+  const cudaStream_t stream;
+  void *const caller_workspace;
+  const size_t workspace_bytes;
+  const DevSortOpts &xo;
   const int kb = key_bytes_of(key_type);
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
+  // set-up
+  int dev = 0, cfg = 0, tile = 0, algo = 0;
+  bool hybrid = false;
   DevInfo di;
-  if (int rc = dev_info(dev, &di)) return rc;
-
-  uint32_t stage_bytes = (uint32_t)kb, rec_bytes = 0;
   StreamSet ss{};
-  ss.n_streams = (int)streams.size();
-  for (size_t s = 0; s < streams.size(); s++) {
-    const uint32_t c = std::min<uint32_t>(chunk_for(streams[s].ptr, streams[s].elem_bytes), (uint32_t)std::max<int64_t>(opt_max_chunk.load(), 1));
-    ss.streams[s].chunk_bytes = c;
-    ss.streams[s].chunks_per_elem = streams[s].elem_bytes / c;
-    ss.streams[s].buf[0] = (unsigned char *)streams[s].ptr;
-    stage_bytes = std::max(stage_bytes, c);
-    rec_bytes += streams[s].elem_bytes;
-  }
-  if (streams[0].elem_bytes != (uint32_t)kb && ((uintptr_t)streams[0].ptr % kb) != 0)
-    return fail(B200SORT_EINVAL, "record array is not aligned to its key type");
-  if (((uintptr_t)streams[0].ptr % kb) != 0) return fail(B200SORT_EINVAL, "key array is not aligned to its key type");
-
-  const int cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, n);
-  const TileCfg tc = kTileCfgs[cfg];
-  const int tile = tc.threads * tc.ipt;
-  const size_t smem = sweep_smem_bytes(tc, stage_bytes);
-  if (smem > di.smem_optin) return fail(B200SORT_ECUDA, "device offers %zu B of shared memory, %zu needed", di.smem_optin, smem);
-
+  uint32_t stage_bytes = 0;
   Layout L;
-  make_layout(streams, std::max(n, layout_n), std::min(tile, HYB_MIN_TILE), &L, xo.layout_landing);
-  void *const caller_workspace = workspace;
+  unsigned char *ws = nullptr;
+  Plan *plan = nullptr;  // (device)
+  HybridCtrl *ctrl = nullptr;
+  KeyOrder ko{};
   CacheGuard cache_guard;  // released (and its event recorded) when this sort has been launched
-  if (workspace == nullptr) {
-    cache_guard.acquire(dev, stream);
-    if (int rc = cached_workspace(dev, L.total, &workspace)) return rc;
-  } else if (workspace_bytes < L.total) {
-    return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", workspace_bytes, L.total);
-  } else if (((uintptr_t)workspace % 256) != 0) {
-    return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
+  // plan
+  Plan hplan{};
+  bool have_plan = false;    // the host knows the plan (hplan): launches only what executes
+  bool landing = false;      // the first executed pass reads the landing arrays (ss_in)
+  StreamSet ss_in{};         // what the key sweeps and the first executed pass read
+  uint32_t hist_sweeps = 1;  // probe (+ exact min/max) (+ exact histogram of the first pass)
+  // passes, finish
+  bool partial = false;      // partial-sort mode: no ordering of the final segments, only a check of their lengths
+  int last_pass = -1;        // the last pass orders the tile-local final segments (junction fix follows)
+  bool fix_flow = false;     // the finish is gated on the device by ctrl->flags[1]
+  bool finish_ran = false;
+
+  // set-up: streams, tile geometry, workspace layout, workspace (and the cache guard if it is the library's)
+  int setup() {
+    CUDA_TRY(cudaGetDevice(&dev));
+    if (int rc = dev_info(dev, &di)) return rc;
+    stage_bytes = make_stream_set(streams, kb, (uint32_t)std::max<int64_t>(opt_max_chunk.load(), 1), &ss);
+    if (streams[0].elem_bytes != (uint32_t)kb && ((uintptr_t)streams[0].ptr % kb) != 0)
+      return fail(B200SORT_EINVAL, "record array is not aligned to its key type");
+    if (((uintptr_t)streams[0].ptr % kb) != 0) return fail(B200SORT_EINVAL, "key array is not aligned to its key type");
+
+    cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, n);
+    const TileCfg tc = kTileCfgs[cfg];
+    tile = tc.threads * tc.ipt;
+    const size_t smem = sweep_smem_bytes(tc, stage_bytes);
+    if (smem > di.smem_optin) return fail(B200SORT_ECUDA, "device offers %zu B of shared memory, %zu needed", di.smem_optin, smem);
+
+    make_layout(streams, std::max(n, xo.layout_n), std::min(tile, HYB_MIN_TILE), &L, xo.layout_landing);
+    void *workspace = caller_workspace;
+    if (workspace == nullptr) {
+      cache_guard.acquire(dev, stream);
+      if (int rc = cached_buffer(CACHE_WORKSPACE, dev, L.total, &workspace)) return rc;
+    } else if (workspace_bytes < L.total) {
+      return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", workspace_bytes, L.total);
+    } else if (((uintptr_t)workspace % 256) != 0) {
+      return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
+    }
+    ws = (unsigned char *)workspace;
+    for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
+    plan = (Plan *)(ws + L.plan_off);
+    ctrl = (HybridCtrl *)(ws + L.hyb_off);
+    if (!xo.forced) prof_reset();
+    if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
+
+    ko = make_key_order(key_type, ascending);
+    algo = xo.force_algo != 0 ? xo.force_algo : (int)opt_algo.load();
+    if (xo.forced) algo = 2;
+    if (algo == 0) algo = (kb == 8 && n >= HYB_MIN_N) ? 2 : 1;
+    if (algo == 2 && kb != 8) algo = 1;
+    hybrid = algo == 2;
+    return 0;
   }
-  unsigned char *ws = (unsigned char *)workspace;
-  for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
-  uint64_t *ghist = (uint64_t *)(ws + L.ghist_off);
-  uint32_t *tile_counter = (uint32_t *)(ws + L.tilectr_off);
-  Plan *plan = (Plan *)(ws + L.plan_off);
-  uint64_t *lookback = (uint64_t *)(ws + L.lookback_off);
 
-  const uint64_t launches_before = g_launches.load();
-  if (!xo.forced) prof_reset();
-  if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
+  // input in the landing arrays, delivered into the caller's arrays by a copy
+  int deliver_landing() {
+    for (size_t s = 0; s < streams.size(); s++)
+      CUDA_TRY(cudaMemcpyAsync(streams[s].ptr, ws + L.land_off[s], (size_t)n * streams[s].elem_bytes, cudaMemcpyDeviceToDevice, stream));
+    return 0;
+  }
 
-  const KeyOrder ko = make_key_order(key_type, ascending);
+  int read_plan(cudaEvent_t ev) {
+    CUDA_TRY(cudaMemcpyAsync(&hplan, plan, sizeof hplan, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaEventRecord(ev, stream));
+    CUDA_TRY(cudaEventSynchronize(ev));
+    return 0;
+  }
 
-  int algo = xo.force_algo != 0 ? xo.force_algo : (int)opt_algo.load();
-  if (xo.forced) algo = 2;
-  if (algo == 0) algo = (kb == 8 && n >= HYB_MIN_N) ? 2 : 1;
-  if (algo == 2 && kb != 8) algo = 1;
-
-  b200sort_stats stt{};
-  stt.num = n;
-  stt.record_bytes = rec_bytes;
-  stt.key_bytes = (uint32_t)kb;
-  stt.algo = (uint32_t)algo;
-
-  const bool hybrid = algo == 2;
-  {
-    // ---- one histogram sweep over all digit positions, the bucket-offset scan (+ pass plan), one
-    //      scatter pass per digit position (skipped ones return at once), segment finish, copy-back ----
-    uint64_t *ghist_exact = (uint64_t *)(ws + L.ghist2_off);
-    ProbeOut *probe = (ProbeOut *)(ws + L.probe_off);
-    // large sorts (any algorithm): the host reads the plan back and launches exactly what executes, with the
-    // plan's values as kernel arguments and the lean kernel instantiations they allow
+  // plan: the probe (sampled histograms + the exact histogram of the guessed first digit) and the scan that makes
+  // the plan.  Large sorts read the plan back (small D2H, one host wait) and launch only what executes: the exact
+  // min/max sweep and a second planning step if asked for, the histogram kernel unless the probe's guess was
+  // right, the passes that are not skipped.  Smaller sorts launch everything; what is not needed returns at once.
+  int make_plan() {
+    uint64_t *ghist = (uint64_t *)(ws + L.ghist_off), *ghist_exact = (uint64_t *)(ws + L.ghist2_off);
     const bool big = xo.forced || n >= (int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_host_plan_min_log2.load(), 0), 62);
     // Input in the landing arrays (multi-GPU): only the large hybrid flow knows on the host which pass runs
     // first; everything else simply starts with a copy into the caller's arrays.
-    bool landing = xo.landing_input;
-    auto copy_landing_to_caller = [&]() -> int {
-      for (size_t s2 = 0; s2 < streams.size(); s2++)
-        CUDA_TRY(cudaMemcpyAsync(streams[s2].ptr, ws + L.land_off[s2], (size_t)n * streams[s2].elem_bytes, cudaMemcpyDeviceToDevice, stream));
-      return 0;
-    };
+    landing = xo.landing_input;
     if (landing && !big) {
-      if (int rc = copy_landing_to_caller()) return rc;
+      if (int rc = deliver_landing()) return rc;
       landing = false;
     }
-    StreamSet ss_in = ss;  // what the key sweeps and the first executed pass read
+    ss_in = ss;
     if (landing)
-      for (size_t s2 = 0; s2 < streams.size(); s2++) ss_in.streams[s2].buf[0] = ws + L.land_off[s2];
+      for (size_t s = 0; s < streams.size(); s++) ss_in.streams[s].buf[0] = ws + L.land_off[s];
     HistArgs ha{};
-    ha.keys = ss_in.streams[0].buf[start_sel];
+    ha.keys = ss_in.streams[0].buf[xo.start_sel];
     ha.stride = streams[0].elem_bytes;
-    ha.n = n; ha.ko = ko; ha.digit_mask = (1u << kb) - 1; ha.ghist = ghist; ha.probe = probe;
-    {
-      const int64_t tile_keys = hist_tile_keys(kb, ha.keys, ha.stride);
-      // entropies from one key per thread of every 16th tile (option probe_sample) once there are plenty of tiles
-      const bool sparse = (n / tile_keys) >= 8192;
-      ha.sample = sparse ? (uint32_t)std::max<int64_t>(1, opt_probe_sample.load()) : 1;
-      ha.sample_one = sparse ? 1 : 0;
-    }
+    ha.n = n; ha.ko = ko; ha.digit_mask = (1u << kb) - 1; ha.ghist = ghist; ha.probe = (ProbeOut *)(ws + L.probe_off);
+    // entropies from one key per thread of every 16th tile (option probe_sample) once there are plenty of tiles
+    const bool sparse = (n / hist_tile_keys(kb, ha.keys, ha.stride)) >= 8192;
+    ha.sample = sparse ? (uint32_t)std::max<int64_t>(1, opt_probe_sample.load()) : 1;
+    ha.sample_one = sparse ? 1 : 0;
     // Large sorts leave the exact key range to a sweep of its own that only runs when the sampled range says
     // range reduction may pay; the others get it from the probe.
     ha.with_minmax = big ? 0 : 1;
     // The digit position the first pass will sweep if the keys are (close to) uniformly distributed: the
     // probe counts it exactly, and if the plan comes out that way hist_kernel is not needed.
-    {
-      uint32_t guess = 0, guess_l = 0;
-      if (hybrid) {
-        // hint_lead_bits: leading bits the caller expects all keys to agree on (a shard of the multi-GPU sort)
-        const double need = std::log2((double)n) + (double)opt_margin_bits.load();
-        const int swept = (int)std::ceil(need / 8.0);
-        const int shift_l = opt_allow_lshift.load() != 0 ? (hint_lead_bits & 7) : 0;
-        const int cut = 8 - hint_lead_bits / 8 - swept;
-        if (cut >= 2) { guess = (uint32_t)cut; guess_l = (uint32_t)shift_l; }
+    // (digit-by-digit path: the least significant digit, guess = 0, is the first pass unless it is constant)
+    uint32_t guess = 0;
+    if (hybrid) {
+      // hint_lead_bits: leading bits the caller expects all keys to agree on (a shard of the multi-GPU sort)
+      const double need = std::log2((double)n) + (double)opt_margin_bits.load();
+      const int cut = 8 - xo.hint_lead_bits / 8 - (int)std::ceil(need / 8.0);
+      if (cut >= 2) {
+        guess = (uint32_t)cut;
+        ha.guess_lshift = opt_allow_lshift.load() != 0 ? (uint32_t)(xo.hint_lead_bits & 7) : 0u;
       }
-      // (digit-by-digit path: the least significant digit, guess = 0, is the first pass unless it is constant)
-      ha.guess_lshift = guess_l;
-      ha.guess_p1 = opt_probe_guess.load() != 0 ? guess + 1 : 0;
-      ha.ghist_exact = ghist_exact;
     }
-    if (!xo.forced) CUDA_TRY(launch_hist(kb, ha, di.sm_count, /*probe=*/1, stream));
+    ha.guess_p1 = opt_probe_guess.load() != 0 ? guess + 1 : 0;
+    ha.ghist_exact = ghist_exact;
+    if (xo.forced) {  // the caller's plan (its probe, scan and first pass ran overlapped with the exchange)
+      hist_sweeps = 0;
+      hplan = forced_plan(kb, xo.forced_cut, xo.forced_lshift);
+      CUDA_TRY(cudaMemcpyAsync(plan, &hplan, sizeof hplan, cudaMemcpyHostToDevice, stream));
+      have_plan = true;
+      return 0;
+    }
+    CUDA_TRY(launch_hist(kb, ha, di.sm_count, /*probe=*/1, stream));
 
     ScanArgs sa{};
-    sa.ghist = ghist; sa.probe = probe; sa.plan = plan; sa.n = n; sa.n_passes = kb;
+    sa.ghist = ghist; sa.probe = ha.probe; sa.plan = plan; sa.n = n; sa.n_passes = kb;
     sa.allow_skip = (int)opt_allow_skip.load();
     sa.hybrid = hybrid ? 1 : 0;
     sa.allow_reduce = (int)opt_allow_reduce.load();
     sa.margin_bits = (float)opt_margin_bits.load();
     sa.have_minmax = (int)ha.with_minmax;
     sa.allow_lshift = (int)opt_allow_lshift.load();
-    sa.start_sel = (uint32_t)start_sel;
+    sa.start_sel = (uint32_t)xo.start_sel;
     sa.guess_p1 = ha.guess_p1; sa.guess_lshift = ha.guess_lshift; sa.ghist_exact = ghist_exact;
-    auto launch_scan = [&]() -> int {
-      {
-        ProfScope ps(PK_SCAN, stream);
-        scan_kernel<<<1, RADIX, 0, stream>>>(sa);
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      return 0;
-    };
-    if (!xo.forced)
-      if (int rc = launch_scan()) return rc;
+    CUDA_TRY(launch(PK_SCAN, scan_kernel, 1, RADIX, 0, stream, sa));
 
-    // Large hybrid sorts read the plan back (small D2H, one host wait) and launch only what executes: the
-    // exact min/max sweep and a second planning step if asked for, the histogram kernel unless the probe's
-    // guess was right, the passes that are not skipped.  Smaller sorts launch everything; what is not
-    // needed returns at once.
-    Plan hplan{};
-    bool have_plan = false;
-    cudaEvent_t plan_event = nullptr;
-    HistArgs hb = ha;
+    HistArgs hb = ha;  // exact histogram of the first executed pass only; every pass counts its successor's digit
     hb.ghist = ghist_exact; hb.plan = plan; hb.probe = nullptr;
-    uint32_t hist_sweeps = 1;
-    if (xo.forced) {
-      // the caller's plan: sweep digit positions forced_cut .. kb-1 in LSD order; the first of them is done
-      hist_sweeps = 0;
-      uint32_t sel = 0, prev = 0;
-      bool any_prev = false;
-      for (int p = 0; p < kb; p++) {
-        hplan.skip[p] = (uint32_t)p < xo.forced_cut ? 1u : 0u;
-        hplan.src_sel[p] = sel;
-        if (!hplan.skip[p]) {
-          sel ^= 1u;
-          hplan.n_exec++;
-          if (!any_prev) hplan.first_exec_p1 = (uint32_t)p + 1; else hplan.next_exec_p1[prev] = (uint32_t)p + 1;
-          prev = (uint32_t)p;
-          any_prev = true;
-        }
-      }
-      hplan.final_sel = sel;
-      hplan.cut_digit = xo.forced_cut;
-      hplan.lshift = xo.forced_lshift;
-      hplan.hist_done = 1;
-      CUDA_TRY(cudaMemcpyAsync(plan, &hplan, sizeof hplan, cudaMemcpyHostToDevice, stream));
-      have_plan = true;
-    } else if (big) {
-      plan_event = plan_event_of(dev);
-      if (plan_event == nullptr) return fail(B200SORT_ECUDA, "cudaEventCreate failed on device %d", dev);
-      CUDA_TRY(cudaMemcpyAsync(&hplan, plan, sizeof hplan, cudaMemcpyDeviceToHost, stream));
-      CUDA_TRY(cudaEventRecord(plan_event, stream));
-      CUDA_TRY(cudaEventSynchronize(plan_event));
+    if (big) {
+      const cudaEvent_t ev = plan_event_of(dev);
+      if (ev == nullptr) return fail(B200SORT_ECUDA, "cudaEventCreate failed on device %d", dev);
+      if (int rc = read_plan(ev)) return rc;
       if (hplan.want_minmax) {
         CUDA_TRY(launch_hist(kb, ha, di.sm_count, /*minmax=*/2, stream));
         hist_sweeps++;
         sa.have_minmax = 1;
-        if (int rc = launch_scan()) return rc;
-        CUDA_TRY(cudaMemcpyAsync(&hplan, plan, sizeof hplan, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaEventRecord(plan_event, stream));
-        CUDA_TRY(cudaEventSynchronize(plan_event));
+        CUDA_TRY(launch(PK_SCAN, scan_kernel, 1, RADIX, 0, stream, sa));
+        if (int rc = read_plan(ev)) return rc;
       }
       have_plan = true;
-      if (!hplan.hist_done) {
-        CUDA_TRY(launch_hist(kb, hb, di.sm_count, /*probe=*/0, stream));
-        hist_sweeps++;
-      }
-    } else {
-      // exact histogram of the first executed pass only; every pass counts its successor's digit
-      CUDA_TRY(launch_hist(kb, hb, di.sm_count, /*probe=*/0, stream));
-      hist_sweeps++;
+      if (hplan.hist_done) return 0;
     }
+    CUDA_TRY(launch_hist(kb, hb, di.sm_count, /*probe=*/0, stream));
+    hist_sweeps++;
+    return 0;
+  }
 
-    const int64_t n_tiles = (n + tile - 1) / tile;
-    HybridCtrl *ctrl = (HybridCtrl *)(ws + L.hyb_off);
-    // With the plan on the host, an 8-byte-key SoA sort lets the LAST pass order the final segments each tile
-    // holds and repairs the tile-straddling ones with junction_fix_kernel; the full segment finish then only
-    // runs if one of them reports a run that is too long.
+  // passes: one scatter pass per digit position (skipped ones return at once, or are not launched if the host
+  // knows the plan).  With the plan on the host, an 8-byte-key SoA sort lets the LAST pass order the final
+  // segments each tile holds and repairs the tile-straddling ones with junction_fix_kernel (see finish).
+  int run_passes() {
     const bool soa = streams[0].elem_bytes == (uint32_t)kb;
-    // partial-sort mode: no ordering of the final segments at all, only a check that none exceeds the threshold
-    const bool partial = have_plan && hplan.cut_digit != 0 && xo.cmp_none_thresh >= CMP_NONE_MIN_THRESH;
-    const bool use_fix = !partial && have_plan && hplan.cut_digit != 0 && (soa || ss.streams[0].chunk_bytes >= (uint32_t)kb) && cfg == kDefaultTileCfg && opt_fix_in_pass.load() != 0;
-    int last_pass = -1;
+    partial = have_plan && hplan.cut_digit != 0 && xo.cmp_none_thresh >= CMP_NONE_MIN_THRESH;
+    const bool use_fix = !partial && have_plan && hplan.cut_digit != 0 && (soa || ss.streams[0].chunk_bytes >= (uint32_t)kb) &&
+                         cfg == kDefaultTileCfg && opt_fix_in_pass.load() != 0;
+    if (landing && hplan.n_exec == 0)  // nothing will move the records: deliver them
+      if (int rc = deliver_landing()) return rc;
     bool first_exec = true;
-    if (landing && hplan.n_exec == 0) {  // nothing will move the records: deliver them
-      if (int rc = copy_landing_to_caller()) return rc;
-    }
     for (int p = 0; p < kb; p++) {
       if (have_plan && hplan.skip[p]) continue;
-      SweepArgs wa{};
-      wa.ss = (landing && first_exec) ? ss_in : ss; wa.n = n;
       const bool was_first = first_exec;
       first_exec = false;
       if (xo.forced && was_first) continue;  // run by the caller, overlapped with the exchange
+      SweepArgs wa{};
+      wa.ss = (landing && was_first) ? ss_in : ss; wa.n = n;
       wa.ko = ko; wa.pass = p; wa.shift = p * RADIX_BITS;
-      wa.bin_base = nullptr; wa.ghist = ghist_exact;
-      wa.lookback = lookback; wa.tile_counter = tile_counter; wa.plan = plan;
+      wa.bin_base = nullptr; wa.ghist = (uint64_t *)(ws + L.ghist2_off);
+      wa.lookback = (uint64_t *)(ws + L.lookback_off); wa.tile_counter = (uint32_t *)(ws + L.tilectr_off); wa.plan = plan;
       wa.tag = (uint32_t)(p + 1); wa.stage_bytes = stage_bytes; wa.spin_ns = (uint32_t)opt_spin_ns.load();
       if (have_plan) {
         wa.plan_in_args = 1; wa.arg_sel = hplan.src_sel[p]; wa.arg_next_p1 = hplan.next_exec_p1[p];
@@ -689,112 +706,119 @@ static int sort_device(int key_type, bool ascending, int64_t n, const std::vecto
       }
       // the first executed pass may rank its keys in any order (nothing has been established yet)
       const bool unordered = have_plan && was_first && hplan.skewed[p] == 0;
-      CUDA_TRY(launch_sweep(kb, cfg, wa, n_tiles, di.smem_optin, di.sm_count, stream, unordered));
+      CUDA_TRY(launch_sweep(kb, cfg, wa, (n + tile - 1) / tile, di.smem_optin, di.sm_count, stream, unordered));
     }
-    auto launch_segfix = [&](const uint32_t *gate) -> int {
-      SegfixArgs fa{};
-      fa.ss = ss; fa.n = n; fa.ko = ko; fa.plan = plan; fa.ctrl = ctrl; fa.gate = gate;
-      if (have_plan) { fa.plan_in_args = 1; fa.arg_cut = hplan.cut_digit; fa.arg_sel = hplan.final_sel; fa.arg_sub = hplan.sub; fa.arg_lshift = hplan.lshift; }
-      bool any = false;
-      for (int s = 0; s < ss.n_streams; s++) any = any || ss.streams[s].chunk_bytes < 4;
-      const unsigned grid = (unsigned)std::min<int64_t>((n + SF_FT - 1) / SF_FT, (int64_t)di.sm_count * 16);
-      {
-        ProfScope ps(PK_SEGFIX, stream);
-        if (any) segfix_kernel<8, true><<<grid, SF_THREADS, 0, stream>>>(fa);
-        else segfix_kernel<8, false><<<grid, SF_THREADS, 0, stream>>>(fa);
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      return 0;
-    };
-    auto launch_copyback = [&](bool force, const uint32_t *skip_if) -> int {
-      CopyBackArgs ca{};
-      ca.ss = ss; ca.n = n; ca.plan = plan; ca.force = force ? 1 : 0; ca.skip_if = skip_if;
-      {
-        ProfScope ps(PK_COPYBACK, stream);
-        copyback_kernel<<<di.sm_count * 8, 256, 0, stream>>>(ca);
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      return 0;
-    };
-    bool finish_ran = false, fix_flow = false;
+    return 0;
+  }
+
+  // the full segment finish (gate: it only runs if *gate != 0), which delivers into the caller's arrays
+  cudaError_t launch_segfix(const uint32_t *gate) {
+    SegfixArgs fa{};
+    fa.ss = ss; fa.n = n; fa.ko = ko; fa.plan = plan; fa.ctrl = ctrl; fa.gate = gate;
+    if (have_plan) { fa.plan_in_args = 1; fa.arg_cut = hplan.cut_digit; fa.arg_sel = hplan.final_sel; fa.arg_sub = hplan.sub; fa.arg_lshift = hplan.lshift; }
+    bool any = false;
+    for (int s = 0; s < ss.n_streams; s++) any = any || ss.streams[s].chunk_bytes < 4;
+    const unsigned grid = (unsigned)std::min<int64_t>((n + SF_FT - 1) / SF_FT, (int64_t)di.sm_count * 16);
+    return launch(PK_SEGFIX, any ? segfix_kernel<8, true> : segfix_kernel<8, false>, grid, SF_THREADS, 0, stream, fa);
+  }
+
+  // the result out of the shadow arrays if it ended there (force: whatever the plan says; skip_if: not if *skip_if)
+  cudaError_t launch_copyback(bool force, const uint32_t *skip_if) {
+    CopyBackArgs ca{};
+    ca.ss = ss; ca.n = n; ca.plan = plan; ca.force = force ? 1 : 0; ca.skip_if = skip_if;
+    return launch(PK_COPYBACK, copyback_kernel, di.sm_count * 8, 256, 0, stream, ca);
+  }
+
+  // finish: the final segments ordered, or checked in partial-sort mode, and the result in the caller's arrays
+  int finish() {
+    const uint32_t *flag = &ctrl->flags[1];
     if (last_pass >= 0) {
+      const int64_t n_tiles = (n + tile - 1) / tile;
       JunctionArgs ja{};
-      ja.ss = ss; ja.n = n; ja.ko = ko; ja.ko.sub = hplan.sub; ja.ko.lshift = hplan.lshift; ja.lookback = lookback; ja.n_tiles = n_tiles;
-      ja.tag = (uint32_t)(last_pass + 1); ja.cut = hplan.cut_digit; ja.sel = hplan.final_sel; ja.flag = &ctrl->flags[1];
+      ja.ss = ss; ja.n = n; ja.ko = ko; ja.ko.sub = hplan.sub; ja.ko.lshift = hplan.lshift; ja.lookback = (uint64_t *)(ws + L.lookback_off);
+      ja.n_tiles = n_tiles; ja.tag = (uint32_t)(last_pass + 1); ja.cut = hplan.cut_digit; ja.sel = hplan.final_sel; ja.flag = &ctrl->flags[1];
       ja.jtable = opt_junction_table.load() != 0 ? (const uint64_t *)(ws + L.jtable_off) : nullptr;
-      const int64_t threads = n_tiles * RADIX;
-      {
-        ProfScope ps(PK_SEGFIX, stream);
-        junction_fix_kernel<8><<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(ja);
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      // Both possible continuations are launched; which one does anything is decided on the device by the flag
-      // the last pass / the junction kernel raise when they meet a run that is too long for them: the full
-      // segment finish repairs everything (and delivers the result into the caller's arrays), else the result
-      // is copied out of the shadow if it ended there.  No host round trip in between.
-      if (int rc = launch_segfix(&ctrl->flags[1])) return rc;
-      if (hplan.final_sel == 1)
-        if (int rc = launch_copyback(true, &ctrl->flags[1])) return rc;
-      fix_flow = true;
+      CUDA_TRY(launch(PK_SEGFIX, junction_fix_kernel<8>, (unsigned)((n_tiles * RADIX + 255) / 256), 256, 0, stream, ja));
     } else if (partial) {
       PartialCheckArgs pa{};
       pa.ss = ss; pa.n = n; pa.ko = ko; pa.ko.sub = hplan.sub; pa.ko.lshift = hplan.lshift; pa.cut = hplan.cut_digit; pa.sel = hplan.final_sel;
       pa.thresh = xo.cmp_none_thresh; pa.flag = &ctrl->flags[1];
-      {
-        ProfScope ps(PK_SEGFIX, stream);
-        partial_check_kernel<8><<<di.sm_count * 8, 256, 0, stream>>>(pa);
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-      if (int rc = launch_segfix(&ctrl->flags[1])) return rc;  // runs only if a segment longer than the threshold is out of order
-      if (hplan.final_sel == 1)
-        if (int rc = launch_copyback(true, &ctrl->flags[1])) return rc;
-      fix_flow = true;
+      CUDA_TRY(launch(PK_SEGFIX, partial_check_kernel<8>, di.sm_count * 8, 256, 0, stream, pa));
     } else {
       if (hybrid && !(have_plan && hplan.cut_digit == 0)) {
-        if (int rc = launch_segfix(nullptr)) return rc;
+        CUDA_TRY(launch_segfix(nullptr));
         finish_ran = true;
       }
-      if (int rc = launch_copyback(false, nullptr)) return rc;
+      CUDA_TRY(launch_copyback(false, nullptr));
+      return 0;
     }
-    stt.passes_planned = (uint32_t)kb;
-    stt.hist_sweeps = hist_sweeps;  // probe (+ exact min/max) (+ exact histogram of the first pass)
-    stt.algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)kb * 2ull * (uint64_t)n * rec_bytes;
-    if (have_plan) {  // the executed passes are known
-      stt.passes_planned = hplan.n_exec;
-      stt.algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)hplan.n_exec * 2ull * (uint64_t)n * rec_bytes;
-    }
+    // Both possible continuations are launched; which one does anything is decided on the device by the flag the
+    // last pass / the junction kernel / the partial check raise when they meet a run that is too long for them:
+    // the full segment finish repairs everything (and delivers the result into the caller's arrays), else the
+    // result is copied out of the shadow if it ended there.  No host round trip in between.
+    CUDA_TRY(launch_segfix(flag));
+    if (hplan.final_sel == 1) CUDA_TRY(launch_copyback(true, flag));
+    fix_flow = true;
+    return 0;
+  }
+
+  // statistics of what ran.  The hybrid path reads its plan (made on the device) and its flags back: its one
+  // host synchronisation.  *fall_back: a long bucket with distinct keys is left for the digit-by-digit path.
+  int statistics(b200sort_stats *stt, bool *fall_back) {
+    HybridCtrl hctrl{};
     if (hybrid) {
-      // The plan was made on the device; read it (and the fall-back flag) back.  This is the one host
-      // synchronisation of the hybrid path.
-      HybridCtrl hctrl{};
       if (!have_plan) CUDA_TRY(cudaMemcpyAsync(&hplan, plan, sizeof hplan, cudaMemcpyDeviceToHost, stream));
       CUDA_TRY(cudaMemcpyAsync(&hctrl, ctrl, sizeof hctrl, cudaMemcpyDeviceToHost, stream));
       CUDA_TRY(cudaStreamSynchronize(stream));
       if (fix_flow) finish_ran = hctrl.flags[1] != 0;
-      stt.passes_planned = hplan.n_exec;
-      stt.segfix_passes = finish_ran ? 1 : 0;
-      stt.cut_digit = hplan.cut_digit;
-      memcpy(&stt.segfix_moved, &hctrl.flags[2], 8);
-      stt.algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)(hplan.n_exec + stt.segfix_passes) * 2ull * (uint64_t)n * rec_bytes;
-      if (hctrl.flags[0] != 0) {
-        // a long bucket with distinct keys: finish with the plain digit-by-digit path (the array is a
-        // permutation of the input, already ordered by its top digits)
-        DevSortOpts fo;
-        fo.layout_n = layout_n; fo.layout_landing = xo.layout_landing; fo.force_algo = 1;
-        const int rc = sort_device(key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo);
-        if (rc != 0) return rc;
-        b200sort_stats s2 = g_last_stats;
-        stt.fell_back = 1;
-        stt.passes_planned += s2.passes_planned;
-        stt.hist_sweeps += s2.hist_sweeps;
-        stt.algorithmic_bytes += s2.algorithmic_bytes;
-      }
     }
+    uint32_t rec_bytes = 0;
+    for (const StreamDesc &s : streams) rec_bytes += s.elem_bytes;
+    *stt = b200sort_stats{};
+    stt->num = n;
+    stt->record_bytes = rec_bytes;
+    stt->key_bytes = (uint32_t)kb;
+    stt->algo = (uint32_t)algo;
+    stt->hist_sweeps = hist_sweeps;
+    stt->passes_planned = (have_plan || hybrid) ? hplan.n_exec : (uint32_t)kb;  // (otherwise every pass is launched)
+    if (hybrid) {
+      stt->segfix_passes = finish_ran ? 1 : 0;
+      stt->cut_digit = hplan.cut_digit;
+      memcpy(&stt->segfix_moved, &hctrl.flags[2], 8);
+    }
+    stt->algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)(stt->passes_planned + stt->segfix_passes) * 2ull * (uint64_t)n * rec_bytes;
+    *fall_back = hybrid && hctrl.flags[0] != 0;
+    return 0;
   }
+
+  // fall-back: finish with the plain digit-by-digit path (the array is a permutation of the input, already ordered
+  // by its top digits)
+  int fall_back(b200sort_stats *stt) {
+    DevSortOpts fo;
+    fo.layout_n = xo.layout_n; fo.layout_landing = xo.layout_landing; fo.force_algo = 1;
+    if (int rc = sort_device(key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo)) return rc;
+    const b200sort_stats &s2 = g_last_stats;
+    stt->fell_back = 1;
+    stt->passes_planned += s2.passes_planned;
+    stt->hist_sweeps += s2.hist_sweeps;
+    stt->algorithmic_bytes += s2.algorithmic_bytes;
+    return 0;
+  }
+};
+
+static int sort_device(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
+                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo) {
+  const uint64_t launches_before = g_launches.load();
+  DevSort s{key_type, ascending, n, streams, stream, workspace, workspace_bytes, xo};
+  if (int rc = s.setup()) return rc;
+  if (int rc = s.make_plan()) return rc;
+  if (int rc = s.run_passes()) return rc;
+  if (int rc = s.finish()) return rc;
+  b200sort_stats stt;
+  bool fall_back = false;
+  if (int rc = s.statistics(&stt, &fall_back)) return rc;
+  if (fall_back)
+    if (int rc = s.fall_back(&stt)) return rc;
   stt.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
   g_last_stats = stt;
   g_have_stats = true;
@@ -856,38 +880,6 @@ __global__ void __launch_bounds__(256) gather_kernel(const uint32_t *__restrict_
   }
 }
 
-static CacheEntry &stage_cache_entry(int dev) {
-  static std::map<int, CacheEntry> g_stage;
-  return g_stage[dev];
-}
-static std::vector<CacheEntry *> g_stage_entries;  // for b200sort_release_cache
-
-static int cached_stage(int dev, size_t bytes, void **out) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  CacheEntry &c = stage_cache_entry(dev);
-  if (c.bytes < bytes) {
-    if (c.ptr) {
-      CUDA_TRY(cudaDeviceSynchronize());
-      CUDA_TRY(cudaFree(c.ptr));
-      c.ptr = nullptr;
-      c.bytes = 0;
-    }
-    void *p = nullptr;
-    cudaError_t e = cudaMalloc(&p, bytes);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(B200SORT_ENOMEM, "cudaMalloc of %zu staging bytes failed: %s", bytes, cudaGetErrorString(e));
-    }
-    c.ptr = p;
-    c.bytes = bytes;
-    bool known = false;
-    for (auto *q : g_stage_entries) known = known || q == &c;
-    if (!known) g_stage_entries.push_back(&c);
-  }
-  *out = c.ptr;
-  return 0;
-}
-
 static bool host_is_pinned(const void *p) {
   cudaPointerAttributes at{};
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -921,7 +913,7 @@ static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const st
   CacheGuard cache_guard;  // the staging buffer is shared per device as well; this call is synchronous anyway
   cache_guard.acquire(dev, caller);
   void *dbuf_v = nullptr;
-  if (int rc = cached_stage(dev, total, &dbuf_v)) return rc;
+  if (int rc = cached_buffer(CACHE_STAGE, dev, total, &dbuf_v)) return rc;
   unsigned char *dbuf = (unsigned char *)dbuf_v;
 
   std::vector<cudaEvent_t> ev;
@@ -960,9 +952,7 @@ static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const st
       if (int r = upload_payloads()) return r;
 
     CUDA_TRY(cudaStreamWaitEvent(st_comp, e_keys, 0));
-    iota_kernel<<<di.sm_count * 8, 256, 0, st_comp>>>((uint32_t *)(dbuf + off_idx), n);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(launch(PK_NONE, iota_kernel, di.sm_count * 8, 256, 0, st_comp, (uint32_t *)(dbuf + off_idx), n));
     std::vector<StreamDesc> ds = {{dbuf + off_keys, (uint32_t)kb}, {dbuf + off_idx, 4u}};
     if (int r = sort_device(key_type, ascending, n, ds, st_comp, nullptr, 0)) return r;
     cudaEvent_t e_sorted = new_event();
@@ -980,15 +970,12 @@ static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const st
       CUDA_TRY(cudaStreamWaitEvent(st_comp, e_pay[s], 0));
       const uint32_t *idx = (const uint32_t *)(dbuf + off_idx);
       const unsigned grid = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)di.sm_count * 16);
-      switch (ck) {
-        case 16: gather_kernel<uint4><<<grid, 256, 0, st_comp>>>(idx, (const uint4 *)(dbuf + off_in[s]), (uint4 *)(dbuf + off_out[s]), n, cpe); break;
-        case 8: gather_kernel<uint64_t><<<grid, 256, 0, st_comp>>>(idx, (const uint64_t *)(dbuf + off_in[s]), (uint64_t *)(dbuf + off_out[s]), n, cpe); break;
-        case 4: gather_kernel<uint32_t><<<grid, 256, 0, st_comp>>>(idx, (const uint32_t *)(dbuf + off_in[s]), (uint32_t *)(dbuf + off_out[s]), n, cpe); break;
-        case 2: gather_kernel<uint16_t><<<grid, 256, 0, st_comp>>>(idx, (const uint16_t *)(dbuf + off_in[s]), (uint16_t *)(dbuf + off_out[s]), n, cpe); break;
-        default: gather_kernel<uint8_t><<<grid, 256, 0, st_comp>>>(idx, (const uint8_t *)(dbuf + off_in[s]), (uint8_t *)(dbuf + off_out[s]), n, cpe); break;
-      }
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
+      auto gather = [&](auto *t) {  // (t: the type of one chunk)
+        using T = std::remove_pointer_t<decltype(t)>;
+        return launch(PK_NONE, gather_kernel<T>, grid, 256, 0, st_comp, idx, (const T *)(dbuf + off_in[s]), (T *)(dbuf + off_out[s]), n, cpe);
+      };
+      CUDA_TRY(ck == 16 ? gather((uint4 *)nullptr) : ck == 8 ? gather((uint64_t *)nullptr) : ck == 4 ? gather((uint32_t *)nullptr)
+               : ck == 2 ? gather((uint16_t *)nullptr) : gather((uint8_t *)nullptr));
       cudaEvent_t e_g = new_event();
       CUDA_TRY(cudaEventRecord(e_g, st_comp));
       CUDA_TRY(cudaStreamWaitEvent(st_out, e_g, 0));
@@ -1042,11 +1029,7 @@ static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<S
     size_t free_b = 0, total_b = 0;
     int cur_dev = 0;
     cudaGetDevice(&cur_dev);
-    size_t staged = 0;
-    {
-      std::lock_guard<std::mutex> lk(g_mu);
-      staged = stage_cache_entry(cur_dev).bytes;
-    }
+    const size_t staged = cache_entry(CACHE_STAGE, cur_dev).bytes;
     if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need < free_b / 10 * 9 + staged)
       return sort_host_pipelined(key_type, ascending, n, streams, stream);
     cudaGetLastError();
@@ -1244,20 +1227,15 @@ int b200sort_last_profile(int *kinds, float *ms, int capacity) {
 
 void b200sort_release_cache(void) {
   std::lock_guard<std::mutex> lk(g_mu);
-  for (auto &kv : g_cache) {
-    if (kv.second.ptr) {
-      int cur = 0;
-      cudaGetDevice(&cur);
-      cudaSetDevice(kv.first);
-      cudaDeviceSynchronize();
-      cudaFree(kv.second.ptr);
-      cudaSetDevice(cur);
+  for (auto &cache : g_cache)
+    for (auto &kv : cache) {
+      CacheEntry &c = kv.second;
+      if (!c.ptr) continue;
+      DeviceScope scope;  // (each buffer is freed on its own device)
+      if (scope.enter(kv.first) == 0) { cudaDeviceSynchronize(); cudaFree(c.ptr); }
+      c.ptr = nullptr;
+      c.bytes = 0;  // (gen survives: a later allocation is a new one for the multi-GPU handle check)
     }
-  }
-  g_cache.clear();
-  for (auto *c : g_stage_entries) {
-    if (c->ptr) { cudaDeviceSynchronize(); cudaFree(c->ptr); c->ptr = nullptr; c->bytes = 0; }
-  }
 }
 
 }  // extern "C"

@@ -126,24 +126,10 @@ __global__ void __launch_bounds__(256) range_kernel(TopHistArgs a) {
 static cudaError_t launch_top_hist(int kb, const TopHistArgs &a, int sm_count, cudaStream_t st, bool range_only = false) {
   const int64_t rows = ((a.n + 31) / 32 + a.sample - 1) / a.sample;
   const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((rows + 7) / 8, (int64_t)sm_count * 16));
-  ProfScope ps(PK_HIST, st);
-  if (range_only) {
-    switch (kb) {
-      case 1: range_kernel<1><<<grid, 256, 0, st>>>(a); break;
-      case 2: range_kernel<2><<<grid, 256, 0, st>>>(a); break;
-      case 4: range_kernel<4><<<grid, 256, 0, st>>>(a); break;
-      default: range_kernel<8><<<grid, 256, 0, st>>>(a); break;
-    }
-  } else {
-    switch (kb) {
-      case 1: top_hist_kernel<1><<<grid, 256, 0, st>>>(a); break;
-      case 2: top_hist_kernel<2><<<grid, 256, 0, st>>>(a); break;
-      case 4: top_hist_kernel<4><<<grid, 256, 0, st>>>(a); break;
-      default: top_hist_kernel<8><<<grid, 256, 0, st>>>(a); break;
-    }
-  }
-  g_launches++;
-  return cudaGetLastError();
+  return with_kb(kb, [&](auto K) {
+    constexpr int KB = decltype(K)::value;
+    return launch(PK_HIST, range_only ? range_kernel<KB> : top_hist_kernel<KB>, grid, 256, 0, st, a);
+  });
 }
 
 // ---- refinement of heavy histogram bins (SURVEY 8e(3)) -------------------------------------------------------
@@ -398,7 +384,7 @@ static cudaError_t launch_dest_count(int kb, const DestCountArgs &a0, int sm_cou
   const int64_t tile_keys = (int64_t)HIST_THREADS * hist_nld(kb) * (16 / kb);
   const int64_t n_tiles = (a.n + tile_keys - 1) / tile_keys;
   if (a.tile_hi <= 0 || a.tile_hi > n_tiles) a.tile_hi = n_tiles;
-  ProfScope ps(PK_HIST, st);
+  ProfScope ps(PK_HIST, st);  // (one profile entry for the one or two kernels)
   const bool dense = a.stride == (uint32_t)kb && (((uintptr_t)a.keys) & 15) == 0;
   if (kb == 8 && a.hi_only && a.world <= 8 && dense) {
     // full tiles through the lean kernel, a partial last tile (if it belongs to this launch) through the general one
@@ -407,23 +393,17 @@ static cudaError_t launch_dest_count(int kb, const DestCountArgs &a0, int sm_cou
       DestCountArgs f = a;
       f.tile_hi = full_hi;
       const int gridf = (int)std::max<int64_t>(1, std::min<int64_t>(full_hi - a.tile_lo, (int64_t)sm_count * 4));
-      dest_count_fast_kernel<hist_nld(8)><<<gridf, HIST_THREADS, 0, st>>>(f);
-      g_launches++;
-      cudaError_t e = cudaGetLastError();
+      const cudaError_t e = launch(PK_NONE, dest_count_fast_kernel<hist_nld(8)>, gridf, HIST_THREADS, 0, st, f);
       if (e != cudaSuccess) return e;
     }
     if (full_hi >= a.tile_hi) return cudaSuccess;
     a.tile_lo = std::max(a.tile_lo, full_hi);
   }
   const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(a.tile_hi - a.tile_lo, (int64_t)sm_count * 8));
-  switch (kb) {
-    case 1: dest_count_kernel<1, hist_nld(1)><<<grid, HIST_THREADS, 0, st>>>(a); break;
-    case 2: dest_count_kernel<2, hist_nld(2)><<<grid, HIST_THREADS, 0, st>>>(a); break;
-    case 4: dest_count_kernel<4, hist_nld(4)><<<grid, HIST_THREADS, 0, st>>>(a); break;
-    default: dest_count_kernel<8, hist_nld(8)><<<grid, HIST_THREADS, 0, st>>>(a); break;
-  }
-  g_launches++;
-  return cudaGetLastError();
+  return with_kb(kb, [&](auto K) {
+    constexpr int KB = decltype(K)::value;
+    return launch(PK_NONE, dest_count_kernel<KB, hist_nld(KB)>, grid, HIST_THREADS, 0, st, a);
+  });
 }
 
 // From the smallest / largest sampled ordered key to the binning of the splitter histogram:
@@ -648,16 +628,27 @@ struct b200sort_comm {
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
 
-// B200SORT_MGPU_TRACE=1: per-phase device times of every multi-GPU sort on stderr (adds a stream sync at the end)
+// B200SORT_MGPU_TRACE=1: per-phase device times of every multi-GPU sort on stderr (adds a stream sync at the end),
+// and for the overlapped exchange a timeline of its two streams: when each chunk's partition kernel, arrival and
+// first-pass kernels finished, relative to the first timeline mark (the fork)
 struct MgpuTrace {
+  using Marks = std::vector<std::pair<std::string, cudaEvent_t>>;
   bool on = false;
   cudaStream_t st = nullptr;
-  std::vector<std::pair<const char *, cudaEvent_t>> ev;
+  Marks phases, timeline;
   explicit MgpuTrace(cudaStream_t s) : st(s) {
     const char *e = getenv("B200SORT_MGPU_TRACE");
     on = e && *e == '1';
     mark("start");
   }
+  void record(Marks &m, const std::string &name, cudaStream_t s) {
+    if (!on) return;
+    cudaEvent_t e;
+    cudaEventCreate(&e);
+    cudaEventRecord(e, s);
+    m.emplace_back(name, e);
+  }
+  // end of a phase on the sort's stream
   void mark(const char *name) {
     static const bool dbg = getenv("B200SORT_MGPU_DEBUG") != nullptr;  // host-side progress lines (locating a hang)
     if (dbg) {
@@ -665,28 +656,33 @@ struct MgpuTrace {
       const cudaError_t e = cudaStreamSynchronize(st);
       fprintf(stderr, " device done (%s)\n", cudaGetErrorString(e));
     }
-    if (!on) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, st);
-    ev.emplace_back(name, e);
+    record(phases, name, st);
   }
+  // a point of the overlapped exchange's timeline, on stream s
+  void mark(const std::string &name, cudaStream_t s) { record(timeline, name, s); }
   void report(int rank) {
     if (!on) return;
     cudaStreamSynchronize(st);
-    std::string line = "[b200sort mgpu rank " + std::to_string(rank) + "]";
-    for (size_t i = 1; i < ev.size(); i++) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, ev[i - 1].second, ev[i].second);
-      char buf[96];
-      snprintf(buf, sizeof buf, " %s=%.3f", ev[i].first, ms);
-      line += buf;
-    }
+    const std::string head = "[b200sort mgpu rank " + std::to_string(rank) + "]";
+    auto line = [](const Marks &m, bool from_first, const char *fmt) {
+      std::string out;
+      for (size_t i = 1; i < m.size(); i++) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, m[from_first ? 0 : i - 1].second, m[i].second);
+        char buf[96];
+        snprintf(buf, sizeof buf, fmt, m[i].first.c_str(), ms);
+        out += buf;
+      }
+      return out;
+    };
+    if (!timeline.empty()) fprintf(stderr, "%s timeline (ms after the fork):%s\n", head.c_str(), line(timeline, true, " %s=%.2f").c_str());
     float tot = 0;
-    cudaEventElapsedTime(&tot, ev.front().second, ev.back().second);
-    fprintf(stderr, "%s total=%.3f ms\n", line.c_str(), tot);
-    for (auto &e : ev) cudaEventDestroy(e.second);
-    ev.clear();
+    cudaEventElapsedTime(&tot, phases.front().second, phases.back().second);
+    fprintf(stderr, "%s%s total=%.3f ms\n", head.c_str(), line(phases, false, " %s=%.3f").c_str(), tot);
+    for (Marks *m : {&phases, &timeline}) {
+      for (auto &e : *m) cudaEventDestroy(e.second);
+      m->clear();
+    }
   }
 };
 
@@ -868,14 +864,7 @@ static int mgpu_refine_hist(void *ctx_v, int n_ranges, const uint64_t *lo, const
   if (ra.n > 0) {
     const int64_t rows = ((ra.n + 31) / 32 + ra.sample - 1) / ra.sample;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((rows + 7) / 8, (int64_t)x->sm_count * 16));
-    switch (x->kb) {
-      case 1: refine_hist_kernel<1><<<grid, 256, 0, x->stream>>>(ra); break;
-      case 2: refine_hist_kernel<2><<<grid, 256, 0, x->stream>>>(ra); break;
-      case 4: refine_hist_kernel<4><<<grid, 256, 0, x->stream>>>(ra); break;
-      default: refine_hist_kernel<8><<<grid, 256, 0, x->stream>>>(ra); break;
-    }
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(with_kb(x->kb, [&](auto K) { return launch(PK_NONE, refine_hist_kernel<decltype(K)::value>, grid, 256, 0, x->stream, ra); }));
   }
   NCCL_TRY(x->api->AllReduce(x->c->d_hist, x->c->d_hist, words, ncclUint64, ncclSum, x->c->comm, x->stream));
   CUDA_TRY(cudaMemcpyAsync(out, x->c->d_hist, words * 8, cudaMemcpyDeviceToHost, x->stream));
@@ -883,199 +872,221 @@ static int mgpu_refine_hist(void *ctx_v, int n_ranges, const uint64_t *lo, const
   return 0;
 }
 
-// The distributed sort of b200sort_mgpu_sort_soa / b200sort_mgpu_sort_aos; streams[0] carries the key at offset 0.
-static int mgpu_sort(b200sort_comm *c, int key_type, const std::vector<StreamDesc> &streams, int64_t num_local, int64_t capacity,
-                     bool ascending, int64_t *out_num_local, cudaStream_t stream) {
-  NcclApi &api = nccl_api();
+// The distributed sort of b200sort_mgpu_sort_soa / b200sort_mgpu_sort_aos, phase by phase (mgpu_sort); streams[0]
+// carries the key at offset 0.
+struct MgpuSort {
+  b200sort_comm *const c;
+  NcclApi &api;
+  const int key_type;
+  const std::vector<StreamDesc> &streams;
+  const int64_t num_local, capacity;
+  const bool ascending;
+  const cudaStream_t stream;
   const int kb = key_bytes_of(key_type);
   const int world = c->world;
   const int bits = std::min(MGPU_MAX_BITS, 8 * kb);
   const uint32_t nb = 1u << bits;
-  const unsigned char *keys = (const unsigned char *)streams[0].ptr;
+  const unsigned char *const keys = (const unsigned char *)streams[0].ptr;
   const uint32_t kstride = streams[0].elem_bytes;
-  DeviceScope dev_scope;  // the communicator's device, whatever the caller's current device is
-  if (dev_scope.enter(c->dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", c->dev);
-  DevInfo di;
-  if (int rc = dev_info(c->dev, &di)) return rc;
-  const KeyOrder ko = make_key_order(key_type, ascending);
-  MgpuTrace trace(stream);
-  c->seq++;
-  c->last_overlap = false;
-
-  // workspace, laid out for `capacity` records on every rank (so that equal capacities give equal layouts
-  // and the local sort below finds what the peers wrote where it expects its shadow arrays)
-  uint32_t stage_bytes = (uint32_t)kb;
-  StreamSet ss{};
-  ss.n_streams = (int)streams.size();
-  for (size_t s = 0; s < streams.size(); s++) {
-    const uint32_t ck = chunk_for(streams[s].ptr, streams[s].elem_bytes);
-    ss.streams[s].chunk_bytes = ck;
-    ss.streams[s].chunks_per_elem = streams[s].elem_bytes / ck;
-    ss.streams[s].buf[0] = (unsigned char *)streams[s].ptr;
-    stage_bytes = std::max(stage_bytes, ck);
-  }
-  const int cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, num_local);
-  const TileCfg tc = kTileCfgs[cfg];
-  const int tile = tc.threads * tc.ipt;
   const int64_t n_ws = std::max<int64_t>(capacity, 1);
-  // Large 8-byte-key sorts receive into a third set of arrays (landing): the local sort then runs
-  // landing -> shadow -> caller -> shadow -> caller and an even number of passes ends in the caller's arrays
-  // without a copy.  The choice depends on nothing but the arguments all ranks share.
-  const bool landing = kb == 8 && n_ws >= ((int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_host_plan_min_log2.load(), 0), 62)) &&
-                       opt_mgpu_landing.load() != 0 && opt_mgpu_p2p.load() != 0;
-  Layout L;
-  make_layout(streams, n_ws, std::min(tile, HYB_MIN_TILE), &L, landing);
-  CacheGuard cache_guard;  // (recursive: the local sort below takes it again)
-  cache_guard.acquire(c->dev, stream);
-  // A rank whose cached workspace is too small is going to free and re-allocate it.  Its peers may still have
-  // the old allocation mapped (cudaIpcOpenMemHandle): they have to let go of it first.  The flag travels with
-  // the first all-reduce below.
-  const bool will_realloc = cached_workspace_bytes(c->dev) < L.total;
-
-  // 1: key range of a sample of all ranks' keys (min / max all-reduced), then the histogram of that range in
-  //    2^bits bins on the same sample, all-reduced
   const int64_t sample = std::max<int64_t>(1, num_local >> 24);  // about 2^24 sampled keys at most
-  unsigned long long range_h[3] = {~0ull, ~0ull, will_realloc ? 0ull : 1ull};
-  CUDA_TRY(cudaMemcpyAsync(c->d_counts, range_h, sizeof range_h, cudaMemcpyHostToDevice, stream));
-  TopHistArgs ha{keys, kstride, num_local, ko, 0, c->d_hist, sample, 0ull, nb, c->d_counts};
-  if (num_local > 0) CUDA_TRY(launch_top_hist(kb, ha, di.sm_count, stream, /*range_only=*/true));
-  NCCL_TRY(api.AllReduce(c->d_counts, c->d_counts, 3, ncclUint64, ncclMin, c->comm, stream));
-  CUDA_TRY(cudaMemcpyAsync(range_h, c->d_counts, sizeof range_h, cudaMemcpyDeviceToHost, stream));
-  CUDA_TRY(cudaMemsetAsync(c->d_hist, 0, sizeof(unsigned long long) * nb, stream));
-  CUDA_TRY(cudaStreamSynchronize(stream));
-  if (range_h[2] == 0) {
-    // somebody re-allocates: every rank drops all its mappings, and nobody frees anything before all have
-    for (int r = 0; r < world; r++) {
-      if (r != c->rank && c->peer_base[r]) cudaIpcCloseMemHandle(c->peer_base[r]);
-      c->peer_base[r] = nullptr;
-    }
-    NCCL_TRY(api.AllReduce(c->d_counts + 4, c->d_counts + 4, 1, ncclUint64, ncclSum, c->comm, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));
-  }
-  void *ws_v = nullptr;
-  if (int rc = cached_workspace(c->dev, L.total, &ws_v)) return rc;
-  unsigned char *ws = (unsigned char *)ws_v;
-  for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
+  const KeyOrder ko = make_key_order(key_type, ascending);
+  MgpuTrace trace{stream};
+  // set-up
+  DevInfo di;
+  StreamSet ss{};
+  uint32_t stage_bytes = 0;
+  int cfg = 0, tile = 0;
+  bool landing = false;
+  Layout L;
+  unsigned char *ws = nullptr;
+  CacheGuard cache_guard;  // (recursive: the local sort takes it again)
+  // splitters
+  std::vector<uint64_t> global_hist;  // reduced histogram of the sampled keys in 2^bits bins: bin(u) = (u - lo) >> shift
+  uint64_t sampled_total = 0;
   unsigned long long lo = 0;
   int shift = 0;
-  choose_range_bins(range_h[0], ~range_h[1], kb, bits, &lo, &shift);
-  ha.lo = lo; ha.shift = shift;
-  if (num_local > 0) CUDA_TRY(launch_top_hist(kb, ha, di.sm_count, stream));
-  std::vector<uint64_t> global_hist(nb);
-  NCCL_TRY(api.AllReduce(c->d_hist, c->d_hist, nb, ncclUint64, ncclSum, c->comm, stream));
-  CUDA_TRY(cudaMemcpyAsync(global_hist.data(), c->d_hist, sizeof(uint64_t) * nb, cudaMemcpyDeviceToHost, stream));
-  CUDA_TRY(cudaStreamSynchronize(stream));
-  trace.mark("hist+allreduce");
+  std::vector<uint32_t> bounds;       // rank r: bins [bounds[r], bounds[r+1])
+  bool heavy = false, has_tie = false;
+  std::vector<unsigned long long> split_key;
+  std::vector<uint32_t> split_blk, split_tie;
+  int blk_shift = 5;
+  PartArgs part{};
+  // overlap decision
+  bool overlap = false;
+  int n_chunks = 1;
+  uint32_t d_lshift[8] = {0}, d_cut[8] = {0};  // per destination: the first digit its local sort sweeps
+  std::vector<int> lead;                        // per rank: leading key bits all keys of its shard agree on
+  std::vector<int64_t> ct;                      // chunk ch = sweep tiles [ct[ch], ct[ch+1]) of the local input
+  // blob exchange, peer mapping
+  std::vector<MgpuBlob> blobs;
+  MgpuBlob *my_slot = nullptr;  // (device) my contribution, behind the gathered array
+  bool my_handle_changed = false, p2p = false;
+  std::vector<int64_t> recv_off, send_off;
+  int64_t recv_total = 0;
 
-  // 2: splitters (same on every rank).  Ordinary case: on bin boundaries of that histogram.  A rank that would
-  //    get more than its share + 1/16 means a bin too heavy to be kept whole (skewed keys, few distinct values,
-  //    SURVEY 8e(3)): the splitters are then refined, 16 key bits per level, down to single key values if need
-  //    be, and the keys EQUAL to such a value are divided by source rank and position.
-  std::vector<uint32_t> bounds(world + 1);
-  compute_splitters(global_hist.data(), bits, world, bounds.data());
-  uint64_t sampled_total = 0;
-  for (uint32_t b = 0; b < nb; b++) sampled_total += global_hist[b];
-  bool heavy = false;
-  {
+  uint64_t m(int src, int dst) const { return blobs[src].counts[dst]; }  // records rank src sends to rank dst
+
+  // set-up: streams, tile geometry, workspace layout, cache guard
+  int setup() {
+    if (int rc = dev_info(c->dev, &di)) return rc;
+    // workspace, laid out for `capacity` records on every rank (so that equal capacities give equal layouts
+    // and the local sort finds what the peers wrote where it expects its shadow arrays)
+    stage_bytes = make_stream_set(streams, kb, 16, &ss);
+    cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, num_local);
+    tile = kTileCfgs[cfg].threads * kTileCfgs[cfg].ipt;
+    // Large 8-byte-key sorts receive into a third set of arrays (landing): the local sort then runs
+    // landing -> shadow -> caller -> shadow -> caller and an even number of passes ends in the caller's arrays
+    // without a copy.  The choice depends on nothing but the arguments all ranks share.
+    landing = kb == 8 && n_ws >= ((int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_host_plan_min_log2.load(), 0), 62)) &&
+              opt_mgpu_landing.load() != 0 && opt_mgpu_p2p.load() != 0;
+    make_layout(streams, n_ws, std::min(tile, HYB_MIN_TILE), &L, landing);
+    cache_guard.acquire(c->dev, stream);
+    return 0;
+  }
+
+  // splitters: key range of a sample of all ranks' keys (min / max all-reduced), then the histogram of that range
+  // in 2^bits bins on the same sample, all-reduced; splitters on its bin boundaries, refined where a bin is too
+  // heavy (down to single key values: ties).  The same on every rank.  Also takes the workspace.
+  int splitters() {
+    // A rank whose cached workspace is too small is going to free and re-allocate it.  Its peers may still have
+    // the old allocation mapped (cudaIpcOpenMemHandle): they have to let go of it first.  The flag travels with
+    // the first all-reduce.
+    const bool will_realloc = cache_entry(CACHE_WORKSPACE, c->dev).bytes < L.total;
+    unsigned long long range_h[3] = {~0ull, ~0ull, will_realloc ? 0ull : 1ull};
+    CUDA_TRY(cudaMemcpyAsync(c->d_counts, range_h, sizeof range_h, cudaMemcpyHostToDevice, stream));
+    TopHistArgs ha{keys, kstride, num_local, ko, 0, c->d_hist, sample, 0ull, nb, c->d_counts};
+    if (num_local > 0) CUDA_TRY(launch_top_hist(kb, ha, di.sm_count, stream, /*range_only=*/true));
+    NCCL_TRY(api.AllReduce(c->d_counts, c->d_counts, 3, ncclUint64, ncclMin, c->comm, stream));
+    CUDA_TRY(cudaMemcpyAsync(range_h, c->d_counts, sizeof range_h, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemsetAsync(c->d_hist, 0, sizeof(unsigned long long) * nb, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (range_h[2] == 0) {
+      // somebody re-allocates: every rank drops all its mappings, and nobody frees anything before all have
+      for (int r = 0; r < world; r++) {
+        if (r != c->rank && c->peer_base[r]) cudaIpcCloseMemHandle(c->peer_base[r]);
+        c->peer_base[r] = nullptr;
+      }
+      NCCL_TRY(api.AllReduce(c->d_counts + 4, c->d_counts + 4, 1, ncclUint64, ncclSum, c->comm, stream));
+      CUDA_TRY(cudaStreamSynchronize(stream));
+    }
+    void *ws_v = nullptr;
+    if (int rc = cached_buffer(CACHE_WORKSPACE, c->dev, L.total, &ws_v)) return rc;
+    ws = (unsigned char *)ws_v;
+    for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
+    choose_range_bins(range_h[0], ~range_h[1], kb, bits, &lo, &shift);
+    ha.lo = lo; ha.shift = shift;
+    if (num_local > 0) CUDA_TRY(launch_top_hist(kb, ha, di.sm_count, stream));
+    global_hist.assign(nb, 0);
+    NCCL_TRY(api.AllReduce(c->d_hist, c->d_hist, nb, ncclUint64, ncclSum, c->comm, stream));
+    CUDA_TRY(cudaMemcpyAsync(global_hist.data(), c->d_hist, sizeof(uint64_t) * nb, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    trace.mark("hist+allreduce");
+
+    // Ordinary case: splitters on bin boundaries of that histogram.  A rank that would get more than its share
+    // + 1/16 means a bin too heavy to be kept whole (skewed keys, few distinct values, SURVEY 8e(3)): the
+    // splitters are then refined, 16 key bits per level, down to single key values if need be, and the keys
+    // EQUAL to such a value are divided by source rank and position.
+    bounds.assign(world + 1, 0);
+    compute_splitters(global_hist.data(), bits, world, bounds.data());
     std::vector<uint64_t> prefix((size_t)nb + 1, 0);
     for (uint32_t b = 0; b < nb; b++) prefix[b + 1] = prefix[b] + global_hist[b];
+    sampled_total = prefix[nb];
     const uint64_t share = sampled_total / (uint64_t)world;
-    for (int r = 0; r < world; r++)
-      heavy = heavy || prefix[bounds[r + 1]] - prefix[bounds[r]] > share + share / 16 + 64;
-  }
-  const int ns = world - 1;
-  std::vector<unsigned long long> split_key(std::max(ns, 1), 0ull);
-  std::vector<uint32_t> split_blk(std::max(ns, 1), 0u), split_tie(std::max(ns, 1), 0u);
-  int blk_shift = 5;
-  while (((int64_t)MGPU_TIE_BLOCKS << blk_shift) < std::max<int64_t>(capacity, 1)) blk_shift++;  // capacity: the same on all ranks
-  bool has_tie = false;
-  if (!heavy || opt_mgpu_refine.load() == 0) {
-    heavy = false;
-    for (int r = 0; r < ns; r++) {
-      const uint32_t b = bounds[r + 1];
-      split_key[r] = b == 0 ? 0ull : (b >= nb ? ~0ull : lo + ((unsigned long long)b << shift));
-    }
-  } else {
-    RefineCtx rx{c, &api, RefineArgs{}, kb, di.sm_count, stream};
-    rx.ra.keys = keys; rx.ra.stride = kstride; rx.ra.n = num_local; rx.ra.ko = ko; rx.ra.sample = sample;
-    std::vector<uint64_t> rk(std::max(ns, 1)), below(std::max(ns, 1));
-    if (int rc = refine_splitters(world, 8 * kb, sampled_total, mgpu_refine_hist, &rx, rk.data(), split_tie.data(), below.data())) return rc;
-    for (int r = 0; r < ns; r++) { split_key[r] = rk[r]; has_tie = has_tie || split_tie[r] != 0; }
-    trace.mark("refine");
-    if (has_tie) {
-      // exact counts around the (distinct) tie values: keys below, equal keys per position block; all-gathered
-      std::vector<unsigned long long> tv;
-      for (int r = 0; r < ns; r++)
-        if (split_tie[r] && (tv.empty() || tv.back() != split_key[r])) tv.push_back(split_key[r]);
-      std::vector<uint32_t> blk_all(std::max(ns, 1), 0u);
-      for (size_t t0 = 0; t0 < tv.size(); t0 += MGPU_MAX_REFINE) {
-        const int nt = (int)std::min<size_t>(MGPU_MAX_REFINE, tv.size() - t0);
-        unsigned long long *my_less = c->d_tie_less + (size_t)world * MGPU_MAX_REFINE;          // my slot, then gathered at 0
-        uint32_t *my_eq = c->d_tie_eq + (size_t)world * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS;
-        CUDA_TRY(cudaMemsetAsync(my_less, 0, sizeof(unsigned long long) * MGPU_MAX_REFINE, stream));
-        CUDA_TRY(cudaMemsetAsync(my_eq, 0, sizeof(uint32_t) * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS, stream));
-        TieCountArgs ta{keys, kstride, num_local, ko, nt, {}, blk_shift, my_less, my_eq};
-        for (int j = 0; j < nt; j++) ta.v[j] = tv[t0 + j];
-        if (num_local > 0) {
-          const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((num_local + 255) / 256, (int64_t)di.sm_count * 16));
-          switch (kb) {
-            case 1: tie_count_kernel<1><<<grid, 256, 0, stream>>>(ta); break;
-            case 2: tie_count_kernel<2><<<grid, 256, 0, stream>>>(ta); break;
-            case 4: tie_count_kernel<4><<<grid, 256, 0, stream>>>(ta); break;
-            default: tie_count_kernel<8><<<grid, 256, 0, stream>>>(ta); break;
-          }
-          g_launches++;
-          CUDA_TRY(cudaGetLastError());
-        }
-        NCCL_TRY(api.AllGather(my_less, c->d_tie_less, MGPU_MAX_REFINE, ncclUint64, c->comm, stream));
-        NCCL_TRY(api.AllGather(my_eq, c->d_tie_eq, (size_t)MGPU_MAX_REFINE * MGPU_TIE_BLOCKS, ncclUint32, c->comm, stream));
-        std::vector<unsigned long long> less_h((size_t)world * MGPU_MAX_REFINE);
-        std::vector<uint32_t> eq_h((size_t)world * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS);
-        unsigned long long tot_h[2] = {(unsigned long long)num_local, 0};
-        CUDA_TRY(cudaMemcpyAsync(c->d_counts + 8, tot_h, 8, cudaMemcpyHostToDevice, stream));
-        NCCL_TRY(api.AllReduce(c->d_counts + 8, c->d_counts + 8, 1, ncclUint64, ncclSum, c->comm, stream));
-        CUDA_TRY(cudaMemcpyAsync(tot_h, c->d_counts + 8, 8, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaMemcpyAsync(less_h.data(), c->d_tie_less, less_h.size() * 8, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaMemcpyAsync(eq_h.data(), c->d_tie_eq, eq_h.size() * 4, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        const uint64_t n_total = tot_h[0];
-        for (int j = 0; j < nt; j++) {
-          uint64_t less_total = 0;
-          std::vector<uint32_t> eq((size_t)world * MGPU_TIE_BLOCKS);
-          for (int s2 = 0; s2 < world; s2++) {
-            less_total += less_h[(size_t)s2 * MGPU_MAX_REFINE + j];
-            memcpy(&eq[(size_t)s2 * MGPU_TIE_BLOCKS], &eq_h[((size_t)s2 * MGPU_MAX_REFINE + j) * MGPU_TIE_BLOCKS], sizeof(uint32_t) * MGPU_TIE_BLOCKS);
-          }
-          std::vector<uint64_t> targets;
-          std::vector<int> which;
-          for (int r = 0; r < ns; r++)
-            if (split_tie[r] && split_key[r] == tv[t0 + j]) {
-              targets.push_back((uint64_t)(((unsigned __int128)n_total * (unsigned)(r + 1)) / (unsigned)world));
-              which.push_back(r);
-            }
-          std::vector<uint32_t> out(targets.size());
-          tie_thresholds(world, c->rank, MGPU_TIE_BLOCKS, less_total, eq.data(), (int)targets.size(), targets.data(), out.data());
-          for (size_t q = 0; q < which.size(); q++) blk_all[which[q]] = out[q];
-        }
+    for (int r = 0; r < world; r++) heavy = heavy || prefix[bounds[r + 1]] - prefix[bounds[r]] > share + share / 16 + 64;
+    const int ns = world - 1;
+    split_key.assign(std::max(ns, 1), 0ull);
+    split_blk.assign(std::max(ns, 1), 0u);
+    split_tie.assign(std::max(ns, 1), 0u);
+    while (((int64_t)MGPU_TIE_BLOCKS << blk_shift) < std::max<int64_t>(capacity, 1)) blk_shift++;  // capacity: the same on all ranks
+    if (!heavy || opt_mgpu_refine.load() == 0) {
+      heavy = false;
+      for (int r = 0; r < ns; r++) {
+        const uint32_t b = bounds[r + 1];
+        split_key[r] = b == 0 ? 0ull : (b >= nb ? ~0ull : lo + ((unsigned long long)b << shift));
       }
-      for (int r = 0; r < ns; r++) split_blk[r] = split_tie[r] ? blk_all[r] : 0u;
-      // (key, block) pairs must ascend: an ordinary splitter on the same key value as a tie keeps the tie's threshold
-      for (int r = 1; r < ns; r++)
-        if (split_key[r] == split_key[r - 1] && split_blk[r] < split_blk[r - 1]) split_blk[r] = split_blk[r - 1];
-      trace.mark("ties");
+    } else {
+      RefineCtx rx{c, &api, RefineArgs{}, kb, di.sm_count, stream};
+      rx.ra.keys = keys; rx.ra.stride = kstride; rx.ra.n = num_local; rx.ra.ko = ko; rx.ra.sample = sample;
+      std::vector<uint64_t> rk(std::max(ns, 1)), below(std::max(ns, 1));
+      if (int rc = refine_splitters(world, 8 * kb, sampled_total, mgpu_refine_hist, &rx, rk.data(), split_tie.data(), below.data())) return rc;
+      for (int r = 0; r < ns; r++) { split_key[r] = rk[r]; has_tie = has_tie || split_tie[r] != 0; }
+      trace.mark("refine");
+      if (has_tie)
+        if (int rc = tie_blocks()) return rc;
     }
+    CUDA_TRY(cudaMemcpyAsync(c->d_split_key, split_key.data(), sizeof(unsigned long long) * std::max(ns, 1), cudaMemcpyHostToDevice, stream));
+    CUDA_TRY(cudaMemcpyAsync(c->d_split_blk, split_blk.data(), sizeof(uint32_t) * std::max(ns, 1), cudaMemcpyHostToDevice, stream));
+    part = PartArgs{c->d_split_key, c->d_split_blk, ns, blk_shift, has_tie ? 1 : 0, 0u, {}};
+    part.hi_only = (kb == 8 && !has_tie && world <= 8) ? 1u : 0u;
+    for (int r = 0; r < 7; r++) {
+      part.hi_m1[r] = 0xffffffffu;
+      if (r < ns) {
+        const unsigned long long kv = split_key[r];
+        if ((uint32_t)kv != 0 || (kv >> 32) == 0) part.hi_only = 0;  // (a splitter at 0 or with low bits: general form)
+        else part.hi_m1[r] = (uint32_t)(kv >> 32) - 1u;
+      }
+    }
+    return 0;
   }
-  CUDA_TRY(cudaMemcpyAsync(c->d_split_key, split_key.data(), sizeof(unsigned long long) * std::max(ns, 1), cudaMemcpyHostToDevice, stream));
-  CUDA_TRY(cudaMemcpyAsync(c->d_split_blk, split_blk.data(), sizeof(uint32_t) * std::max(ns, 1), cudaMemcpyHostToDevice, stream));
-  PartArgs part{c->d_split_key, c->d_split_blk, ns, blk_shift, has_tie ? 1 : 0, 0u, {}};
-  part.hi_only = (kb == 8 && !has_tie && world <= 8) ? 1u : 0u;
-  for (int r = 0; r < 7; r++) {
-    part.hi_m1[r] = 0xffffffffu;
-    if (r < ns) {
-      const unsigned long long kv = split_key[r];
-      if ((uint32_t)kv != 0 || (kv >> 32) == 0) part.hi_only = 0;  // (a splitter at 0 or with low bits: general form)
-      else part.hi_m1[r] = (uint32_t)(kv >> 32) - 1u;
+
+  // ties: exact counts around the (distinct) tie values -- keys below, equal keys per position block -- all-gathered,
+  // and from them this rank's position-block threshold of every splitter that sits on a tie
+  int tie_blocks() {
+    const int ns = world - 1;
+    std::vector<unsigned long long> tv;
+    for (int r = 0; r < ns; r++)
+      if (split_tie[r] && (tv.empty() || tv.back() != split_key[r])) tv.push_back(split_key[r]);
+    std::vector<uint32_t> blk_all(std::max(ns, 1), 0u);
+    for (size_t t0 = 0; t0 < tv.size(); t0 += MGPU_MAX_REFINE) {
+      const int nt = (int)std::min<size_t>(MGPU_MAX_REFINE, tv.size() - t0);
+      unsigned long long *my_less = c->d_tie_less + (size_t)world * MGPU_MAX_REFINE;          // my slot, then gathered at 0
+      uint32_t *my_eq = c->d_tie_eq + (size_t)world * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS;
+      CUDA_TRY(cudaMemsetAsync(my_less, 0, sizeof(unsigned long long) * MGPU_MAX_REFINE, stream));
+      CUDA_TRY(cudaMemsetAsync(my_eq, 0, sizeof(uint32_t) * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS, stream));
+      TieCountArgs ta{keys, kstride, num_local, ko, nt, {}, blk_shift, my_less, my_eq};
+      for (int j = 0; j < nt; j++) ta.v[j] = tv[t0 + j];
+      if (num_local > 0) {
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((num_local + 255) / 256, (int64_t)di.sm_count * 16));
+        CUDA_TRY(with_kb(kb, [&](auto K) { return launch(PK_NONE, tie_count_kernel<decltype(K)::value>, grid, 256, 0, stream, ta); }));
+      }
+      NCCL_TRY(api.AllGather(my_less, c->d_tie_less, MGPU_MAX_REFINE, ncclUint64, c->comm, stream));
+      NCCL_TRY(api.AllGather(my_eq, c->d_tie_eq, (size_t)MGPU_MAX_REFINE * MGPU_TIE_BLOCKS, ncclUint32, c->comm, stream));
+      std::vector<unsigned long long> less_h((size_t)world * MGPU_MAX_REFINE);
+      std::vector<uint32_t> eq_h((size_t)world * MGPU_MAX_REFINE * MGPU_TIE_BLOCKS);
+      unsigned long long tot_h[2] = {(unsigned long long)num_local, 0};
+      CUDA_TRY(cudaMemcpyAsync(c->d_counts + 8, tot_h, 8, cudaMemcpyHostToDevice, stream));
+      NCCL_TRY(api.AllReduce(c->d_counts + 8, c->d_counts + 8, 1, ncclUint64, ncclSum, c->comm, stream));
+      CUDA_TRY(cudaMemcpyAsync(tot_h, c->d_counts + 8, 8, cudaMemcpyDeviceToHost, stream));
+      CUDA_TRY(cudaMemcpyAsync(less_h.data(), c->d_tie_less, less_h.size() * 8, cudaMemcpyDeviceToHost, stream));
+      CUDA_TRY(cudaMemcpyAsync(eq_h.data(), c->d_tie_eq, eq_h.size() * 4, cudaMemcpyDeviceToHost, stream));
+      CUDA_TRY(cudaStreamSynchronize(stream));
+      const uint64_t n_total = tot_h[0];
+      for (int j = 0; j < nt; j++) {
+        uint64_t less_total = 0;
+        std::vector<uint32_t> eq((size_t)world * MGPU_TIE_BLOCKS);
+        for (int s2 = 0; s2 < world; s2++) {
+          less_total += less_h[(size_t)s2 * MGPU_MAX_REFINE + j];
+          memcpy(&eq[(size_t)s2 * MGPU_TIE_BLOCKS], &eq_h[((size_t)s2 * MGPU_MAX_REFINE + j) * MGPU_TIE_BLOCKS], sizeof(uint32_t) * MGPU_TIE_BLOCKS);
+        }
+        std::vector<uint64_t> targets;
+        std::vector<int> which;
+        for (int r = 0; r < ns; r++)
+          if (split_tie[r] && split_key[r] == tv[t0 + j]) {
+            targets.push_back((uint64_t)(((unsigned __int128)n_total * (unsigned)(r + 1)) / (unsigned)world));
+            which.push_back(r);
+          }
+        std::vector<uint32_t> out(targets.size());
+        tie_thresholds(world, c->rank, MGPU_TIE_BLOCKS, less_total, eq.data(), (int)targets.size(), targets.data(), out.data());
+        for (size_t q = 0; q < which.size(); q++) blk_all[which[q]] = out[q];
+      }
     }
+    for (int r = 0; r < ns; r++) split_blk[r] = split_tie[r] ? blk_all[r] : 0u;
+    // (key, block) pairs must ascend: an ordinary splitter on the same key value as a tie keeps the tie's threshold
+    for (int r = 1; r < ns; r++)
+      if (split_key[r] == split_key[r - 1] && split_blk[r] < split_blk[r - 1]) split_blk[r] = split_blk[r - 1];
+    trace.mark("ties");
+    return 0;
   }
 
   // Overlapped exchange (the headline shape): full-width 8-byte keys, close to uniform, one box, peer memory.
@@ -1083,246 +1094,234 @@ static int mgpu_sort(b200sort_comm *c, int key_type, const std::vector<StreamDes
   // below its shard's common leading bits), the senders count the first of those digits per destination while
   // they count the records, and the destination runs its first pass chunk by chunk while later chunks are
   // still on the NVLink.
-  const int64_t chunk_min = (int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunk_min_log2.load(), 12), 40);
-  int n_chunks = (int)std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunks.load(), 1), MGPU_MAX_CHUNKS);
-  bool overlap = landing && !heavy && kb == 8 && world <= 8 && (world >= 2 || opt_mgpu_overlap.load() == 2) && lo == 0 && shift == 8 * kb - bits &&
-                 opt_mgpu_overlap.load() != 0 && opt_mgpu_p2p.load() != 0 && !c->p2p_failed && cfg == kDefaultTileCfg &&
-                 streams[0].elem_bytes == (uint32_t)kb;
-  uint32_t d_lshift[8] = {0}, d_cut[8] = {0};
-  if (overlap) {
-    // flat enough?  (by the top 8 bits of the sampled histogram inside every shard)
-    std::vector<uint64_t> g256(256, 0);
-    for (uint32_t b = 0; b < nb; b++) g256[b >> (bits - 8)] += global_hist[b];
-    uint64_t mx = 0, mn = ~0ull;
-    for (int g = 0; g < 256; g++) { mx = std::max(mx, g256[g]); mn = std::min(mn, g256[g]); }
-    overlap = mn > 0 && mx <= mn + mn / 4;
-    for (int r = 0; r < world && overlap; r++) {
-      if (bounds[r + 1] <= bounds[r]) { overlap = false; break; }
-      const uint32_t x = bounds[r] ^ (bounds[r + 1] - 1);
-      const int lead = x ? __builtin_clz(x) - (32 - bits) : bits;
-      const double est_n = (double)sampled_total * (double)sample / (double)world;
-      const int swept = (int)std::ceil((std::log2(std::max(est_n, 2.0)) + (double)opt_margin_bits.load()) / 8.0);
-      const int cut = 8 - lead / 8 - swept;
-      if (cut < 2 || opt_allow_lshift.load() == 0) { overlap = false; break; }
-      d_lshift[r] = (uint32_t)(lead & 7);
-      d_cut[r] = (uint32_t)cut;
+  void decide_overlap() {
+    // leading key bits each rank's range [bounds[r], bounds[r+1]) of top-`bits` values has in common (bins aligned
+    // with the key's own leading bits only)
+    const bool aligned = !heavy && kb == 8 && lo == 0 && shift == 8 * kb - bits;
+    lead.assign(world, 0);
+    for (int r = 0; r < world; r++)
+      if (aligned && bounds[r + 1] > bounds[r]) {
+        const uint32_t x = bounds[r] ^ (bounds[r + 1] - 1);
+        lead[r] = x ? __builtin_clz(x) - (32 - bits) : bits;
+      }
+    const int64_t chunk_min = (int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunk_min_log2.load(), 12), 40);
+    n_chunks = (int)std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunks.load(), 1), MGPU_MAX_CHUNKS);
+    overlap = landing && aligned && world <= 8 && (world >= 2 || opt_mgpu_overlap.load() == 2) && opt_mgpu_overlap.load() != 0 &&
+              opt_mgpu_p2p.load() != 0 && !c->p2p_failed && cfg == kDefaultTileCfg && streams[0].elem_bytes == (uint32_t)kb;
+    if (overlap) {
+      // flat enough?  (by the top 8 bits of the sampled histogram inside every shard)
+      std::vector<uint64_t> g256(256, 0);
+      for (uint32_t b = 0; b < nb; b++) g256[b >> (bits - 8)] += global_hist[b];
+      uint64_t mx = 0, mn = ~0ull;
+      for (int g = 0; g < 256; g++) { mx = std::max(mx, g256[g]); mn = std::min(mn, g256[g]); }
+      overlap = mn > 0 && mx <= mn + mn / 4;
+      for (int r = 0; r < world && overlap; r++) {
+        if (bounds[r + 1] <= bounds[r]) { overlap = false; break; }
+        const double est_n = (double)sampled_total * (double)sample / (double)world;
+        const int swept = (int)std::ceil((std::log2(std::max(est_n, 2.0)) + (double)opt_margin_bits.load()) / 8.0);
+        const int cut = 8 - lead[r] / 8 - swept;
+        if (cut < 2 || opt_allow_lshift.load() == 0) { overlap = false; break; }
+        d_lshift[r] = (uint32_t)(lead[r] & 7);
+        d_cut[r] = (uint32_t)cut;
+      }
+      // (all ranks took the same decision: it depends on the reduced histogram and shared arguments only; the
+      //  records per rank must be large enough for chunks to make sense, which is also a shared quantity here)
+      overlap = overlap && capacity >= chunk_min;
+      while (n_chunks > 1 && capacity / n_chunks < chunk_min / 2) n_chunks--;
     }
-    // (all ranks took the same decision: it depends on the reduced histogram and shared arguments only; the
-    //  records per rank must be large enough for chunks to make sense, which is also a shared quantity here)
-    overlap = overlap && capacity >= chunk_min;
-    while (n_chunks > 1 && capacity / n_chunks < chunk_min / 2) n_chunks--;
+    const int64_t n_tiles_local = (num_local + tile - 1) / tile;
+    ct.assign(n_chunks + 1, 0);
+    for (int ch = 0; ch <= n_chunks; ch++) ct[ch] = overlap ? (n_tiles_local * ch) / n_chunks : (ch == 0 ? 0 : n_tiles_local);
   }
 
-  // 3: my blob = {workspace handle, layout size, capacity, exact send counts (+ first-digit histograms)}; all-gather
-  MgpuBlob *mine_h = nullptr;
-  std::vector<unsigned char> mine_buf(sizeof(MgpuBlob), 0);
-  mine_h = (MgpuBlob *)mine_buf.data();
-  const bool want_p2p = opt_mgpu_p2p.load() != 0 && !c->p2p_failed;
-  bool my_handle_changed = false;
-  if (want_p2p) {
-    const uint64_t gen = cached_workspace_gen(c->dev);
-    if (c->my_handle_of != ws || c->my_handle_gen != gen) {  // (a slow driver call: once per workspace allocation)
-      cudaError_t e = cudaIpcGetMemHandle(&c->my_handle, ws);
-      if (e != cudaSuccess) { cudaGetLastError(); c->p2p_failed = true; }
-      else { c->my_handle_of = ws; c->my_handle_gen = gen; my_handle_changed = true; }
+  // blob exchange: my blob = {workspace handle, layout size, capacity, exact send counts (+ first-digit
+  // histograms)}, all-gathered; the send and receive offsets from them
+  int exchange_blobs() {
+    auto mine = std::make_unique<MgpuBlob>();
+    const bool want_p2p = opt_mgpu_p2p.load() != 0 && !c->p2p_failed;
+    if (want_p2p) {
+      const uint64_t gen = cache_entry(CACHE_WORKSPACE, c->dev).gen;
+      if (c->my_handle_of != ws || c->my_handle_gen != gen) {  // (a slow driver call: once per workspace allocation)
+        cudaError_t e = cudaIpcGetMemHandle(&c->my_handle, ws);
+        if (e != cudaSuccess) { cudaGetLastError(); c->p2p_failed = true; }
+        else { c->my_handle_of = ws; c->my_handle_gen = gen; my_handle_changed = true; }
+      }
+      mine->handle = c->my_handle;
     }
-    mine_h->handle = c->my_handle;
-  }
-  // arrival flags of the overlapped exchange: cleared by their owner before the all-gather below, i.e. before
-  // any peer can write this sort's flags (the previous sort's are dead: its waits are stream-ordered before this)
-  CUDA_TRY(cudaMemsetAsync(ws + L.flags_off, 0, 4096, stream));
-  mine_h->ws_bytes = L.total;
-  mine_h->capacity = capacity;
-  mine_h->p2p = (want_p2p && !c->p2p_failed) ? 1 : 0;
-  MgpuBlob *my_slot = c->d_blob + world;  // my contribution lives behind the gathered array
-  CUDA_TRY(cudaMemcpyAsync(my_slot, mine_h, sizeof(MgpuBlob), cudaMemcpyHostToDevice, stream));  // counts zeroed with it
-  trace.mark("host_prep");
-  const int64_t ktile_keys = (int64_t)HIST_THREADS * hist_nld(kb) * (16 / kb);
-  // chunk c = sweep tiles [ct[c], ct[c+1]) of the local input (multiples of both tile sizes)
-  const int64_t n_tiles_local = (num_local + tile - 1) / tile;
-  std::vector<int64_t> ct(n_chunks + 1, 0);
-  for (int ch = 0; ch <= n_chunks; ch++) ct[ch] = overlap ? (n_tiles_local * ch) / n_chunks : (ch == 0 ? 0 : n_tiles_local);
-  if (num_local > 0) {
-    DestCountArgs da{};
-    da.keys = keys; da.stride = kstride; da.n = num_local; da.ko = ko; da.part = part; da.world = world;
-    da.hi_only = part.hi_only;
-    for (int r = 0; r < 8; r++) da.hi_m1[r] = r < 7 ? part.hi_m1[r] : 0xffffffffu;
-    if (!overlap) {
-      da.counts = my_slot->counts; da.tile_lo = 0; da.tile_hi = 0;
-      CUDA_TRY(launch_dest_count(kb, da, di.sm_count, stream));
-    } else {
-      for (int r = 0; r < world; r++) { da.digit_lshift[r] = d_lshift[r]; da.digit_shift[r] = d_cut[r] * RADIX_BITS; }
+    // arrival flags of the overlapped exchange: cleared by their owner before the all-gather below, i.e. before
+    // any peer can write this sort's flags (the previous sort's are dead: its waits are stream-ordered before this)
+    CUDA_TRY(cudaMemsetAsync(ws + L.flags_off, 0, 4096, stream));
+    mine->ws_bytes = L.total;
+    mine->capacity = capacity;
+    mine->p2p = (want_p2p && !c->p2p_failed) ? 1 : 0;
+    my_slot = c->d_blob + world;
+    CUDA_TRY(cudaMemcpyAsync(my_slot, mine.get(), sizeof(MgpuBlob), cudaMemcpyHostToDevice, stream));  // counts zeroed with it
+    trace.mark("host_prep");
+    if (num_local > 0) {
+      DestCountArgs da{};
+      da.keys = keys; da.stride = kstride; da.n = num_local; da.ko = ko; da.part = part; da.world = world;
       da.hi_only = part.hi_only;
       for (int r = 0; r < 8; r++) da.hi_m1[r] = r < 7 ? part.hi_m1[r] : 0xffffffffu;
-      for (int ch = 0; ch < n_chunks; ch++) {
-        // (sweep tiles are a multiple of the counting kernel's tiles: 4096 vs 2048 keys)
-        da.counts = my_slot->chunk_counts[ch];  // [8] used, the kernel's [RADIX] view stays inside the blob
-        da.digit_hist = &my_slot->chunk_hist[ch][0][0];
-        da.tile_lo = ct[ch] * tile / ktile_keys;
-        da.tile_hi = std::min<int64_t>(ct[ch + 1] * tile / ktile_keys, (num_local + ktile_keys - 1) / ktile_keys);
-        if (da.tile_hi > da.tile_lo) CUDA_TRY(launch_dest_count(kb, da, di.sm_count, stream));
+      if (!overlap) {
+        da.counts = my_slot->counts; da.tile_lo = 0; da.tile_hi = 0;
+        CUDA_TRY(launch_dest_count(kb, da, di.sm_count, stream));
+      } else {
+        const int64_t ktile_keys = (int64_t)HIST_THREADS * hist_nld(kb) * (16 / kb);
+        for (int r = 0; r < world; r++) { da.digit_lshift[r] = d_lshift[r]; da.digit_shift[r] = d_cut[r] * RADIX_BITS; }
+        for (int ch = 0; ch < n_chunks; ch++) {
+          // (sweep tiles are a multiple of the counting kernel's tiles: 4096 vs 2048 keys)
+          da.counts = my_slot->chunk_counts[ch];  // [8] used, the kernel's [RADIX] view stays inside the blob
+          da.digit_hist = &my_slot->chunk_hist[ch][0][0];
+          da.tile_lo = ct[ch] * tile / ktile_keys;
+          da.tile_hi = std::min<int64_t>(ct[ch + 1] * tile / ktile_keys, (num_local + ktile_keys - 1) / ktile_keys);
+          if (da.tile_hi > da.tile_lo) CUDA_TRY(launch_dest_count(kb, da, di.sm_count, stream));
+        }
       }
     }
-  }
-  trace.mark("count");
-  NCCL_TRY(api.AllGather(my_slot, c->d_blob, sizeof(MgpuBlob), ncclUint8, c->comm, stream));
-  std::vector<unsigned char> blobs_buf(sizeof(MgpuBlob) * (size_t)world);
-  MgpuBlob *blobs = (MgpuBlob *)blobs_buf.data();
-  CUDA_TRY(cudaMemcpyAsync(blobs, c->d_blob, sizeof(MgpuBlob) * world, cudaMemcpyDeviceToHost, stream));
-  CUDA_TRY(cudaStreamSynchronize(stream));
-  trace.mark("allgather");
-  if (overlap)  // totals per destination from the chunks
-    for (int s2 = 0; s2 < world; s2++)
-      for (int r = 0; r < world; r++) {
-        uint64_t t = 0;
-        for (int ch = 0; ch < n_chunks; ch++) t += blobs[s2].chunk_counts[ch][r];
-        blobs[s2].counts[r] = t;
-      }
-
-  auto m = [&](int src, int dst) -> uint64_t { return blobs[src].counts[dst]; };
-  std::vector<uint64_t> send(world);
-  for (int r = 0; r < world; r++) send[r] = m(c->rank, r);
-  int64_t recv_total = 0;
-  std::vector<int64_t> recv_off(world), send_off(world);
-  for (int s = 0; s < world; s++) { recv_off[s] = recv_total; recv_total += (int64_t)m(s, c->rank); }
-  {
-    int64_t o = 0;
-    for (int r = 0; r < world; r++) { send_off[r] = o; o += (int64_t)send[r]; }
-  }
-  // every rank can evaluate every rank's receive total, so all ranks fail together
-  for (int r = 0; r < world; r++) {
-    int64_t t = 0;
-    for (int s = 0; s < world; s++) t += (int64_t)m(s, r);
-    if (t > blobs[r].capacity)
-      return fail(B200SORT_ENOMEM, "rank %d would receive %lld records, its capacity is %lld", r, (long long)t, (long long)blobs[r].capacity);
-  }
-
-  // peer-memory path: everybody willing, equal layouts; map the workspaces that changed since the last sort
-  bool p2p = true;
-  for (int r = 0; r < world; r++) p2p = p2p && blobs[r].p2p == 1 && blobs[r].ws_bytes == L.total && blobs[r].capacity == capacity;
-  if (p2p) {
-    bool ok = true;
-    bool changed = false;
+    trace.mark("count");
+    NCCL_TRY(api.AllGather(my_slot, c->d_blob, sizeof(MgpuBlob), ncclUint8, c->comm, stream));
+    blobs.resize(world);
+    CUDA_TRY(cudaMemcpyAsync(blobs.data(), c->d_blob, sizeof(MgpuBlob) * world, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    trace.mark("allgather");
+    if (overlap)  // totals per destination from the chunks
+      for (int s2 = 0; s2 < world; s2++)
+        for (int r = 0; r < world; r++) {
+          uint64_t t = 0;
+          for (int ch = 0; ch < n_chunks; ch++) t += blobs[s2].chunk_counts[ch][r];
+          blobs[s2].counts[r] = t;
+        }
+    recv_off.assign(world, 0);
+    send_off.assign(world, 0);
+    for (int s = 0; s < world; s++) { recv_off[s] = recv_total; recv_total += (int64_t)m(s, c->rank); }
+    for (int r = 1; r < world; r++) send_off[r] = send_off[r - 1] + (int64_t)m(c->rank, r - 1);
+    // every rank can evaluate every rank's receive total, so all ranks fail together
     for (int r = 0; r < world; r++) {
-      if (r == c->rank) { c->peer_base[r] = ws; continue; }
-      if (c->peer_base[r] && memcmp(&c->peer_handle[r], &blobs[r].handle, sizeof(cudaIpcMemHandle_t)) == 0) continue;
-      changed = true;
-      if (c->peer_base[r]) { cudaIpcCloseMemHandle(c->peer_base[r]); c->peer_base[r] = nullptr; }
-      void *pp = nullptr;
-      cudaError_t e = cudaIpcOpenMemHandle(&pp, blobs[r].handle, cudaIpcMemLazyEnablePeerAccess);
-      if (e != cudaSuccess) { cudaGetLastError(); ok = false; continue; }
-      c->peer_base[r] = pp;
-      c->peer_handle[r] = blobs[r].handle;
+      int64_t t = 0;
+      for (int s = 0; s < world; s++) t += (int64_t)m(s, r);
+      if (t > blobs[r].capacity)
+        return fail(B200SORT_ENOMEM, "rank %d would receive %lld records, its capacity is %lld", r, (long long)t, (long long)blobs[r].capacity);
     }
-    // agreement: one failed mapping anywhere sends everybody to the NCCL path for good.  Every rank sees every
-    // handle, so all ranks know alike whether any mapping had to be (re)opened -- a rank's own new handle is new
-    // for all the others at once -- and the all-reduce is only paid then.
-    if (changed || my_handle_changed) {
-      unsigned long long flag = ok ? 0ull : 1ull;
-      CUDA_TRY(cudaMemcpyAsync(c->d_counts, &flag, sizeof flag, cudaMemcpyHostToDevice, stream));
-      NCCL_TRY(api.AllReduce(c->d_counts, c->d_counts, 1, ncclUint64, ncclSum, c->comm, stream));
-      CUDA_TRY(cudaMemcpyAsync(&flag, c->d_counts, sizeof flag, cudaMemcpyDeviceToHost, stream));
-      CUDA_TRY(cudaStreamSynchronize(stream));
-      if (flag != 0) { c->p2p_failed = true; p2p = false; }
-    }
+    return 0;
   }
-  trace.mark("map");
-  c->last_p2p = p2p;
-  overlap = overlap && p2p;  // (p2p is an agreed value)
-  c->last_overlap = overlap;
 
-  *out_num_local = recv_total;
-  CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
-  uint64_t *lookback = (uint64_t *)(ws + L.lookback_off);
-  uint32_t *tile_counter = (uint32_t *)(ws + L.tilectr_off);
-  int64_t peer_delta[RADIX] = {0};
-  for (int r = 0; r < world; r++) peer_delta[r] = p2p ? (int64_t)((intptr_t)c->peer_base[r] - (intptr_t)ws) : 0;
-  CUDA_TRY(cudaMemcpyAsync(c->d_peer_delta, peer_delta, sizeof peer_delta, cudaMemcpyHostToDevice, stream));
-  Plan plan{};
-  plan.final_sel = 1; plan.n_exec = 1;
-  CUDA_TRY(cudaMemcpyAsync(c->d_plan, &plan, sizeof plan, cudaMemcpyHostToDevice, stream));
-  // leading key bits this rank's range [bounds[rank], bounds[rank+1]) of top-`bits` values has in common
-  int lead = 0;
-  if (!heavy && kb == 8 && lo == 0 && shift == 8 * kb - bits && bounds[c->rank + 1] > bounds[c->rank]) {
-    const uint32_t x = bounds[c->rank] ^ (bounds[c->rank + 1] - 1);
-    lead = x ? __builtin_clz(x) - (32 - bits) : bits;
+  // peer mapping: the peer-memory path if everybody is willing and has an equal layout; maps the workspaces that
+  // changed since the last sort
+  int map_peers() {
+    p2p = true;
+    for (int r = 0; r < world; r++) p2p = p2p && blobs[r].p2p == 1 && blobs[r].ws_bytes == L.total && blobs[r].capacity == capacity;
+    if (p2p) {
+      bool ok = true;
+      bool changed = false;
+      for (int r = 0; r < world; r++) {
+        if (r == c->rank) { c->peer_base[r] = ws; continue; }
+        if (c->peer_base[r] && memcmp(&c->peer_handle[r], &blobs[r].handle, sizeof(cudaIpcMemHandle_t)) == 0) continue;
+        changed = true;
+        if (c->peer_base[r]) { cudaIpcCloseMemHandle(c->peer_base[r]); c->peer_base[r] = nullptr; }
+        void *pp = nullptr;
+        cudaError_t e = cudaIpcOpenMemHandle(&pp, blobs[r].handle, cudaIpcMemLazyEnablePeerAccess);
+        if (e != cudaSuccess) { cudaGetLastError(); ok = false; continue; }
+        c->peer_base[r] = pp;
+        c->peer_handle[r] = blobs[r].handle;
+      }
+      // agreement: one failed mapping anywhere sends everybody to the NCCL path for good.  Every rank sees every
+      // handle, so all ranks know alike whether any mapping had to be (re)opened -- a rank's own new handle is new
+      // for all the others at once -- and the all-reduce is only paid then.
+      if (changed || my_handle_changed) {
+        unsigned long long flag = ok ? 0ull : 1ull;
+        CUDA_TRY(cudaMemcpyAsync(c->d_counts, &flag, sizeof flag, cudaMemcpyHostToDevice, stream));
+        NCCL_TRY(api.AllReduce(c->d_counts, c->d_counts, 1, ncclUint64, ncclSum, c->comm, stream));
+        CUDA_TRY(cudaMemcpyAsync(&flag, c->d_counts, sizeof flag, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaStreamSynchronize(stream));
+        if (flag != 0) { c->p2p_failed = true; p2p = false; }
+      }
+    }
+    trace.mark("map");
+    c->last_p2p = p2p;
+    overlap = overlap && p2p;  // (p2p is an agreed value)
+    c->last_overlap = overlap;
+    return 0;
   }
-  auto partition_args = [&](int pass, int64_t t_first, int64_t n_end) -> SweepArgs {
+
+  // what the partition pass(es) need on the device: cleared control block, peer offsets, a one-pass plan, and the
+  // bucket offsets -- one table per chunk: where my records (of chunk ch) go inside rank r's receive range (peer
+  // path), or inside my own shadow arrays (NCCL path); buckets past the world take none
+  int prepare_partition() {
+    CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
+    int64_t peer_delta[RADIX] = {0};
+    for (int r = 0; r < world; r++) peer_delta[r] = p2p ? (int64_t)((intptr_t)c->peer_base[r] - (intptr_t)ws) : 0;
+    CUDA_TRY(cudaMemcpyAsync(c->d_peer_delta, peer_delta, sizeof peer_delta, cudaMemcpyHostToDevice, stream));
+    Plan plan{};
+    plan.final_sel = 1; plan.n_exec = 1;
+    CUDA_TRY(cudaMemcpyAsync(c->d_plan, &plan, sizeof plan, cudaMemcpyHostToDevice, stream));
+    const int n_tables = overlap ? n_chunks : 1;
+    std::vector<uint64_t> bb((size_t)n_tables * RADIX, (uint64_t)num_local);
+    for (int r = 0; r < world; r++) {
+      int64_t o = p2p ? 0 : send_off[r];
+      for (int s2 = 0; p2p && s2 < c->rank; s2++) o += (int64_t)m(s2, r);
+      for (int ch = 0; ch < n_tables; ch++) {
+        bb[(size_t)ch * RADIX + r] = (uint64_t)o;
+        if (overlap) o += (int64_t)blobs[c->rank].chunk_counts[ch][r];
+      }
+    }
+    CUDA_TRY(cudaMemcpyAsync(c->d_bin_base, bb.data(), bb.size() * 8, cudaMemcpyHostToDevice, stream));
+    return 0;
+  }
+
+  // the partition pass over my tiles from t_first on (records < n_end): bucket d = what goes to rank d
+  SweepArgs partition_args(int pass, int64_t t_first, int64_t n_end) {
     SweepArgs wa{};
     wa.ss = ss; wa.n = n_end; wa.ko = ko; wa.pass = pass; wa.shift = 0;
     if (p2p && landing)
       for (size_t s2 = 0; s2 < streams.size(); s2++) wa.ss.streams[s2].buf[1] = ws + L.land_off[s2];
-    wa.bin_base = c->d_bin_base + (size_t)pass * RADIX; wa.lookback = lookback;
+    wa.bin_base = c->d_bin_base + (size_t)pass * RADIX; wa.lookback = (uint64_t *)(ws + L.lookback_off);
     // (look-back tags 16.. : the local sort's passes, tags 1..8, reuse the same table later)
-    wa.tile_counter = tile_counter; wa.plan = c->d_plan; wa.tag = 16u + (uint32_t)pass; wa.stage_bytes = stage_bytes;
+    wa.tile_counter = (uint32_t *)(ws + L.tilectr_off); wa.plan = c->d_plan; wa.tag = 16u + (uint32_t)pass; wa.stage_bytes = stage_bytes;
     wa.part = part; wa.lut_world = world; wa.tile_first = (uint32_t)t_first; wa.peer_wide = opt_mgpu_wide.load() != 0 ? 1u : 0u;
     wa.peer_delta = p2p ? c->d_peer_delta : nullptr;
     return wa;
-  };
+  }
 
-  if (!overlap) {
-    // 4: partition by destination: one scatter pass; bucket d = what goes to rank d.
-    //    peer path : caller arrays -> shadow (or landing) arrays OF RANK d, at the offset where this rank's records belong
-    //    NCCL path : caller arrays -> own shadow arrays, then send/recv
-    uint64_t bin_base[RADIX] = {0};
-    for (int r = 0; r < RADIX; r++) {
-      if (r < world) {
-        if (p2p) {
-          int64_t o = 0;
-          for (int s2 = 0; s2 < c->rank; s2++) o += (int64_t)m(s2, r);  // my region inside rank r's receive range
-          bin_base[r] = (uint64_t)o;
-        } else {
-          bin_base[r] = (uint64_t)send_off[r];
-        }
-      } else {
-        bin_base[r] = (uint64_t)num_local;
-      }
-    }
-    CUDA_TRY(cudaMemcpyAsync(c->d_bin_base, bin_base, sizeof bin_base, cudaMemcpyHostToDevice, stream));
+  // plain exchange: one partition pass.  Peer path: caller arrays -> shadow (or landing) arrays OF RANK d, at the
+  // offset where this rank's records belong.  NCCL path: caller arrays -> own shadow arrays, then send/recv.
+  // Then the local sort of what arrived.
+  int plain_exchange() {
     if (num_local > 0) {
       SweepArgs wa = partition_args(0, 0, num_local);
-      CUDA_TRY(launch_sweep(kb, cfg, wa, n_tiles_local, di.smem_optin, di.sm_count, stream));
+      CUDA_TRY(launch_sweep(kb, cfg, wa, ct[n_chunks], di.smem_optin, di.sm_count, stream));
     }
     trace.mark(p2p ? "partition+exchange" : "partition");
+    DevSortOpts so;
+    so.layout_n = n_ws;
+    so.layout_landing = landing;
     if (p2p) {
       // barrier: nobody reads its shadow arrays before every rank's scatter kernel has finished (the
       // all-reduce is ordered after the local kernel on each rank's stream and completes when all joined)
       NCCL_TRY(api.AllReduce(c->d_counts, c->d_counts, 1, ncclUint64, ncclSum, c->comm, stream));
       trace.mark("barrier");
-      // 5: local sort, input in the shadow arrays, result in the caller's arrays
-      if (recv_total > 0) {
-        DevSortOpts so;
-        so.start_sel = landing ? 0 : 1;
-        so.layout_n = n_ws;
-        so.hint_lead_bits = lead;
-        so.layout_landing = landing;
-        so.landing_input = landing;
-        int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so);
-        if (rc != 0) return rc;
-      }
+      // local sort, input in the shadow (or landing) arrays, result in the caller's arrays
+      so.start_sel = landing ? 0 : 1;
+      so.hint_lead_bits = lead[c->rank];
+      so.landing_input = landing;
+      if (recv_total > 0)
+        if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
     } else {
       // all-to-all-v, shadow -> caller arrays
       NCCL_TRY(api.GroupStart());
       for (size_t s = 0; s < streams.size(); s++) {
         const size_t eb = streams[s].elem_bytes;
         for (int p = 0; p < world; p++) {
-          const size_t sb = (size_t)send[p] * eb, rb = (size_t)m(p, c->rank) * eb;
+          const size_t sb = (size_t)m(c->rank, p) * eb, rb = (size_t)m(p, c->rank) * eb;
           if (sb) NCCL_TRY(api.Send(ss.streams[s].buf[1] + (size_t)send_off[p] * eb, sb, ncclUint8, p, c->comm, stream));
           if (rb) NCCL_TRY(api.Recv(ss.streams[s].buf[0] + (size_t)recv_off[p] * eb, rb, ncclUint8, p, c->comm, stream));
         }
       }
       NCCL_TRY(api.GroupEnd());
       trace.mark("exchange");
-      if (recv_total > 1) {
-        DevSortOpts so;
-        so.layout_n = n_ws;
-        so.layout_landing = landing;
-        int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so);
-        if (rc != 0) return rc;
-      }
+      if (recv_total > 1)
+        if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
     }
     trace.mark("local_sort");
-    trace.report(c->rank);
     return 0;
   }
 
@@ -1330,172 +1329,145 @@ static int mgpu_sort(b200sort_comm *c, int key_type, const std::vector<StreamDes
   // main stream : partition kernel of chunk 0, signal, chunk 1, signal, ...
   // side stream : wait for all sources' chunk 0, first-pass kernels over the eight regions of it, wait chunk 1, ...
   // then the main stream joins and runs the remaining passes of the local sort.
-  const uint32_t my_cut = d_cut[c->rank], my_lshift = d_lshift[c->rank];
-  const int n_launch = n_chunks * world;
-  {
-    // where my records of chunk ch go inside rank r's receive range
-    std::vector<uint64_t> bb((size_t)n_chunks * RADIX, 0);
-    for (int r = 0; r < world; r++) {
-      int64_t o = 0;
-      for (int s2 = 0; s2 < c->rank; s2++) o += (int64_t)m(s2, r);
-      for (int ch = 0; ch < n_chunks; ch++) {
-        bb[(size_t)ch * RADIX + r] = (uint64_t)o;
-        o += (int64_t)blobs[c->rank].chunk_counts[ch][r];
-      }
-    }
-    for (int ch = 0; ch < n_chunks; ch++)
-      for (int r = world; r < RADIX; r++) bb[(size_t)ch * RADIX + r] = (uint64_t)num_local;
-    CUDA_TRY(cudaMemcpyAsync(c->d_bin_base, bb.data(), bb.size() * 8, cudaMemcpyHostToDevice, stream));
-    // bucket offsets of my first pass: launch (ch, s2) sweeps what source s2 sent me in chunk ch; its keys of digit d
-    // go behind those of all earlier launches (any order is fine for a first pass)
-    std::vector<uint64_t> cb((size_t)n_launch * RADIX, 0);
-    uint64_t tot[RADIX] = {0};
-    for (int ch = 0; ch < n_chunks; ch++)
-      for (int s2 = 0; s2 < world; s2++)
-        for (int d = 0; d < RADIX; d++) tot[d] += blobs[s2].chunk_hist[ch][c->rank][d];
-    uint64_t run[RADIX];
-    uint64_t acc = 0;
-    for (int d = 0; d < RADIX; d++) { run[d] = acc; acc += tot[d]; }
-    if ((int64_t)acc != recv_total) return fail(B200SORT_ECUDA, "internal: first-digit histograms (%llu) disagree with the record counts (%lld)", (unsigned long long)acc, (long long)recv_total);
-    for (int ch = 0; ch < n_chunks; ch++)
-      for (int s2 = 0; s2 < world; s2++) {
-        const int Lx = ch * world + s2;
-        for (int d = 0; d < RADIX; d++) { cb[(size_t)Lx * RADIX + d] = run[d]; run[d] += blobs[s2].chunk_hist[ch][c->rank][d]; }
-      }
-    CUDA_TRY(cudaMemcpyAsync(c->d_cons_base, cb.data(), cb.size() * 8, cudaMemcpyHostToDevice, stream));
-    CUDA_TRY(cudaMemsetAsync(c->d_cons_ctr, 0, sizeof(uint32_t) * (MGPU_MAX_CHUNKS * 8 + MGPU_MAX_CHUNKS), stream));
-    // the first pass's look-back table: the junction table's memory (unused until the last pass)
-    CUDA_TRY(cudaMemsetAsync(ws + L.jtable_off, 0, (size_t)L.n_tiles * RADIX * 8, stream));
-  }
-  CUDA_TRY(cudaEventRecord(c->ev_fork, stream));
-  CUDA_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-  // (trace: when each chunk's partition kernel, arrival and first-pass kernels finished, relative to the fork)
-  std::vector<std::pair<std::string, cudaEvent_t>> tl;
-  auto tl_mark = [&](const std::string &name, cudaStream_t st2) {
-    if (!trace.on) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, st2);
-    tl.emplace_back(name, e);
-  };
-  tl_mark("fork", stream);
-  SignalArgs sg{};
-  sg.world = world; sg.me = c->rank;
-  for (int r = 0; r < world; r++) sg.peer_flags[r] = (uint32_t *)((unsigned char *)c->peer_base[r] + L.flags_off);
-  const uint32_t epoch = c->seq * 16u;
-  // ONE partition kernel for all chunks, launched with about one and a half CTAs per SM that loop over the tile
-  // tickets (so that the first-pass kernels of the side stream find room on every SM the whole time); the CTA
-  // that delivers the last tile of a chunk writes the chunk's arrival flag into every destination's flag array.
-  // (A chunk without tiles is signalled from here.)
-  for (int ch = 0; ch < n_chunks; ch++)
-    if (ct[ch + 1] == ct[ch]) {
-      sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
-      mgpu_signal_kernel<<<1, 32, 0, stream>>>(sg);
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-    }
-  const int64_t persist_x2 = opt_mgpu_persist_x2.load();
-  if (persist_x2 <= 0) {
-    // variant: one ordinary partition kernel per chunk (one CTA per tile), each followed by a one-warp kernel
-    // that writes the chunk's flags (the first-pass kernels of the high-priority side stream then alternate with
-    // the chunks' partition kernels rather than run beside them)
-    std::vector<uint64_t> bb((size_t)n_chunks * RADIX, 0);
-    for (int r = 0; r < world; r++) {
-      int64_t o = 0;
-      for (int s2 = 0; s2 < c->rank; s2++) o += (int64_t)m(s2, r);
-      for (int ch = 0; ch < n_chunks; ch++) {
-        bb[(size_t)ch * RADIX + r] = (uint64_t)o;
-        o += (int64_t)blobs[c->rank].chunk_counts[ch][r];
-      }
-    }
-    for (int ch = 0; ch < n_chunks; ch++)
-      for (int r = world; r < RADIX; r++) bb[(size_t)ch * RADIX + r] = (uint64_t)num_local;
-    CUDA_TRY(cudaMemcpyAsync(c->d_bin_base, bb.data(), bb.size() * 8, cudaMemcpyHostToDevice, stream));
-    for (int ch = 0; ch < n_chunks; ch++) {
-      if (ct[ch + 1] == ct[ch]) continue;  // (signalled above)
-      SweepArgs wa = partition_args(ch, ct[ch], std::min<int64_t>(num_local, ct[ch + 1] * tile));
-      CUDA_TRY(launch_sweep(kb, cfg, wa, ct[ch + 1] - ct[ch], di.smem_optin, di.sm_count, stream));
-      sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
-      mgpu_signal_kernel<<<1, 32, 0, stream>>>(sg);
-      g_launches++;
-      CUDA_TRY(cudaGetLastError());
-    }
-  } else if (n_tiles_local > 0) {
-    SweepArgs wa = partition_args(0, 0, num_local);
-    wa.sig_n = (uint32_t)n_chunks;
-    for (int ch = 0; ch <= n_chunks; ch++) wa.sig_ct[ch] = (uint32_t)ct[ch];
-    wa.sig_done = c->d_cons_ctr + MGPU_MAX_CHUNKS * 8;
-    for (int r = 0; r < world; r++) wa.sig_flags[r] = sg.peer_flags[r];
-    wa.sig_me = (uint32_t)c->rank; wa.sig_value = epoch + 1u;
-    const int64_t cap = std::max<int64_t>(1, (int64_t)di.sm_count * persist_x2 / 2);
-    CUDA_TRY(launch_sweep(kb, cfg, wa, n_tiles_local, di.smem_optin, di.sm_count, stream, false, 0, cap));
-  }
-  tl_mark("sent_all", stream);
-  for (int ch = 0; ch < n_chunks; ch++) {
-    // receiver side of the same chunk
-    mgpu_wait_kernel<<<1, 32, 0, c->side>>>((const uint32_t *)(ws + L.flags_off), world, ch, epoch + (uint32_t)ch + 1u);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    tl_mark("arrived" + std::to_string(ch), c->side);
-    int64_t tiles_before = 0;
-    for (int c2 = 0; c2 < ch; c2++)
-      for (int s2 = 0; s2 < world; s2++) tiles_before += ((int64_t)blobs[s2].chunk_counts[c2][c->rank] + tile - 1) / tile;
-    for (int s2 = 0; s2 < world; s2++) {
-      const int64_t cnt = (int64_t)blobs[s2].chunk_counts[ch][c->rank];
-      const int64_t tiles_here = (cnt + tile - 1) / tile;
-      if (cnt > 0) {
-        int64_t lo_rec = recv_off[s2];
-        for (int c2 = 0; c2 < ch; c2++) lo_rec += (int64_t)blobs[s2].chunk_counts[c2][c->rank];
-        SweepArgs wa{};
-        wa.ss = ss;
-        for (size_t q = 0; q < streams.size(); q++) {  // landing sub-range in, shadow arrays out
-          wa.ss.streams[q].buf[0] = ws + L.land_off[q] + (size_t)lo_rec * streams[q].elem_bytes;
-          wa.ss.streams[q].buf[1] = ws + L.shadow_off[q];
+  int overlapped_exchange() {
+    const uint32_t my_cut = d_cut[c->rank], my_lshift = d_lshift[c->rank];
+    const int n_launch = n_chunks * world;
+    {
+      // bucket offsets of my first pass: launch (ch, s2) sweeps what source s2 sent me in chunk ch; its keys of digit d
+      // go behind those of all earlier launches (any order is fine for a first pass)
+      std::vector<uint64_t> cb((size_t)n_launch * RADIX, 0);
+      uint64_t tot[RADIX] = {0};
+      for (int ch = 0; ch < n_chunks; ch++)
+        for (int s2 = 0; s2 < world; s2++)
+          for (int d = 0; d < RADIX; d++) tot[d] += blobs[s2].chunk_hist[ch][c->rank][d];
+      uint64_t run[RADIX];
+      uint64_t acc = 0;
+      for (int d = 0; d < RADIX; d++) { run[d] = acc; acc += tot[d]; }
+      if ((int64_t)acc != recv_total) return fail(B200SORT_ECUDA, "internal: first-digit histograms (%llu) disagree with the record counts (%lld)", (unsigned long long)acc, (long long)recv_total);
+      for (int ch = 0; ch < n_chunks; ch++)
+        for (int s2 = 0; s2 < world; s2++) {
+          const int Lx = ch * world + s2;
+          for (int d = 0; d < RADIX; d++) { cb[(size_t)Lx * RADIX + d] = run[d]; run[d] += blobs[s2].chunk_hist[ch][c->rank][d]; }
         }
-        wa.n = cnt; wa.ko = ko; wa.pass = ch * world + s2; wa.shift = (int)my_cut * RADIX_BITS;
-        wa.bin_base = c->d_cons_base + (size_t)(ch * world + s2) * RADIX;
-        wa.ghist = (uint64_t *)(ws + L.ghist2_off);
-        wa.lookback = (uint64_t *)(ws + L.jtable_off) + (size_t)tiles_before * RADIX;
-        wa.tile_counter = c->d_cons_ctr; wa.plan = c->d_plan; wa.tag = my_cut + 1; wa.stage_bytes = stage_bytes;
-        wa.plan_in_args = 1; wa.arg_sel = 0; wa.arg_next_p1 = my_cut + 2; wa.arg_next_skewed = 0; wa.arg_sub = 0; wa.arg_lshift = my_lshift;
-        // (high-priority stream: without a bound on its CTAs per SM the first pass would take every slot that frees
-        //  up and starve the partition kernel -- measured: the two then simply alternate)
-        CUDA_TRY(launch_sweep(kb, cfg, wa, tiles_here, di.smem_optin, di.sm_count, c->side, /*first_pass_unordered=*/true,
-                              (size_t)std::max<int64_t>(opt_mgpu_cons_smem_kb.load(), 0) << 10));
+      CUDA_TRY(cudaMemcpyAsync(c->d_cons_base, cb.data(), cb.size() * 8, cudaMemcpyHostToDevice, stream));
+      CUDA_TRY(cudaMemsetAsync(c->d_cons_ctr, 0, sizeof(uint32_t) * (MGPU_MAX_CHUNKS * 8 + MGPU_MAX_CHUNKS), stream));
+      // the first pass's look-back table: the junction table's memory (unused until the last pass)
+      CUDA_TRY(cudaMemsetAsync(ws + L.jtable_off, 0, (size_t)L.n_tiles * RADIX * 8, stream));
+    }
+    CUDA_TRY(cudaEventRecord(c->ev_fork, stream));
+    CUDA_TRY(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
+    trace.mark("fork", stream);
+    SignalArgs sg{};
+    sg.world = world; sg.me = c->rank;
+    for (int r = 0; r < world; r++) sg.peer_flags[r] = (uint32_t *)((unsigned char *)c->peer_base[r] + L.flags_off);
+    const uint32_t epoch = c->seq * 16u;
+    // ONE partition kernel for all chunks, launched with about one and a half CTAs per SM that loop over the tile
+    // tickets (so that the first-pass kernels of the side stream find room on every SM the whole time); the CTA
+    // that delivers the last tile of a chunk writes the chunk's arrival flag into every destination's flag array.
+    // (A chunk without tiles is signalled from here.)
+    for (int ch = 0; ch < n_chunks; ch++)
+      if (ct[ch + 1] == ct[ch]) {
+        sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
+        CUDA_TRY(launch(PK_NONE, mgpu_signal_kernel, 1, 32, 0, stream, sg));
       }
-      tiles_before += tiles_here;
+    const int64_t persist_x2 = opt_mgpu_persist_x2.load();
+    if (persist_x2 <= 0) {
+      // variant: one ordinary partition kernel per chunk (one CTA per tile), each followed by a one-warp kernel
+      // that writes the chunk's flags (the first-pass kernels of the high-priority side stream then alternate with
+      // the chunks' partition kernels rather than run beside them)
+      for (int ch = 0; ch < n_chunks; ch++) {
+        if (ct[ch + 1] == ct[ch]) continue;  // (signalled above)
+        SweepArgs wa = partition_args(ch, ct[ch], std::min<int64_t>(num_local, ct[ch + 1] * tile));
+        CUDA_TRY(launch_sweep(kb, cfg, wa, ct[ch + 1] - ct[ch], di.smem_optin, di.sm_count, stream));
+        sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
+        CUDA_TRY(launch(PK_NONE, mgpu_signal_kernel, 1, 32, 0, stream, sg));
+      }
+    } else if (ct[n_chunks] > 0) {
+      SweepArgs wa = partition_args(0, 0, num_local);
+      wa.sig_n = (uint32_t)n_chunks;
+      for (int ch = 0; ch <= n_chunks; ch++) wa.sig_ct[ch] = (uint32_t)ct[ch];
+      wa.sig_done = c->d_cons_ctr + MGPU_MAX_CHUNKS * 8;
+      for (int r = 0; r < world; r++) wa.sig_flags[r] = sg.peer_flags[r];
+      wa.sig_me = (uint32_t)c->rank; wa.sig_value = epoch + 1u;
+      const int64_t cap = std::max<int64_t>(1, (int64_t)di.sm_count * persist_x2 / 2);
+      CUDA_TRY(launch_sweep(kb, cfg, wa, ct[n_chunks], di.smem_optin, di.sm_count, stream, false, 0, cap));
     }
-    tl_mark("swept" + std::to_string(ch), c->side);
-  }
-  CUDA_TRY(cudaEventRecord(c->ev_join, c->side));
-  CUDA_TRY(cudaStreamWaitEvent(stream, c->ev_join, 0));
-  trace.mark("exchange+first_pass");
-  if (recv_total > 0) {
-    DevSortOpts so;
-    so.layout_n = n_ws;
-    so.layout_landing = landing;
-    so.landing_input = true;
-    so.forced = true;
-    so.forced_cut = my_cut;
-    so.forced_lshift = my_lshift;
-    int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so);
-    if (rc != 0) return rc;
-  }
-  trace.mark("local_sort_rest");
-  if (trace.on) {
-    cudaStreamSynchronize(stream);
-    std::string line = "[b200sort mgpu rank " + std::to_string(c->rank) + "] timeline (ms after the fork):";
-    for (size_t i = 1; i < tl.size(); i++) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, tl[0].second, tl[i].second);
-      char buf[64];
-      snprintf(buf, sizeof buf, " %s=%.2f", tl[i].first.c_str(), ms);
-      line += buf;
+    trace.mark("sent_all", stream);
+    int64_t tiles_before = 0;
+    for (int ch = 0; ch < n_chunks; ch++) {
+      // receiver side of the same chunk
+      CUDA_TRY(launch(PK_NONE, mgpu_wait_kernel, 1, 32, 0, c->side, (const uint32_t *)(ws + L.flags_off), world, ch, epoch + (uint32_t)ch + 1u));
+      trace.mark("arrived" + std::to_string(ch), c->side);
+      for (int s2 = 0; s2 < world; s2++) {
+        const int64_t cnt = (int64_t)blobs[s2].chunk_counts[ch][c->rank];
+        const int64_t tiles_here = (cnt + tile - 1) / tile;
+        if (cnt > 0) {
+          int64_t lo_rec = recv_off[s2];
+          for (int c2 = 0; c2 < ch; c2++) lo_rec += (int64_t)blobs[s2].chunk_counts[c2][c->rank];
+          SweepArgs wa{};
+          wa.ss = ss;
+          for (size_t q = 0; q < streams.size(); q++) {  // landing sub-range in, shadow arrays out
+            wa.ss.streams[q].buf[0] = ws + L.land_off[q] + (size_t)lo_rec * streams[q].elem_bytes;
+            wa.ss.streams[q].buf[1] = ws + L.shadow_off[q];
+          }
+          wa.n = cnt; wa.ko = ko; wa.pass = ch * world + s2; wa.shift = (int)my_cut * RADIX_BITS;
+          wa.bin_base = c->d_cons_base + (size_t)(ch * world + s2) * RADIX;
+          wa.ghist = (uint64_t *)(ws + L.ghist2_off);
+          wa.lookback = (uint64_t *)(ws + L.jtable_off) + (size_t)tiles_before * RADIX;
+          wa.tile_counter = c->d_cons_ctr; wa.plan = c->d_plan; wa.tag = my_cut + 1; wa.stage_bytes = stage_bytes;
+          wa.plan_in_args = 1; wa.arg_sel = 0; wa.arg_next_p1 = my_cut + 2; wa.arg_next_skewed = 0; wa.arg_sub = 0; wa.arg_lshift = my_lshift;
+          // (high-priority stream: without a bound on its CTAs per SM the first pass would take every slot that frees
+          //  up and starve the partition kernel -- measured: the two then simply alternate)
+          CUDA_TRY(launch_sweep(kb, cfg, wa, tiles_here, di.smem_optin, di.sm_count, c->side, /*first_pass_unordered=*/true,
+                                (size_t)std::max<int64_t>(opt_mgpu_cons_smem_kb.load(), 0) << 10));
+        }
+        tiles_before += tiles_here;
+      }
+      trace.mark("swept" + std::to_string(ch), c->side);
     }
-    fprintf(stderr, "%s\n", line.c_str());
-    for (auto &e : tl) cudaEventDestroy(e.second);
+    CUDA_TRY(cudaEventRecord(c->ev_join, c->side));
+    CUDA_TRY(cudaStreamWaitEvent(stream, c->ev_join, 0));
+    trace.mark("exchange+first_pass");
+    if (recv_total > 0) {
+      DevSortOpts so;
+      so.layout_n = n_ws;
+      so.layout_landing = landing;
+      so.landing_input = true;
+      so.forced = true;
+      so.forced_cut = my_cut;
+      so.forced_lshift = my_lshift;
+      if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
+    }
+    trace.mark("local_sort_rest");
+    return 0;
   }
-  trace.report(c->rank);
+};
+
+static int mgpu_sort(b200sort_comm *c, int key_type, const std::vector<StreamDesc> &streams, int64_t num_local, int64_t capacity,
+                     bool ascending, int64_t *out_num_local, cudaStream_t stream) {
+  DeviceScope dev_scope;  // the communicator's device, whatever the caller's current device is
+  if (dev_scope.enter(c->dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", c->dev);
+  MgpuSort s{c, nccl_api(), key_type, streams, num_local, capacity, ascending, stream};
+  c->seq++;
+  c->last_overlap = false;
+  if (int rc = s.setup()) return rc;
+  if (int rc = s.splitters()) return rc;
+  s.decide_overlap();
+  if (int rc = s.exchange_blobs()) return rc;
+  if (int rc = s.map_peers()) return rc;
+  *out_num_local = s.recv_total;
+  if (int rc = s.prepare_partition()) return rc;
+  if (int rc = s.overlap ? s.overlapped_exchange() : s.plain_exchange()) return rc;
+  s.trace.report(c->rank);
+  return 0;
+}
+
+// what both multi-GPU entry points check before anything else
+static int mgpu_check(const b200sort_comm *c, int64_t num_local, int64_t capacity, const int64_t *out_num_local) {
+  NcclApi &api = nccl_api();
+  if (!api.ok) return fail(B200SORT_ENCCL, "NCCL unavailable: %s", api.why.c_str());
+  if (!c || !out_num_local) return fail(B200SORT_EINVAL, "comm/out_num_local is NULL");
+  if (capacity < num_local) return fail(B200SORT_EINVAL, "capacity smaller than num_local");
   return 0;
 }
 
@@ -1507,11 +1479,8 @@ int b200sort_mgpu_sort_soa(b200sort_comm *c, void *keys, int key_type, int64_t n
                            int ascending, int n_payloads, void *const *payloads, const uint32_t *payload_elem_bytes,
                            int64_t *out_num_local, void *stream_v) {
   using namespace b200sort;
-  NcclApi &api = nccl_api();
-  if (!api.ok) return fail(B200SORT_ENCCL, "NCCL unavailable: %s", api.why.c_str());
-  if (!c || !out_num_local) return fail(B200SORT_EINVAL, "comm/out_num_local is NULL");
-  if (capacity < num_local) return fail(B200SORT_EINVAL, "capacity smaller than num_local");
   std::vector<StreamDesc> streams;
+  if (int rc = mgpu_check(c, num_local, capacity, out_num_local)) return rc;
   if (int rc = check_soa(keys, key_type, num_local, n_payloads, payloads, payload_elem_bytes, &streams)) return rc;
   if (!keys) return fail(B200SORT_EINVAL, "keys is NULL");
   return mgpu_sort(c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v);
@@ -1520,11 +1489,8 @@ int b200sort_mgpu_sort_soa(b200sort_comm *c, void *keys, int key_type, int64_t n
 int b200sort_mgpu_sort_aos(b200sort_comm *c, void *records, int key_type, uint32_t record_bytes, int64_t num_local,
                            int64_t capacity, int ascending, int64_t *out_num_local, void *stream_v) {
   using namespace b200sort;
-  NcclApi &api = nccl_api();
-  if (!api.ok) return fail(B200SORT_ENCCL, "NCCL unavailable: %s", api.why.c_str());
-  if (!c || !out_num_local) return fail(B200SORT_EINVAL, "comm/out_num_local is NULL");
-  if (capacity < num_local) return fail(B200SORT_EINVAL, "capacity smaller than num_local");
   std::vector<StreamDesc> streams;
+  if (int rc = mgpu_check(c, num_local, capacity, out_num_local)) return rc;
   if (int rc = check_aos(records, key_type, record_bytes, num_local, &streams)) return rc;
   if (!records) return fail(B200SORT_EINVAL, "records is NULL");
   return mgpu_sort(c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v);
