@@ -113,10 +113,10 @@ int b200sort_version(void);
  * for its gpu_launches field). */
 uint64_t b200sort_launch_count(void);
 
-/* Tuning/ablation knobs, process-wide.  Known names: "algo" (0 auto, 1 LSD one-sweep passes,
+/* Tuning/ablation knobs: process-wide defaults, read once when a call starts.  Known names: "algo" (0 auto, 1 LSD one-sweep passes,
  * 2 hybrid MSB), "tile_cfg" (index of the scatter tile geometry), "first_atomic", "tma_keys", "bytewise",
  * "hist_match", "allow_skip", "profile", "mgpu_overlap", "mgpu_chunks", "mgpu_refine" (INTEGRATION.md lists them
- * all).  Returns 0, or B200SORT_EINVAL for an unknown name. */
+ * all).  Returns 0, or B200SORT_EINVAL for an unknown name or a value "max_chunk" does not take. */
 int b200sort_set_option(const char *name, int64_t value);
 int64_t b200sort_get_option(const char *name);
 

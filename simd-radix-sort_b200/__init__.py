@@ -9,8 +9,8 @@ Both sort IN PLACE, like the reference, and go through the C ABI of include/b200
 (libb200sort.so, hand-written CUDA for sm_100a).  There is no CPU implementation in this package:
 if the library is missing or no CUDA device is usable the calls raise.
 """
-from ._api import (B200SortError, KEY_TYPES, last_profile, last_stats, launch_count, lib, lib_path, set_option, get_option, sort,
-                   sort_combined, workspace_bytes, version)
+from ._api import (B200SortError, KEY_TYPES, last_profile, last_stats, launch_count, lib, lib_path, options, set_option, get_option,
+                   sort, sort_combined, workspace_bytes, version)
 
-__all__ = ["B200SortError", "KEY_TYPES", "last_profile", "last_stats", "launch_count", "lib", "lib_path", "set_option",
+__all__ = ["B200SortError", "KEY_TYPES", "last_profile", "last_stats", "launch_count", "lib", "lib_path", "options", "set_option",
            "get_option", "sort", "sort_combined", "workspace_bytes", "version"]

@@ -1,6 +1,7 @@
 """ctypes binding of include/b200sort.h + the Python mirror of the reference's sort<> overloads."""
 from __future__ import annotations
 
+import contextlib
 import ctypes
 from pathlib import Path
 
@@ -113,6 +114,24 @@ def set_option(name: str, value: int):
 
 def get_option(name: str) -> int:
     return int(lib().b200sort_get_option(name.encode()))
+
+
+@contextlib.contextmanager
+def options(**values):
+    """Sets options for the body of a `with` block: `with options(algo=2, margin_bits=-2): ...`.
+
+    The values they had before are restored on the way out, also when the body raises.  Options are
+    process-wide defaults that a sort reads once when it starts."""
+    saved = {}
+    try:
+        for name, value in values.items():
+            before = get_option(name)
+            set_option(name, value)
+            saved[name] = before
+        yield
+    finally:
+        for name, value in saved.items():
+            set_option(name, value)
 
 
 def last_stats() -> dict:

@@ -33,38 +33,71 @@ namespace b200sort {
 // errors, options, counters
 // ------------------------------------------------------------------------------------------------
 static thread_local std::string g_last_error;
-static thread_local b200sort_stats g_last_stats{};
-static thread_local bool g_have_stats = false;
+static thread_local b200sort_stats g_last_stats = {-1};  // what the last successful sort on this thread did (num < 0: none yet)
 static std::atomic<uint64_t> g_launches{0};
 
-static std::atomic<int64_t> opt_algo{0};       // 0 auto, 1 LSD, 2 hybrid
-static std::atomic<int64_t> opt_tile_cfg{-1};  // -1 auto
-static std::atomic<int64_t> opt_allow_skip{1};
-static std::atomic<int64_t> opt_allow_reduce{1};
-static std::atomic<int64_t> opt_spin_ns{0};
-static std::atomic<int64_t> opt_fix_in_pass{1};  // order tile-local segments in the last pass + junction fix instead of the full finish
-static std::atomic<int64_t> opt_hist_match{0};
-static std::atomic<int64_t> opt_margin_bits{2};
-static std::atomic<int64_t> opt_probe_guess{1};
-static std::atomic<int64_t> opt_probe_sample{16};  // large sorts: every this-many-th tile feeds the sampled histograms
-static std::atomic<int64_t> opt_allow_lshift{1};
-static std::atomic<int64_t> opt_junction_table{1};  // junction kernel compares fingerprints left by the last pass
-static std::atomic<int64_t> opt_host_pipeline{1};  // host SoA arrays: sort keys + index while the payloads upload
-static std::atomic<int64_t> opt_mgpu_landing{1};  // multi-GPU: receive into a third set of arrays (saves the final copy)
-static std::atomic<int64_t> opt_mgpu_p2p{1};  // multi-GPU: scatter straight into peer memory (0: NCCL send/recv)
-static std::atomic<int64_t> opt_mgpu_refine{1};   // multi-GPU: refine heavy splitter bins / split heavy key values (0: fail with ENOMEM)
-static std::atomic<int64_t> opt_mgpu_overlap{0};  // multi-GPU: chunked exchange overlapped with the receivers' first pass (measured: no gain, see DESIGN.md)
-static std::atomic<int64_t> opt_mgpu_chunks{4};   // ... in this many chunks
-static std::atomic<int64_t> opt_mgpu_wide{1};     // multi-GPU: 16-byte peer stores of element pairs
-static std::atomic<int64_t> opt_mgpu_cons_smem_kb{0};   // overlapped first pass: shared memory requested per CTA (bounds its CTAs per SM; 0 = what it needs)
-static std::atomic<int64_t> opt_mgpu_persist_x2{0};     // overlapped exchange: CTAs per SM of the looping partition kernel, times two
-static std::atomic<int64_t> opt_mgpu_chunk_min_log2{24};  // ... when a rank holds at least 2^this records
-static std::atomic<int64_t> opt_host_plan_min_log2{24};  // hybrid sorts of at least 2^this records read the plan back
+constexpr int MGPU_MAX_CHUNKS = 8;  // multi-GPU overlapped exchange: at most this many chunks (mgpu.cuh)
+
+// The tuning options of b200sort_set_option; the member initialisers are the defaults.  The process-wide values
+// are read once when a sort call starts (options()) and that snapshot is passed down.
+struct Options {
+  int64_t algo = 0, tile_cfg = -1;  // algo: 0 auto, 1 LSD, 2 hybrid; tile_cfg: -1 auto, else the index of a tile geometry
+  int64_t wide_tiles = 1;     // 4-byte keys, all chunks <= 4 bytes: 8192-key tiles
+  int64_t nstage = 0;         // 0 auto, 1 single staging buffer, 2 double-buffered columns
+  int64_t max_chunk = 16;     // largest chunk a stream is moved in (ablation: 8 = AoS records as 8-byte columns)
+  int64_t tma_keys = 1;       // key tiles arrive by one TMA bulk copy per tile (cp.async.bulk + mbarrier)
+  int64_t prefetch_cols = 1;  // the tile's part of the payload columns is prefetched into L2 when the tile starts
+  int64_t bytewise = 1;       // lean kernels when the host knows the plan (no range reduction / shift)
+  int64_t first_atomic = 1;   // first executed pass of a large sort: unstable atomicAdd ranking
+  int64_t allow_skip = 1, allow_reduce = 1, allow_lshift = 1, spin_ns = 0, hist_match = 0, margin_bits = 2, probe_guess = 1;
+  // the last pass orders tile-local segments + junction fix instead of the full finish; the junction kernel compares
+  // fingerprints left by the last pass
+  int64_t fix_in_pass = 1, junction_table = 1;
+  int64_t probe_sample = 16;  // large sorts: every this-many-th tile feeds the sampled histograms
+  int64_t host_plan_min_log2 = 24;  // hybrid sorts of at least 2^this records read the plan back
+  int64_t host_pipeline = 1;  // host SoA arrays: sort keys + index while the payloads upload
+  int64_t profile = 0;        // CUDA events around every launch of the sort (b200sort_last_profile)
+  int64_t mgpu_landing = 1;  // multi-GPU: receive into a third set of arrays (saves the final copy)
+  int64_t mgpu_p2p = 1;      // multi-GPU: scatter straight into peer memory (0: NCCL send/recv)
+  int64_t mgpu_refine = 1;   // multi-GPU: refine heavy splitter bins / split heavy key values (0: fail with ENOMEM)
+  int64_t mgpu_wide = 1;     // multi-GPU: 16-byte peer stores of element pairs
+  // multi-GPU: chunked exchange overlapped with the receivers' first pass (measured: no gain, see DESIGN.md), in
+  // mgpu_chunks chunks when a rank holds at least 2^mgpu_chunk_min_log2 records
+  int64_t mgpu_overlap = 0, mgpu_chunks = 4, mgpu_chunk_min_log2 = 24;
+  int64_t mgpu_cons_smem_kb = 0;   // overlapped first pass: shared memory requested per CTA (bounds its CTAs per SM; 0 = what it needs)
+  int64_t mgpu_persist_x2 = 0;     // overlapped exchange: CTAs per SM of the looping partition kernel, times two
+};
+static const struct { const char *name; int64_t Options::*member; } kOptionNames[] = {
+    {"algo", &Options::algo}, {"tile_cfg", &Options::tile_cfg}, {"wide_tiles", &Options::wide_tiles}, {"nstage", &Options::nstage},
+    {"max_chunk", &Options::max_chunk}, {"tma_keys", &Options::tma_keys}, {"prefetch_cols", &Options::prefetch_cols},
+    {"bytewise", &Options::bytewise}, {"first_atomic", &Options::first_atomic}, {"allow_skip", &Options::allow_skip},
+    {"allow_reduce", &Options::allow_reduce}, {"allow_lshift", &Options::allow_lshift}, {"spin_ns", &Options::spin_ns},
+    {"hist_match", &Options::hist_match}, {"margin_bits", &Options::margin_bits}, {"probe_guess", &Options::probe_guess},
+    {"fix_in_pass", &Options::fix_in_pass}, {"junction_table", &Options::junction_table}, {"probe_sample", &Options::probe_sample},
+    {"host_plan_min_log2", &Options::host_plan_min_log2}, {"host_pipeline", &Options::host_pipeline}, {"profile", &Options::profile},
+    {"mgpu_landing", &Options::mgpu_landing}, {"mgpu_p2p", &Options::mgpu_p2p}, {"mgpu_refine", &Options::mgpu_refine},
+    {"mgpu_wide", &Options::mgpu_wide}, {"mgpu_overlap", &Options::mgpu_overlap}, {"mgpu_chunks", &Options::mgpu_chunks},
+    {"mgpu_chunk_min_log2", &Options::mgpu_chunk_min_log2}, {"mgpu_cons_smem_kb", &Options::mgpu_cons_smem_kb},
+    {"mgpu_persist_x2", &Options::mgpu_persist_x2}};
+static std::mutex g_opt_mu;
+static Options g_opt;  // (under g_opt_mu) the values b200sort_set_option set
+
+// the options a sort call runs with: the values set when it starts, brought into their valid ranges
+static Options options() {
+  Options o;
+  { std::lock_guard<std::mutex> lk(g_opt_mu); o = g_opt; }
+  o.host_plan_min_log2 = std::clamp<int64_t>(o.host_plan_min_log2, 0, 62);
+  o.probe_sample = std::max<int64_t>(o.probe_sample, 1);
+  o.mgpu_chunks = std::clamp<int64_t>(o.mgpu_chunks, 1, MGPU_MAX_CHUNKS);
+  o.mgpu_chunk_min_log2 = std::clamp<int64_t>(o.mgpu_chunk_min_log2, 12, 40);
+  o.mgpu_cons_smem_kb = std::max<int64_t>(o.mgpu_cons_smem_kb, 0);
+  return o;
+}
 
 // optional per-kernel timing (option "profile"): CUDA events around every launch of the last sort
 enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5 };
 struct ProfEntry { int kind; cudaEvent_t e0, e1; int dev; };
-static std::atomic<int64_t> opt_profile{0};
+static thread_local bool g_prof_on = false;  // the sort running on this thread has option "profile" set
 static thread_local std::vector<ProfEntry> g_prof;
 static thread_local std::map<int, std::vector<cudaEvent_t>> g_prof_pool;  // per device: events belong to one
 
@@ -79,7 +112,7 @@ static cudaEvent_t prof_event(int dev) {
 }
 struct ProfScope {  // (kind PK_NONE: records nothing)
   bool on; ProfEntry pe; cudaStream_t st;
-  ProfScope(int kind, cudaStream_t s) : on(kind != PK_NONE && opt_profile.load() != 0), st(s), kind_(kind) {
+  ProfScope(int kind, cudaStream_t s) : on(kind != PK_NONE && g_prof_on), st(s), kind_(kind) {
     if (on) { pe.dev = 0; cudaGetDevice(&pe.dev); pe.kind = kind; pe.e0 = prof_event(pe.dev); pe.e1 = prof_event(pe.dev); cudaEventRecord(pe.e0, st); }
   }
   ~ProfScope() {
@@ -171,14 +204,6 @@ static size_t sweep_smem_bytes(const TileCfg &c, uint32_t stage_bytes, int nstag
          (lut ? RADIX * 8 : 0);   // LUT: peer byte offsets
 }
 
-static std::atomic<int64_t> opt_nstage{0};  // 0 auto, 1 single staging buffer, 2 double-buffered columns
-static std::atomic<int64_t> opt_prefetch_cols{1};  // the tile's part of the payload columns is prefetched into L2 when the tile starts
-static std::atomic<int64_t> opt_max_chunk{16};     // largest chunk a stream is moved in (ablation: 8 = AoS records as 8-byte columns)
-static std::atomic<int64_t> opt_wide_tiles{1};    // 4-byte keys, all chunks <= 4 bytes: 8192-key tiles
-static std::atomic<int64_t> opt_tma_keys{1};      // key tiles arrive by one TMA bulk copy per tile (cp.async.bulk + mbarrier)
-static std::atomic<int64_t> opt_bytewise{1};      // lean kernels when the host knows the plan (no range reduction / shift)
-static std::atomic<int64_t> opt_first_atomic{1};  // first executed pass of a large sort: unstable atomicAdd ranking
-
 inline SweepFn sweep_fn(int kb, int cfg, const SweepSel &s) {
   switch (kb * 2 + cfg) {
     case 2: return sweep_fn_inst<1, 0>(s);
@@ -197,7 +222,7 @@ inline SweepFn sweep_fn(int kb, int cfg, const SweepSel &s) {
 // digit's histogram is not skewed -- the unstable ranking may be used
 // smem_floor: request at least this much dynamic shared memory (bounds how many CTAs of this launch an SM holds:
 // the overlapped first pass of the multi-GPU sort must leave room for the partition kernel's CTAs)
-static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_tiles, size_t smem_optin, int sm_count, cudaStream_t st,
+static cudaError_t launch_sweep(const Options &o, int kb, int cfg, const SweepArgs &a, int64_t n_tiles, size_t smem_optin, cudaStream_t st,
                                 bool first_pass_unordered = false, size_t smem_floor = 0, int64_t grid_cap = 0) {
   bool any = false;  // a stream with 1- or 2-byte chunks in the move loop needs the ANYCHUNK instantiation
   int n_cols = 0;
@@ -212,10 +237,10 @@ static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_t
   const bool fix = !lut && a.fix_cut != 0;  // (the caller only sets fix_cut where the FIX instantiation exists)
   int rank = RANK_BALLOT;
   // digits are whole bytes of the raw key when the host knows that the plan has no range reduction and no shift
-  const bool bytewise = !lut && a.plan_in_args != 0 && a.arg_sub == 0 && a.arg_lshift == 0 && opt_bytewise.load() != 0;
-  if (first_pass_unordered && a.plan_in_args != 0 && !lut && !fix && opt_first_atomic.load() != 0) rank = RANK_ATOMIC;
+  const bool bytewise = !lut && a.plan_in_args != 0 && a.arg_sub == 0 && a.arg_lshift == 0 && o.bytewise != 0;
+  if (first_pass_unordered && a.plan_in_args != 0 && !lut && !fix && o.first_atomic != 0) rank = RANK_ATOMIC;
   // double-buffer the columns when there is more than one and minb CTAs still fit on an SM
-  int nstage = (int)opt_nstage.load();
+  int nstage = (int)o.nstage;
   if (nstage != 1 && nstage != 2)
     nstage = (n_cols >= 2 && (sweep_smem_bytes(tc, a.stage_bytes, 2) + 1024) * tc.minb <= smem_optin + 1024) ? 2 : 1;
   if (nstage == 2 && sweep_smem_bytes(tc, a.stage_bytes, 2) > smem_optin) nstage = 1;
@@ -223,7 +248,7 @@ static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_t
   SweepSel sel{nstage, any || lut, lut, fix, rank, bytewise};
   SweepArgs a2 = a;
   // TMA bulk load of the key tile: SoA keys whose arrays (both sides of the ping-pong) are 16-byte aligned
-  a2.tma_keys = (opt_tma_keys.load() != 0 && soa && (((uintptr_t)a.ss.streams[0].buf[0] | (uintptr_t)a.ss.streams[0].buf[1]) & 15) == 0 &&
+  a2.tma_keys = (o.tma_keys != 0 && soa && (((uintptr_t)a.ss.streams[0].buf[0] | (uintptr_t)a.ss.streams[0].buf[1]) & 15) == 0 &&
                  ((size_t)tc.threads * tc.ipt * kb) % 16 == 0) ? 1u : 0u;
   SweepFn k = sweep_fn(kb, cfg, sel);
   const size_t smem = std::min(std::max(sweep_smem_bytes(tc, a.stage_bytes, nstage, fix, lut), smem_floor), smem_optin);
@@ -232,17 +257,15 @@ static cudaError_t launch_sweep(int kb, int cfg, const SweepArgs &a, int64_t n_t
   // one shared-memory carve-out for every instantiation: kernels that want different L1 / shared-memory splits
   // cannot be resident on an SM together (the overlapped exchange runs two of them side by side)
   // (only for the kernels of the overlapped exchange: a maximal carve-out leaves the other sorts 28 KB of L1,
-  //  which costs them 4 % -- 38.2 vs 36.8 ms at 1e9 records)
-  if (smem_floor != 0 || grid_cap != 0 || opt_mgpu_overlap.load() != 0) {
-    e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-  }
-  (void)sm_count;
+  //  which costs them 4 % -- 38.2 vs 36.8 ms at 1e9 records).  Set on every launch: the setting outlives the sort.
+  e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, (smem_floor != 0 || grid_cap != 0 || o.mgpu_overlap != 0)
+                           ? (int)cudaSharedmemCarveoutMaxShared : (int)cudaSharedmemCarveoutDefault);
+  if (e != cudaSuccess) return e;
   // L2 prefetch of the tile's part of the first column after the keys (16-byte aligned on both sides)
   a2.prefetch_cols = 0;
   {
     const int s2 = a2.tma_keys ? 1 : 0;
-    if (opt_prefetch_cols.load() != 0 && s2 < a.ss.n_streams) {
+    if (o.prefetch_cols != 0 && s2 < a.ss.n_streams) {
       const Stream &st2 = a.ss.streams[s2];
       const size_t bytes = (size_t)tc.threads * tc.ipt * st2.chunk_bytes * st2.chunks_per_elem;
       if ((((uintptr_t)st2.buf[0] | (uintptr_t)st2.buf[1] | bytes) & 15) == 0) {
@@ -275,11 +298,11 @@ static int64_t hist_tile_keys(int kb, const void *keys, uint32_t stride) {
   return (int64_t)HIST_THREADS * nld * (16 / kb);
 }
 
-cudaError_t launch_hist(int kb, const HistArgs &a, int sm_count, int probe, cudaStream_t st) {
+static cudaError_t launch_hist(const Options &o, int kb, const HistArgs &a, int sm_count, int probe, cudaStream_t st) {
   const int64_t tile_keys = hist_tile_keys(kb, a.keys, a.stride);
   const int64_t tiles = (a.n + tile_keys - 1) / tile_keys;
   const int grid = (int)std::min<int64_t>(tiles, (int64_t)sm_count * 8);
-  const bool m = opt_hist_match.load() != 0;
+  const bool m = o.hist_match != 0;
   return with_kb(kb, [&](auto K) {
     constexpr int KB = decltype(K)::value;
     if constexpr (KB == 8)
@@ -385,11 +408,11 @@ struct Layout {
   int64_t n_tiles;
 };
 
-static int pick_tile_cfg(int kb, uint32_t stage_bytes, size_t smem_optin, int64_t n) {
-  int cfg = (int)opt_tile_cfg.load();
+static int pick_tile_cfg(const Options &o, int kb, uint32_t stage_bytes, size_t smem_optin, int64_t n) {
+  int cfg = (int)o.tile_cfg;
   const bool automatic = cfg < 0 || cfg >= kNumTileCfgs;
   // (wide tiles only where there are plenty of them: 10^6 records are 123 wide tiles for 148 SMs -- 0.18 vs 0.13 ms)
-  if (automatic) cfg = (kb == 4 && stage_bytes <= 4 && n >= ((int64_t)1 << 24) && opt_wide_tiles.load() != 0) ? kWideTileCfg : kDefaultTileCfg;
+  if (automatic) cfg = (kb == 4 && stage_bytes <= 4 && n >= ((int64_t)1 << 24) && o.wide_tiles != 0) ? kWideTileCfg : kDefaultTileCfg;
   if (cfg == kWideTileCfg && (kb != 4 || stage_bytes > 4)) cfg = kDefaultTileCfg;  // (only instantiated for that shape)
   // fall back to the smaller tile if the staging buffer would not fit
   if (sweep_smem_bytes(kTileCfgs[cfg], stage_bytes) > smem_optin) cfg = 1;
@@ -426,8 +449,8 @@ static void make_layout(const std::vector<StreamDesc> &streams, int64_t n, int t
 }
 
 // The arrays as the streams the scatter kernel moves: each one in chunks of the largest power of two <= max_chunk
-// (and <= 16) dividing both its address and its element size.  Returns the staging buffer's element size: the
-// largest chunk, at least the key.
+// (and <= 16) dividing both its address and its element size; the key stream (keys or records) in chunks no narrower
+// than the key, whatever max_chunk says.  Returns the staging buffer's element size: the largest chunk, at least the key.
 static uint32_t make_stream_set(const std::vector<StreamDesc> &streams, int kb, uint32_t max_chunk, StreamSet *ss) {
   uint32_t stage_bytes = (uint32_t)kb;
   *ss = StreamSet{};
@@ -435,7 +458,7 @@ static uint32_t make_stream_set(const std::vector<StreamDesc> &streams, int kb, 
   for (size_t s = 0; s < streams.size(); s++) {
     uint32_t c = 16;
     while (c > 1 && ((streams[s].elem_bytes % c) != 0 || ((uintptr_t)streams[s].ptr % c) != 0)) c >>= 1;
-    c = std::min(c, max_chunk);
+    if (c > max_chunk) c = std::max(max_chunk, s == 0 ? (uint32_t)kb : 1u);
     ss->streams[s].chunk_bytes = c;
     ss->streams[s].chunks_per_elem = streams[s].elem_bytes / c;
     ss->streams[s].buf[0] = (unsigned char *)streams[s].ptr;
@@ -453,7 +476,6 @@ struct DevSortOpts {
   bool landing_input = false;   // the input lies in the landing arrays: the first executed pass reads it from
                                 // there (landing -> shadow -> caller -> ...), so that an even number of passes
                                 // ends in the caller's arrays without a copy
-  int force_algo = 0;           // 1 / 2: use this algorithm whatever option "algo" says (the hybrid path's fall-back)
   // Multi-GPU sort with the exchange overlapped (mgpu.cuh): the plan is fixed by the caller (forced_plan), the
   // control block has been cleared by the caller, and the FIRST executed pass has already been run by the
   // caller (landing arrays -> shadow arrays, its successor's digit counted into the exact histograms).
@@ -498,12 +520,10 @@ static Plan forced_plan(int kb, uint32_t cut, uint32_t lshift) {
   return p;
 }
 
-static int sort_device(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
-                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo = DevSortOpts());
-
 // One sort of device arrays, phase by phase: one histogram sweep over all digit positions, the bucket-offset scan
 // (+ pass plan), one scatter pass per digit position, the segment finish, the copy-back.
 struct DevSort {
+  const Options &o;
   const int key_type;
   const bool ascending;
   const int64_t n;
@@ -541,12 +561,12 @@ struct DevSort {
   int setup() {
     CUDA_TRY(cudaGetDevice(&dev));
     if (int rc = dev_info(dev, &di)) return rc;
-    stage_bytes = make_stream_set(streams, kb, (uint32_t)std::max<int64_t>(opt_max_chunk.load(), 1), &ss);
+    stage_bytes = make_stream_set(streams, kb, (uint32_t)o.max_chunk, &ss);
     if (streams[0].elem_bytes != (uint32_t)kb && ((uintptr_t)streams[0].ptr % kb) != 0)
       return fail(B200SORT_EINVAL, "record array is not aligned to its key type");
     if (((uintptr_t)streams[0].ptr % kb) != 0) return fail(B200SORT_EINVAL, "key array is not aligned to its key type");
 
-    cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, n);
+    cfg = pick_tile_cfg(o, kb, stage_bytes, di.smem_optin, n);
     const TileCfg tc = kTileCfgs[cfg];
     tile = tc.threads * tc.ipt;
     const size_t smem = sweep_smem_bytes(tc, stage_bytes);
@@ -566,12 +586,12 @@ struct DevSort {
     for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
     plan = (Plan *)(ws + L.plan_off);
     ctrl = (HybridCtrl *)(ws + L.hyb_off);
+    g_prof_on = o.profile != 0;
     if (!xo.forced) prof_reset();
     if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
 
     ko = make_key_order(key_type, ascending);
-    algo = xo.force_algo != 0 ? xo.force_algo : (int)opt_algo.load();
-    if (xo.forced) algo = 2;
+    algo = xo.forced ? 2 : (int)o.algo;
     if (algo == 0) algo = (kb == 8 && n >= HYB_MIN_N) ? 2 : 1;
     if (algo == 2 && kb != 8) algo = 1;
     hybrid = algo == 2;
@@ -598,7 +618,7 @@ struct DevSort {
   // right, the passes that are not skipped.  Smaller sorts launch everything; what is not needed returns at once.
   int make_plan() {
     uint64_t *ghist = (uint64_t *)(ws + L.ghist_off), *ghist_exact = (uint64_t *)(ws + L.ghist2_off);
-    const bool big = xo.forced || n >= (int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_host_plan_min_log2.load(), 0), 62);
+    const bool big = xo.forced || n >= (int64_t)1 << o.host_plan_min_log2;
     // Input in the landing arrays (multi-GPU): only the large hybrid flow knows on the host which pass runs
     // first; everything else simply starts with a copy into the caller's arrays.
     landing = xo.landing_input;
@@ -615,7 +635,7 @@ struct DevSort {
     ha.n = n; ha.ko = ko; ha.digit_mask = (1u << kb) - 1; ha.ghist = ghist; ha.probe = (ProbeOut *)(ws + L.probe_off);
     // entropies from one key per thread of every 16th tile (option probe_sample) once there are plenty of tiles
     const bool sparse = (n / hist_tile_keys(kb, ha.keys, ha.stride)) >= 8192;
-    ha.sample = sparse ? (uint32_t)std::max<int64_t>(1, opt_probe_sample.load()) : 1;
+    ha.sample = sparse ? (uint32_t)o.probe_sample : 1;
     ha.sample_one = sparse ? 1 : 0;
     // Large sorts leave the exact key range to a sweep of its own that only runs when the sampled range says
     // range reduction may pay; the others get it from the probe.
@@ -626,14 +646,14 @@ struct DevSort {
     uint32_t guess = 0;
     if (hybrid) {
       // hint_lead_bits: leading bits the caller expects all keys to agree on (a shard of the multi-GPU sort)
-      const double need = std::log2((double)n) + (double)opt_margin_bits.load();
+      const double need = std::log2((double)n) + (double)o.margin_bits;
       const int cut = 8 - xo.hint_lead_bits / 8 - (int)std::ceil(need / 8.0);
       if (cut >= 2) {
         guess = (uint32_t)cut;
-        ha.guess_lshift = opt_allow_lshift.load() != 0 ? (uint32_t)(xo.hint_lead_bits & 7) : 0u;
+        ha.guess_lshift = o.allow_lshift != 0 ? (uint32_t)(xo.hint_lead_bits & 7) : 0u;
       }
     }
-    ha.guess_p1 = opt_probe_guess.load() != 0 ? guess + 1 : 0;
+    ha.guess_p1 = o.probe_guess != 0 ? guess + 1 : 0;
     ha.ghist_exact = ghist_exact;
     if (xo.forced) {  // the caller's plan (its probe, scan and first pass ran overlapped with the exchange)
       hist_sweeps = 0;
@@ -642,16 +662,16 @@ struct DevSort {
       have_plan = true;
       return 0;
     }
-    CUDA_TRY(launch_hist(kb, ha, di.sm_count, /*probe=*/1, stream));
+    CUDA_TRY(launch_hist(o, kb, ha, di.sm_count, /*probe=*/1, stream));
 
     ScanArgs sa{};
     sa.ghist = ghist; sa.probe = ha.probe; sa.plan = plan; sa.n = n; sa.n_passes = kb;
-    sa.allow_skip = (int)opt_allow_skip.load();
+    sa.allow_skip = (int)o.allow_skip;
     sa.hybrid = hybrid ? 1 : 0;
-    sa.allow_reduce = (int)opt_allow_reduce.load();
-    sa.margin_bits = (float)opt_margin_bits.load();
+    sa.allow_reduce = (int)o.allow_reduce;
+    sa.margin_bits = (float)o.margin_bits;
     sa.have_minmax = (int)ha.with_minmax;
-    sa.allow_lshift = (int)opt_allow_lshift.load();
+    sa.allow_lshift = (int)o.allow_lshift;
     sa.start_sel = (uint32_t)xo.start_sel;
     sa.guess_p1 = ha.guess_p1; sa.guess_lshift = ha.guess_lshift; sa.ghist_exact = ghist_exact;
     CUDA_TRY(launch(PK_SCAN, scan_kernel, 1, RADIX, 0, stream, sa));
@@ -663,7 +683,7 @@ struct DevSort {
       if (ev == nullptr) return fail(B200SORT_ECUDA, "cudaEventCreate failed on device %d", dev);
       if (int rc = read_plan(ev)) return rc;
       if (hplan.want_minmax) {
-        CUDA_TRY(launch_hist(kb, ha, di.sm_count, /*minmax=*/2, stream));
+        CUDA_TRY(launch_hist(o, kb, ha, di.sm_count, /*minmax=*/2, stream));
         hist_sweeps++;
         sa.have_minmax = 1;
         CUDA_TRY(launch(PK_SCAN, scan_kernel, 1, RADIX, 0, stream, sa));
@@ -672,7 +692,7 @@ struct DevSort {
       have_plan = true;
       if (hplan.hist_done) return 0;
     }
-    CUDA_TRY(launch_hist(kb, hb, di.sm_count, /*probe=*/0, stream));
+    CUDA_TRY(launch_hist(o, kb, hb, di.sm_count, /*probe=*/0, stream));
     hist_sweeps++;
     return 0;
   }
@@ -684,7 +704,7 @@ struct DevSort {
     const bool soa = streams[0].elem_bytes == (uint32_t)kb;
     partial = have_plan && hplan.cut_digit != 0 && xo.cmp_none_thresh >= CMP_NONE_MIN_THRESH;
     const bool use_fix = !partial && have_plan && hplan.cut_digit != 0 && (soa || ss.streams[0].chunk_bytes >= (uint32_t)kb) &&
-                         cfg == kDefaultTileCfg && opt_fix_in_pass.load() != 0;
+                         cfg == kDefaultTileCfg && o.fix_in_pass != 0;
     if (landing && hplan.n_exec == 0)  // nothing will move the records: deliver them
       if (int rc = deliver_landing()) return rc;
     bool first_exec = true;
@@ -698,7 +718,7 @@ struct DevSort {
       wa.ko = ko; wa.pass = p; wa.shift = p * RADIX_BITS;
       wa.bin_base = nullptr; wa.ghist = (uint64_t *)(ws + L.ghist2_off);
       wa.lookback = (uint64_t *)(ws + L.lookback_off); wa.tile_counter = (uint32_t *)(ws + L.tilectr_off); wa.plan = plan;
-      wa.tag = (uint32_t)(p + 1); wa.stage_bytes = stage_bytes; wa.spin_ns = (uint32_t)opt_spin_ns.load();
+      wa.tag = (uint32_t)(p + 1); wa.stage_bytes = stage_bytes; wa.spin_ns = (uint32_t)o.spin_ns;
       if (have_plan) {
         wa.plan_in_args = 1; wa.arg_sel = hplan.src_sel[p]; wa.arg_next_p1 = hplan.next_exec_p1[p];
         wa.arg_next_skewed = hplan.next_exec_p1[p] ? hplan.skewed[hplan.next_exec_p1[p] - 1] : 0; wa.arg_sub = hplan.sub; wa.arg_lshift = hplan.lshift;
@@ -706,7 +726,7 @@ struct DevSort {
       }
       // the first executed pass may rank its keys in any order (nothing has been established yet)
       const bool unordered = have_plan && was_first && hplan.skewed[p] == 0;
-      CUDA_TRY(launch_sweep(kb, cfg, wa, (n + tile - 1) / tile, di.smem_optin, di.sm_count, stream, unordered));
+      CUDA_TRY(launch_sweep(o, kb, cfg, wa, (n + tile - 1) / tile, di.smem_optin, stream, unordered));
     }
     return 0;
   }
@@ -737,7 +757,7 @@ struct DevSort {
       JunctionArgs ja{};
       ja.ss = ss; ja.n = n; ja.ko = ko; ja.ko.sub = hplan.sub; ja.ko.lshift = hplan.lshift; ja.lookback = (uint64_t *)(ws + L.lookback_off);
       ja.n_tiles = n_tiles; ja.tag = (uint32_t)(last_pass + 1); ja.cut = hplan.cut_digit; ja.sel = hplan.final_sel; ja.flag = &ctrl->flags[1];
-      ja.jtable = opt_junction_table.load() != 0 ? (const uint64_t *)(ws + L.jtable_off) : nullptr;
+      ja.jtable = o.junction_table != 0 ? (const uint64_t *)(ws + L.jtable_off) : nullptr;
       CUDA_TRY(launch(PK_SEGFIX, junction_fix_kernel<8>, (unsigned)((n_tiles * RADIX + 255) / 256), 256, 0, stream, ja));
     } else if (partial) {
       PartialCheckArgs pa{};
@@ -794,35 +814,39 @@ struct DevSort {
   // fall-back: finish with the plain digit-by-digit path (the array is a permutation of the input, already ordered
   // by its top digits)
   int fall_back(b200sort_stats *stt) {
+    Options lsd = o; lsd.algo = 1;  // (whatever option "algo" says)
     DevSortOpts fo;
-    fo.layout_n = xo.layout_n; fo.layout_landing = xo.layout_landing; fo.force_algo = 1;
-    if (int rc = sort_device(key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo)) return rc;
-    const b200sort_stats &s2 = g_last_stats;
+    fo.layout_n = xo.layout_n; fo.layout_landing = xo.layout_landing;
+    b200sort_stats s2;
+    if (int rc = DevSort{lsd, key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo}.run(&s2)) return rc;
     stt->fell_back = 1;
     stt->passes_planned += s2.passes_planned;
     stt->hist_sweeps += s2.hist_sweeps;
     stt->algorithmic_bytes += s2.algorithmic_bytes;
     return 0;
   }
+
+  // the sort, phase by phase; *stats: what ran (written when the sort succeeds)
+  int run(b200sort_stats *stats) {
+    const uint64_t launches_before = g_launches.load();
+    if (int rc = setup()) return rc;
+    if (int rc = make_plan()) return rc;
+    if (int rc = run_passes()) return rc;
+    if (int rc = finish()) return rc;
+    b200sort_stats stt;
+    bool fell_back = false;
+    if (int rc = statistics(&stt, &fell_back)) return rc;
+    if (fell_back)
+      if (int rc = fall_back(&stt)) return rc;
+    stt.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
+    *stats = stt;
+    return B200SORT_OK;
+  }
 };
 
-static int sort_device(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
-                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo) {
-  const uint64_t launches_before = g_launches.load();
-  DevSort s{key_type, ascending, n, streams, stream, workspace, workspace_bytes, xo};
-  if (int rc = s.setup()) return rc;
-  if (int rc = s.make_plan()) return rc;
-  if (int rc = s.run_passes()) return rc;
-  if (int rc = s.finish()) return rc;
-  b200sort_stats stt;
-  bool fall_back = false;
-  if (int rc = s.statistics(&stt, &fall_back)) return rc;
-  if (fall_back)
-    if (int rc = s.fall_back(&stt)) return rc;
-  stt.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
-  g_last_stats = stt;
-  g_have_stats = true;
-  return B200SORT_OK;
+static int sort_device(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
+                       cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo, b200sort_stats *stats) {
+  return DevSort{o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, xo}.run(stats);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -886,7 +910,8 @@ static bool host_is_pinned(const void *p) {
   return at.type == cudaMemoryTypeHost;
 }
 
-static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, cudaStream_t caller) {
+static int sort_host_pipelined(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
+                               cudaStream_t caller, b200sort_stats *stats) {
   const int kb = key_bytes_of(key_type);
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
@@ -954,7 +979,7 @@ static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const st
     CUDA_TRY(cudaStreamWaitEvent(st_comp, e_keys, 0));
     CUDA_TRY(launch(PK_NONE, iota_kernel, di.sm_count * 8, 256, 0, st_comp, (uint32_t *)(dbuf + off_idx), n));
     std::vector<StreamDesc> ds = {{dbuf + off_keys, (uint32_t)kb}, {dbuf + off_idx, 4u}};
-    if (int r = sort_device(key_type, ascending, n, ds, st_comp, nullptr, 0)) return r;
+    if (int r = sort_device(o, key_type, ascending, n, ds, st_comp, nullptr, 0, DevSortOpts(), stats)) return r;
     cudaEvent_t e_sorted = new_event();
     CUDA_TRY(cudaEventRecord(e_sorted, st_comp));
     if (!pinned)
@@ -993,8 +1018,8 @@ static int sort_host_pipelined(int key_type, bool ascending, int64_t n, const st
   return rc;
 }
 
-static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
-                    void *workspace, size_t workspace_bytes, const DevSortOpts &base = DevSortOpts()) {
+static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
+                    void *workspace, size_t workspace_bytes, const DevSortOpts &base, b200sort_stats *stats) {
   cudaStream_t stream = (cudaStream_t)stream_v;
   if (n <= 1) return B200SORT_OK;  // src/radix_sort.hpp:276: nothing to do for 0 or 1 element
   int ndev = 0;
@@ -1017,11 +1042,11 @@ static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<S
   if (side0 == SIDE_DEVICE) {
     DeviceScope scope;  // sort on the device that owns the arrays (include/b200sort.h)
     if (scope.enter(dev0) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", dev0);
-    return sort_device(key_type, ascending, n, streams, stream, workspace, workspace_bytes, base);
+    return sort_device(o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, base, stats);
   }
 
   // ---- host arrays, SoA with payloads, big enough to care: pipelined staging --------------------------
-  if (opt_host_pipeline.load() != 0 && base.cmp_none_thresh == 0 && workspace == nullptr && streams.size() >= 2 &&
+  if (o.host_pipeline != 0 && base.cmp_none_thresh == 0 && workspace == nullptr && streams.size() >= 2 &&
       streams[0].elem_bytes == (uint32_t)key_bytes_of(key_type) && n >= ((int64_t)1 << 20) && n < ((int64_t)1 << 32)) {
     size_t need = 0;
     for (size_t s = 0; s < streams.size(); s++) need += (size_t)n * streams[s].elem_bytes * (s ? 2 : 1);
@@ -1031,7 +1056,7 @@ static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<S
     cudaGetDevice(&cur_dev);
     const size_t staged = cache_entry(CACHE_STAGE, cur_dev).bytes;
     if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need < free_b / 10 * 9 + staged)
-      return sort_host_pipelined(key_type, ascending, n, streams, stream);
+      return sort_host_pipelined(o, key_type, ascending, n, streams, stream, stats);
     cudaGetLastError();
   }
   // ---- host arrays: stage through device memory ---------------------------------------------------
@@ -1054,7 +1079,7 @@ static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<S
     e = cudaMemcpyAsync(dstreams[s].ptr, streams[s].ptr, (size_t)n * streams[s].elem_bytes, cudaMemcpyHostToDevice, stream);
     if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "H2D copy failed: %s", cudaGetErrorString(e));
   }
-  if (rc == 0) rc = sort_device(key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base);
+  if (rc == 0) rc = sort_device(o, key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base, stats);
   for (size_t s = 0; s < streams.size() && rc == 0; s++) {
     e = cudaMemcpyAsync(streams[s].ptr, dstreams[s].ptr, (size_t)n * streams[s].elem_bytes, cudaMemcpyDeviceToHost, stream);
     if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "D2H copy failed: %s", cudaGetErrorString(e));
@@ -1111,7 +1136,7 @@ int b200sort_sort_soa_ex(void *keys, int key_type, int64_t num, int ascending, i
   if (cmp_sorter == B200SORT_CMP_NONE && cmp_sort_threshold >= CMP_NONE_MIN_THRESH) base.cmp_none_thresh = cmp_sort_threshold;
   std::vector<StreamDesc> streams;
   if (int rc = check_soa(keys, key_type, num, n_payloads, payloads, payload_elem_bytes, &streams)) return rc;
-  return sort_any(key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base);
+  return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
 }
 
 int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int64_t num, int ascending,
@@ -1123,7 +1148,7 @@ int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int
   if (cmp_sorter == B200SORT_CMP_NONE && cmp_sort_threshold >= CMP_NONE_MIN_THRESH) base.cmp_none_thresh = cmp_sort_threshold;
   std::vector<StreamDesc> streams;
   if (int rc = check_aos(records, key_type, record_bytes, num, &streams)) return rc;
-  return sort_any(key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base);
+  return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
 }
 
 int b200sort_sort_soa(void *keys, int key_type, int64_t num, int ascending, int n_payloads, void *const *payloads,
@@ -1159,54 +1184,27 @@ const char *b200sort_last_error(void) { return g_last_error.c_str(); }
 int b200sort_version(void) { return B200SORT_VERSION; }
 uint64_t b200sort_launch_count(void) { return g_launches.load(); }
 
-static std::atomic<int64_t> *find_opt(const char *name) {
-  if (!name) return nullptr;
-  if (!strcmp(name, "algo")) return &opt_algo;
-  if (!strcmp(name, "tile_cfg")) return &opt_tile_cfg;
-  if (!strcmp(name, "first_atomic")) return &opt_first_atomic;
-  if (!strcmp(name, "tma_keys")) return &opt_tma_keys;
-  if (!strcmp(name, "prefetch_cols")) return &opt_prefetch_cols;
-  if (!strcmp(name, "wide_tiles")) return &opt_wide_tiles;
-  if (!strcmp(name, "max_chunk")) return &opt_max_chunk;
-  if (!strcmp(name, "bytewise")) return &opt_bytewise;
-  if (!strcmp(name, "allow_skip")) return &opt_allow_skip;
-  if (!strcmp(name, "allow_reduce")) return &opt_allow_reduce;
-  if (!strcmp(name, "spin_ns")) return &opt_spin_ns;
-  if (!strcmp(name, "fix_in_pass")) return &opt_fix_in_pass;
-  if (!strcmp(name, "hist_match")) return &opt_hist_match;
-  if (!strcmp(name, "profile")) return &opt_profile;
-  if (!strcmp(name, "margin_bits")) return &opt_margin_bits;
-  if (!strcmp(name, "probe_guess")) return &opt_probe_guess;
-  if (!strcmp(name, "probe_sample")) return &opt_probe_sample;
-  if (!strcmp(name, "allow_lshift")) return &opt_allow_lshift;
-  if (!strcmp(name, "mgpu_p2p")) return &opt_mgpu_p2p;
-  if (!strcmp(name, "mgpu_landing")) return &opt_mgpu_landing;
-  if (!strcmp(name, "mgpu_refine")) return &opt_mgpu_refine;
-  if (!strcmp(name, "mgpu_overlap")) return &opt_mgpu_overlap;
-  if (!strcmp(name, "mgpu_chunks")) return &opt_mgpu_chunks;
-  if (!strcmp(name, "mgpu_wide")) return &opt_mgpu_wide;
-  if (!strcmp(name, "mgpu_cons_smem_kb")) return &opt_mgpu_cons_smem_kb;
-  if (!strcmp(name, "mgpu_persist_x2")) return &opt_mgpu_persist_x2;
-  if (!strcmp(name, "mgpu_chunk_min_log2")) return &opt_mgpu_chunk_min_log2;
-  if (!strcmp(name, "host_pipeline")) return &opt_host_pipeline;
-  if (!strcmp(name, "junction_table")) return &opt_junction_table;
-  if (!strcmp(name, "host_plan_min_log2")) return &opt_host_plan_min_log2;
-  if (!strcmp(name, "nstage")) return &opt_nstage;
+static int64_t Options::*find_opt(const char *name) {
+  for (const auto &e : kOptionNames) if (name && !strcmp(name, e.name)) return e.member;
   return nullptr;
 }
 int b200sort_set_option(const char *name, int64_t value) {
-  auto *o = find_opt(name);
-  if (!o) return fail(B200SORT_EINVAL, "unknown option '%s'", name ? name : "(null)");
-  o->store(value);
+  int64_t Options::*m = find_opt(name);
+  if (!m) return fail(B200SORT_EINVAL, "unknown option '%s'", name ? name : "(null)");
+  if (m == &Options::max_chunk && (value < 1 || value > 16 || (value & (value - 1)) != 0))
+    return fail(B200SORT_EINVAL, "max_chunk must be a power of two in [1, 16], not %lld", (long long)value);
+  std::lock_guard<std::mutex> lk(g_opt_mu);
+  g_opt.*m = value;
   return 0;
 }
 int64_t b200sort_get_option(const char *name) {
-  auto *o = find_opt(name);
-  return o ? o->load() : INT64_MIN;
+  int64_t Options::*m = find_opt(name);
+  std::lock_guard<std::mutex> lk(g_opt_mu);
+  return m ? g_opt.*m : INT64_MIN;
 }
 
 int b200sort_last_stats(b200sort_stats *out) {
-  if (!out || !g_have_stats) return B200SORT_EINVAL;
+  if (!out || g_last_stats.num < 0) return B200SORT_EINVAL;
   *out = g_last_stats;
   return 0;
 }

@@ -587,7 +587,6 @@ static void tie_thresholds(int world, int rank, int n_blocks, uint64_t less_tota
 }  // namespace b200sort
 
 // what every rank tells the others before the exchange (all-gathered in one go)
-constexpr int MGPU_MAX_CHUNKS = 8;
 struct MgpuBlob {
   cudaIpcMemHandle_t handle;        // its workspace allocation
   unsigned long long ws_bytes;      // size of that allocation's layout (equal layouts <=> equal shadow offsets)
@@ -875,6 +874,7 @@ static int mgpu_refine_hist(void *ctx_v, int n_ranges, const uint64_t *lo, const
 // The distributed sort of b200sort_mgpu_sort_soa / b200sort_mgpu_sort_aos, phase by phase (mgpu_sort); streams[0]
 // carries the key at offset 0.
 struct MgpuSort {
+  const Options &o;
   b200sort_comm *const c;
   NcclApi &api;
   const int key_type;
@@ -882,6 +882,7 @@ struct MgpuSort {
   const int64_t num_local, capacity;
   const bool ascending;
   const cudaStream_t stream;
+  b200sort_stats *const stats;  // of the local sort
   const int kb = key_bytes_of(key_type);
   const int world = c->world;
   const int bits = std::min(MGPU_MAX_BITS, 8 * kb);
@@ -932,14 +933,14 @@ struct MgpuSort {
     if (int rc = dev_info(c->dev, &di)) return rc;
     // workspace, laid out for `capacity` records on every rank (so that equal capacities give equal layouts
     // and the local sort finds what the peers wrote where it expects its shadow arrays)
+    g_prof_on = o.profile != 0;
     stage_bytes = make_stream_set(streams, kb, 16, &ss);
-    cfg = pick_tile_cfg(kb, stage_bytes, di.smem_optin, num_local);
+    cfg = pick_tile_cfg(o, kb, stage_bytes, di.smem_optin, num_local);
     tile = kTileCfgs[cfg].threads * kTileCfgs[cfg].ipt;
     // Large 8-byte-key sorts receive into a third set of arrays (landing): the local sort then runs
     // landing -> shadow -> caller -> shadow -> caller and an even number of passes ends in the caller's arrays
     // without a copy.  The choice depends on nothing but the arguments all ranks share.
-    landing = kb == 8 && n_ws >= ((int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_host_plan_min_log2.load(), 0), 62)) &&
-              opt_mgpu_landing.load() != 0 && opt_mgpu_p2p.load() != 0;
+    landing = kb == 8 && n_ws >= ((int64_t)1 << o.host_plan_min_log2) && o.mgpu_landing != 0 && o.mgpu_p2p != 0;
     make_layout(streams, n_ws, std::min(tile, HYB_MIN_TILE), &L, landing);
     cache_guard.acquire(c->dev, stream);
     return 0;
@@ -999,7 +1000,7 @@ struct MgpuSort {
     split_blk.assign(std::max(ns, 1), 0u);
     split_tie.assign(std::max(ns, 1), 0u);
     while (((int64_t)MGPU_TIE_BLOCKS << blk_shift) < std::max<int64_t>(capacity, 1)) blk_shift++;  // capacity: the same on all ranks
-    if (!heavy || opt_mgpu_refine.load() == 0) {
+    if (!heavy || o.mgpu_refine == 0) {
       heavy = false;
       for (int r = 0; r < ns; r++) {
         const uint32_t b = bounds[r + 1];
@@ -1104,10 +1105,10 @@ struct MgpuSort {
         const uint32_t x = bounds[r] ^ (bounds[r + 1] - 1);
         lead[r] = x ? __builtin_clz(x) - (32 - bits) : bits;
       }
-    const int64_t chunk_min = (int64_t)1 << std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunk_min_log2.load(), 12), 40);
-    n_chunks = (int)std::min<int64_t>(std::max<int64_t>(opt_mgpu_chunks.load(), 1), MGPU_MAX_CHUNKS);
-    overlap = landing && aligned && world <= 8 && (world >= 2 || opt_mgpu_overlap.load() == 2) && opt_mgpu_overlap.load() != 0 &&
-              opt_mgpu_p2p.load() != 0 && !c->p2p_failed && cfg == kDefaultTileCfg && streams[0].elem_bytes == (uint32_t)kb;
+    const int64_t chunk_min = (int64_t)1 << o.mgpu_chunk_min_log2;
+    n_chunks = (int)o.mgpu_chunks;
+    overlap = landing && aligned && world <= 8 && (world >= 2 || o.mgpu_overlap == 2) && o.mgpu_overlap != 0 &&
+              o.mgpu_p2p != 0 && !c->p2p_failed && cfg == kDefaultTileCfg && streams[0].elem_bytes == (uint32_t)kb;
     if (overlap) {
       // flat enough?  (by the top 8 bits of the sampled histogram inside every shard)
       std::vector<uint64_t> g256(256, 0);
@@ -1118,9 +1119,9 @@ struct MgpuSort {
       for (int r = 0; r < world && overlap; r++) {
         if (bounds[r + 1] <= bounds[r]) { overlap = false; break; }
         const double est_n = (double)sampled_total * (double)sample / (double)world;
-        const int swept = (int)std::ceil((std::log2(std::max(est_n, 2.0)) + (double)opt_margin_bits.load()) / 8.0);
+        const int swept = (int)std::ceil((std::log2(std::max(est_n, 2.0)) + (double)o.margin_bits) / 8.0);
         const int cut = 8 - lead[r] / 8 - swept;
-        if (cut < 2 || opt_allow_lshift.load() == 0) { overlap = false; break; }
+        if (cut < 2 || o.allow_lshift == 0) { overlap = false; break; }
         d_lshift[r] = (uint32_t)(lead[r] & 7);
         d_cut[r] = (uint32_t)cut;
       }
@@ -1138,7 +1139,7 @@ struct MgpuSort {
   // histograms)}, all-gathered; the send and receive offsets from them
   int exchange_blobs() {
     auto mine = std::make_unique<MgpuBlob>();
-    const bool want_p2p = opt_mgpu_p2p.load() != 0 && !c->p2p_failed;
+    const bool want_p2p = o.mgpu_p2p != 0 && !c->p2p_failed;
     if (want_p2p) {
       const uint64_t gen = cache_entry(CACHE_WORKSPACE, c->dev).gen;
       if (c->my_handle_of != ws || c->my_handle_gen != gen) {  // (a slow driver call: once per workspace allocation)
@@ -1277,7 +1278,7 @@ struct MgpuSort {
     wa.bin_base = c->d_bin_base + (size_t)pass * RADIX; wa.lookback = (uint64_t *)(ws + L.lookback_off);
     // (look-back tags 16.. : the local sort's passes, tags 1..8, reuse the same table later)
     wa.tile_counter = (uint32_t *)(ws + L.tilectr_off); wa.plan = c->d_plan; wa.tag = 16u + (uint32_t)pass; wa.stage_bytes = stage_bytes;
-    wa.part = part; wa.lut_world = world; wa.tile_first = (uint32_t)t_first; wa.peer_wide = opt_mgpu_wide.load() != 0 ? 1u : 0u;
+    wa.part = part; wa.lut_world = world; wa.tile_first = (uint32_t)t_first; wa.peer_wide = o.mgpu_wide != 0 ? 1u : 0u;
     wa.peer_delta = p2p ? c->d_peer_delta : nullptr;
     return wa;
   }
@@ -1288,7 +1289,7 @@ struct MgpuSort {
   int plain_exchange() {
     if (num_local > 0) {
       SweepArgs wa = partition_args(0, 0, num_local);
-      CUDA_TRY(launch_sweep(kb, cfg, wa, ct[n_chunks], di.smem_optin, di.sm_count, stream));
+      CUDA_TRY(launch_sweep(o, kb, cfg, wa, ct[n_chunks], di.smem_optin, stream));
     }
     trace.mark(p2p ? "partition+exchange" : "partition");
     DevSortOpts so;
@@ -1304,7 +1305,7 @@ struct MgpuSort {
       so.hint_lead_bits = lead[c->rank];
       so.landing_input = landing;
       if (recv_total > 0)
-        if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
+        if (int rc = sort_device(o, key_type, ascending, recv_total, streams, stream, nullptr, 0, so, stats)) return rc;
     } else {
       // all-to-all-v, shadow -> caller arrays
       NCCL_TRY(api.GroupStart());
@@ -1319,7 +1320,7 @@ struct MgpuSort {
       NCCL_TRY(api.GroupEnd());
       trace.mark("exchange");
       if (recv_total > 1)
-        if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
+        if (int rc = sort_device(o, key_type, ascending, recv_total, streams, stream, nullptr, 0, so, stats)) return rc;
     }
     trace.mark("local_sort");
     return 0;
@@ -1370,7 +1371,7 @@ struct MgpuSort {
         sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
         CUDA_TRY(launch(PK_NONE, mgpu_signal_kernel, 1, 32, 0, stream, sg));
       }
-    const int64_t persist_x2 = opt_mgpu_persist_x2.load();
+    const int64_t persist_x2 = o.mgpu_persist_x2;
     if (persist_x2 <= 0) {
       // variant: one ordinary partition kernel per chunk (one CTA per tile), each followed by a one-warp kernel
       // that writes the chunk's flags (the first-pass kernels of the high-priority side stream then alternate with
@@ -1378,7 +1379,7 @@ struct MgpuSort {
       for (int ch = 0; ch < n_chunks; ch++) {
         if (ct[ch + 1] == ct[ch]) continue;  // (signalled above)
         SweepArgs wa = partition_args(ch, ct[ch], std::min<int64_t>(num_local, ct[ch + 1] * tile));
-        CUDA_TRY(launch_sweep(kb, cfg, wa, ct[ch + 1] - ct[ch], di.smem_optin, di.sm_count, stream));
+        CUDA_TRY(launch_sweep(o, kb, cfg, wa, ct[ch + 1] - ct[ch], di.smem_optin, stream));
         sg.chunk = ch; sg.value = epoch + (uint32_t)ch + 1u;
         CUDA_TRY(launch(PK_NONE, mgpu_signal_kernel, 1, 32, 0, stream, sg));
       }
@@ -1390,7 +1391,7 @@ struct MgpuSort {
       for (int r = 0; r < world; r++) wa.sig_flags[r] = sg.peer_flags[r];
       wa.sig_me = (uint32_t)c->rank; wa.sig_value = epoch + 1u;
       const int64_t cap = std::max<int64_t>(1, (int64_t)di.sm_count * persist_x2 / 2);
-      CUDA_TRY(launch_sweep(kb, cfg, wa, ct[n_chunks], di.smem_optin, di.sm_count, stream, false, 0, cap));
+      CUDA_TRY(launch_sweep(o, kb, cfg, wa, ct[n_chunks], di.smem_optin, stream, false, 0, cap));
     }
     trace.mark("sent_all", stream);
     int64_t tiles_before = 0;
@@ -1418,8 +1419,8 @@ struct MgpuSort {
           wa.plan_in_args = 1; wa.arg_sel = 0; wa.arg_next_p1 = my_cut + 2; wa.arg_next_skewed = 0; wa.arg_sub = 0; wa.arg_lshift = my_lshift;
           // (high-priority stream: without a bound on its CTAs per SM the first pass would take every slot that frees
           //  up and starve the partition kernel -- measured: the two then simply alternate)
-          CUDA_TRY(launch_sweep(kb, cfg, wa, tiles_here, di.smem_optin, di.sm_count, c->side, /*first_pass_unordered=*/true,
-                                (size_t)std::max<int64_t>(opt_mgpu_cons_smem_kb.load(), 0) << 10));
+          CUDA_TRY(launch_sweep(o, kb, cfg, wa, tiles_here, di.smem_optin, c->side, /*first_pass_unordered=*/true,
+                                (size_t)o.mgpu_cons_smem_kb << 10));
         }
         tiles_before += tiles_here;
       }
@@ -1436,18 +1437,18 @@ struct MgpuSort {
       so.forced = true;
       so.forced_cut = my_cut;
       so.forced_lshift = my_lshift;
-      if (int rc = sort_device(key_type, ascending, recv_total, streams, stream, nullptr, 0, so)) return rc;
+      if (int rc = sort_device(o, key_type, ascending, recv_total, streams, stream, nullptr, 0, so, stats)) return rc;
     }
     trace.mark("local_sort_rest");
     return 0;
   }
 };
 
-static int mgpu_sort(b200sort_comm *c, int key_type, const std::vector<StreamDesc> &streams, int64_t num_local, int64_t capacity,
-                     bool ascending, int64_t *out_num_local, cudaStream_t stream) {
+static int mgpu_sort(const Options &o, b200sort_comm *c, int key_type, const std::vector<StreamDesc> &streams, int64_t num_local,
+                     int64_t capacity, bool ascending, int64_t *out_num_local, cudaStream_t stream, b200sort_stats *stats) {
   DeviceScope dev_scope;  // the communicator's device, whatever the caller's current device is
   if (dev_scope.enter(c->dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", c->dev);
-  MgpuSort s{c, nccl_api(), key_type, streams, num_local, capacity, ascending, stream};
+  MgpuSort s{o, c, nccl_api(), key_type, streams, num_local, capacity, ascending, stream, stats};
   c->seq++;
   c->last_overlap = false;
   if (int rc = s.setup()) return rc;
@@ -1483,7 +1484,7 @@ int b200sort_mgpu_sort_soa(b200sort_comm *c, void *keys, int key_type, int64_t n
   if (int rc = mgpu_check(c, num_local, capacity, out_num_local)) return rc;
   if (int rc = check_soa(keys, key_type, num_local, n_payloads, payloads, payload_elem_bytes, &streams)) return rc;
   if (!keys) return fail(B200SORT_EINVAL, "keys is NULL");
-  return mgpu_sort(c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v);
+  return mgpu_sort(options(), c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v, &g_last_stats);
 }
 
 int b200sort_mgpu_sort_aos(b200sort_comm *c, void *records, int key_type, uint32_t record_bytes, int64_t num_local,
@@ -1493,7 +1494,7 @@ int b200sort_mgpu_sort_aos(b200sort_comm *c, void *records, int key_type, uint32
   if (int rc = mgpu_check(c, num_local, capacity, out_num_local)) return rc;
   if (int rc = check_aos(records, key_type, record_bytes, num_local, &streams)) return rc;
   if (!records) return fail(B200SORT_EINVAL, "records is NULL");
-  return mgpu_sort(c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v);
+  return mgpu_sort(options(), c, key_type, streams, num_local, capacity, ascending != 0, out_num_local, (cudaStream_t)stream_v, &g_last_stats);
 }
 
 }  // extern "C"

@@ -51,22 +51,15 @@ def main():
     rng = np.random.default_rng(1)
     run(O.make_keys("Uniform", np.uint64, n, 1), True, "plain u64")
     run(O.make_keys("Gaussian", np.float32, n, 2), False, "plain f32 desc")
-    S.set_option("host_plan_min_log2", 0)
-    run(O.make_keys("Uniform", np.uint64, n, 3), True, "landing u64", 0)
-    S.set_option("mgpu_chunk_min_log2", 12)
-    S.set_option("mgpu_overlap", 2)   # 2: also with a world of one (this vehicle)
-    for chunks, persist in ((4, 0), (1, 3), (3, 4), (8, 2)):
-        S.set_option("mgpu_chunks", chunks)
-        S.set_option("mgpu_persist_x2", persist)
-        run(O.make_keys("Uniform", np.uint64, n, 4 + chunks), True, f"overlap u64 chunks={chunks}", 1)
-        run(O.make_keys("Uniform", np.int64, n, 14 + chunks), False, f"overlap i64 desc chunks={chunks}", 1)
-    S.set_option("mgpu_overlap", 0)
-    S.set_option("mgpu_persist_x2", 0)
-    S.set_option("mgpu_chunk_min_log2", 24)
-    S.set_option("mgpu_chunks", 4)
-    run(np.zeros(n, np.int64), True, "zero")
-    run(rng.integers(-8, 8, size=n, dtype=np.int64), False, "few unique")
-    S.set_option("host_plan_min_log2", 24)
+    with S.options(host_plan_min_log2=0):
+        run(O.make_keys("Uniform", np.uint64, n, 3), True, "landing u64", 0)
+        with S.options(mgpu_chunk_min_log2=12, mgpu_overlap=2):   # 2: also with a world of one (this vehicle)
+            for chunks, persist in ((4, 0), (1, 3), (3, 4), (8, 2)):
+                with S.options(mgpu_chunks=chunks, mgpu_persist_x2=persist):
+                    run(O.make_keys("Uniform", np.uint64, n, 4 + chunks), True, f"overlap u64 chunks={chunks}", 1)
+                    run(O.make_keys("Uniform", np.int64, n, 14 + chunks), False, f"overlap i64 desc chunks={chunks}", 1)
+        run(np.zeros(n, np.int64), True, "zero")
+        run(rng.integers(-8, 8, size=n, dtype=np.int64), False, "few unique")
     assert L.b200sort_mgpu_comm_destroy(comm) == 0
     print("MGPU_SINGLE_OK", flush=True)
 

@@ -2,8 +2,10 @@
 include/b200sort.h declares, validates its arguments like the reference's static_asserts do, and fails
 loudly (no CPU fallback) when no CUDA device is present.  No compute happens here."""
 import ctypes
+import json
 import re
 import subprocess
+import sys
 from pathlib import Path
 
 import numpy as np
@@ -159,3 +161,53 @@ def test_range_bins_make_narrow_key_ranges_splittable():
         assert loads.max() <= ideal * (1 + 1 / 32) + hist.max() + 1, (name, loads)
         if name != "small_u32":
             assert loads.max() <= 1.2 * ideal, (name, loads)  # what the default capacity (1.125x + slack) tolerates
+
+
+def _documented_options() -> dict:
+    """{name: bracketed default} of the option list in INTEGRATION.md section 6"""
+    doc = (ROOT / "INTEGRATION.md").read_text()
+    sec = doc[doc.index("## 6. Options"):].split("\n## ")[0]
+    return {name: int(v) for name, v in re.findall(r"`(\w+)` \[(-?\d+)", sec)}
+
+
+def test_documented_option_defaults_in_a_fresh_process():
+    documented = _documented_options()
+    code = ("import json, simd_radix_sort_b200 as S; "
+            f"print(json.dumps({{n: S.get_option(n) for n in {sorted(documented)!r}}}))")
+    out = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, check=True).stdout
+    assert json.loads(out) == documented
+
+
+def test_option_table_matches_the_documented_names():
+    src = (ROOT / "simd-radix-sort_b200" / "csrc" / "b200sort.cu").read_text()
+    table = re.findall(r'\{"(\w+)", &Options::(\w+)\}', src)
+    assert all(name == member for name, member in table), table
+    names = [name for name, _ in table]
+    assert len(names) == len(set(names))
+    assert set(names) == set(_documented_options())
+
+
+def test_max_chunk_takes_powers_of_two_up_to_16():
+    L = S.lib()
+    before = S.get_option("max_chunk")
+    for v in (0, 3, 12, 32):
+        assert L.b200sort_set_option(b"max_chunk", v) == -1, v
+        assert S.get_option("max_chunk") == before
+    for v in (1, 2, 4, 8, 16):
+        with S.options(max_chunk=v):
+            assert S.get_option("max_chunk") == v
+    assert S.get_option("max_chunk") == before
+
+
+def test_options_restores_the_earlier_values_when_the_body_raises():
+    before = {"algo": S.get_option("algo"), "margin_bits": S.get_option("margin_bits")}
+    with pytest.raises(ZeroDivisionError):
+        with S.options(algo=2, margin_bits=-3):
+            assert S.get_option("algo") == 2 and S.get_option("margin_bits") == -3
+            1 / 0
+    assert {n: S.get_option(n) for n in before} == before
+    # a name the library does not know raises, and what was already set is restored
+    with pytest.raises(S.B200SortError):
+        with S.options(algo=1, no_such_option=1):
+            pass
+    assert S.get_option("algo") == before["algo"]

@@ -224,34 +224,53 @@ def test_tile_geometries_agree():
     n = 300_000
     keys = O.make_keys("Uniform", np.uint64, n, seed=77)
     want = np.sort(keys)
-    try:
-        for cfg in range(2):
-            S.set_option("tile_cfg", cfg)
+    for cfg in range(2):
+        with S.options(tile_cfg=cfg):
             k, (p,) = gpu_sort_soa(keys, [np.arange(n, dtype=np.uint32)], True)
             assert k.tobytes() == want.tobytes(), cfg
             assert keys[p].tobytes() == k.tobytes(), cfg
-    finally:
-        S.set_option("tile_cfg", -1)
 
 
 def test_wide_tiles_for_4_byte_keys():
     """8192-key tiles (tile geometry 2): chosen automatically for 4-byte keys with <= 4-byte chunks from 2^24 records
     (test_gpu_large covers that size), forced here at sizes with full, partial and single tiles"""
-    try:
-        S.set_option("tile_cfg", 2)
+    with S.options(tile_cfg=2):
         for n in (5, 8191, 8193, 300_000, (1 << 22) + 4099):
             for dt, up in ((np.uint32, True), (np.float32, False), (np.int32, False)):
                 keys = O.make_keys("Uniform" if n % 2 else "Gaussian", dt, n, seed=n % 97)
                 a, b = np.arange(n, dtype=np.uint32), (np.arange(n) % 251).astype(np.uint8)
                 for big in (24, 0):
-                    S.set_option("host_plan_min_log2", big)
-                    k, (pa, pb) = gpu_sort_soa(keys, [a, b], up)
-                    assert k.tobytes() == O.total_order_sorted_keys(keys, up).tobytes(), (n, dt, up, big)
-                    assert keys[pa].tobytes() == k.tobytes() and np.array_equal(np.sort(pa), a), (n, dt, up, big)
-                    assert np.array_equal(pb, (pa % 251).astype(np.uint8)), (n, dt, up, big)
-    finally:
-        S.set_option("tile_cfg", -1)
-        S.set_option("host_plan_min_log2", 24)
+                    with S.options(host_plan_min_log2=big):
+                        k, (pa, pb) = gpu_sort_soa(keys, [a, b], up)
+                        assert k.tobytes() == O.total_order_sorted_keys(keys, up).tobytes(), (n, dt, up, big)
+                        assert keys[pa].tobytes() == k.tobytes() and np.array_equal(np.sort(pa), a), (n, dt, up, big)
+                        assert np.array_equal(pb, (pa % 251).astype(np.uint8)), (n, dt, up, big)
+
+
+@pytest.mark.parametrize("max_chunk", [1, 2, 4, 8])
+def test_max_chunk_below_the_key_width(max_chunk):
+    """option max_chunk narrower than the key: payloads move in chunks that narrow, keys and whole records never in
+    chunks narrower than the key (large-sort flow, whose lean kernels read the key from the record's first chunk)"""
+    n = (1 << 20) + 77
+    rng = np.random.default_rng(max_chunk)
+    with S.options(host_plan_min_log2=0, max_chunk=max_chunk):
+        keys = rng.integers(0, 2**64, size=n, dtype=np.uint64)
+        keys[::13] = keys[7]  # duplicates of one value
+        idx = np.arange(n, dtype=np.uint64)
+        k, (p,) = gpu_sort_soa(keys, [idx], True)
+        assert k.tobytes() == O.total_order_sorted_keys(keys, True).tobytes()
+        assert np.array_equal(np.sort(p), idx) and keys[p.astype(np.int64)].tobytes() == k.tobytes()
+        rk = rng.integers(-2**63, 2**63 - 1, size=n, dtype=np.int64)
+        rec = np.zeros((n, 16), np.uint8)
+        rec[:, :8] = rk.view(np.uint8).reshape(n, 8)
+        rec[:, 8:] = np.arange(n, dtype=np.int64).view(np.uint8).reshape(n, 8)
+        r = dev(rec)
+        S.sort_combined(n, r, np.int64, up=True)
+        out = host(r)
+        ok = np.ascontiguousarray(out[:, :8]).reshape(-1).view(np.int64)
+        op = np.ascontiguousarray(out[:, 8:]).reshape(-1).view(np.int64)
+        assert ok.tobytes() == O.total_order_sorted_keys(rk, True).tobytes()
+        assert np.array_equal(np.sort(op), np.arange(n)) and np.array_equal(rk[op], ok)
 
 
 @pytest.mark.parametrize("first_atomic", [0, 1])
@@ -260,10 +279,7 @@ def test_unstable_first_pass_ranking(first_atomic):
     every later pass stays stable -- same result either way, payloads follow their keys"""
     n = (1 << 20) + 4099
     rng = np.random.default_rng(5 + first_atomic)
-    try:
-        S.set_option("host_plan_min_log2", 0)
-        S.set_option("first_atomic", first_atomic)
-        S.set_option("algo", 2)
+    with S.options(host_plan_min_log2=0, first_atomic=first_atomic, algo=2):
         for dt in (np.uint64, np.int64, np.float64):
             keys = O.make_keys("Uniform", dt, n, seed=21)
             keys[::11] = keys[5]  # duplicates of one value
@@ -272,10 +288,6 @@ def test_unstable_first_pass_ranking(first_atomic):
                 k, (p,) = gpu_sort_soa(keys, [idx], up)
                 assert k.tobytes() == O.total_order_sorted_keys(keys, up).tobytes(), (dt, up)
                 assert np.array_equal(np.sort(p), idx) and keys[p.astype(np.int64)].tobytes() == k.tobytes(), (dt, up)
-    finally:
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("first_atomic", 1)
-        S.set_option("algo", 0)
 
 
 @pytest.mark.parametrize("up", [True, False])
@@ -285,10 +297,7 @@ def test_last_pass_window_at_tile_edges_with_32_bit_cut(up):
     ordering looks one slot outside the tile.  Slots outside the tile must never pair with a key."""
     n = (1 << 20) + 4099
     rng = np.random.default_rng(32)
-    try:
-        S.set_option("algo", 2)
-        S.set_option("host_plan_min_log2", 0)
-        S.set_option("margin_bits", 11)   # log2(n) + 11 = 31.01 -> four swept digits, cut at bit 32
+    with S.options(algo=2, host_plan_min_log2=0, margin_bits=11):  # log2(n) + 11 = 31.01 -> four swept digits, cut at bit 32
         hi = rng.integers(0, 2**32, size=n, dtype=np.uint64)
         # plenty of keys with raw high word 1 (and 0, 2: neighbours), in runs so that they also meet in one tile
         hi[rng.integers(0, n, size=n // 8)] = 1
@@ -311,10 +320,6 @@ def test_last_pass_window_at_tile_edges_with_32_bit_cut(up):
         assert S.last_stats()["cut_digit"] == 4, S.last_stats()
         assert k.tobytes() == O.total_order_sorted_keys(keys2, up).tobytes()
         assert kk is not None and keys2[p].tobytes() == k.tobytes()
-    finally:
-        S.set_option("algo", 0)
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("margin_bits", 2)
 
 
 def test_caller_workspace_and_stats():
@@ -361,8 +366,7 @@ def _hybrid_cases(n, rng):
 @pytest.mark.parametrize("n", [1, 17, 2049, 300_000, (1 << 20) + 77])
 def test_hybrid_msb_path_matches_total_order(n):
     rng = np.random.default_rng(n)
-    try:
-        S.set_option("algo", 2)
+    with S.options(algo=2):
         for name, keys, dt in _hybrid_cases(n, rng):
             keys = np.ascontiguousarray(keys.astype(dt))
             for up in (True, False):
@@ -376,15 +380,12 @@ def test_hybrid_msb_path_matches_total_order(n):
             if name == "uniform_u64" and n >= 300_000:
                 st = S.last_stats()
                 assert st["algo"] == 2 and st["fell_back"] == 0 and st["cut_digit"] >= 2 and st["segfix_passes"] == 1
-    finally:
-        S.set_option("algo", 0)
 
 
 def test_hybrid_aos_and_multi_stream():
     n = 500_000
     rng = np.random.default_rng(5)
-    try:
-        S.set_option("algo", 2)
+    with S.options(algo=2):
         keys = rng.integers(-2**63, 2**63 - 1, size=n, dtype=np.int64)
         keys[::7] = keys[3]  # duplicates
         rec = np.zeros((n, 32), np.uint8)
@@ -403,8 +404,6 @@ def test_hybrid_aos_and_multi_stream():
         k, (pa, pb_, pc) = gpu_sort_soa(fk, [a, b, c], True)
         assert k.tobytes() == np.sort(fk).tobytes() and fk[pa].tobytes() == k.tobytes()
         assert np.array_equal(pb_, pa.astype(np.float64)) and np.array_equal(pc, (pa % 65536).astype(np.uint16))
-    finally:
-        S.set_option("algo", 0)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -414,10 +413,7 @@ def test_hybrid_aos_and_multi_stream():
 @pytest.mark.parametrize("n,margin", [(300_000, 2), ((1 << 20) + 77, 2), ((1 << 20) + 77, -2), ((1 << 20) + 77, -5)])
 def test_hybrid_host_plan_tile_local_ordering_and_junctions(n, margin):
     rng = np.random.default_rng(n + margin)
-    try:
-        S.set_option("algo", 2)
-        S.set_option("host_plan_min_log2", 0)
-        S.set_option("margin_bits", margin)
+    with S.options(algo=2, host_plan_min_log2=0, margin_bits=margin):
         for name, keys, dt in _hybrid_cases(n, rng):
             keys = np.ascontiguousarray(keys.astype(dt))
             for up in (True, False):
@@ -429,19 +425,12 @@ def test_hybrid_host_plan_tile_local_ordering_and_junctions(n, margin):
             if name == "uniform_u64" and margin == 2:
                 st = S.last_stats()  # no full segment finish: the last pass and the junction kernel did it
                 assert st["algo"] == 2 and st["fell_back"] == 0 and st["cut_digit"] >= 2 and st["segfix_passes"] == 0
-    finally:
-        S.set_option("algo", 0)
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("margin_bits", 2)
 
 
 def test_hybrid_host_plan_aos_and_multi_stream():
     n = (1 << 19) + 4099
     rng = np.random.default_rng(77)
-    try:
-        S.set_option("algo", 2)
-        S.set_option("host_plan_min_log2", 0)
-        S.set_option("margin_bits", -2)  # about four keys per final segment: plenty of runs and junctions
+    with S.options(algo=2, host_plan_min_log2=0, margin_bits=-2):  # about four keys per final segment: plenty of runs and junctions
         for rec_bytes in (16, 32, 64):
             keys = rng.integers(-2**63, 2**63 - 1, size=n, dtype=np.int64)
             keys[::5] = keys[1::5][: len(keys[::5])]  # duplicates
@@ -465,10 +454,6 @@ def test_hybrid_host_plan_aos_and_multi_stream():
             k, (pa, pb_, pc) = gpu_sort_soa(fk, [a, b, c], up)
             assert k.tobytes() == O.total_order_sorted_keys(fk, up).tobytes() and fk[pa].tobytes() == k.tobytes()
             assert np.array_equal(pb_, pa.astype(np.float64)) and np.array_equal(pc, (pa % 65536).astype(np.uint16))
-    finally:
-        S.set_option("algo", 0)
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("margin_bits", 2)
 
 
 @pytest.mark.parametrize("host_plan", [0, 24])
@@ -479,28 +464,20 @@ def test_hybrid_left_shift_plan_for_common_leading_bits(host_plan):
     rng = np.random.default_rng(9)
     body = rng.integers(0, 2**58, size=n, dtype=np.uint64)
     passes = {}
-    try:
-        S.set_option("algo", 2)
-        S.set_option("host_plan_min_log2", host_plan)
-        S.set_option("margin_bits", -1)
+    with S.options(algo=2, host_plan_min_log2=host_plan, margin_bits=-1):
         for name, keys in (("u64_top6", body | np.uint64(0b101011 << 58)),
                            ("i64_neg", (body | np.uint64(0b111111 << 58)).view(np.int64)),
                            ("f64", (body >> np.uint64(2) | np.uint64(0x3FF << 52)).view(np.float64))):
             keys = np.ascontiguousarray(keys)
             for allow in (1, 0):
-                S.set_option("allow_lshift", allow)
-                for up in (True, False):
-                    idx = np.arange(n, dtype=np.uint32)
-                    k, (p,) = gpu_sort_soa(keys, [idx], up)
-                    assert k.tobytes() == O.total_order_sorted_keys(keys, up).tobytes(), (name, allow, up)
-                    assert np.array_equal(np.sort(p), idx) and keys[p].tobytes() == k.tobytes(), (name, allow, up)
-                passes[(name, allow)] = S.last_stats()["passes_planned"]
+                with S.options(allow_lshift=allow):
+                    for up in (True, False):
+                        idx = np.arange(n, dtype=np.uint32)
+                        k, (p,) = gpu_sort_soa(keys, [idx], up)
+                        assert k.tobytes() == O.total_order_sorted_keys(keys, up).tobytes(), (name, allow, up)
+                        assert np.array_equal(np.sort(p), idx) and keys[p].tobytes() == k.tobytes(), (name, allow, up)
+                    passes[(name, allow)] = S.last_stats()["passes_planned"]
         assert passes[("u64_top6", 1)] < passes[("u64_top6", 0)], passes
-    finally:
-        S.set_option("algo", 0)
-        S.set_option("allow_lshift", 1)
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("margin_bits", 2)
 
 
 @pytest.mark.parametrize("pinned", [False, True])
@@ -553,10 +530,9 @@ def test_cmp_sorter_none_partial_sort_contract(thresh):
     n = (1 << 20) + 333
     rng = np.random.default_rng(thresh)
     CMP_NONE = 1
-    try:
-        S.set_option("algo", 2)           # (the MSB hybrid path is the default from 2^22 records)
-        S.set_option("host_plan_min_log2", 0)
-        S.set_option("margin_bits", -2)   # about four keys per final segment: plenty of unordered small buckets
+    with S.options(algo=2,            # (the MSB hybrid path is the default from 2^22 records)
+                   host_plan_min_log2=0,
+                   margin_bits=-2):   # about four keys per final segment: plenty of unordered small buckets
         for dt, up in ((np.uint64, True), (np.int64, False), (np.float64, True)):
             keys = O.make_keys("Uniform", dt, n, seed=9 + thresh)
             idx = np.arange(n, dtype=np.uint32)
@@ -598,7 +574,3 @@ def test_cmp_sorter_none_partial_sort_contract(thresh):
         ok = np.ascontiguousarray(out[:, :8]).reshape(-1).view(np.int64)
         assert _within_thresh_of_sorted(O.order_key(ok, True), O.order_key(np.sort(ok), True), 32)
         assert out.tobytes() == O.make_records(ok, 16).tobytes()   # records stayed whole
-    finally:
-        S.set_option("algo", 0)
-        S.set_option("host_plan_min_log2", 24)
-        S.set_option("margin_bits", 2)
