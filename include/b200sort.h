@@ -18,7 +18,8 @@
  *    result overwrites keys/payloads/records.  Scratch (one shadow copy of every stream + per-tile
  *    status words) comes from `workspace` or, when that is NULL, from a per-device cache owned by
  *    the library.  Sorts that use that cache (and all host-memory calls, which stage through a cached
- *    buffer) are serialised per device by the library; give concurrent sorts their own workspaces.
+ *    buffer) are serialised per device by the library; give concurrent sorts of device arrays their own
+ *    workspaces.  Both cached buffers are kept until b200sort_release_cache().
  *  - return value: 0 on success, a negative B200SORT_E* code otherwise; b200sort_last_error() gives
  *    a thread-local human-readable message.  There is NO CPU fallback: without a usable CUDA device
  *    every sort call fails with B200SORT_ECUDA.
@@ -142,7 +143,8 @@ int b200sort_last_stats(b200sort_stats *out);
  * 4 segment finish, 5 other.  Returns the number of entries written (<= capacity) or a negative code. */
 int b200sort_last_profile(int *kinds, float *ms, int capacity);
 
-/* Releases the per-device workspace caches held by the library. */
+/* Releases the per-device workspace and host-staging buffers held by the library.  A sort another thread
+ * is launching on them is queued first; the call then waits for each device to be idle. */
 void b200sort_release_cache(void);
 
 /* ---- multi-GPU: one process per GPU, NCCL over NVLink (SURVEY.md 8e) -------------------------

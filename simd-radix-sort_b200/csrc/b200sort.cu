@@ -94,19 +94,27 @@ static Options options() {
   return o;
 }
 
+// What one host thread keeps for one device, created on first use: events and streams belong to the device they
+// were created on, and two host threads sorting on one device (with their own workspaces) must not share them.
+struct ThreadDeviceState {
+  cudaEvent_t plan_event = nullptr;          // the plan read-back of large sorts
+  std::vector<cudaEvent_t> prof_pool;        // free events of option "profile"
+  cudaStream_t in = nullptr, comp = nullptr, out = nullptr;  // the pipelined host path: upload, sort, download
+};
+static thread_local std::map<int, ThreadDeviceState> t_dev;
+
 // optional per-kernel timing (option "profile"): CUDA events around every launch of the last sort
 enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5 };
 struct ProfEntry { int kind; cudaEvent_t e0, e1; int dev; };
 static thread_local bool g_prof_on = false;  // the sort running on this thread has option "profile" set
 static thread_local std::vector<ProfEntry> g_prof;
-static thread_local std::map<int, std::vector<cudaEvent_t>> g_prof_pool;  // per device: events belong to one
 
 static void prof_reset() {
-  for (auto &p : g_prof) { g_prof_pool[p.dev].push_back(p.e0); g_prof_pool[p.dev].push_back(p.e1); }
+  for (auto &p : g_prof) { t_dev[p.dev].prof_pool.push_back(p.e0); t_dev[p.dev].prof_pool.push_back(p.e1); }
   g_prof.clear();
 }
 static cudaEvent_t prof_event(int dev) {
-  auto &pool = g_prof_pool[dev];
+  auto &pool = t_dev[dev].prof_pool;
   if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
   cudaEvent_t e; cudaEventCreate(&e); return e;
 }
@@ -312,45 +320,52 @@ static cudaError_t launch_hist(const Options &o, int kb, const HistArgs &a, int 
 }
 
 // ------------------------------------------------------------------------------------------------
-// device properties + per-device workspace cache
+// per-device state: device properties, the library-owned caches and their guard
 // ------------------------------------------------------------------------------------------------
 struct DevInfo { int sm_count = 0; size_t smem_optin = 0; bool ok = false; };
-static std::mutex g_mu;
-static std::map<int, DevInfo> g_dev;
 struct CacheEntry { void *ptr = nullptr; size_t bytes = 0; uint64_t gen = 0; };  // gen: bumped by every (re)allocation
-enum CacheKind { CACHE_WORKSPACE = 0, CACHE_STAGE = 1 };  // the sort's workspace, the staging of host arrays
-static std::map<int, CacheEntry> g_cache[2];              // [kind][device]
 
-// The library-owned caches (workspace, host staging) are one allocation per device.  Sorts that use them are
-// serialised: a per-device (recursive) mutex covers the launching of a sort, and the stream of the next sort
-// waits for an event recorded at the end of the previous one, so that two host threads, or two streams, never
-// have kernels in flight on the same scratch memory.  Callers who want concurrent sorts pass their own workspace.
-struct CacheGuardState { std::recursive_mutex mu; cudaEvent_t last_use = nullptr; };
-static CacheGuardState &cache_guard_state(int dev) {
-  static std::map<int, CacheGuardState> g_guard;
+// What the library keeps for one device, process-wide.  The caches (the sort's workspace, the staging of host
+// arrays) are one allocation each, and the sorts that use them are serialised, so that two host threads, or two
+// streams, never have kernels in flight on the same scratch memory.  Callers who want concurrent sorts of device
+// arrays pass their own workspace.  Rule: a device's cache entries are read and written only while its guard
+// (`mu`, taken by CacheGuard) is held.
+struct DeviceState {
+  DevInfo info;                    // filled once, on first use (under g_mu)
+  std::recursive_mutex mu;         // held from acquiring a cache until the sort's work is queued
+  cudaEvent_t last_use = nullptr;  // recorded when the guard is released; the next user's stream waits for it
+  CacheEntry workspace, stage;
+};
+static std::mutex g_mu;                    // guards the map and every record's `info`; never held while waiting for `mu`
+static std::map<int, DeviceState> g_devs;  // (std::map nodes are stable: a reference to a record stays valid)
+
+static DeviceState &device_state(int dev) {
   std::lock_guard<std::mutex> lk(g_mu);
-  return g_guard[dev];  // (std::map nodes are stable)
+  return g_devs[dev];
 }
+
+// holds a device's DeviceState::mu from acquire() until it is destroyed, which records `last_use` on the stream
 struct CacheGuard {
-  CacheGuardState *st = nullptr;
+  DeviceState *state = nullptr;
   cudaStream_t stream = nullptr;
-  void acquire(int dev, cudaStream_t s) {
-    st = &cache_guard_state(dev);
+  DeviceState &acquire(int dev, cudaStream_t s) {
+    state = &device_state(dev);
     stream = s;
-    st->mu.lock();
-    if (st->last_use == nullptr) cudaEventCreateWithFlags(&st->last_use, cudaEventDisableTiming);
-    else cudaStreamWaitEvent(stream, st->last_use, 0);
+    state->mu.lock();
+    if (state->last_use == nullptr) cudaEventCreateWithFlags(&state->last_use, cudaEventDisableTiming);
+    else cudaStreamWaitEvent(stream, state->last_use, 0);
+    return *state;
   }
   ~CacheGuard() {
-    if (!st) return;
-    cudaEventRecord(st->last_use, stream);
-    st->mu.unlock();
+    if (!state) return;
+    cudaEventRecord(state->last_use, stream);
+    state->mu.unlock();
   }
 };
 
 static int dev_info(int dev, DevInfo *out) {
   std::lock_guard<std::mutex> lk(g_mu);
-  DevInfo &d = g_dev[dev];
+  DevInfo &d = g_devs[dev].info;
   if (!d.ok) {
     int v = 0;
     CUDA_TRY(cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev));
@@ -363,10 +378,8 @@ static int dev_info(int dev, DevInfo *out) {
   return 0;
 }
 
-// the cached buffer of this kind on the current device `dev`, grown to at least `bytes`
-static int cached_buffer(CacheKind kind, int dev, size_t bytes, void **out) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  CacheEntry &c = g_cache[kind][dev];
+// the buffer of cache entry `c` of the current device (its guard held), grown to at least `bytes`; `what` names it
+static int cached_buffer(CacheEntry &c, size_t bytes, const char *what, void **out) {
   if (c.bytes < bytes) {
     if (c.ptr) {
       CUDA_TRY(cudaDeviceSynchronize());
@@ -378,8 +391,7 @@ static int cached_buffer(CacheKind kind, int dev, size_t bytes, void **out) {
     cudaError_t e = cudaMalloc(&p, bytes);
     if (e != cudaSuccess) {
       cudaGetLastError();
-      return fail(B200SORT_ENOMEM, "cudaMalloc of %zu %s bytes failed: %s", bytes, kind == CACHE_STAGE ? "staging" : "workspace",
-                  cudaGetErrorString(e));
+      return fail(B200SORT_ENOMEM, "cudaMalloc of %zu %s bytes failed: %s", bytes, what, cudaGetErrorString(e));
     }
     c.ptr = p;
     c.bytes = bytes;
@@ -387,11 +399,6 @@ static int cached_buffer(CacheKind kind, int dev, size_t bytes, void **out) {
   }
   *out = c.ptr;
   return 0;
-}
-
-static CacheEntry cache_entry(CacheKind kind, int dev) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return g_cache[kind][dev];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -487,15 +494,6 @@ struct DevSortOpts {
 };
 constexpr int64_t CMP_NONE_MIN_THRESH = 8;  // below it nearly every sort would need the finish anyway: full sort
 
-// one event per (host thread, device) for the plan read-back of large sorts: an event belongs to the device it was
-// created on, and two host threads sorting on one device (with their own workspaces) must not share one
-static cudaEvent_t plan_event_of(int dev) {
-  static thread_local std::map<int, cudaEvent_t> t_plan_events;
-  cudaEvent_t &e = t_plan_events[dev];
-  if (e == nullptr && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) e = nullptr;
-  return e;
-}
-
 // The plan of the overlapped multi-GPU exchange's local sort: the hybrid sweep of digit positions cut .. kb-1 of
 // the key shifted left by lshift, in LSD order, without range reduction; the first of them is run by the caller.
 static Plan forced_plan(int kb, uint32_t cut, uint32_t lshift) {
@@ -575,8 +573,7 @@ struct DevSort {
     make_layout(streams, std::max(n, xo.layout_n), std::min(tile, HYB_MIN_TILE), &L, xo.layout_landing);
     void *workspace = caller_workspace;
     if (workspace == nullptr) {
-      cache_guard.acquire(dev, stream);
-      if (int rc = cached_buffer(CACHE_WORKSPACE, dev, L.total, &workspace)) return rc;
+      if (int rc = cached_buffer(cache_guard.acquire(dev, stream).workspace, L.total, "workspace", &workspace)) return rc;
     } else if (workspace_bytes < L.total) {
       return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", workspace_bytes, L.total);
     } else if (((uintptr_t)workspace % 256) != 0) {
@@ -679,8 +676,11 @@ struct DevSort {
     HistArgs hb = ha;  // exact histogram of the first executed pass only; every pass counts its successor's digit
     hb.ghist = ghist_exact; hb.plan = plan; hb.probe = nullptr;
     if (big) {
-      const cudaEvent_t ev = plan_event_of(dev);
-      if (ev == nullptr) return fail(B200SORT_ECUDA, "cudaEventCreate failed on device %d", dev);
+      cudaEvent_t &ev = t_dev[dev].plan_event;
+      if (ev == nullptr && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+        ev = nullptr;
+        return fail(B200SORT_ECUDA, "cudaEventCreate failed on device %d", dev);
+      }
       if (int rc = read_plan(ev)) return rc;
       if (hplan.want_minmax) {
         CUDA_TRY(launch_hist(o, kb, ha, di.sm_count, /*minmax=*/2, stream));
@@ -910,21 +910,19 @@ static bool host_is_pinned(const void *p) {
   return at.type == cudaMemoryTypeHost;
 }
 
-static int sort_host_pipelined(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
-                               cudaStream_t caller, b200sort_stats *stats) {
+// `stage`: the staging cache entry of the current device `dev`, whose guard the caller holds
+static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int key_type, bool ascending, int64_t n,
+                               const std::vector<StreamDesc> &streams, cudaStream_t caller, b200sort_stats *stats) {
   const int kb = key_bytes_of(key_type);
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
   DevInfo di;
   if (int rc = dev_info(dev, &di)) return rc;
-  static thread_local cudaStream_t st_in = nullptr, st_comp = nullptr, st_out = nullptr;
-  static thread_local int st_dev = -1;
-  if (st_in == nullptr || st_dev != dev) {
-    CUDA_TRY(cudaStreamCreateWithFlags(&st_in, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamCreateWithFlags(&st_comp, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamCreateWithFlags(&st_out, cudaStreamNonBlocking));
-    st_dev = dev;
+  ThreadDeviceState &t = t_dev[dev];
+  if (t.in == nullptr) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&t.in, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&t.comp, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&t.out, cudaStreamNonBlocking));
   }
+  const cudaStream_t st_in = t.in, st_comp = t.comp, st_out = t.out;
   const size_t np = streams.size() - 1;
   // device staging: keys | index | payload s in | payload s out
   std::vector<size_t> off_in(np), off_out(np);
@@ -935,10 +933,8 @@ static int sort_host_pipelined(const Options &o, int key_type, bool ascending, i
     off_in[s] = total;  total = align_up(total + (size_t)n * streams[s + 1].elem_bytes, 256);
     off_out[s] = total; total = align_up(total + (size_t)n * streams[s + 1].elem_bytes, 256);
   }
-  CacheGuard cache_guard;  // the staging buffer is shared per device as well; this call is synchronous anyway
-  cache_guard.acquire(dev, caller);
   void *dbuf_v = nullptr;
-  if (int rc = cached_buffer(CACHE_STAGE, dev, total, &dbuf_v)) return rc;
+  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
   unsigned char *dbuf = (unsigned char *)dbuf_v;
 
   std::vector<cudaEvent_t> ev;
@@ -1045,21 +1041,23 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
     return sort_device(o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, base, stats);
   }
 
-  // ---- host arrays, SoA with payloads, big enough to care: pipelined staging --------------------------
+  // ---- host arrays: staged on the current device, through its cached staging buffer ----------------
+  int dev = 0;
+  CUDA_TRY(cudaGetDevice(&dev));
+  CacheGuard cache_guard;  // the staging buffer is the library's, like the workspace; this call is synchronous anyway
+  CacheEntry &stage = cache_guard.acquire(dev, stream).stage;
+  // SoA with payloads, big enough to care: pipelined staging
   if (o.host_pipeline != 0 && base.cmp_none_thresh == 0 && workspace == nullptr && streams.size() >= 2 &&
       streams[0].elem_bytes == (uint32_t)key_bytes_of(key_type) && n >= ((int64_t)1 << 20) && n < ((int64_t)1 << 32)) {
     size_t need = 0;
     for (size_t s = 0; s < streams.size(); s++) need += (size_t)n * streams[s].elem_bytes * (s ? 2 : 1);
     need += (size_t)n * 4 + 2 * ((size_t)n * (key_bytes_of(key_type) + 4));  // index + the sort's own workspace
     size_t free_b = 0, total_b = 0;
-    int cur_dev = 0;
-    cudaGetDevice(&cur_dev);
-    const size_t staged = cache_entry(CACHE_STAGE, cur_dev).bytes;
-    if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need < free_b / 10 * 9 + staged)
-      return sort_host_pipelined(o, key_type, ascending, n, streams, stream, stats);
+    if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need < free_b / 10 * 9 + stage.bytes)
+      return sort_host_pipelined(o, dev, stage, key_type, ascending, n, streams, stream, stats);
     cudaGetLastError();
   }
-  // ---- host arrays: stage through device memory ---------------------------------------------------
+  // everything else: the whole arrays up, the sort, the whole arrays down
   std::vector<StreamDesc> dstreams(streams.size());
   size_t total = 0;
   std::vector<size_t> offs(streams.size());
@@ -1067,12 +1065,9 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
     offs[s] = total;
     total = align_up(total + (size_t)n * streams[s].elem_bytes, 256);
   }
-  unsigned char *dbuf = nullptr;
-  e = cudaMalloc((void **)&dbuf, total);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail(B200SORT_ENOMEM, "cudaMalloc of %zu staging bytes failed: %s", total, cudaGetErrorString(e));
-  }
+  void *dbuf_v = nullptr;
+  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
+  unsigned char *dbuf = (unsigned char *)dbuf_v;
   int rc = B200SORT_OK;
   for (size_t s = 0; s < streams.size() && rc == 0; s++) {
     dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
@@ -1086,7 +1081,6 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
   }
   e = cudaStreamSynchronize(stream);
   if (e != cudaSuccess && rc == 0) rc = fail(B200SORT_ECUDA, "sort failed on the device: %s", cudaGetErrorString(e));
-  cudaFree(dbuf);
   return rc;
 }
 
@@ -1224,16 +1218,21 @@ int b200sort_last_profile(int *kinds, float *ms, int capacity) {
 }
 
 void b200sort_release_cache(void) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  for (auto &cache : g_cache)
-    for (auto &kv : cache) {
-      CacheEntry &c = kv.second;
-      if (!c.ptr) continue;
+  std::vector<std::pair<int, DeviceState *>> devs;
+  {
+    std::lock_guard<std::mutex> lk(g_mu);
+    for (auto &kv : g_devs) devs.push_back({kv.first, &kv.second});
+  }
+  for (auto [dev, ds] : devs) {
+    std::lock_guard<std::recursive_mutex> guard(ds->mu);  // (a sort being launched on the caches finishes that first)
+    for (CacheEntry *c : {&ds->workspace, &ds->stage}) {
+      if (!c->ptr) continue;
       DeviceScope scope;  // (each buffer is freed on its own device)
-      if (scope.enter(kv.first) == 0) { cudaDeviceSynchronize(); cudaFree(c.ptr); }
-      c.ptr = nullptr;
-      c.bytes = 0;  // (gen survives: a later allocation is a new one for the multi-GPU handle check)
+      if (scope.enter(dev) == 0) { cudaDeviceSynchronize(); cudaFree(c->ptr); }
+      c->ptr = nullptr;
+      c->bytes = 0;  // (gen survives: a later allocation is a new one for the multi-GPU handle check)
     }
+  }
 }
 
 }  // extern "C"

@@ -741,9 +741,13 @@ int b200sort_mgpu_comm_create(b200sort_comm **out, int world_size, int rank, con
     return fail(B200SORT_EINVAL, "bad communicator arguments");
   ncclUniqueId id;
   memcpy(&id, id_bytes, sizeof id);
-  b200sort_comm *c = new b200sort_comm();
+  // (a failing step returns; the communicator is then destroyed with whatever the steps before it created)
+  std::unique_ptr<b200sort_comm, decltype(&b200sort_mgpu_comm_destroy)> c(new b200sort_comm(), b200sort_mgpu_comm_destroy);
   c->world = world_size;
   c->rank = rank;
+  c->peer_handle.resize(world_size);
+  c->peer_base.assign(world_size, nullptr);
+  for (auto &h : c->peer_handle) memset(&h, 0, sizeof h);
   CUDA_TRY(cudaGetDevice(&c->dev));
   NCCL_TRY(api.CommInitRank(&c->comm, world_size, id, rank));
   CUDA_TRY(cudaMalloc(&c->d_hist, (sizeof(unsigned long long) * MGPU_MAX_REFINE) << MGPU_MAX_BITS));
@@ -763,10 +767,7 @@ int b200sort_mgpu_comm_create(b200sort_comm **out, int world_size, int rank, con
   CUDA_TRY(cudaStreamCreateWithPriority(&c->side, cudaStreamNonBlocking, hi_prio));
   CUDA_TRY(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
   CUDA_TRY(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
-  c->peer_handle.resize(world_size);
-  c->peer_base.assign(world_size, nullptr);
-  for (auto &h : c->peer_handle) memset(&h, 0, sizeof h);
-  *out = c;
+  *out = c.release();
   return 0;
 }
 
@@ -953,7 +954,7 @@ struct MgpuSort {
     // A rank whose cached workspace is too small is going to free and re-allocate it.  Its peers may still have
     // the old allocation mapped (cudaIpcOpenMemHandle): they have to let go of it first.  The flag travels with
     // the first all-reduce.
-    const bool will_realloc = cache_entry(CACHE_WORKSPACE, c->dev).bytes < L.total;
+    const bool will_realloc = cache_guard.state->workspace.bytes < L.total;
     unsigned long long range_h[3] = {~0ull, ~0ull, will_realloc ? 0ull : 1ull};
     CUDA_TRY(cudaMemcpyAsync(c->d_counts, range_h, sizeof range_h, cudaMemcpyHostToDevice, stream));
     TopHistArgs ha{keys, kstride, num_local, ko, 0, c->d_hist, sample, 0ull, nb, c->d_counts};
@@ -972,7 +973,7 @@ struct MgpuSort {
       CUDA_TRY(cudaStreamSynchronize(stream));
     }
     void *ws_v = nullptr;
-    if (int rc = cached_buffer(CACHE_WORKSPACE, c->dev, L.total, &ws_v)) return rc;
+    if (int rc = cached_buffer(cache_guard.state->workspace, L.total, "workspace", &ws_v)) return rc;
     ws = (unsigned char *)ws_v;
     for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
     choose_range_bins(range_h[0], ~range_h[1], kb, bits, &lo, &shift);
@@ -1141,7 +1142,7 @@ struct MgpuSort {
     auto mine = std::make_unique<MgpuBlob>();
     const bool want_p2p = o.mgpu_p2p != 0 && !c->p2p_failed;
     if (want_p2p) {
-      const uint64_t gen = cache_entry(CACHE_WORKSPACE, c->dev).gen;
+      const uint64_t gen = cache_guard.state->workspace.gen;
       if (c->my_handle_of != ws || c->my_handle_gen != gen) {  // (a slow driver call: once per workspace allocation)
         cudaError_t e = cudaIpcGetMemHandle(&c->my_handle, ws);
         if (e != cudaSuccess) { cudaGetLastError(); c->p2p_failed = true; }
