@@ -31,6 +31,8 @@
  *        the end: the device-made plan may ask the host for the digit-by-digit fall-back);
  *      * any sort of >= 2^24 records: additionally waits once, early, for the 200-byte pass plan made
  *        on the device, so that only the passes that execute are launched.
+ *      * a segmented sort: one wait for the segment classification, two with 8-byte keys and a segment
+ *        longer than 8192 records, plus the waits above of the whole-array sorts it runs for long segments.
  *    These calls therefore cannot be captured into a CUDA graph; everything between the two waits
  *    (all passes, the junction kernel, the flag-gated segment finish / copy-back) is queued without one.
  *  - device arrays are sorted on the device that owns them, whatever the caller's current device is;
@@ -105,6 +107,39 @@ int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int
 size_t b200sort_workspace_bytes(int key_type, int64_t num, int n_payloads,
                                 const uint32_t *payload_elem_bytes, uint32_t record_bytes);
 
+/* ---- segmented sort: many independent segments of one array in one call ---------------------------
+ * (An extension: the reference has no counterpart.)
+ *  - Segments: segment i is records [offsets[i], offsets[i+1]).  `offsets` holds n_segments + 1 values,
+ *    non-decreasing, with 0 <= offsets[0] and offsets[n_segments] <= num.
+ *  - Result: each segment is sorted on its own, with the order and payload contract of b200sort_sort_soa /
+ *    _aos (the total order on bit patterns; not stable).  Records outside [offsets[0], offsets[n_segments])
+ *    are not touched.  n_segments == 0 and empty segments are no-ops; with num <= 1 nothing moves, but the offsets
+ *    are still checked.  There is no partial-sort mode.
+ *  - Memory side: `offsets` lives where the arrays do (host memory, or the arrays' device).  Host arrays are
+ *    staged whole through the device's staging cache, and the call returns when the data is back.
+ *  - Errors: offsets that decrease, are negative or pass num: B200SORT_EINVAL, and no record has moved.
+ *    n_segments outside [0, 2^31 - 1] or offsets NULL: B200SORT_EINVAL.  Key type, payload shapes and record
+ *    size are checked as in b200sort_sort_soa / _aos.
+ *  - Workspace: NULL (the library's per-device cache) or a 256-byte aligned buffer of at least
+ *    b200sort_segmented_workspace_bytes(...) bytes.
+ *  - Host waits: a device-array call reads a few bytes of segment classification back (one wait; two when keys
+ *    of 8 bytes have segments longer than CAP = 8192 records), plus the waits of the whole-array sorts below.
+ *  - Segments of up to CAP records (16384 for keys of <= 4 bytes, 8192 for 8-byte keys) are sorted in shared
+ *    memory.  With a longer segment, keys of <= 4 bytes are sorted as ONE whole-array sort of u64 (segment
+ *    index, key) pairs over [offsets[0], offsets[n_segments]); 8-byte keys cost one whole-array sort per long
+ *    segment (b200sort_sort_soa's sequence and host waits each).
+ *  - b200sort_last_stats afterwards: algo = 3, num, record_bytes, key_bytes and kernel_launches of the whole call;
+ *    every other field 0. */
+int b200sort_sort_segmented_soa(void *keys, int key_type, int64_t num, int64_t n_segments, const int64_t *offsets,
+                                int ascending, int n_payloads, void *const *payloads,
+                                const uint32_t *payload_elem_bytes, void *stream, void *workspace, size_t workspace_bytes);
+int b200sort_sort_segmented_aos(void *records, int key_type, uint32_t record_bytes, int64_t num, int64_t n_segments,
+                                const int64_t *offsets, int ascending, void *stream, void *workspace, size_t workspace_bytes);
+/* Bytes of device scratch a segmented call with these shapes needs, whatever the segment lengths (record_bytes = 0
+ * for the SoA form). */
+size_t b200sort_segmented_workspace_bytes(int key_type, int64_t num, int64_t n_segments, int n_payloads,
+                                          const uint32_t *payload_elem_bytes, uint32_t record_bytes);
+
 /* Thread-local message of the last failing call on this thread ("" if none). */
 const char *b200sort_last_error(void);
 
@@ -126,7 +161,8 @@ typedef struct b200sort_stats {
   int64_t num;
   uint32_t record_bytes;      /* sum of all stream element sizes */
   uint32_t key_bytes;
-  uint32_t algo;              /* 1 LSD, 2 hybrid */
+  uint32_t algo;              /* 1 LSD, 2 hybrid, 3 segmented sort (then only num, record_bytes, key_bytes and
+                                 kernel_launches are set) */
   uint32_t passes_planned;    /* scatter passes executed (hybrid) / launched (LSD; constant digits return at once) */
   uint32_t hist_sweeps;       /* key-only sweeps launched */
   uint32_t kernel_launches;   /* kernels launched by this call */
@@ -140,7 +176,7 @@ int b200sort_last_stats(b200sort_stats *out);
 
 /* Per-kernel device times of the last sort on this thread, recorded with CUDA events on the sort's
  * stream when option "profile" is 1.  kinds[i]: 0 histogram, 1 scan, 2 scatter pass, 3 copy-back,
- * 4 segment finish, 5 other.  Returns the number of entries written (<= capacity) or a negative code. */
+ * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments.  Returns the number of entries written (<= capacity) or a negative code. */
 int b200sort_last_profile(int *kinds, float *ms, int capacity);
 
 /* Releases the per-device workspace and host-staging buffers held by the library.  A sort another thread

@@ -138,5 +138,23 @@ void sort(const SortIndex num, K *const keys, Ps *const... payloads) {
   sort<Up, BitSorterSIMD, CmpSorterInsertionSort>(16, num, keys, payloads...);
 }
 
+// An extension with no counterpart in the reference: sorts every segment [offsets[i], offsets[i+1]) of
+// keys[0, num) on its own (b200sort_sort_segmented_soa; `offsets` holds n_segments + 1 values and lives
+// where the arrays do).
+template <bool Up = true, typename K, typename... Ps>
+void sort_segmented(const SortIndex num, const int64_t n_segments, const int64_t *const offsets, K *const keys,
+                    Ps *const... payloads) {
+  static_assert(internal::key_type_code<K>() >= 0,
+                "key type must be one of (u)int8/16/32/64, float, double");
+  static_assert(((std::is_trivially_copyable_v<Ps> && sizeof(Ps) >= 1 && sizeof(Ps) <= 64) && ...),
+                "payload types must be trivially copyable and at most 64 bytes");
+  static_assert(sizeof...(Ps) <= 63, "at most 63 payload streams");
+  void *ptrs[sizeof...(Ps) + 1] = {const_cast<void *>(static_cast<const void *>(payloads))..., nullptr};
+  const uint32_t sizes[sizeof...(Ps) + 1] = {static_cast<uint32_t>(sizeof(Ps))..., 0u};
+  internal::check(b200sort_sort_segmented_soa(const_cast<std::remove_cv_t<K> *>(keys), internal::key_type_code<K>(), num,
+                                              n_segments, offsets, Up ? 1 : 0, static_cast<int>(sizeof...(Ps)), ptrs, sizes,
+                                              nullptr, nullptr, 0));
+}
+
 }  // namespace radix_sort
 }  // namespace simd_sort

@@ -59,6 +59,12 @@ def lib():
         L.b200sort_sort_aos_ex.restype = i32
         L.b200sort_workspace_bytes.argtypes = [i32, i64, i32, u32p, u32]
         L.b200sort_workspace_bytes.restype = sz
+        L.b200sort_sort_segmented_soa.argtypes = [vp, i32, i64, i64, vp, i32, i32, vpp, u32p, vp, vp, sz]
+        L.b200sort_sort_segmented_soa.restype = i32
+        L.b200sort_sort_segmented_aos.argtypes = [vp, i32, u32, i64, i64, vp, i32, vp, vp, sz]
+        L.b200sort_sort_segmented_aos.restype = i32
+        L.b200sort_segmented_workspace_bytes.argtypes = [i32, i64, i64, i32, u32p, u32]
+        L.b200sort_segmented_workspace_bytes.restype = sz
         L.b200sort_last_error.restype = ctypes.c_char_p
         L.b200sort_version.restype = i32
         L.b200sort_launch_count.restype = ctypes.c_uint64
@@ -140,7 +146,7 @@ def last_stats() -> dict:
     return {f: getattr(s, f) for f, _ in _Stats._fields_}
 
 
-PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other"]
+PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other", "segment"]
 
 
 def last_profile():
@@ -259,3 +265,83 @@ def workspace_bytes(key_dtype, num: int, payload_itemsizes=(), record_bytes: int
     n = len(payload_itemsizes)
     sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
     return int(lib().b200sort_workspace_bytes(_key_code(kname), num, n, sizes, record_bytes))
+
+
+def _offsets_arg(offsets):
+    """-> (address, n_segments) of a contiguous 1-D int64 offsets array (n_segments + 1 values)"""
+    addr, name, _, count, _ = _describe(offsets)
+    if name != "int64":
+        raise TypeError(f"offsets must be int64, not {name}")
+    if count < 1:
+        raise ValueError("offsets holds n_segments + 1 values, at least one")
+    return addr, count - 1
+
+
+def sort_segmented(offsets, keys, *payloads, up: bool = True, stream=None, workspace=None):
+    """Sorts every segment keys[offsets[i]:offsets[i+1]] on its own, in place, and applies each segment's
+    permutation to the payload arrays (b200sort_sort_segmented_soa; an extension, the reference has none).
+
+    `offsets` is a 1-D int64 array or tensor of n_segments + 1 non-decreasing values in [0, len(keys)],
+    on the same side (and device) as the arrays.  Records outside [offsets[0], offsets[-1]) are not touched."""
+    kaddr, kname, _, num, _ = _describe(keys)
+    oaddr, n_seg = _offsets_arg(offsets)
+    n = len(payloads)
+    ptrs = (ctypes.c_void_p * max(n, 1))()
+    sizes = (ctypes.c_uint32 * max(n, 1))()
+    for i, p in enumerate(payloads):
+        addr, _, item, pn, _ = _describe(p)
+        if pn < num:
+            raise ValueError(f"payload {i} is shorter than the keys")
+        ptrs[i], sizes[i] = addr, item
+    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
+    with _device_guard((keys,) + payloads):
+        st = _stream_for((keys,) + payloads, stream)
+        rc = lib().b200sort_sort_segmented_soa(kaddr, _key_code(kname), num, n_seg, oaddr, int(up), n, ptrs, sizes, st, ws_ptr, ws_bytes)
+    _check(rc)
+
+
+def sort_segmented_combined(offsets, records, key_dtype, up: bool = True, stream=None, workspace=None):
+    """sort_segmented for combined records (b200sort_sort_segmented_aos): `records` as in sort_combined."""
+    addr, _, record_bytes, num, _ = _describe(records)
+    oaddr, n_seg = _offsets_arg(offsets)
+    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
+    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
+    with _device_guard((records,)):
+        st = _stream_for((records,), stream)
+        rc = lib().b200sort_sort_segmented_aos(addr, _key_code(kname), record_bytes, num, n_seg, oaddr, int(up), st, ws_ptr, ws_bytes)
+    _check(rc)
+
+
+def segmented_workspace_bytes(key_dtype, num: int, n_segments: int, payload_itemsizes=(), record_bytes: int = 0) -> int:
+    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
+    n = len(payload_itemsizes)
+    sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
+    return int(lib().b200sort_segmented_workspace_bytes(_key_code(kname), num, n_segments, n, sizes, record_bytes))
+
+
+def sort_rows(keys, *payloads, up: bool = True, stream=None):
+    """Sorts every row of a contiguous (B, L) array or tensor in place, like torch.sort(keys, dim=-1), and
+    applies each row's permutation to the payloads, whose first two dimensions are (B, L)."""
+    if keys.ndim != 2:
+        raise ValueError("keys must be 2-D (B, L)")
+    B, L = int(keys.shape[0]), int(keys.shape[1])
+    for i, p in enumerate(payloads):
+        if p.ndim < 2 or tuple(p.shape[:2]) != (B, L):
+            raise ValueError(f"payload {i} does not have the keys' (B, L) shape")
+
+    # 2-D arrays are streams of row-sized elements (_describe): pass flat views, one element per (row, column)
+    def flat(x):
+        return x.reshape(B * L) if x.ndim == 2 else x.reshape(B * L, -1)
+
+    if _is_torch(keys):
+        import torch
+        if keys.is_cuda and stream is not None:
+            # the offsets are made on the stream the sort runs on, and freed only after it
+            with torch.cuda.stream(torch.cuda.ExternalStream(int(stream), device=keys.device)):
+                offsets = torch.arange(B + 1, dtype=torch.int64, device=keys.device) * L
+                sort_segmented(offsets, flat(keys), *[flat(p) for p in payloads], up=up, stream=stream)
+            return
+        offsets = torch.arange(B + 1, dtype=torch.int64, device=keys.device) * L
+    else:
+        offsets = np.arange(B + 1, dtype=np.int64) * L
+    sort_segmented(offsets, flat(keys), *[flat(p) for p in payloads], up=up, stream=stream)

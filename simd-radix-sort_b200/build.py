@@ -17,11 +17,11 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libb200sort.so"
 # (source, object stem, extra defines): sweep_inst.cu is compiled once per (key bytes, tile geometry)
-UNITS = [(CSRC / "b200sort.cu", "b200sort", [])] + [
+UNITS = [(CSRC / "b200sort.cu", "b200sort", []), (CSRC / "segmented_inst.cu", "segmented_inst", [])] + [
     (CSRC / "sweep_inst.cu", f"sweep_kb{k}_c{c}", [f"-DSWEEP_KB={k}", f"-DSWEEP_CFG={c}"]) for k in (8, 4, 2, 1) for c in (0, 1)] + [
     (CSRC / "sweep_inst.cu", "sweep_kb4_c2", ["-DSWEEP_KB=4", "-DSWEEP_CFG=2"])]
-SOURCES = [CSRC / "b200sort.cu", CSRC / "sweep_inst.cu"]
-HEADERS = [CSRC / "kernels.cuh", CSRC / "hybrid.cuh", CSRC / "mgpu.cuh", CSRC / "sweep_select.cuh", PKG.parent / "include" / "b200sort.h"]
+SOURCES = [CSRC / "b200sort.cu", CSRC / "sweep_inst.cu", CSRC / "segmented_inst.cu"]
+HEADERS = [CSRC / "kernels.cuh", CSRC / "hybrid.cuh", CSRC / "mgpu.cuh", CSRC / "segmented.cuh", CSRC / "segmented_host.cuh", CSRC / "sweep_select.cuh", PKG.parent / "include" / "b200sort.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-lineinfo",

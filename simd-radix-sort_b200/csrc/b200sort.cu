@@ -26,6 +26,7 @@
 #include "kernels.cuh"
 #include "sweep_select.cuh"
 #include "hybrid.cuh"
+#include "segmented.cuh"
 
 namespace b200sort {
 
@@ -104,7 +105,7 @@ struct ThreadDeviceState {
 static thread_local std::map<int, ThreadDeviceState> t_dev;
 
 // optional per-kernel timing (option "profile"): CUDA events around every launch of the last sort
-enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5 };
+enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5, PK_SEGMENT = 6 };
 struct ProfEntry { int kind; cudaEvent_t e0, e1; int dev; };
 static thread_local bool g_prof_on = false;  // the sort running on this thread has option "profile" set
 static thread_local std::vector<ProfEntry> g_prof;
@@ -127,8 +128,8 @@ struct ProfScope {  // (kind PK_NONE: records nothing)
     if (on) { cudaEventRecord(pe.e1, st); g_prof.push_back(pe); }
     static const bool dbg = getenv("B200SORT_DEBUG_SYNC") != nullptr;  // development: wait for every kernel, say which one
     if (dbg && kind_ != PK_NONE) {
-      static const char *names[] = {"hist", "scan", "sweep", "copyback", "segfix", "other"};
-      fprintf(stderr, "[b200sort] %s launched ...", names[kind_ < 6 ? kind_ : 5]);
+      static const char *names[] = {"hist", "scan", "sweep", "copyback", "segfix", "other", "segment"};
+      fprintf(stderr, "[b200sort] %s launched ...", names[kind_ < 7 ? kind_ : 5]);
       const cudaError_t e = cudaStreamSynchronize(st);
       fprintf(stderr, " done (%s)\n", cudaGetErrorString(e));
     }
@@ -491,6 +492,7 @@ struct DevSortOpts {
   // Partial-sort mode (B200SORT_CMP_NONE with a threshold >= CMP_NONE_MIN_THRESH): the segments below the plan's
   // cut need not be ordered as long as none has more than this many keys (0 = full sort)
   int64_t cmp_none_thresh = 0;
+  bool keep_profile = false;  // part of a larger call (a segmented sort): add to its profile entries, do not reset them
 };
 constexpr int64_t CMP_NONE_MIN_THRESH = 8;  // below it nearly every sort would need the finish anyway: full sort
 
@@ -584,7 +586,7 @@ struct DevSort {
     plan = (Plan *)(ws + L.plan_off);
     ctrl = (HybridCtrl *)(ws + L.hyb_off);
     g_prof_on = o.profile != 0;
-    if (!xo.forced) prof_reset();
+    if (!xo.forced && !xo.keep_profile) prof_reset();
     if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
 
     ko = make_key_order(key_type, ascending);
@@ -1014,10 +1016,8 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
   return rc;
 }
 
-static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
-                    void *workspace, size_t workspace_bytes, const DevSortOpts &base, b200sort_stats *stats) {
-  cudaStream_t stream = (cudaStream_t)stream_v;
-  if (n <= 1) return B200SORT_OK;  // src/radix_sort.hpp:276: nothing to do for 0 or 1 element
+// where the arrays of one call live: all in host memory, or all on one device (*dev); fails without a device
+static int arrays_side(const std::vector<StreamDesc> &streams, Side *side, int *dev) {
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0) {
@@ -1025,16 +1025,24 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
     return fail(B200SORT_ECUDA, "no CUDA device available (%s); libb200sort has no CPU fallback",
                 e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
   }
-  Side side0;
-  int dev0 = 0;
-  if (int rc = side_of(streams[0].ptr, &side0, &dev0)) return rc;
+  if (int rc = side_of(streams[0].ptr, side, dev)) return rc;
   for (size_t s = 1; s < streams.size(); s++) {
     Side sd;
     int dv = 0;
     if (int rc = side_of(streams[s].ptr, &sd, &dv)) return rc;
-    if (sd != side0) return fail(B200SORT_EINVAL, "arrays must be all in host memory or all in device memory");
-    if (sd == SIDE_DEVICE && dv != dev0) return fail(B200SORT_EINVAL, "device arrays live on different devices (%d and %d)", dev0, dv);
+    if (sd != *side) return fail(B200SORT_EINVAL, "arrays must be all in host memory or all in device memory");
+    if (sd == SIDE_DEVICE && dv != *dev) return fail(B200SORT_EINVAL, "device arrays live on different devices (%d and %d)", *dev, dv);
   }
+  return 0;
+}
+
+static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
+                    void *workspace, size_t workspace_bytes, const DevSortOpts &base, b200sort_stats *stats) {
+  cudaStream_t stream = (cudaStream_t)stream_v;
+  if (n <= 1) return B200SORT_OK;  // src/radix_sort.hpp:276: nothing to do for 0 or 1 element
+  Side side0;
+  int dev0 = 0;
+  if (int rc = arrays_side(streams, &side0, &dev0)) return rc;
   if (side0 == SIDE_DEVICE) {
     DeviceScope scope;  // sort on the device that owns the arrays (include/b200sort.h)
     if (scope.enter(dev0) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", dev0);
@@ -1069,6 +1077,7 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
   if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
   unsigned char *dbuf = (unsigned char *)dbuf_v;
   int rc = B200SORT_OK;
+  cudaError_t e = cudaSuccess;
   for (size_t s = 0; s < streams.size() && rc == 0; s++) {
     dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
     e = cudaMemcpyAsync(dstreams[s].ptr, streams[s].ptr, (size_t)n * streams[s].elem_bytes, cudaMemcpyHostToDevice, stream);
@@ -1238,3 +1247,4 @@ void b200sort_release_cache(void) {
 }  // extern "C"
 
 #include "mgpu.cuh"
+#include "segmented_host.cuh"
