@@ -26,11 +26,13 @@ def main():
     assert L.b200sort_mgpu_comm_create(ctypes.byref(comm), 1, 0, buf) == 0, L.b200sort_last_error()
     st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
-    def run(keys, up, tag, want_overlap=None):
+    def run(keys, up, tag, want_overlap=None, offset=0):
+        """offset: keys and payloads are views that start `offset` elements into their allocations"""
         n = len(keys)
         cap = n + 4096
-        k = torch.zeros(cap, dtype=torch.from_numpy(keys[:1]).dtype, device=dev)
-        p = torch.zeros(cap, dtype=torch.uint64, device=dev)
+        kbuf = torch.zeros(cap + offset, dtype=torch.from_numpy(keys[:1]).dtype, device=dev)
+        pbuf = torch.zeros(cap + offset, dtype=torch.uint64, device=dev)
+        k, p = kbuf[offset:], pbuf[offset:]
         k[:n].copy_(torch.from_numpy(keys))
         p[:n].copy_(torch.from_numpy(np.arange(n, dtype=np.uint64)))
         ptrs = (ctypes.c_void_p * 1)(p.data_ptr())
@@ -51,6 +53,9 @@ def main():
     rng = np.random.default_rng(1)
     run(O.make_keys("Uniform", np.uint64, n, 1), True, "plain u64")
     run(O.make_keys("Gaussian", np.float32, n, 2), False, "plain f32 desc")
+    # keys and payloads at 8 mod 16: the count and partition kernels take their paths for keys that are not dense and
+    # 16-byte aligned
+    run(O.make_keys("Uniform", np.uint64, n, 30), True, "u64 at offset 1", offset=1)
     with S.options(host_plan_min_log2=0):
         run(O.make_keys("Uniform", np.uint64, n, 3), True, "landing u64", 0)
         with S.options(mgpu_chunk_min_log2=12, mgpu_overlap=2):   # 2: also with a world of one (this vehicle)
@@ -59,6 +64,7 @@ def main():
                     run(O.make_keys("Uniform", np.uint64, n, 4 + chunks), True, f"overlap u64 chunks={chunks}", 1)
                     run(O.make_keys("Uniform", np.int64, n, 14 + chunks), False, f"overlap i64 desc chunks={chunks}", 1)
         run(np.zeros(n, np.int64), True, "zero")
+        run(O.make_keys("Gaussian", np.int64, n, 31), False, "i64 desc at offset 1", offset=1)
         run(rng.integers(-8, 8, size=n, dtype=np.int64), False, "few unique")
     assert L.b200sort_mgpu_comm_destroy(comm) == 0
     print("MGPU_SINGLE_OK", flush=True)

@@ -44,6 +44,15 @@ def keys_of(dt, n, rng, specials=True):
     return rng.integers(max(int(info.min), -hi - 1), hi, size=n, dtype=dt, endpoint=True)
 
 
+def full_range_keys(dt, n, rng):
+    """random bit patterns (for floats with +-0, +-inf and NaN among them): a long segment of these keys has digits
+    below the hybrid path's cut, so its sort runs the segment finish"""
+    k = rng.integers(0, 2**64, n, dtype=np.uint64).view(dt)
+    if k.dtype.kind == "f":
+        k[rng.integers(0, n, 15)] = np.repeat(np.array([0.0, -0.0, np.inf, -np.inf, np.nan]), 3)
+    return k
+
+
 def offsets_of(lengths, first=0):
     return np.concatenate([[first], first + np.cumsum(lengths)]).astype(np.int64)
 
@@ -69,6 +78,33 @@ def check(keys_in, keys_out, pays_in, pays_out, offsets, up):
         assert po[:lo].tobytes() == pi[:lo].tobytes() and po[hi:].tobytes() == pi[hi:].tobytes()
     if pays_in:
         assert O.runs_multiset_equal(runs, [p[lo:hi] for p in pays_out], [p[lo:hi][perm] for p in pays_in])
+
+
+def check_with_index(keys_in, keys_out, pays_in, pays_out, offsets, up):
+    """check() for calls too large for the lexsort of expected().  pays_in[0] is the index np.arange(n), and pays_out[0]
+    must be a permutation of the covered range that keeps every record in its segment, with keys_out == keys_in[idx]
+    and the ordered keys non-decreasing inside every segment.  Equal ordered keys have equal bytes, so that is
+    expected()'s key sequence byte for byte.  Every other payload must equal its input at that index."""
+    lo, hi = int(offsets[0]), int(offsets[-1])
+    for a, b in [(keys_in, keys_out)] + list(zip(pays_in, pays_out)):
+        assert b[:lo].tobytes() == a[:lo].tobytes() and b[hi:].tobytes() == a[hi:].tobytes()
+    seg = np.repeat(np.arange(len(offsets) - 1), np.diff(offsets))
+    idx = pays_out[0][lo:hi].astype(np.int64)
+    assert idx.min() >= lo and idx.max() < hi and np.all(np.bincount(idx - lo, minlength=hi - lo) == 1), "not a permutation"
+    assert np.array_equal(seg[idx - lo], seg), "a record left its segment"
+    assert keys_out[lo:hi].tobytes() == keys_in[idx].tobytes()
+    ok = O.order_key(keys_out[lo:hi], up)
+    assert np.all((ok[1:] >= ok[:-1]) | (seg[1:] != seg[:-1])), "a segment is not sorted"
+    for pi, po in zip(pays_in[1:], pays_out[1:]):
+        assert np.array_equal(po[lo:hi], pi[idx])
+
+
+def odd_starts(lens, first, which):
+    """lengthens the segment before each of `which` by one where needed, so that those segments start at odd records"""
+    for j in sorted(which):
+        if (first + int(lens[:j].sum())) % 2 == 0:
+            lens[j - 1] += 1
+    return offsets_of(lens, first)
 
 
 def run_soa(keys, pays, offsets, up=True, on_device=True, **kw):
@@ -193,22 +229,58 @@ def test_composite_branch(dt):
         sort_and_check(keys, [], offsets, up)
 
 
+def test_composite_branch_above_2p24():
+    """u16 keys: 2^20 short segments and one long one, a span above 2^24 records from an odd offsets[0] (so the payload
+    streams of the composite sort start at odd records); the segment index fills 20 bits of the composite key"""
+    rng = np.random.default_rng(56)
+    lens = rng.integers(0, 24, 1 << 20)
+    lens[1000] = 5_000_000
+    offsets = offsets_of(lens, first=7)
+    assert offsets[-1] - offsets[0] >= 1 << 24
+    n = int(offsets[-1]) + 5
+    keys = keys_of(np.uint16, n, rng)
+    pays = [np.arange(n, dtype=np.uint64), rng.integers(0, 256, (n, 12), dtype=np.uint8)]
+    for up in (True, False):
+        with S.options(profile=1):
+            k, ps = run_soa(keys, pays, offsets, up)
+        assert S.last_stats()["algo"] == 3
+        check_with_index(keys, k, pays, ps, offsets, up)
+        kinds = [kd for kd, _ in S.last_profile()]
+        # the composite sort read its plan back: the smaller flow always launches one full segment finish; this one
+        # launches none (nothing left below the cut) or the junction kernel and the gated finish
+        assert "sweep" in kinds and kinds.count("segfix") in (0, 2), kinds
+
+
 def test_sort_rows_matches_torch_sort_on_sampling_shape():
+    """f32 rows are one composite-key sort of all rows: (64, 128256) below 2^24 records, whose sort launches one full
+    segment finish, and (136, 128256) and (68, 250001) above, where that sort reads its plan back and launches none
+    (nothing left below the cut) or two (the junction kernel and the gated finish).  f64 rows of odd length are one
+    whole-array sort per row, every other row at 8 mod 16."""
     g = torch.Generator(device="cuda").manual_seed(3)
-    logits = torch.randn(64, 128256, device="cuda", generator=g)
-    logits[:, :17] = logits[:, 17:34]  # duplicates inside every row
-    idx = torch.arange(128256, device="cuda", dtype=torch.int64).repeat(64, 1).contiguous()
-    want_v, _ = torch.sort(logits, dim=-1, descending=True)
-    k = logits.clone()
-    S.sort_rows(k, idx, up=False)
-    torch.cuda.synchronize()
-    assert torch.equal(k, want_v)
-    assert torch.equal(torch.gather(logits, 1, idx), k)
-    assert torch.equal(idx.sort(dim=-1).values, torch.arange(128256, device="cuda").repeat(64, 1))
+    for B, L, dt, n_segfix in ((64, 128256, torch.float32, (1,)), (136, 128256, torch.float32, (0, 2)), (68, 250001, torch.float32, (0, 2)),
+                               (68, 250001, torch.float64, (0,))):
+        logits = torch.randn(B, L, device="cuda", generator=g, dtype=dt)
+        logits[:, :17] = logits[:, 17:34]  # duplicates inside every row
+        for up in (False, True):
+            want_v, _ = torch.sort(logits, dim=-1, descending=not up)
+            idx = torch.arange(L, device="cuda", dtype=torch.int64).repeat(B, 1).contiguous()
+            k = logits.clone()
+            with S.options(profile=1):
+                S.sort_rows(k, idx, up=up)
+            torch.cuda.synchronize()
+            assert torch.equal(k, want_v), (B, L, dt, up)
+            assert torch.equal(torch.gather(logits, 1, idx), k), (B, L, dt, up)
+            assert torch.equal(idx.sort(dim=-1).values, torch.arange(L, device="cuda").repeat(B, 1)), (B, L, dt, up)
+            kinds = [kd for kd, _ in S.last_profile()]
+            assert "sweep" in kinds and kinds.count("segfix") in n_segfix, (B, L, dt, kinds)
+            del want_v, idx, k
     # the same through numpy host arrays, ascending
-    kh, ih = logits[:4].cpu().numpy().copy(), idx[:4].cpu().numpy().copy()
-    S.sort_rows(kh, ih)
+    logits = torch.randn(64, 128256, device="cuda", generator=g)
+    idx = torch.arange(128256, dtype=torch.int64).repeat(4, 1).numpy()
+    kh = logits[:4].cpu().numpy().copy()
+    S.sort_rows(kh, idx)
     assert np.array_equal(kh, torch.sort(logits[:4], dim=-1).values.cpu().numpy())
+    assert np.array_equal(np.take_along_axis(logits[:4].cpu().numpy(), idx, 1), kh)
 
 
 @pytest.mark.parametrize("dt", [np.uint64, np.int64, np.float64], ids=lambda d: np.dtype(d).name)
@@ -221,6 +293,52 @@ def test_wide_keys_with_long_segments(dt):
     keys = keys_of(dt, int(offsets[-1]), rng)
     for up in (True, False):
         sort_and_check(keys, [np.arange(len(keys), dtype=np.uint32), rng.integers(0, 2**60, len(keys), dtype=np.uint64)], offsets, up)
+
+
+@pytest.mark.parametrize("dt", [np.int64, np.float64], ids=lambda d: np.dtype(d).name)
+def test_wide_keys_with_hybrid_long_segments(dt):
+    """8-byte keys: long segments of 2^22 + 5 and 2^24 + 3 records starting at odd records (8 mod 16), among short and
+    CAP + 1 segments.  Their whole-array sorts take the hybrid path, the longer one reading its plan back: one
+    "segfix" entry for the first, two (the junction kernel and the gated full segment finish) for the second."""
+    dt = np.dtype(dt)
+    rng = np.random.default_rng(dt.num + 90)
+    lens = mixed_lengths(rng, 600)
+    lens[[10, 200, 400, 599]] = [CAP[8] + 1, (1 << 22) + 5, (1 << 24) + 3, CAP[8] + 1]
+    offsets = odd_starts(lens, 3, [200, 400])
+    n = int(offsets[-1]) + 2
+    keys = full_range_keys(dt, n, rng)
+    pays = [np.arange(n, dtype=np.uint64), rng.integers(0, 2**16, n, dtype=np.uint16)]
+    for up in (True, False):
+        with S.options(profile=1):
+            k, ps = run_soa(keys, pays, offsets, up)
+        assert S.last_stats()["algo"] == 3
+        check_with_index(keys, k, pays, ps, offsets, up)
+        kinds = [kd for kd, _ in S.last_profile()]
+        assert "sweep" in kinds and "segment" in kinds and kinds.count("segfix") == 3, kinds
+
+
+def test_combined_records_with_a_hybrid_long_segment():
+    """16-byte i64 records with one segment of 2^22 + 1 records at an odd start: its whole-array sort of records takes
+    the hybrid path"""
+    rng = np.random.default_rng(91)
+    lens = mixed_lengths(rng, 300)
+    lens[100] = (1 << 22) + 1
+    offsets = odd_starts(lens, 1, [100])
+    n = int(offsets[-1]) + 1
+    keys = full_range_keys(np.int64, n, rng)
+    rec = np.empty((n, 16), np.uint8)
+    rec[:, :8] = keys.view(np.uint8).reshape(n, 8)
+    rec[:, 8:] = np.arange(n, dtype=np.uint64).view(np.uint8).reshape(n, 8)
+    r = dev(rec)
+    with S.options(profile=1):
+        S.sort_segmented_combined(dev(offsets), r, np.int64, up=False)
+    got = r.cpu().numpy()
+    assert S.last_stats()["algo"] == 3
+    kinds = [kd for kd, _ in S.last_profile()]
+    assert "sweep" in kinds and "segment" in kinds and kinds.count("segfix") == 1, kinds
+    idx = np.ascontiguousarray(got[:, 8:]).view(np.uint64).reshape(-1)
+    check_with_index(keys, np.ascontiguousarray(got[:, :8]).view(np.int64).reshape(-1), [np.arange(n, dtype=np.uint64), rec], [idx, got],
+                     offsets, False)
 
 
 def test_one_segment_equals_sort():
