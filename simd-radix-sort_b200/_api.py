@@ -202,14 +202,37 @@ def _device_guard(arrays):
         if _is_torch(x) and x.is_cuda:
             import torch
             return torch.cuda.device(x.device)
-    import contextlib
     return contextlib.nullcontext()
 
 
-def _key_code(name: str) -> int:
+def _key_code(key_dtype) -> int:
+    """The key type code of a dtype (numpy, or anything np.dtype takes) or a dtype name such as "int32"."""
+    name = key_dtype if isinstance(key_dtype, str) else np.dtype(key_dtype).name
     if name not in KEY_TYPES:
         raise TypeError(f"unsupported key type {name}; the reference sorts {sorted(KEY_TYPES)}")
     return KEY_TYPES[name]
+
+
+def _payload_args(payloads, num: int):
+    """-> (count, addresses, element sizes) of the payload arrays, as the C calls take them; each has at least num rows"""
+    n = len(payloads)
+    ptrs = (ctypes.c_void_p * max(n, 1))()
+    sizes = (ctypes.c_uint32 * max(n, 1))()
+    for i, p in enumerate(payloads):
+        addr, _, item, pn, _ = _describe(p)
+        if pn < num:
+            raise ValueError(f"payload {i} has fewer than {num} rows")
+        ptrs[i], sizes[i] = addr, item
+    return n, ptrs, sizes
+
+
+def _call(fn, arrays, stream, workspace, *args):
+    """fn(*args, stream, workspace address, workspace bytes) on the device and stream of the arrays (unless `stream` is
+    given); raises B200SortError when it fails."""
+    ws = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
+    with _device_guard(arrays):
+        rc = fn(*args, _stream_for(arrays, stream), *ws)
+    _check(rc)
 
 
 def sort(num, keys, *payloads, up: bool = True, stream=None, cmp_sort_threshold: int | None = None,
@@ -223,23 +246,12 @@ def sort(num, keys, *payloads, up: bool = True, stream=None, cmp_sort_threshold:
     kaddr, kname, _, kn, _ = _describe(keys)
     if num < 0 or num > kn:
         raise ValueError("num exceeds the key array")
-    n = len(payloads)
-    ptrs = (ctypes.c_void_p * max(n, 1))()
-    sizes = (ctypes.c_uint32 * max(n, 1))()
-    for i, p in enumerate(payloads):
-        addr, _, item, pn, _ = _describe(p)
-        if pn < num:
-            raise ValueError(f"payload {i} is shorter than num")
-        ptrs[i], sizes[i] = addr, item
-    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
-    with _device_guard((keys,) + payloads):
-        st = _stream_for((keys,) + payloads, stream)
-        if cmp_sort_threshold is None:
-            rc = lib().b200sort_sort_soa(kaddr, _key_code(kname), num, int(up), n, ptrs, sizes, st, ws_ptr, ws_bytes)
-        else:
-            rc = lib().b200sort_sort_soa_ex(kaddr, _key_code(kname), num, int(up), n, ptrs, sizes,
-                                            cmp_sort_threshold, cmp_sorter, st, ws_ptr, ws_bytes)
-    _check(rc)
+    pay = _payload_args(payloads, num)
+    args = (kaddr, _key_code(kname), num, int(up), *pay)
+    if cmp_sort_threshold is None:
+        _call(lib().b200sort_sort_soa, (keys,) + payloads, stream, workspace, *args)
+    else:
+        _call(lib().b200sort_sort_soa_ex, (keys,) + payloads, stream, workspace, *args, cmp_sort_threshold, cmp_sorter)
 
 
 def sort_combined(num, records, key_dtype, up: bool = True, stream=None, workspace=None):
@@ -252,19 +264,13 @@ def sort_combined(num, records, key_dtype, up: bool = True, stream=None, workspa
     addr, _, record_bytes, rows, _ = _describe(records)
     if rows < num:
         raise ValueError("num exceeds the record array")
-    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
-    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
-    with _device_guard((records,)):
-        st = _stream_for((records,), stream)
-        rc = lib().b200sort_sort_aos(addr, _key_code(kname), record_bytes, num, int(up), st, ws_ptr, ws_bytes)
-    _check(rc)
+    _call(lib().b200sort_sort_aos, (records,), stream, workspace, addr, _key_code(key_dtype), record_bytes, num, int(up))
 
 
 def workspace_bytes(key_dtype, num: int, payload_itemsizes=(), record_bytes: int = 0) -> int:
-    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
     n = len(payload_itemsizes)
     sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
-    return int(lib().b200sort_workspace_bytes(_key_code(kname), num, n, sizes, record_bytes))
+    return int(lib().b200sort_workspace_bytes(_key_code(key_dtype), num, n, sizes, record_bytes))
 
 
 def _offsets_arg(offsets):
@@ -285,38 +291,23 @@ def sort_segmented(offsets, keys, *payloads, up: bool = True, stream=None, works
     on the same side (and device) as the arrays.  Records outside [offsets[0], offsets[-1]) are not touched."""
     kaddr, kname, _, num, _ = _describe(keys)
     oaddr, n_seg = _offsets_arg(offsets)
-    n = len(payloads)
-    ptrs = (ctypes.c_void_p * max(n, 1))()
-    sizes = (ctypes.c_uint32 * max(n, 1))()
-    for i, p in enumerate(payloads):
-        addr, _, item, pn, _ = _describe(p)
-        if pn < num:
-            raise ValueError(f"payload {i} is shorter than the keys")
-        ptrs[i], sizes[i] = addr, item
-    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
-    with _device_guard((keys,) + payloads):
-        st = _stream_for((keys,) + payloads, stream)
-        rc = lib().b200sort_sort_segmented_soa(kaddr, _key_code(kname), num, n_seg, oaddr, int(up), n, ptrs, sizes, st, ws_ptr, ws_bytes)
-    _check(rc)
+    pay = _payload_args(payloads, num)
+    _call(lib().b200sort_sort_segmented_soa, (keys,) + payloads, stream, workspace, kaddr, _key_code(kname), num, n_seg, oaddr, int(up),
+          *pay)
 
 
 def sort_segmented_combined(offsets, records, key_dtype, up: bool = True, stream=None, workspace=None):
     """sort_segmented for combined records (b200sort_sort_segmented_aos): `records` as in sort_combined."""
     addr, _, record_bytes, num, _ = _describe(records)
     oaddr, n_seg = _offsets_arg(offsets)
-    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
-    ws_ptr, ws_bytes = (None, 0) if workspace is None else (workspace.data_ptr(), workspace.numel() * workspace.element_size())
-    with _device_guard((records,)):
-        st = _stream_for((records,), stream)
-        rc = lib().b200sort_sort_segmented_aos(addr, _key_code(kname), record_bytes, num, n_seg, oaddr, int(up), st, ws_ptr, ws_bytes)
-    _check(rc)
+    _call(lib().b200sort_sort_segmented_aos, (records,), stream, workspace, addr, _key_code(key_dtype), record_bytes, num, n_seg, oaddr,
+          int(up))
 
 
 def segmented_workspace_bytes(key_dtype, num: int, n_segments: int, payload_itemsizes=(), record_bytes: int = 0) -> int:
-    kname = np.dtype(key_dtype).name if not isinstance(key_dtype, str) else key_dtype
     n = len(payload_itemsizes)
     sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
-    return int(lib().b200sort_segmented_workspace_bytes(_key_code(kname), num, n_segments, n, sizes, record_bytes))
+    return int(lib().b200sort_segmented_workspace_bytes(_key_code(key_dtype), num, n_segments, n, sizes, record_bytes))
 
 
 def sort_rows(keys, *payloads, up: bool = True, stream=None):

@@ -114,6 +114,12 @@ static void prof_reset() {
   for (auto &p : g_prof) { t_dev[p.dev].prof_pool.push_back(p.e0); t_dev[p.dev].prof_pool.push_back(p.e1); }
   g_prof.clear();
 }
+// a sort call starts timing its launches if option "profile" is set; keep: it is part of a larger call (a
+// segmented sort, a multi-GPU sort) and adds to that call's entries instead of starting over
+static void start_profile(const Options &o, bool keep) {
+  g_prof_on = o.profile != 0;
+  if (!keep) prof_reset();
+}
 static cudaEvent_t prof_event(int dev) {
   auto &pool = t_dev[dev].prof_pool;
   if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
@@ -202,6 +208,18 @@ KeyOrder make_key_order(int key_type, bool ascending) {
 }
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// arrays of these sizes placed back to back at 256-byte boundaries: their offsets; *total: the bytes they span
+static std::vector<size_t> back_to_back(const std::vector<size_t> &bytes, size_t *total) {
+  std::vector<size_t> offs(bytes.size());
+  size_t off = 0;
+  for (size_t i = 0; i < bytes.size(); i++) {
+    offs[i] = off;
+    off = align_up(off + bytes[i], 256);
+  }
+  *total = off;
+  return offs;
+}
 
 // ------------------------------------------------------------------------------------------------
 // tile geometries of the scatter kernel
@@ -402,6 +420,22 @@ static int cached_buffer(CacheEntry &c, size_t bytes, const char *what, void **o
   return 0;
 }
 
+// The workspace of a sort of `bytes` on the current device `dev`: the caller's (`caller_ws`, NULL for none), or the
+// library's cached one, taken through `guard` (which the caller holds until the sort's work is queued).
+static int acquire_workspace(int dev, cudaStream_t stream, void *caller_ws, size_t caller_bytes, size_t bytes, CacheGuard &guard,
+                             unsigned char **out) {
+  void *ws = caller_ws;
+  if (ws == nullptr) {
+    if (int rc = cached_buffer(guard.acquire(dev, stream).workspace, bytes, "workspace", &ws)) return rc;
+  } else if (caller_bytes < bytes) {
+    return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", caller_bytes, bytes);
+  } else if (((uintptr_t)ws % 256) != 0) {
+    return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
+  }
+  *out = (unsigned char *)ws;
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // job description
 // ------------------------------------------------------------------------------------------------
@@ -454,6 +488,33 @@ static void make_layout(const std::vector<StreamDesc> &streams, int64_t n, int t
     if (landing) off = align_up(off + (size_t)n * streams[s].elem_bytes, 256);
   }
   L->total = align_up(off, 256);
+}
+
+// the streams of a call of this shape, without addresses: SoA keys of kb bytes and n_payloads payloads of the given
+// sizes, or (record_bytes != 0) records
+static std::vector<StreamDesc> streams_of_shape(int kb, int n_payloads, const uint32_t *sizes, uint32_t record_bytes) {
+  if (record_bytes) return {{nullptr, record_bytes}};
+  std::vector<StreamDesc> streams = {{nullptr, (uint32_t)kb}};
+  for (int p = 0; p < n_payloads; p++) streams.push_back({nullptr, sizes[p]});
+  return streams;
+}
+
+// the workspace a sort_device of these streams needs, whatever tile geometry it picks
+static size_t sort_workspace_bytes(const std::vector<StreamDesc> &streams, int64_t n) {
+  Layout L;
+  // the smallest tile any geometry uses bounds the look-back size from above
+  make_layout(streams, std::max<int64_t>(n, 1), HYB_MIN_TILE, &L);
+  return L.total;
+}
+
+// the stats fields every sort reports: what it sorted, and the kernels launched since `launches_before`
+static b200sort_stats call_stats(int64_t n, const std::vector<StreamDesc> &streams, int kb, uint64_t launches_before) {
+  b200sort_stats s{};
+  s.num = n;
+  for (const StreamDesc &d : streams) s.record_bytes += d.elem_bytes;
+  s.key_bytes = (uint32_t)kb;
+  s.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
+  return s;
 }
 
 // The arrays as the streams the scatter kernel moves: each one in chunks of the largest power of two <= max_chunk
@@ -534,6 +595,7 @@ struct DevSort {
   const DevSortOpts &xo;
   const int kb = key_bytes_of(key_type);
   // set-up
+  uint64_t launches_before = 0;  // the launch counter when the sort started
   int dev = 0, cfg = 0, tile = 0, algo = 0;
   bool hybrid = false;
   DevInfo di;
@@ -573,20 +635,11 @@ struct DevSort {
     if (smem > di.smem_optin) return fail(B200SORT_ECUDA, "device offers %zu B of shared memory, %zu needed", di.smem_optin, smem);
 
     make_layout(streams, std::max(n, xo.layout_n), std::min(tile, HYB_MIN_TILE), &L, xo.layout_landing);
-    void *workspace = caller_workspace;
-    if (workspace == nullptr) {
-      if (int rc = cached_buffer(cache_guard.acquire(dev, stream).workspace, L.total, "workspace", &workspace)) return rc;
-    } else if (workspace_bytes < L.total) {
-      return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", workspace_bytes, L.total);
-    } else if (((uintptr_t)workspace % 256) != 0) {
-      return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
-    }
-    ws = (unsigned char *)workspace;
+    if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, L.total, cache_guard, &ws)) return rc;
     for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
     plan = (Plan *)(ws + L.plan_off);
     ctrl = (HybridCtrl *)(ws + L.hyb_off);
-    g_prof_on = o.profile != 0;
-    if (!xo.forced && !xo.keep_profile) prof_reset();
+    start_profile(o, xo.forced || xo.keep_profile);
     if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
 
     ko = make_key_order(key_type, ascending);
@@ -794,12 +847,7 @@ struct DevSort {
       CUDA_TRY(cudaStreamSynchronize(stream));
       if (fix_flow) finish_ran = hctrl.flags[1] != 0;
     }
-    uint32_t rec_bytes = 0;
-    for (const StreamDesc &s : streams) rec_bytes += s.elem_bytes;
-    *stt = b200sort_stats{};
-    stt->num = n;
-    stt->record_bytes = rec_bytes;
-    stt->key_bytes = (uint32_t)kb;
+    *stt = call_stats(n, streams, kb, launches_before);
     stt->algo = (uint32_t)algo;
     stt->hist_sweeps = hist_sweeps;
     stt->passes_planned = (have_plan || hybrid) ? hplan.n_exec : (uint32_t)kb;  // (otherwise every pass is launched)
@@ -808,7 +856,7 @@ struct DevSort {
       stt->cut_digit = hplan.cut_digit;
       memcpy(&stt->segfix_moved, &hctrl.flags[2], 8);
     }
-    stt->algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)(stt->passes_planned + stt->segfix_passes) * 2ull * (uint64_t)n * rec_bytes;
+    stt->algorithmic_bytes = (uint64_t)hist_sweeps * (uint64_t)n * kb + (uint64_t)(stt->passes_planned + stt->segfix_passes) * 2ull * (uint64_t)n * stt->record_bytes;
     *fall_back = hybrid && hctrl.flags[0] != 0;
     return 0;
   }
@@ -825,12 +873,13 @@ struct DevSort {
     stt->passes_planned += s2.passes_planned;
     stt->hist_sweeps += s2.hist_sweeps;
     stt->algorithmic_bytes += s2.algorithmic_bytes;
+    stt->kernel_launches += s2.kernel_launches;
     return 0;
   }
 
   // the sort, phase by phase; *stats: what ran (written when the sort succeeds)
   int run(b200sort_stats *stats) {
-    const uint64_t launches_before = g_launches.load();
+    launches_before = g_launches.load();
     if (int rc = setup()) return rc;
     if (int rc = make_plan()) return rc;
     if (int rc = run_passes()) return rc;
@@ -840,7 +889,6 @@ struct DevSort {
     if (int rc = statistics(&stt, &fell_back)) return rc;
     if (fell_back)
       if (int rc = fall_back(&stt)) return rc;
-    stt.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
     *stats = stt;
     return B200SORT_OK;
   }
@@ -862,11 +910,11 @@ struct DeviceScope {
   int prev = -1;
   bool switched = false;
   int enter(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) { cudaGetLastError(); return -1; }
-    if (prev != dev) {
-      if (cudaSetDevice(dev) != cudaSuccess) { cudaGetLastError(); return -1; }
-      switched = true;
+    if (cudaGetDevice(&prev) != cudaSuccess || (prev != dev && cudaSetDevice(dev) != cudaSuccess)) {
+      cudaGetLastError();
+      return fail(B200SORT_ECUDA, "cannot make device %d current", dev);
     }
+    switched = prev != dev;
     return 0;
   }
   ~DeviceScope() { if (switched) cudaSetDevice(prev); }
@@ -927,14 +975,13 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
   const cudaStream_t st_in = t.in, st_comp = t.comp, st_out = t.out;
   const size_t np = streams.size() - 1;
   // device staging: keys | index | payload s in | payload s out
-  std::vector<size_t> off_in(np), off_out(np);
+  std::vector<size_t> bytes = {(size_t)n * kb, (size_t)n * 4};
+  for (size_t s = 0; s < np; s++) bytes.insert(bytes.end(), 2, (size_t)n * streams[s + 1].elem_bytes);
   size_t total = 0;
-  const size_t off_keys = total; total = align_up(total + (size_t)n * kb, 256);
-  const size_t off_idx = total;  total = align_up(total + (size_t)n * 4, 256);
-  for (size_t s = 0; s < np; s++) {
-    off_in[s] = total;  total = align_up(total + (size_t)n * streams[s + 1].elem_bytes, 256);
-    off_out[s] = total; total = align_up(total + (size_t)n * streams[s + 1].elem_bytes, 256);
-  }
+  const std::vector<size_t> offs = back_to_back(bytes, &total);
+  const size_t off_keys = offs[0], off_idx = offs[1];
+  auto off_in = [&](size_t s) { return offs[2 + 2 * s]; };
+  auto off_out = [&](size_t s) { return offs[3 + 2 * s]; };
   void *dbuf_v = nullptr;
   if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
   unsigned char *dbuf = (unsigned char *)dbuf_v;
@@ -961,7 +1008,7 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
     std::vector<cudaEvent_t> e_pay(np);
     auto upload_payloads = [&]() -> int {
       for (size_t s = 0; s < np; s++) {
-        CUDA_TRY(cudaMemcpyAsync(dbuf + off_in[s], streams[s + 1].ptr, (size_t)n * streams[s + 1].elem_bytes, cudaMemcpyHostToDevice, st_in));
+        CUDA_TRY(cudaMemcpyAsync(dbuf + off_in(s), streams[s + 1].ptr, (size_t)n * streams[s + 1].elem_bytes, cudaMemcpyHostToDevice, st_in));
         e_pay[s] = new_event();
         CUDA_TRY(cudaEventRecord(e_pay[s], st_in));
       }
@@ -995,14 +1042,14 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
       const unsigned grid = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)di.sm_count * 16);
       auto gather = [&](auto *t) {  // (t: the type of one chunk)
         using T = std::remove_pointer_t<decltype(t)>;
-        return launch(PK_NONE, gather_kernel<T>, grid, 256, 0, st_comp, idx, (const T *)(dbuf + off_in[s]), (T *)(dbuf + off_out[s]), n, cpe);
+        return launch(PK_NONE, gather_kernel<T>, grid, 256, 0, st_comp, idx, (const T *)(dbuf + off_in(s)), (T *)(dbuf + off_out(s)), n, cpe);
       };
       CUDA_TRY(ck == 16 ? gather((uint4 *)nullptr) : ck == 8 ? gather((uint64_t *)nullptr) : ck == 4 ? gather((uint32_t *)nullptr)
                : ck == 2 ? gather((uint16_t *)nullptr) : gather((uint8_t *)nullptr));
       cudaEvent_t e_g = new_event();
       CUDA_TRY(cudaEventRecord(e_g, st_comp));
       CUDA_TRY(cudaStreamWaitEvent(st_out, e_g, 0));
-      CUDA_TRY(cudaMemcpyAsync(streams[s + 1].ptr, dbuf + off_out[s], (size_t)n * eb, cudaMemcpyDeviceToHost, st_out));
+      CUDA_TRY(cudaMemcpyAsync(streams[s + 1].ptr, dbuf + off_out(s), (size_t)n * eb, cudaMemcpyDeviceToHost, st_out));
     }
     return 0;
   };
@@ -1016,8 +1063,8 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
   return rc;
 }
 
-// where the arrays of one call live: all in host memory, or all on one device (*dev); fails without a device
-static int arrays_side(const std::vector<StreamDesc> &streams, Side *side, int *dev) {
+// fails unless a CUDA device is usable
+static int require_device() {
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0) {
@@ -1025,6 +1072,13 @@ static int arrays_side(const std::vector<StreamDesc> &streams, Side *side, int *
     return fail(B200SORT_ECUDA, "no CUDA device available (%s); libb200sort has no CPU fallback",
                 e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
   }
+  return 0;
+}
+
+// where the arrays of one call, and the offsets of a segmented sort (NULL for none), live: all in host memory, or all
+// on one device (*dev); fails without a device
+static int arrays_side(const std::vector<StreamDesc> &streams, const int64_t *offsets, Side *side, int *dev) {
+  if (int rc = require_device()) return rc;
   if (int rc = side_of(streams[0].ptr, side, dev)) return rc;
   for (size_t s = 1; s < streams.size(); s++) {
     Side sd;
@@ -1033,7 +1087,47 @@ static int arrays_side(const std::vector<StreamDesc> &streams, Side *side, int *
     if (sd != *side) return fail(B200SORT_EINVAL, "arrays must be all in host memory or all in device memory");
     if (sd == SIDE_DEVICE && dv != *dev) return fail(B200SORT_EINVAL, "device arrays live on different devices (%d and %d)", *dev, dv);
   }
+  if (offsets != nullptr) {
+    Side sd;
+    int dv = 0;
+    if (int rc = side_of(offsets, &sd, &dv)) return rc;
+    if (sd != *side || (sd == SIDE_DEVICE && dv != *dev))
+      return fail(B200SORT_EINVAL, "offsets must live where the arrays do (host memory, or the arrays' device)");
+  }
   return 0;
+}
+
+// Host arrays sorted whole on the current device: the arrays, and `upload_bytes` at `upload` (NULL for none) that the
+// sort only reads, copied up into the staging buffer (cache entry `stage`, whose guard the caller holds);
+// sort(the arrays' device streams, the device copy of `upload`); the arrays copied back unless it failed.  Returns
+// when they are back.
+template <typename SortFn>
+static int sort_staged(CacheEntry &stage, int64_t n, const std::vector<StreamDesc> &streams, const void *upload, size_t upload_bytes,
+                       cudaStream_t stream, SortFn &&sort) {
+  std::vector<size_t> bytes;
+  for (const StreamDesc &s : streams) bytes.push_back((size_t)n * s.elem_bytes);
+  if (upload != nullptr) bytes.push_back(upload_bytes);
+  size_t total = 0;
+  const std::vector<size_t> offs = back_to_back(bytes, &total);
+  void *dbuf_v = nullptr;
+  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
+  unsigned char *dbuf = (unsigned char *)dbuf_v;
+  std::vector<StreamDesc> dstreams(streams.size());
+  for (size_t s = 0; s < streams.size(); s++) dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
+  int rc = B200SORT_OK;
+  cudaError_t e = cudaSuccess;
+  for (size_t i = 0; i < bytes.size() && rc == 0; i++) {
+    e = cudaMemcpyAsync(dbuf + offs[i], i < streams.size() ? streams[i].ptr : upload, bytes[i], cudaMemcpyHostToDevice, stream);
+    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "H2D copy failed: %s", cudaGetErrorString(e));
+  }
+  if (rc == 0) rc = sort(dstreams, upload != nullptr ? dbuf + offs.back() : nullptr);
+  for (size_t s = 0; s < streams.size() && rc == 0; s++) {
+    e = cudaMemcpyAsync(streams[s].ptr, dstreams[s].ptr, bytes[s], cudaMemcpyDeviceToHost, stream);
+    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "D2H copy failed: %s", cudaGetErrorString(e));
+  }
+  e = cudaStreamSynchronize(stream);
+  if (e != cudaSuccess && rc == 0) rc = fail(B200SORT_ECUDA, "sort failed on the device: %s", cudaGetErrorString(e));
+  return rc;
 }
 
 static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
@@ -1042,10 +1136,10 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
   if (n <= 1) return B200SORT_OK;  // src/radix_sort.hpp:276: nothing to do for 0 or 1 element
   Side side0;
   int dev0 = 0;
-  if (int rc = arrays_side(streams, &side0, &dev0)) return rc;
+  if (int rc = arrays_side(streams, nullptr, &side0, &dev0)) return rc;
   if (side0 == SIDE_DEVICE) {
     DeviceScope scope;  // sort on the device that owns the arrays (include/b200sort.h)
-    if (scope.enter(dev0) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", dev0);
+    if (int rc = scope.enter(dev0)) return rc;
     return sort_device(o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, base, stats);
   }
 
@@ -1066,31 +1160,9 @@ static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, c
     cudaGetLastError();
   }
   // everything else: the whole arrays up, the sort, the whole arrays down
-  std::vector<StreamDesc> dstreams(streams.size());
-  size_t total = 0;
-  std::vector<size_t> offs(streams.size());
-  for (size_t s = 0; s < streams.size(); s++) {
-    offs[s] = total;
-    total = align_up(total + (size_t)n * streams[s].elem_bytes, 256);
-  }
-  void *dbuf_v = nullptr;
-  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
-  unsigned char *dbuf = (unsigned char *)dbuf_v;
-  int rc = B200SORT_OK;
-  cudaError_t e = cudaSuccess;
-  for (size_t s = 0; s < streams.size() && rc == 0; s++) {
-    dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
-    e = cudaMemcpyAsync(dstreams[s].ptr, streams[s].ptr, (size_t)n * streams[s].elem_bytes, cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-  }
-  if (rc == 0) rc = sort_device(o, key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base, stats);
-  for (size_t s = 0; s < streams.size() && rc == 0; s++) {
-    e = cudaMemcpyAsync(streams[s].ptr, dstreams[s].ptr, (size_t)n * streams[s].elem_bytes, cudaMemcpyDeviceToHost, stream);
-    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "D2H copy failed: %s", cudaGetErrorString(e));
-  }
-  e = cudaStreamSynchronize(stream);
-  if (e != cudaSuccess && rc == 0) rc = fail(B200SORT_ECUDA, "sort failed on the device: %s", cudaGetErrorString(e));
-  return rc;
+  return sort_staged(stage, n, streams, nullptr, 0, stream, [&](const std::vector<StreamDesc> &dstreams, const void *) {
+    return sort_device(o, key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base, stats);
+  });
 }
 
 static int check_soa(void *keys, int key_type, int64_t num, int n_payloads, void *const *payloads,
@@ -1122,6 +1194,16 @@ static int check_aos(void *records, int key_type, uint32_t record_bytes, int64_t
   return 0;
 }
 
+// the options of the _ex calls' comparison sorter.  CmpSorterInsertionSort: the full sort whatever the threshold.
+// CmpSorterNoSort: buckets of at most cmp_sort_threshold elements may stay unordered (src/radix_sort.hpp:279,
+// src/cmp_sorters.hpp:66-78).
+static int cmp_sorter_opts(int64_t cmp_sort_threshold, int cmp_sorter, DevSortOpts *out) {
+  if (cmp_sorter != B200SORT_CMP_INSERTION && cmp_sorter != B200SORT_CMP_NONE)
+    return fail(B200SORT_EINVAL, "unknown cmp_sorter %d", cmp_sorter);
+  if (cmp_sorter == B200SORT_CMP_NONE && cmp_sort_threshold >= CMP_NONE_MIN_THRESH) out->cmp_none_thresh = cmp_sort_threshold;
+  return 0;
+}
+
 }  // namespace b200sort
 
 using namespace b200sort;
@@ -1131,12 +1213,8 @@ extern "C" {
 int b200sort_sort_soa_ex(void *keys, int key_type, int64_t num, int ascending, int n_payloads, void *const *payloads,
                          const uint32_t *payload_elem_bytes, int64_t cmp_sort_threshold, int cmp_sorter, void *stream,
                          void *workspace, size_t workspace_bytes) {
-  if (cmp_sorter != B200SORT_CMP_INSERTION && cmp_sorter != B200SORT_CMP_NONE)
-    return fail(B200SORT_EINVAL, "unknown cmp_sorter %d", cmp_sorter);
-  // CmpSorterInsertionSort: the full sort whatever the threshold.  CmpSorterNoSort: buckets of at most
-  // cmp_sort_threshold elements may stay unordered (src/radix_sort.hpp:279, src/cmp_sorters.hpp:66-78).
   DevSortOpts base;
-  if (cmp_sorter == B200SORT_CMP_NONE && cmp_sort_threshold >= CMP_NONE_MIN_THRESH) base.cmp_none_thresh = cmp_sort_threshold;
+  if (int rc = cmp_sorter_opts(cmp_sort_threshold, cmp_sorter, &base)) return rc;
   std::vector<StreamDesc> streams;
   if (int rc = check_soa(keys, key_type, num, n_payloads, payloads, payload_elem_bytes, &streams)) return rc;
   return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
@@ -1145,10 +1223,8 @@ int b200sort_sort_soa_ex(void *keys, int key_type, int64_t num, int ascending, i
 int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int64_t num, int ascending,
                          int64_t cmp_sort_threshold, int cmp_sorter, void *stream, void *workspace,
                          size_t workspace_bytes) {
-  if (cmp_sorter != B200SORT_CMP_INSERTION && cmp_sorter != B200SORT_CMP_NONE)
-    return fail(B200SORT_EINVAL, "unknown cmp_sorter %d", cmp_sorter);
   DevSortOpts base;
-  if (cmp_sorter == B200SORT_CMP_NONE && cmp_sort_threshold >= CMP_NONE_MIN_THRESH) base.cmp_none_thresh = cmp_sort_threshold;
+  if (int rc = cmp_sorter_opts(cmp_sort_threshold, cmp_sorter, &base)) return rc;
   std::vector<StreamDesc> streams;
   if (int rc = check_aos(records, key_type, record_bytes, num, &streams)) return rc;
   return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
@@ -1170,17 +1246,7 @@ size_t b200sort_workspace_bytes(int key_type, int64_t num, int n_payloads, const
                                 uint32_t record_bytes) {
   const int kb = key_bytes_of(key_type);
   if (kb == 0 || num < 0) return 0;
-  std::vector<StreamDesc> streams;
-  if (record_bytes) {
-    streams.push_back({nullptr, record_bytes});
-  } else {
-    streams.push_back({nullptr, (uint32_t)kb});
-    for (int p = 0; p < n_payloads; p++) streams.push_back({nullptr, payload_elem_bytes[p]});
-  }
-  Layout L;
-  // the smallest tile any geometry uses bounds the look-back size from above
-  make_layout(streams, std::max<int64_t>(num, 1), HYB_MIN_TILE, &L);
-  return L.total;
+  return sort_workspace_bytes(streams_of_shape(kb, n_payloads, payload_elem_bytes, record_bytes), num);
 }
 
 const char *b200sort_last_error(void) { return g_last_error.c_str(); }

@@ -1448,7 +1448,7 @@ struct MgpuSort {
 static int mgpu_sort(const Options &o, b200sort_comm *c, int key_type, const std::vector<StreamDesc> &streams, int64_t num_local,
                      int64_t capacity, bool ascending, int64_t *out_num_local, cudaStream_t stream, b200sort_stats *stats) {
   DeviceScope dev_scope;  // the communicator's device, whatever the caller's current device is
-  if (dev_scope.enter(c->dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", c->dev);
+  if (int rc = dev_scope.enter(c->dev)) return rc;
   MgpuSort s{o, c, nccl_api(), key_type, streams, num_local, capacity, ascending, stream, stats};
   c->seq++;
   c->last_overlap = false;

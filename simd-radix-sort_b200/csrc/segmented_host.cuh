@@ -11,13 +11,6 @@ struct SegLayout {
   size_t comp_off, sort_off;  // (inside the region) composite keys, whole-array sort workspace
 };
 
-// the workspace a sort_device of these streams needs (what b200sort_workspace_bytes computes)
-static size_t sort_workspace_bytes(const std::vector<StreamDesc> &streams, int64_t n) {
-  Layout L;
-  make_layout(streams, std::max<int64_t>(n, 1), HYB_MIN_TILE, &L);
-  return L.total;
-}
-
 static SegLayout seg_layout(int kb, int64_t num, int64_t n_segments, const std::vector<StreamDesc> &streams, bool soa) {
   SegLayout s{};
   const int64_t cap = (int64_t)1 << seg_cap_log2(kb);
@@ -82,17 +75,9 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
   if (((uintptr_t)streams[0].ptr % kb) != 0) return fail(B200SORT_EINVAL, "key array is not aligned to its key type");
   const SegLayout sl = seg_layout(kb, num, n_segments, streams, soa);
   CacheGuard cache_guard;
-  void *workspace = caller_workspace;
-  if (workspace == nullptr) {
-    if (int rc = cached_buffer(cache_guard.acquire(dev, stream).workspace, sl.total, "workspace", &workspace)) return rc;
-  } else if (workspace_bytes < sl.total) {
-    return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", workspace_bytes, sl.total);
-  } else if (((uintptr_t)workspace % 256) != 0) {
-    return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
-  }
-  unsigned char *ws = (unsigned char *)workspace;
-  g_prof_on = o.profile != 0;
-  prof_reset();
+  unsigned char *ws = nullptr;
+  if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, sl.total, cache_guard, &ws)) return rc;
+  start_profile(o, false);
 
   // classify (one host wait: the bin counts, the validity flag, the longest segment)
   const int cap_log2 = seg_cap_log2(kb);
@@ -156,25 +141,15 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
       CUDA_TRY(seg_launch_bin(kb, b, sa, di.sm_count, stream));
     }
   }
-  uint32_t rec_bytes = 0;
-  for (const StreamDesc &s : streams) rec_bytes += s.elem_bytes;
-  *stats = b200sort_stats{};
-  stats->num = num;
-  stats->record_bytes = rec_bytes;
-  stats->key_bytes = (uint32_t)kb;
+  *stats = call_stats(num, streams, kb, launches_before);
   stats->algo = 3;
-  stats->kernel_launches = (uint32_t)(g_launches.load() - launches_before);
   return B200SORT_OK;
 }
 
 // num <= 1: no segment has two records, but invalid offsets are still an error.  The offsets are checked on the
 // host (device offsets are copied there first: the arrays may be empty, so there is nothing to sort on the device).
 static int check_offsets_only(int64_t num, int64_t n_segments, const int64_t *offsets, cudaStream_t stream) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    return fail(B200SORT_ECUDA, "no CUDA device available; libb200sort has no CPU fallback");
-  }
+  if (int rc = require_device()) return rc;
   Side side;
   int dev = 0;
   if (int rc = side_of(offsets, &side, &dev)) return rc;
@@ -182,7 +157,7 @@ static int check_offsets_only(int64_t num, int64_t n_segments, const int64_t *of
   const int64_t *v = offsets;
   if (side == SIDE_DEVICE) {
     DeviceScope scope;
-    if (scope.enter(dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", dev);
+    if (int rc = scope.enter(dev)) return rc;
     h.resize((size_t)n_segments + 1);
     CUDA_TRY(cudaMemcpyAsync(h.data(), offsets, h.size() * 8, cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
@@ -204,55 +179,21 @@ static int sort_segmented_any(int key_type, bool ascending, int64_t num, int64_t
   const Options o = options();
   Side side;
   int dev = 0;
-  if (int rc = arrays_side(streams, &side, &dev)) return rc;
-  Side oside;
-  int odev = 0;
-  if (int rc = side_of(offsets, &oside, &odev)) return rc;
-  if (oside != side || (side == SIDE_DEVICE && odev != dev))
-    return fail(B200SORT_EINVAL, "offsets must live where the arrays do (host memory, or the arrays' device)");
+  if (int rc = arrays_side(streams, offsets, &side, &dev)) return rc;
   if (side == SIDE_DEVICE) {
     DeviceScope scope;
-    if (scope.enter(dev) != 0) return fail(B200SORT_ECUDA, "cannot make device %d current", dev);
+    if (int rc = scope.enter(dev)) return rc;
     return sort_segmented_device(o, key_type, ascending, num, n_segments, offsets, streams, soa, stream, workspace, workspace_bytes,
                                  &g_last_stats);
   }
   // host arrays: the whole arrays and the offsets up, the sort, the arrays down (not when it failed)
   CUDA_TRY(cudaGetDevice(&dev));
   CacheGuard cache_guard;
-  CacheEntry &stage = cache_guard.acquire(dev, stream).stage;
-  std::vector<size_t> offs(streams.size());
-  size_t total = 0;
-  for (size_t s = 0; s < streams.size(); s++) {
-    offs[s] = total;
-    total = align_up(total + (size_t)num * streams[s].elem_bytes, 256);
-  }
-  const size_t off_offsets = total;
-  total += (size_t)(n_segments + 1) * 8;
-  void *dbuf_v = nullptr;
-  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
-  unsigned char *dbuf = (unsigned char *)dbuf_v;
-  std::vector<StreamDesc> dstreams(streams.size());
-  int rc = B200SORT_OK;
-  cudaError_t e = cudaSuccess;
-  for (size_t s = 0; s < streams.size() && rc == 0; s++) {
-    dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
-    e = cudaMemcpyAsync(dstreams[s].ptr, streams[s].ptr, (size_t)num * streams[s].elem_bytes, cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-  }
-  if (rc == 0) {
-    e = cudaMemcpyAsync(dbuf + off_offsets, offsets, (size_t)(n_segments + 1) * 8, cudaMemcpyHostToDevice, stream);
-    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-  }
-  if (rc == 0)
-    rc = sort_segmented_device(o, key_type, ascending, num, n_segments, (const int64_t *)(dbuf + off_offsets), dstreams, soa, stream,
-                               workspace, workspace_bytes, &g_last_stats);
-  for (size_t s = 0; s < streams.size() && rc == 0; s++) {
-    e = cudaMemcpyAsync(streams[s].ptr, dstreams[s].ptr, (size_t)num * streams[s].elem_bytes, cudaMemcpyDeviceToHost, stream);
-    if (e != cudaSuccess) rc = fail(B200SORT_ECUDA, "D2H copy failed: %s", cudaGetErrorString(e));
-  }
-  e = cudaStreamSynchronize(stream);
-  if (e != cudaSuccess && rc == 0) rc = fail(B200SORT_ECUDA, "segmented sort failed on the device: %s", cudaGetErrorString(e));
-  return rc;
+  return sort_staged(cache_guard.acquire(dev, stream).stage, num, streams, offsets, (size_t)(n_segments + 1) * 8, stream,
+                     [&](const std::vector<StreamDesc> &dstreams, const void *doffsets) {
+                       return sort_segmented_device(o, key_type, ascending, num, n_segments, (const int64_t *)doffsets, dstreams, soa,
+                                                    stream, workspace, workspace_bytes, &g_last_stats);
+                     });
 }
 
 }  // namespace b200sort
@@ -278,14 +219,7 @@ size_t b200sort_segmented_workspace_bytes(int key_type, int64_t num, int64_t n_s
                                           uint32_t record_bytes) {
   const int kb = key_bytes_of(key_type);
   if (kb == 0 || num < 0 || n_segments < 0) return 0;
-  std::vector<StreamDesc> streams;
-  if (record_bytes) {
-    streams.push_back({nullptr, record_bytes});
-  } else {
-    streams.push_back({nullptr, (uint32_t)kb});
-    for (int p = 0; p < n_payloads; p++) streams.push_back({nullptr, payload_elem_bytes[p]});
-  }
-  return seg_layout(kb, num, n_segments, streams, record_bytes == 0).total;
+  return seg_layout(kb, num, n_segments, streams_of_shape(kb, n_payloads, payload_elem_bytes, record_bytes), record_bytes == 0).total;
 }
 
 }  // extern "C"

@@ -317,7 +317,7 @@ def test_last_pass_window_at_tile_edges_with_32_bit_cut(up):
 def test_caller_workspace_and_stats():
     n = 200_000
     keys = O.make_keys("Uniform", np.int64, n, seed=5)
-    ws = torch.empty(S.workspace_bytes(np.int64, n, [8]) + 256, dtype=torch.uint8, device="cuda")
+    ws = torch.empty(S.workspace_bytes(np.int64, n, [8]) + 512, dtype=torch.uint8, device="cuda")
     off = (-ws.data_ptr()) % 256
     k, p = dev(keys), dev(np.arange(n, dtype=np.int64))
     S.sort(n, k, p, up=False, workspace=ws[off:])
@@ -328,6 +328,12 @@ def test_caller_workspace_and_stats():
     with pytest.raises(S.B200SortError) as ei:
         S.sort(n, k, p, workspace=small)
     assert ei.value.code == -4
+    # big enough, but 128 bytes past a 256-byte boundary: rejected, nothing moves
+    k0, p0 = host(k), host(p)
+    with pytest.raises(S.B200SortError) as ei:
+        S.sort(n, k, p, workspace=ws[off + 128:])
+    assert ei.value.code == -1
+    assert host(k).tobytes() == k0.tobytes() and host(p).tobytes() == p0.tobytes()
 
 
 # ------------------------------------------------------------------------------------------------

@@ -410,6 +410,14 @@ def test_caller_workspace(dt):
     with pytest.raises(S.B200SortError) as ei:
         run_soa(keys, [pay], offsets, workspace=short)
     assert ei.value.code == -4
+    # big enough, but 128 bytes past a 256-byte boundary: rejected, nothing moves
+    big = torch.empty(need + 512, dtype=torch.uint8, device="cuda")
+    off = (-big.data_ptr()) % 256 + 128
+    k, p, o = dev(keys), dev(pay), dev(offsets)
+    with pytest.raises(S.B200SortError) as ei:
+        S.sort_segmented(o, k, p, workspace=big[off:])
+    assert ei.value.code == -1
+    assert k.cpu().numpy().tobytes() == keys.tobytes() and p.cpu().numpy().tobytes() == pay.tobytes()
 
 
 def test_back_to_back_on_a_non_default_stream():
