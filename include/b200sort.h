@@ -13,7 +13,8 @@
  *  - plain pointers and sizes only; no C++/torch types.
  *  - every array may live in HOST memory (sorted through a staged copy on the current CUDA device) or
  *    in DEVICE memory (sorted in place on the device that owns it: the fast path).  All arrays of
- *    one call must be on the same side.
+ *    one call must be on the same side.  The one exception is the top-k selection, which takes device arrays only
+ *    (B200SORT_EUNSUPPORTED otherwise): staging a whole row over PCIe to return k records of it is the wrong tool.
  *  - the sort is in place from the caller's point of view (reference: radix_sort.hpp:297-337): the
  *    result overwrites keys/payloads/records.  Scratch (one shadow copy of every stream + per-tile
  *    status words) comes from `workspace` or, when that is NULL, from a per-device cache owned by
@@ -33,6 +34,8 @@
  *        on the device, so that only the passes that execute are launched.
  *      * a segmented sort: one wait for the segment classification, two with 8-byte keys and a segment
  *        longer than 8192 records, plus the waits above of the whole-array sorts it runs for long segments.
+ *      * a top-k: the selection waits for nothing; its ordering step is a segmented sort of n_rows segments of
+ *        k records and adds that sort's waits (one; more with 8-byte keys and k > 8192; none when k = 1).
  *    These calls therefore cannot be captured into a CUDA graph; everything between the two waits
  *    (all passes, the junction kernel, the flag-gated segment finish / copy-back) is queued without one.
  *  - device arrays are sorted on the device that owns them, whatever the caller's current device is;
@@ -140,6 +143,48 @@ int b200sort_sort_segmented_aos(void *records, int key_type, uint32_t record_byt
 size_t b200sort_segmented_workspace_bytes(int key_type, int64_t num, int64_t n_segments, int n_payloads,
                                           const uint32_t *payload_elem_bytes, uint32_t record_bytes);
 
+/* ---- top-k selection: the k smallest or largest records of every row -------------------------------------------
+ * (An extension: the reference has no counterpart.)
+ *  - Input: n_rows contiguous rows of row_len records (a whole array is n_rows = 1).  Payload streams have one
+ *    element per record, as in b200sort_sort_soa; AoS records follow the rules of b200sort_sort_aos.  The inputs are
+ *    only read.
+ *  - Result: row r of every output holds k records.  out_keys[r k + j] equals, byte for byte, the j-th key of row r
+ *    after b200sort_sort_soa(row r, ascending = !largest): largest = 1 gives the k largest in descending order (like
+ *    torch.topk(sorted=True)), largest = 0 the k smallest in ascending order, in the total order on bit patterns
+ *    (-NaN < -inf < ... < -0.0 < +0.0 < ... < +inf < +NaN).  out_index[r k + j] (int64, required) is the record's
+ *    position inside its row; the indices of a row are distinct, keys[r row_len + out_index[r k + j]] equals
+ *    out_keys[r k + j], and every output payload element (or AoS record) is the input's element at that position.
+ *    When equal keys straddle the k-th place, which of them are chosen is unspecified.
+ *  - Errors, checked before any device work: B200SORT_EINVAL for a negative n_rows, row_len or k, k > row_len,
+ *    n_rows > 2^31 - 1, an n_rows * row_len that overflows, a NULL input, output or out_index when k > 0, a key
+ *    array, key output or record array not aligned to the key type, out_index not 8-byte aligned, and an output
+ *    whose address range overlaps an input's.  Payload shapes (up to 63 streams) and record sizes are checked as for
+ *    the sort (B200SORT_ESHAPE / B200SORT_ERECORD).  k == 0 or n_rows == 0 is a no-op that returns 0.
+ *  - Memory side: device arrays only, all on one device (the call runs on it); an array in host memory gives
+ *    B200SORT_EUNSUPPORTED.
+ *  - Workspace: NULL (the library's per-device cache) or a 256-byte aligned buffer of at least
+ *    b200sort_topk_workspace_bytes(...) bytes, which covers any key distribution.  All work is ordered on `stream`;
+ *    host waits: see the conventions above.
+ *  - Method: radix select on 8-bit digits of the order-mapped key, most significant first: key-width + 1 passes of
+ *    one fused kernel (select below the threshold's bucket, keep the candidates equal to it, count their next
+ *    digit), each followed but the last by a decision kernel.  Each row has two candidate buffers of
+ *    ceil(row_len / 16) entries; candidates that do not fit are found again by re-reading the row.  Uniform keys cost
+ *    about two reads of the keys, adversarial ones (all equal, a constant top byte) at most key-width + 1.  The k
+ *    winners of every row are then ordered by the segmented sort, and one gather moves the payloads / records.
+ *  - b200sort_last_stats afterwards: algo = 4, num = n_rows * row_len, record_bytes, key_bytes and kernel_launches;
+ *    every other field 0.  No tuning option applies. */
+int b200sort_topk_soa(const void *keys, int key_type, int64_t n_rows, int64_t row_len, int64_t k, int largest,
+                      int n_payloads, const void *const *payloads, const uint32_t *payload_elem_bytes,
+                      void *out_keys, int64_t *out_index, void *const *out_payloads,
+                      void *stream, void *workspace, size_t workspace_bytes);
+int b200sort_topk_aos(const void *records, int key_type, uint32_t record_bytes, int64_t n_rows, int64_t row_len,
+                      int64_t k, int largest, void *out_records, int64_t *out_index,
+                      void *stream, void *workspace, size_t workspace_bytes);
+/* Bytes of device scratch a top-k call with these shapes needs (record_bytes = 0 for the SoA form); 0 for an unknown
+ * key type or invalid counts. */
+size_t b200sort_topk_workspace_bytes(int key_type, int64_t n_rows, int64_t row_len, int64_t k, int n_payloads,
+                                     const uint32_t *payload_elem_bytes, uint32_t record_bytes);
+
 /* Thread-local message of the last failing call on this thread ("" if none). */
 const char *b200sort_last_error(void);
 
@@ -161,8 +206,8 @@ typedef struct b200sort_stats {
   int64_t num;
   uint32_t record_bytes;      /* sum of all stream element sizes */
   uint32_t key_bytes;
-  uint32_t algo;              /* 1 LSD, 2 hybrid, 3 segmented sort (then only num, record_bytes, key_bytes and
-                                 kernel_launches are set) */
+  uint32_t algo;              /* 1 LSD, 2 hybrid, 3 segmented sort, 4 top-k (3 and 4: only num, record_bytes,
+                                 key_bytes and kernel_launches are set) */
   uint32_t passes_planned;    /* scatter passes executed (hybrid) / launched (LSD; constant digits return at once) */
   uint32_t hist_sweeps;       /* key-only sweeps launched */
   uint32_t kernel_launches;   /* kernels launched by this call */
@@ -176,7 +221,7 @@ int b200sort_last_stats(b200sort_stats *out);
 
 /* Per-kernel device times of the last sort on this thread, recorded with CUDA events on the sort's
  * stream when option "profile" is 1.  kinds[i]: 0 histogram, 1 scan, 2 scatter pass, 3 copy-back,
- * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments.  Returns the number of entries written (<= capacity) or a negative code. */
+ * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments, 7 top-k selection and gather.  Returns the number of entries written (<= capacity) or a negative code. */
 int b200sort_last_profile(int *kinds, float *ms, int capacity);
 
 /* Releases the per-device workspace and host-staging buffers held by the library.  A sort another thread

@@ -11,14 +11,19 @@ and, as an extension without a counterpart there, segmented sorts of many indepe
     sort_segmented_combined(offsets, records, key_dtype, up=True)
     sort_rows(keys, *payloads, up=True)              <- every row of a (B, L) array, like torch.sort(dim=-1)
 
-Both sort IN PLACE, like the reference, and go through the C ABI of include/b200sort.h
+and a top-k selection that returns new arrays (device arrays only):
+
+    topk(keys, k, *payloads, largest=True)           <- the k largest / smallest of a row or of every row, like torch.topk
+    topk_combined(records, key_dtype, k, largest=True)
+
+The sorts work IN PLACE, like the reference, and go through the C ABI of include/b200sort.h
 (libb200sort.so, hand-written CUDA for sm_100a).  There is no CPU implementation in this package:
 if the library is missing or no CUDA device is usable the calls raise.
 """
 from ._api import (B200SortError, KEY_TYPES, last_profile, last_stats, launch_count, lib, lib_path, options, set_option, get_option,
-                   segmented_workspace_bytes, sort, sort_combined, sort_rows, sort_segmented, sort_segmented_combined, workspace_bytes,
-                   version)
+                   segmented_workspace_bytes, sort, sort_combined, sort_rows, sort_segmented, sort_segmented_combined, topk, topk_combined,
+                   topk_workspace_bytes, workspace_bytes, version)
 
 __all__ = ["B200SortError", "KEY_TYPES", "last_profile", "last_stats", "launch_count", "lib", "lib_path", "options", "set_option",
            "get_option", "segmented_workspace_bytes", "sort", "sort_combined", "sort_rows", "sort_segmented", "sort_segmented_combined",
-           "workspace_bytes", "version"]
+           "topk", "topk_combined", "topk_workspace_bytes", "workspace_bytes", "version"]

@@ -65,6 +65,12 @@ def lib():
         L.b200sort_sort_segmented_aos.restype = i32
         L.b200sort_segmented_workspace_bytes.argtypes = [i32, i64, i64, i32, u32p, u32]
         L.b200sort_segmented_workspace_bytes.restype = sz
+        L.b200sort_topk_soa.argtypes = [vp, i32, i64, i64, i64, i32, i32, vpp, u32p, vp, vp, vpp, vp, vp, sz]
+        L.b200sort_topk_soa.restype = i32
+        L.b200sort_topk_aos.argtypes = [vp, i32, u32, i64, i64, i64, i32, vp, vp, vp, vp, sz]
+        L.b200sort_topk_aos.restype = i32
+        L.b200sort_topk_workspace_bytes.argtypes = [i32, i64, i64, i64, i32, u32p, u32]
+        L.b200sort_topk_workspace_bytes.restype = sz
         L.b200sort_last_error.restype = ctypes.c_char_p
         L.b200sort_version.restype = i32
         L.b200sort_launch_count.restype = ctypes.c_uint64
@@ -146,7 +152,7 @@ def last_stats() -> dict:
     return {f: getattr(s, f) for f, _ in _Stats._fields_}
 
 
-PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other", "segment"]
+PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other", "segment", "select"]
 
 
 def last_profile():
@@ -336,3 +342,104 @@ def sort_rows(keys, *payloads, up: bool = True, stream=None):
     else:
         offsets = np.arange(B + 1, dtype=np.int64) * L
     sort_segmented(offsets, flat(keys), *[flat(p) for p in payloads], up=up, stream=stream)
+
+
+def _empty(like, shape, dtype=None):
+    """a new array of `shape` where `like` lives (a torch tensor on its device, or a numpy array); `like`'s dtype unless given"""
+    if _is_torch(like):
+        import torch
+        return torch.empty(shape, dtype=like.dtype if dtype is None else dtype, device=like.device)
+    return np.empty(shape, dtype=like.dtype if dtype is None else dtype)
+
+
+def _index_dtype(like):
+    if _is_torch(like):
+        import torch
+        return torch.int64
+    return np.int64
+
+
+def _itemsize(x) -> int:
+    return x.element_size() if _is_torch(x) else x.dtype.itemsize
+
+
+def _on_stream(like, stream, fn):
+    """fn() with a given CUDA `stream` current, so that the arrays fn allocates belong to the stream the call runs on"""
+    if stream is not None and _is_torch(like) and like.is_cuda:
+        import torch
+        with torch.cuda.stream(torch.cuda.ExternalStream(int(stream), device=like.device)):
+            return fn()
+    return fn()
+
+
+def _topk_shape(lead, k):
+    """-> (n_rows, row_len) of keys of shape `lead` (1-D: one row; 2-D: (B, L)); k must be in [0, L]"""
+    if len(lead) not in (1, 2):
+        raise ValueError("keys must be 1-D (one row) or 2-D (B, L)")
+    n_rows, row_len = (1, lead[0]) if len(lead) == 1 else lead
+    if not 0 <= k <= row_len:
+        raise ValueError(f"k = {k} is not in [0, {row_len}]")
+    return n_rows, row_len
+
+
+def topk(keys, k: int, *payloads, largest: bool = True, stream=None, workspace=None):
+    """The k largest (or smallest) keys of a 1-D array, or of every row of a 2-D (B, L) one, like torch.topk(dim=-1):
+    -> (values, indices, *payload outputs), new arrays of shape (..., k) (plus each payload's trailing dimensions)
+    where the keys are (b200sort_topk_soa).
+
+    values are in descending order for largest=True and ascending otherwise, in the library's total order of bit
+    patterns; indices are int64 positions inside the row; every payload's leading dimensions equal the keys' shape,
+    and its output holds the elements at the selected positions.  The keys must be on a CUDA device: host arrays
+    raise B200SortError with code -7."""
+    kaddr, kname, _, _, _ = _describe(keys)
+    lead, k = tuple(int(d) for d in keys.shape), int(k)
+    n_rows, row_len = _topk_shape(lead, k)
+    for i, p in enumerate(payloads):
+        if tuple(p.shape[:len(lead)]) != lead:
+            raise ValueError(f"payload {i} does not have the keys' leading shape {lead}")
+    code = _key_code(kname)
+    out_shape = lead[:-1] + (k,)
+    sizes = (ctypes.c_uint32 * max(len(payloads), 1))()
+    ptrs = (ctypes.c_void_p * max(len(payloads), 1))()
+    for i, p in enumerate(payloads):
+        ptrs[i] = _describe(p)[0]
+        sizes[i] = _itemsize(p) * int(np.prod(p.shape[len(lead):], dtype=np.int64))
+
+    def run():
+        values, indices = _empty(keys, out_shape), _empty(keys, out_shape, _index_dtype(keys))
+        outs = [_empty(p, out_shape + tuple(p.shape[len(lead):])) for p in payloads]
+        out_ptrs = (ctypes.c_void_p * max(len(outs), 1))(*[_describe(o)[0] for o in outs])
+        _call(lib().b200sort_topk_soa, (keys,) + payloads, stream, workspace, kaddr, code, n_rows, row_len, k, int(largest),
+              len(payloads), ptrs, sizes, _describe(values)[0], _describe(indices)[0], out_ptrs)
+        return (values, indices, *outs)
+
+    return _on_stream(keys, stream, run)
+
+
+def topk_combined(records, key_dtype, k: int, largest: bool = True, stream=None, workspace=None):
+    """topk for combined records (b200sort_topk_aos): `records` is (L, R) for one row or (B, L, R) for rows, whose last
+    dimension holds the record's bytes (a power of two, key of `key_dtype` at byte offset 0).  -> (records_out,
+    indices) of shapes (..., k, R) and (..., k)."""
+    addr, _, _, _, _ = _describe(records)
+    if records.ndim not in (2, 3):
+        raise ValueError("records must be (L, R) or (B, L, R)")
+    lead, k = tuple(int(d) for d in records.shape[:-1]), int(k)
+    n_rows, row_len = _topk_shape(lead, k)
+    record_bytes = _itemsize(records) * int(records.shape[-1])
+    code = _key_code(key_dtype)
+
+    def run():
+        out = _empty(records, lead[:-1] + (k, int(records.shape[-1])))
+        indices = _empty(records, lead[:-1] + (k,), _index_dtype(records))
+        _call(lib().b200sort_topk_aos, (records,), stream, workspace, addr, code, record_bytes, n_rows, row_len, k, int(largest),
+              _describe(out)[0], _describe(indices)[0])
+        return out, indices
+
+    return _on_stream(records, stream, run)
+
+
+def topk_workspace_bytes(key_dtype, n_rows: int, row_len: int, k: int, payload_itemsizes=(), record_bytes: int = 0) -> int:
+    """Bytes of workspace a topk (record_bytes = 0) or topk_combined call of these shapes needs, whatever the keys."""
+    n = len(payload_itemsizes)
+    sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
+    return int(lib().b200sort_topk_workspace_bytes(_key_code(key_dtype), n_rows, row_len, k, n, sizes, record_bytes))

@@ -62,10 +62,11 @@ static cudaError_t seg_launch_bin(int kb, int b, const SegSortArgs &a, int sm_co
   return with_kb(kb, [&](auto K) { return launch(PK_SEGMENT, seg_tiny_kernel<decltype(K)::value>, grid, SEG_TINY_THREADS, 0, st, a); });
 }
 
-// The segmented sort of arrays that are all in device memory (the current device), offsets included.
+// The segmented sort of arrays that are all in device memory (the current device), offsets included.  keep_profile:
+// part of a larger call (a top-k), whose profile entries it adds to.
 static int sort_segmented_device(const Options &o, int key_type, bool ascending, int64_t num, int64_t n_segments, const int64_t *offsets,
                                  const std::vector<StreamDesc> &streams, bool soa, cudaStream_t stream, void *caller_workspace,
-                                 size_t workspace_bytes, b200sort_stats *stats) {
+                                 size_t workspace_bytes, b200sort_stats *stats, bool keep_profile = false) {
   const int kb = key_bytes_of(key_type);
   const uint64_t launches_before = g_launches.load();
   int dev = 0;
@@ -77,7 +78,7 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
   CacheGuard cache_guard;
   unsigned char *ws = nullptr;
   if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, sl.total, cache_guard, &ws)) return rc;
-  start_profile(o, false);
+  start_profile(o, keep_profile);
 
   // classify (one host wait: the bin counts, the validity flag, the longest segment)
   const int cap_log2 = seg_cap_log2(kb);
