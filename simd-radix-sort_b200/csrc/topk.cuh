@@ -59,6 +59,7 @@ struct TopkRow {
 struct TopkCtrl {
   unsigned long long items[MAX_PASSES];  // work items of pass p (p >= 1), counted up by the decision before it
 };
+static_assert(sizeof(TopkRow) == 80 && sizeof(TopkCtrl) == 8 * MAX_PASSES, "mirrored by tests/topk_model.py");
 
 struct TopkArgs {
   const unsigned char *keys;   // the input's keys (SoA keys, or AoS records with the key at offset 0)
