@@ -13,8 +13,9 @@
  *  - plain pointers and sizes only; no C++/torch types.
  *  - every array may live in HOST memory (sorted through a staged copy on the current CUDA device) or
  *    in DEVICE memory (sorted in place on the device that owns it: the fast path).  All arrays of
- *    one call must be on the same side.  The one exception is the top-k selection, which takes device arrays only
- *    (B200SORT_EUNSUPPORTED otherwise): staging a whole row over PCIe to return k records of it is the wrong tool.
+ *    one call must be on the same side.  The exceptions are the top-k selection and unique, which take device arrays
+ *    only (B200SORT_EUNSUPPORTED otherwise): staging a whole row over PCIe to return k records of it is the wrong tool,
+ *    and unique returns results whose size only the device knows.
  *  - the sort is in place from the caller's point of view (reference: radix_sort.hpp:297-337): the
  *    result overwrites keys/payloads/records.  Scratch (one shadow copy of every stream + per-tile
  *    status words) comes from `workspace` or, when that is NULL, from a per-device cache owned by
@@ -36,6 +37,8 @@
  *        longer than 8192 records, plus the waits above of the whole-array sorts it runs for long segments.
  *      * a top-k: the selection waits for nothing; its ordering step is a segmented sort of n_rows segments of
  *        k records and adds that sort's waits (one; more with 8-byte keys and k > 8192; none when k = 1).
+ *      * a unique: consecutive mode waits for nothing; sorted mode adds the waits of the whole-array sort of num
+ *        records it runs.
  *    These calls therefore cannot be captured into a CUDA graph; everything between the two waits
  *    (all passes, the junction kernel, the flag-gated segment finish / copy-back) is queued without one.
  *  - device arrays are sorted on the device that owns them, whatever the caller's current device is;
@@ -185,6 +188,42 @@ int b200sort_topk_aos(const void *records, int key_type, uint32_t record_bytes, 
 size_t b200sort_topk_workspace_bytes(int key_type, int64_t n_rows, int64_t row_len, int64_t k, int n_payloads,
                                      const uint32_t *payload_elem_bytes, uint32_t record_bytes);
 
+/* ---- unique: the distinct keys of an array, with their counts and inverse map --------------------------------------
+ * (An extension: the reference has no counterpart.)
+ *  - Equality is bit-pattern equality, consistent with the library's total order: +0.0 and -0.0 are two values, NaNs
+ *    with the same bits are one value, NaNs with different payloads are different values.  (torch.unique merges
+ *    +-0.0 and keeps every NaN apart.)
+ *  - consecutive = 0, like torch.unique(sorted=True): out_keys[0, U) holds the distinct keys in ascending total order
+ *    (-NaN < -inf < ... < -0.0 < +0.0 < ... < +inf < +NaN).
+ *    consecutive = 1, like torch.unique_consecutive: every maximal run of equal adjacent keys, in input order, gives
+ *    one entry, and no sort runs.
+ *  - out_counts[j] (int64, optional: NULL for none) is the number of input keys equal to entry j, or the length of
+ *    run j.  out_inverse[i] (int64, optional) is the j whose entry equals keys[i], or the run that contains i.
+ *  - *out_num_unique = U (int64, required) is written on `stream` into device memory.  Every output has room for num
+ *    entries; entries >= U are not written.  The input is only read.
+ *  - Errors, checked before any device work: B200SORT_EINVAL for an unknown key type, a negative num, a NULL keys,
+ *    out_keys or out_num_unique when num > 0, keys or out_keys not aligned to the key type, an int64 output not
+ *    8-byte aligned, and an output whose address range overlaps the input or another output.  With num == 0 only
+ *    *out_num_unique = 0 is written (nothing at all when out_num_unique is NULL).
+ *  - Memory side: device arrays only, all on one device (the call runs on it); an array in host memory gives
+ *    B200SORT_EUNSUPPORTED.
+ *  - Workspace: NULL (the library's per-device cache) or a 256-byte aligned buffer of at least
+ *    b200sort_unique_workspace_bytes(key_type, num, consecutive, with_inverse = out_inverse != NULL) bytes, which
+ *    depends on the shape only.  Host waits: consecutive = 1 waits for nothing; consecutive = 0 adds exactly the waits
+ *    of the whole-array sort it runs (see the conventions above).
+ *  - Method: consecutive = 0 copies the keys into the workspace (with their positions, u32 up to 2^32 records and u64
+ *    above, when the inverse is wanted) and sorts the copy with the whole-array sort.  Then one pass over the keys
+ *    compares each with its predecessor, numbers the runs (warp ballots, a block scan and a decoupled look-back over
+ *    tiles of 4096 keys) and writes the entries, the run starts and the inverse (a scatter through the positions after
+ *    the sort); a second small kernel turns the run starts into counts.
+ *  - b200sort_last_stats afterwards: algo = 5, num, record_bytes = key_bytes, kernel_launches (the sort's included);
+ *    every other field 0. */
+int b200sort_unique(const void *keys, int key_type, int64_t num, int consecutive,
+                    void *out_keys, int64_t *out_counts, int64_t *out_inverse, int64_t *out_num_unique,
+                    void *stream, void *workspace, size_t workspace_bytes);
+/* Bytes of device scratch a unique call with this shape needs; 0 for an unknown key type or a negative num. */
+size_t b200sort_unique_workspace_bytes(int key_type, int64_t num, int consecutive, int with_inverse);
+
 /* Thread-local message of the last failing call on this thread ("" if none). */
 const char *b200sort_last_error(void);
 
@@ -206,7 +245,7 @@ typedef struct b200sort_stats {
   int64_t num;
   uint32_t record_bytes;      /* sum of all stream element sizes */
   uint32_t key_bytes;
-  uint32_t algo;              /* 1 LSD, 2 hybrid, 3 segmented sort, 4 top-k (3 and 4: only num, record_bytes,
+  uint32_t algo;              /* 1 LSD, 2 hybrid, 3 segmented sort, 4 top-k, 5 unique (3 to 5: only num, record_bytes,
                                  key_bytes and kernel_launches are set) */
   uint32_t passes_planned;    /* scatter passes executed (hybrid) / launched (LSD; constant digits return at once) */
   uint32_t hist_sweeps;       /* key-only sweeps launched */
@@ -221,7 +260,8 @@ int b200sort_last_stats(b200sort_stats *out);
 
 /* Per-kernel device times of the last sort on this thread, recorded with CUDA events on the sort's
  * stream when option "profile" is 1.  kinds[i]: 0 histogram, 1 scan, 2 scatter pass, 3 copy-back,
- * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments, 7 top-k selection and gather.  Returns the number of entries written (<= capacity) or a negative code. */
+ * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments, 7 top-k selection and gather,
+ * 8 unique (index, run compaction, counts; the sort it runs keeps its own kinds).  Returns the number of entries written (<= capacity) or a negative code. */
 int b200sort_last_profile(int *kinds, float *ms, int capacity);
 
 /* Releases the per-device workspace and host-staging buffers held by the library.  A sort another thread

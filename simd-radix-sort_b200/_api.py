@@ -71,6 +71,10 @@ def lib():
         L.b200sort_topk_aos.restype = i32
         L.b200sort_topk_workspace_bytes.argtypes = [i32, i64, i64, i64, i32, u32p, u32]
         L.b200sort_topk_workspace_bytes.restype = sz
+        L.b200sort_unique.argtypes = [vp, i32, i64, i32, vp, vp, vp, vp, vp, vp, sz]
+        L.b200sort_unique.restype = i32
+        L.b200sort_unique_workspace_bytes.argtypes = [i32, i64, i32, i32]
+        L.b200sort_unique_workspace_bytes.restype = sz
         L.b200sort_last_error.restype = ctypes.c_char_p
         L.b200sort_version.restype = i32
         L.b200sort_launch_count.restype = ctypes.c_uint64
@@ -152,7 +156,7 @@ def last_stats() -> dict:
     return {f: getattr(s, f) for f, _ in _Stats._fields_}
 
 
-PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other", "segment", "select"]
+PROFILE_KINDS = ["hist", "scan", "sweep", "copyback", "segfix", "other", "segment", "select", "unique"]
 
 
 def last_profile():
@@ -443,3 +447,47 @@ def topk_workspace_bytes(key_dtype, n_rows: int, row_len: int, k: int, payload_i
     n = len(payload_itemsizes)
     sizes = (ctypes.c_uint32 * max(n, 1))(*payload_itemsizes)
     return int(lib().b200sort_topk_workspace_bytes(_key_code(key_dtype), n_rows, row_len, k, n, sizes, record_bytes))
+
+
+def _unique(x, consecutive: bool, return_inverse: bool, return_counts: bool, stream, workspace):
+    flat = x.reshape(-1)
+    kaddr, kname, _, num, _ = _describe(flat)
+    code = _key_code(kname)
+
+    def run():
+        values, n_unique = _empty(flat, (num,)), _empty(flat, (1,), _index_dtype(flat))
+        inverse = _empty(flat, tuple(x.shape), _index_dtype(flat)) if return_inverse else None
+        counts = _empty(flat, (num,), _index_dtype(flat)) if return_counts else None
+        _call(lib().b200sort_unique, (flat,), stream, workspace, kaddr, code, num, int(consecutive), _describe(values)[0],
+              None if counts is None else _describe(counts)[0], None if inverse is None else _describe(inverse)[0],
+              _describe(n_unique)[0])
+        u = int(n_unique[0])  # (the call's one host wait)
+        out = (values[:u],) + ((inverse,) if return_inverse else ()) + ((counts[:u],) if return_counts else ())
+        return out[0] if len(out) == 1 else out
+
+    return _on_stream(flat, stream, run)
+
+
+def unique(x, return_inverse: bool = False, return_counts: bool = False, stream=None, workspace=None):
+    """The distinct keys of `x` (flattened) in ascending order, like torch.unique(sorted=True) (b200sort_unique): -> values,
+    or a tuple (values, inverse, counts) holding the ones asked for, in torch's order.
+
+    Keys are equal when their bit patterns are: +0.0 and -0.0 are two values, and NaNs with the same bits are one (torch
+    merges +-0.0 and keeps every NaN apart).  The order is the library's total order of bit patterns.  inverse has x's
+    shape and dtype int64 (values[inverse] == x); counts are int64.  values and counts are views of the first U entries of
+    arrays sized for x.numel(): they keep that storage alive.  Reading U waits for the device once.  The keys must be on
+    a CUDA device: host arrays raise B200SortError with code -7."""
+    return _unique(x, False, return_inverse, return_counts, stream, workspace)
+
+
+def unique_consecutive(x, return_inverse: bool = False, return_counts: bool = False, stream=None, workspace=None):
+    """One entry per maximal run of equal adjacent keys of `x` (flattened), in input order, like torch.unique_consecutive
+    (b200sort_unique with consecutive = 1; no sort runs).  Returns and conventions as for unique."""
+    return _unique(x, True, return_inverse, return_counts, stream, workspace)
+
+
+def unique_workspace_bytes(key_dtype, num: int, consecutive: bool = False, return_inverse: bool = False) -> int:
+    """Bytes of workspace a unique (or unique_consecutive) call on num keys needs, whatever the keys."""
+    if num < 0:
+        raise ValueError(f"num = {num} is negative")
+    return int(lib().b200sort_unique_workspace_bytes(_key_code(key_dtype), num, int(consecutive), int(return_inverse)))

@@ -28,6 +28,7 @@
 #include "hybrid.cuh"
 #include "segmented.cuh"
 #include "topk.cuh"
+#include "unique.cuh"
 
 namespace b200sort {
 
@@ -106,7 +107,7 @@ struct ThreadDeviceState {
 static thread_local std::map<int, ThreadDeviceState> t_dev;
 
 // optional per-kernel timing (option "profile"): CUDA events around every launch of the last sort
-enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5, PK_SEGMENT = 6, PK_SELECT = 7 };
+enum ProfKind { PK_NONE = -1, PK_HIST = 0, PK_SCAN = 1, PK_SWEEP = 2, PK_COPYBACK = 3, PK_SEGFIX = 4, PK_OTHER = 5, PK_SEGMENT = 6, PK_SELECT = 7, PK_UNIQUE = 8 };
 struct ProfEntry { int kind; cudaEvent_t e0, e1; int dev; };
 static thread_local bool g_prof_on = false;  // the sort running on this thread has option "profile" set
 static thread_local std::vector<ProfEntry> g_prof;
@@ -135,8 +136,8 @@ struct ProfScope {  // (kind PK_NONE: records nothing)
     if (on) { cudaEventRecord(pe.e1, st); g_prof.push_back(pe); }
     static const bool dbg = getenv("B200SORT_DEBUG_SYNC") != nullptr;  // development: wait for every kernel, say which one
     if (dbg && kind_ != PK_NONE) {
-      static const char *names[] = {"hist", "scan", "sweep", "copyback", "segfix", "other", "segment", "select"};
-      fprintf(stderr, "[b200sort] %s launched ...", names[kind_ < 8 ? kind_ : 5]);
+      static const char *names[] = {"hist", "scan", "sweep", "copyback", "segfix", "other", "segment", "select", "unique"};
+      fprintf(stderr, "[b200sort] %s launched ...", names[kind_ < 9 ? kind_ : 5]);
       const cudaError_t e = cudaStreamSynchronize(st);
       fprintf(stderr, " done (%s)\n", cudaGetErrorString(e));
     }
@@ -1316,3 +1317,4 @@ void b200sort_release_cache(void) {
 #include "mgpu.cuh"
 #include "segmented_host.cuh"
 #include "topk_host.cuh"
+#include "unique_host.cuh"
