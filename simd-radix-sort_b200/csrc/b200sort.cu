@@ -854,7 +854,8 @@ struct DevSort {
     stt->hist_sweeps = hist_sweeps;
     stt->passes_planned = (have_plan || hybrid) ? hplan.n_exec : (uint32_t)kb;  // (otherwise every pass is launched)
     if (hybrid) {
-      stt->segfix_passes = finish_ran ? 1 : 0;
+      // (the flow that plans on the device launches the finish whatever the plan is; without a cut it returns at once)
+      stt->segfix_passes = (finish_ran && hplan.cut_digit != 0) ? 1 : 0;
       stt->cut_digit = hplan.cut_digit;
       memcpy(&stt->segfix_moved, &hctrl.flags[2], 8);
     }
