@@ -161,8 +161,9 @@ size_t b200sort_segmented_workspace_bytes(int key_type, int64_t num, int64_t n_s
  *  - Errors, checked before any device work: B200SORT_EINVAL for a negative n_rows, row_len or k, k > row_len,
  *    n_rows > 2^31 - 1, an n_rows * row_len that overflows, a NULL input, output or out_index when k > 0, a key
  *    array, key output or record array not aligned to the key type, out_index not 8-byte aligned, and an output
- *    whose address range overlaps an input's.  Payload shapes (up to 63 streams) and record sizes are checked as for
- *    the sort (B200SORT_ESHAPE / B200SORT_ERECORD).  k == 0 or n_rows == 0 is a no-op that returns 0.
+ *    whose address range overlaps an input's or another output's.  Payload shapes (up to 63 streams) and record
+ *    sizes are checked as for the sort (B200SORT_ESHAPE / B200SORT_ERECORD).  k == 0 or n_rows == 0 is a no-op that
+ *    returns 0.
  *  - Memory side: device arrays only, all on one device (the call runs on it); an array in host memory gives
  *    B200SORT_EUNSUPPORTED.
  *  - Workspace: NULL (the library's per-device cache) or a 256-byte aligned buffer of at least
@@ -261,7 +262,9 @@ int b200sort_last_stats(b200sort_stats *out);
 /* Per-kernel device times of the last sort on this thread, recorded with CUDA events on the sort's
  * stream when option "profile" is 1.  kinds[i]: 0 histogram, 1 scan, 2 scatter pass, 3 copy-back,
  * 4 segment finish, 5 other, 6 segmented-sort kernels of short segments, 7 top-k selection and gather,
- * 8 unique (index, run compaction, counts; the sort it runs keeps its own kinds).  Returns the number of entries written (<= capacity) or a negative code. */
+ * 8 unique (index, run compaction, counts; the sort it runs keeps its own kinds).  A single-GPU call lists one entry
+ * per kernel its kernel_launches counts, those of the sorts it runs inside and of a fall-back included.  Returns the
+ * number of entries written (<= capacity) or a negative code. */
 int b200sort_last_profile(int *kinds, float *ms, int capacity);
 
 /* Releases the per-device workspace and host-staging buffers held by the library.  A sort another thread

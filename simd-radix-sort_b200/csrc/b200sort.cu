@@ -41,10 +41,13 @@ static std::atomic<uint64_t> g_launches{0};
 
 constexpr int MGPU_MAX_CHUNKS = 8;  // multi-GPU overlapped exchange: at most this many chunks (mgpu.cuh)
 
+// b200sort_stats::algo (include/b200sort.h), and the values of option "algo", which picks one of the first two
+enum Algo { ALGO_AUTO = 0, ALGO_LSD = 1, ALGO_HYBRID = 2, ALGO_SEGMENTED = 3, ALGO_TOPK = 4, ALGO_UNIQUE = 5 };
+
 // The tuning options of b200sort_set_option; the member initialisers are the defaults.  The process-wide values
 // are read once when a sort call starts (options()) and that snapshot is passed down.
 struct Options {
-  int64_t algo = 0, tile_cfg = -1;  // algo: 0 auto, 1 LSD, 2 hybrid; tile_cfg: -1 auto, else the index of a tile geometry
+  int64_t algo = ALGO_AUTO, tile_cfg = -1;  // algo: auto, LSD or hybrid; tile_cfg: -1 auto, else the index of a tile geometry
   int64_t wide_tiles = 1;     // 4-byte keys, all chunks <= 4 bytes: 8192-key tiles
   int64_t nstage = 0;         // 0 auto, 1 single staging buffer, 2 double-buffered columns
   int64_t max_chunk = 16;     // largest chunk a stream is moved in (ablation: 8 = AoS records as 8-byte columns)
@@ -116,11 +119,11 @@ static void prof_reset() {
   for (auto &p : g_prof) { t_dev[p.dev].prof_pool.push_back(p.e0); t_dev[p.dev].prof_pool.push_back(p.e1); }
   g_prof.clear();
 }
-// a sort call starts timing its launches if option "profile" is set; keep: it is part of a larger call (a
-// segmented sort, a multi-GPU sort) and adds to that call's entries instead of starting over
-static void start_profile(const Options &o, bool keep) {
+// a public call starts over and times its launches if option "profile" is set; the calls it makes inside (the
+// fall-back, the sorts a segmented sort, top-k or unique runs) add to its entries
+static void start_profile(const Options &o) {
   g_prof_on = o.profile != 0;
-  if (!keep) prof_reset();
+  prof_reset();
 }
 static cudaEvent_t prof_event(int dev) {
   auto &pool = t_dev[dev].prof_pool;
@@ -422,22 +425,6 @@ static int cached_buffer(CacheEntry &c, size_t bytes, const char *what, void **o
   return 0;
 }
 
-// The workspace of a sort of `bytes` on the current device `dev`: the caller's (`caller_ws`, NULL for none), or the
-// library's cached one, taken through `guard` (which the caller holds until the sort's work is queued).
-static int acquire_workspace(int dev, cudaStream_t stream, void *caller_ws, size_t caller_bytes, size_t bytes, CacheGuard &guard,
-                             unsigned char **out) {
-  void *ws = caller_ws;
-  if (ws == nullptr) {
-    if (int rc = cached_buffer(guard.acquire(dev, stream).workspace, bytes, "workspace", &ws)) return rc;
-  } else if (caller_bytes < bytes) {
-    return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", caller_bytes, bytes);
-  } else if (((uintptr_t)ws % 256) != 0) {
-    return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
-  }
-  *out = (unsigned char *)ws;
-  return 0;
-}
-
 // ------------------------------------------------------------------------------------------------
 // job description
 // ------------------------------------------------------------------------------------------------
@@ -509,15 +496,44 @@ static size_t sort_workspace_bytes(const std::vector<StreamDesc> &streams, int64
   return L.total;
 }
 
-// the stats fields every sort reports: what it sorted, and the kernels launched since `launches_before`
-static b200sort_stats call_stats(int64_t n, const std::vector<StreamDesc> &streams, int kb, uint64_t launches_before) {
-  b200sort_stats s{};
-  s.num = n;
-  for (const StreamDesc &d : streams) s.record_bytes += d.elem_bytes;
-  s.key_bytes = (uint32_t)kb;
-  s.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
-  return s;
-}
+// What the work on device arrays of the current device (DevSort, sort_segmented_device, topk_device, unique_device)
+// starts with: open() finds the device and its properties; workspace() takes the caller's workspace, or the library's
+// cached one through `guard`, which is held until the work is queued.
+struct DevSetup {
+  uint64_t launches_before = g_launches.load();  // the launch counter when the function started
+  int dev = 0;
+  DevInfo di;
+  CacheGuard guard;
+  unsigned char *ws = nullptr;
+
+  int open() {
+    CUDA_TRY(cudaGetDevice(&dev));
+    return dev_info(dev, &di);
+  }
+  // ws: `bytes` of workspace, from `caller_ws` (NULL for none) of `caller_bytes` or from the cache
+  int workspace(cudaStream_t stream, void *caller_ws, size_t caller_bytes, size_t bytes) {
+    if (caller_ws == nullptr) {
+      void *p = nullptr;
+      if (int rc = cached_buffer(guard.acquire(dev, stream).workspace, bytes, "workspace", &p)) return rc;
+      ws = (unsigned char *)p;
+      return 0;
+    }
+    if (caller_bytes < bytes) return fail(B200SORT_ENOMEM, "workspace of %zu bytes given, %zu needed", caller_bytes, bytes);
+    if (((uintptr_t)caller_ws % 256) != 0) return fail(B200SORT_EINVAL, "workspace must be 256-byte aligned");
+    ws = (unsigned char *)caller_ws;
+    return 0;
+  }
+  // the stats fields every call reports: what it worked on, and the kernels launched since the function started
+  b200sort_stats stats(int64_t n, const std::vector<StreamDesc> &streams, int kb, int algo) const {
+    b200sort_stats s{};
+    s.num = n;
+    for (const StreamDesc &d : streams) s.record_bytes += d.elem_bytes;
+    s.key_bytes = (uint32_t)kb;
+    s.algo = (uint32_t)algo;
+    s.kernel_launches = (uint32_t)(g_launches.load() - launches_before);
+    return s;
+  }
+};
 
 // The arrays as the streams the scatter kernel moves: each one in chunks of the largest power of two <= max_chunk
 // (and <= 16) dividing both its address and its element size; the key stream (keys or records) in chunks no narrower
@@ -555,7 +571,6 @@ struct DevSortOpts {
   // Partial-sort mode (B200SORT_CMP_NONE with a threshold >= CMP_NONE_MIN_THRESH): the segments below the plan's
   // cut need not be ordered as long as none has more than this many keys (0 = full sort)
   int64_t cmp_none_thresh = 0;
-  bool keep_profile = false;  // part of a larger call (a segmented sort): add to its profile entries, do not reset them
 };
 constexpr int64_t CMP_NONE_MIN_THRESH = 8;  // below it nearly every sort would need the finish anyway: full sort
 
@@ -585,7 +600,7 @@ static Plan forced_plan(int kb, uint32_t cut, uint32_t lshift) {
 
 // One sort of device arrays, phase by phase: one histogram sweep over all digit positions, the bucket-offset scan
 // (+ pass plan), one scatter pass per digit position, the segment finish, the copy-back.
-struct DevSort {
+struct DevSort : DevSetup {
   const Options &o;
   const int key_type;
   const bool ascending;
@@ -597,18 +612,14 @@ struct DevSort {
   const DevSortOpts &xo;
   const int kb = key_bytes_of(key_type);
   // set-up
-  uint64_t launches_before = 0;  // the launch counter when the sort started
-  int dev = 0, cfg = 0, tile = 0, algo = 0;
+  int cfg = 0, tile = 0, algo = ALGO_AUTO;
   bool hybrid = false;
-  DevInfo di;
   StreamSet ss{};
   uint32_t stage_bytes = 0;
   Layout L;
-  unsigned char *ws = nullptr;
   Plan *plan = nullptr;  // (device)
   HybridCtrl *ctrl = nullptr;
   KeyOrder ko{};
-  CacheGuard cache_guard;  // released (and its event recorded) when this sort has been launched
   // plan
   Plan hplan{};
   bool have_plan = false;    // the host knows the plan (hplan): launches only what executes
@@ -623,8 +634,7 @@ struct DevSort {
 
   // set-up: streams, tile geometry, workspace layout, workspace (and the cache guard if it is the library's)
   int setup() {
-    CUDA_TRY(cudaGetDevice(&dev));
-    if (int rc = dev_info(dev, &di)) return rc;
+    if (int rc = open()) return rc;
     stage_bytes = make_stream_set(streams, kb, (uint32_t)o.max_chunk, &ss);
     if (streams[0].elem_bytes != (uint32_t)kb && ((uintptr_t)streams[0].ptr % kb) != 0)
       return fail(B200SORT_EINVAL, "record array is not aligned to its key type");
@@ -637,18 +647,17 @@ struct DevSort {
     if (smem > di.smem_optin) return fail(B200SORT_ECUDA, "device offers %zu B of shared memory, %zu needed", di.smem_optin, smem);
 
     make_layout(streams, std::max(n, xo.layout_n), std::min(tile, HYB_MIN_TILE), &L, xo.layout_landing);
-    if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, L.total, cache_guard, &ws)) return rc;
+    if (int rc = workspace(stream, caller_workspace, workspace_bytes, L.total)) return rc;
     for (size_t s = 0; s < streams.size(); s++) ss.streams[s].buf[1] = ws + L.shadow_off[s];
     plan = (Plan *)(ws + L.plan_off);
     ctrl = (HybridCtrl *)(ws + L.hyb_off);
-    start_profile(o, xo.forced || xo.keep_profile);
     if (!xo.forced) CUDA_TRY(cudaMemsetAsync(ws + L.ctrl_off, 0, L.ctrl_bytes, stream));
 
     ko = make_key_order(key_type, ascending);
-    algo = xo.forced ? 2 : (int)o.algo;
-    if (algo == 0) algo = (kb == 8 && n >= HYB_MIN_N) ? 2 : 1;
-    if (algo == 2 && kb != 8) algo = 1;
-    hybrid = algo == 2;
+    algo = xo.forced ? ALGO_HYBRID : (int)o.algo;
+    if (algo == ALGO_AUTO) algo = (kb == 8 && n >= HYB_MIN_N) ? ALGO_HYBRID : ALGO_LSD;
+    if (algo == ALGO_HYBRID && kb != 8) algo = ALGO_LSD;
+    hybrid = algo == ALGO_HYBRID;
     return 0;
   }
 
@@ -849,8 +858,7 @@ struct DevSort {
       CUDA_TRY(cudaStreamSynchronize(stream));
       if (fix_flow) finish_ran = hctrl.flags[1] != 0;
     }
-    *stt = call_stats(n, streams, kb, launches_before);
-    stt->algo = (uint32_t)algo;
+    *stt = stats(n, streams, kb, algo);
     stt->hist_sweeps = hist_sweeps;
     stt->passes_planned = (have_plan || hybrid) ? hplan.n_exec : (uint32_t)kb;  // (otherwise every pass is launched)
     if (hybrid) {
@@ -867,11 +875,11 @@ struct DevSort {
   // fall-back: finish with the plain digit-by-digit path (the array is a permutation of the input, already ordered
   // by its top digits)
   int fall_back(b200sort_stats *stt) {
-    Options lsd = o; lsd.algo = 1;  // (whatever option "algo" says)
+    Options lsd = o; lsd.algo = ALGO_LSD;  // (whatever option "algo" says)
     DevSortOpts fo;
     fo.layout_n = xo.layout_n; fo.layout_landing = xo.layout_landing;
     b200sort_stats s2;
-    if (int rc = DevSort{lsd, key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo}.run(&s2)) return rc;
+    if (int rc = DevSort{{}, lsd, key_type, ascending, n, streams, stream, caller_workspace, workspace_bytes, fo}.run(&s2)) return rc;
     stt->fell_back = 1;
     stt->passes_planned += s2.passes_planned;
     stt->hist_sweeps += s2.hist_sweeps;
@@ -882,7 +890,6 @@ struct DevSort {
 
   // the sort, phase by phase; *stats: what ran (written when the sort succeeds)
   int run(b200sort_stats *stats) {
-    launches_before = g_launches.load();
     if (int rc = setup()) return rc;
     if (int rc = make_plan()) return rc;
     if (int rc = run_passes()) return rc;
@@ -899,7 +906,7 @@ struct DevSort {
 
 static int sort_device(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams,
                        cudaStream_t stream, void *workspace, size_t workspace_bytes, const DevSortOpts &xo, b200sort_stats *stats) {
-  return DevSort{o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, xo}.run(stats);
+  return DevSort{{}, o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, xo}.run(stats);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -923,7 +930,7 @@ struct DeviceScope {
   ~DeviceScope() { if (switched) cudaSetDevice(prev); }
 };
 
-static int side_of(const void *p, Side *out, int *dev_out = nullptr) {
+static int side_of(const void *p, Side *out, int *dev_out) {
   cudaPointerAttributes at{};
   cudaError_t e = cudaPointerGetAttributes(&at, p);
   if (e != cudaSuccess) {
@@ -932,9 +939,63 @@ static int side_of(const void *p, Side *out, int *dev_out = nullptr) {
                 cudaGetErrorString(e));
   }
   *out = (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) ? SIDE_DEVICE : SIDE_HOST;
-  if (dev_out) *dev_out = at.device;
+  *dev_out = at.device;
   return 0;
 }
+
+// Where the arrays of one call live, each pointer asked once: all in host memory, or all on one device (*dev).
+// offsets (NULL for none): a segmented sort's, which must live where the arrays do.  device_only (NULL for none): the
+// name of a call that takes device arrays only, for the error that refuses host arrays.  Fails without a device.
+static int place_arrays(const std::vector<StreamDesc> &arrays, const int64_t *offsets, const char *device_only, Side *side, int *dev) {
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev == 0) {
+    cudaGetLastError();
+    return fail(B200SORT_ECUDA, "no CUDA device available (%s); libb200sort has no CPU fallback",
+                e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
+  }
+  std::vector<Side> sd(arrays.size() + (offsets != nullptr ? 1 : 0));  // (the offsets last)
+  std::vector<int> dv(sd.size());
+  for (size_t i = 0; i < sd.size(); i++)
+    if (int rc = side_of(i < arrays.size() ? arrays[i].ptr : offsets, &sd[i], &dv[i])) return rc;
+  if (device_only != nullptr && std::count(sd.begin(), sd.end(), SIDE_HOST) != 0)
+    return fail(B200SORT_EUNSUPPORTED, "%s takes device arrays only; an array is in host memory", device_only);
+  *side = sd[0];
+  *dev = dv[0];
+  for (size_t i = 1; i < arrays.size(); i++) {
+    if (sd[i] != *side) return fail(B200SORT_EINVAL, "arrays must be all in host memory or all in device memory");
+    if (sd[i] == SIDE_DEVICE && dv[i] != *dev) return fail(B200SORT_EINVAL, "device arrays live on different devices (%d and %d)", *dev, dv[i]);
+  }
+  if (offsets != nullptr && (sd.back() != *side || (*side == SIDE_DEVICE && dv.back() != *dev)))
+    return fail(B200SORT_EINVAL, "offsets must live where the arrays do (host memory, or the arrays' device)");
+  return 0;
+}
+
+// What every public single-GPU call does once its arguments have passed their checks: it takes the options snapshot,
+// places its arrays (place_arrays), runs on their device (host arrays: on the current one) and starts its profile.
+// done(rc) makes `stats` the call's statistics (b200sort_last_stats) when the call succeeded.
+struct CallScope {
+  const Options o = options();
+  Side side = SIDE_HOST;
+  int dev = 0;
+  b200sort_stats stats{};
+  DeviceScope device;
+
+  int enter(const std::vector<StreamDesc> &arrays, const int64_t *offsets, const char *device_only) {
+    if (int rc = place_arrays(arrays, offsets, device_only, &side, &dev)) return rc;
+    if (side == SIDE_DEVICE) {
+      if (int rc = device.enter(dev)) return rc;
+    } else {
+      CUDA_TRY(cudaGetDevice(&dev));
+    }
+    start_profile(o);
+    return 0;
+  }
+  int done(int rc) {
+    if (rc == B200SORT_OK) g_last_stats = stats;
+    return rc;
+  }
+};
 
 // ------------------------------------------------------------------------------------------------
 // Host arrays, SoA with payloads: pipelined staging (SURVEY 8f rank 2).  PCIe is the bottleneck of a sort
@@ -1066,54 +1127,20 @@ static int sort_host_pipelined(const Options &o, int dev, CacheEntry &stage, int
   return rc;
 }
 
-// fails unless a CUDA device is usable
-static int require_device() {
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    return fail(B200SORT_ECUDA, "no CUDA device available (%s); libb200sort has no CPU fallback",
-                e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
-  }
-  return 0;
-}
-
-// where the arrays of one call, and the offsets of a segmented sort (NULL for none), live: all in host memory, or all
-// on one device (*dev); fails without a device
-static int arrays_side(const std::vector<StreamDesc> &streams, const int64_t *offsets, Side *side, int *dev) {
-  if (int rc = require_device()) return rc;
-  if (int rc = side_of(streams[0].ptr, side, dev)) return rc;
-  for (size_t s = 1; s < streams.size(); s++) {
-    Side sd;
-    int dv = 0;
-    if (int rc = side_of(streams[s].ptr, &sd, &dv)) return rc;
-    if (sd != *side) return fail(B200SORT_EINVAL, "arrays must be all in host memory or all in device memory");
-    if (sd == SIDE_DEVICE && dv != *dev) return fail(B200SORT_EINVAL, "device arrays live on different devices (%d and %d)", *dev, dv);
-  }
-  if (offsets != nullptr) {
-    Side sd;
-    int dv = 0;
-    if (int rc = side_of(offsets, &sd, &dv)) return rc;
-    if (sd != *side || (sd == SIDE_DEVICE && dv != *dev))
-      return fail(B200SORT_EINVAL, "offsets must live where the arrays do (host memory, or the arrays' device)");
-  }
-  return 0;
-}
-
-// Host arrays sorted whole on the current device: the arrays, and `upload_bytes` at `upload` (NULL for none) that the
-// sort only reads, copied up into the staging buffer (cache entry `stage`, whose guard the caller holds);
-// sort(the arrays' device streams, the device copy of `upload`); the arrays copied back unless it failed.  Returns
-// when they are back.
+// Host arrays sorted whole on the current device `dev`: the arrays, and `upload_bytes` at `upload` (NULL for none)
+// that the sort only reads, copied up into the device's staging buffer; sort(the arrays' device streams, the device
+// copy of `upload`); the arrays copied back unless it failed.  Returns when they are back.
 template <typename SortFn>
-static int sort_staged(CacheEntry &stage, int64_t n, const std::vector<StreamDesc> &streams, const void *upload, size_t upload_bytes,
+static int sort_staged(int dev, int64_t n, const std::vector<StreamDesc> &streams, const void *upload, size_t upload_bytes,
                        cudaStream_t stream, SortFn &&sort) {
   std::vector<size_t> bytes;
   for (const StreamDesc &s : streams) bytes.push_back((size_t)n * s.elem_bytes);
   if (upload != nullptr) bytes.push_back(upload_bytes);
   size_t total = 0;
   const std::vector<size_t> offs = back_to_back(bytes, &total);
+  CacheGuard guard;  // the staging buffer is the library's, like the workspace; the call is synchronous anyway
   void *dbuf_v = nullptr;
-  if (int rc = cached_buffer(stage, total, "staging", &dbuf_v)) return rc;
+  if (int rc = cached_buffer(guard.acquire(dev, stream).stage, total, "staging", &dbuf_v)) return rc;
   unsigned char *dbuf = (unsigned char *)dbuf_v;
   std::vector<StreamDesc> dstreams(streams.size());
   for (size_t s = 0; s < streams.size(); s++) dstreams[s] = {dbuf + offs[s], streams[s].elem_bytes};
@@ -1133,39 +1160,34 @@ static int sort_staged(CacheEntry &stage, int64_t n, const std::vector<StreamDes
   return rc;
 }
 
-static int sort_any(const Options &o, int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
-                    void *workspace, size_t workspace_bytes, const DevSortOpts &base, b200sort_stats *stats) {
+static int sort_any(int key_type, bool ascending, int64_t n, const std::vector<StreamDesc> &streams, void *stream_v,
+                    void *workspace, size_t workspace_bytes, const DevSortOpts &base) {
   cudaStream_t stream = (cudaStream_t)stream_v;
   if (n <= 1) return B200SORT_OK;  // src/radix_sort.hpp:276: nothing to do for 0 or 1 element
-  Side side0;
-  int dev0 = 0;
-  if (int rc = arrays_side(streams, nullptr, &side0, &dev0)) return rc;
-  if (side0 == SIDE_DEVICE) {
-    DeviceScope scope;  // sort on the device that owns the arrays (include/b200sort.h)
-    if (int rc = scope.enter(dev0)) return rc;
-    return sort_device(o, key_type, ascending, n, streams, stream, workspace, workspace_bytes, base, stats);
-  }
+  CallScope call;  // device arrays: sorted on the device that owns them (include/b200sort.h)
+  if (int rc = call.enter(streams, nullptr, nullptr)) return rc;
+  const Options &o = call.o;
+  auto sort = [&](const std::vector<StreamDesc> &dstreams, const void *) {
+    return sort_device(o, key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base, &call.stats);
+  };
+  if (call.side == SIDE_DEVICE) return call.done(sort(streams, nullptr));
 
   // ---- host arrays: staged on the current device, through its cached staging buffer ----------------
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  CacheGuard cache_guard;  // the staging buffer is the library's, like the workspace; this call is synchronous anyway
-  CacheEntry &stage = cache_guard.acquire(dev, stream).stage;
   // SoA with payloads, big enough to care: pipelined staging
   if (o.host_pipeline != 0 && base.cmp_none_thresh == 0 && workspace == nullptr && streams.size() >= 2 &&
       streams[0].elem_bytes == (uint32_t)key_bytes_of(key_type) && n >= ((int64_t)1 << 20) && n < ((int64_t)1 << 32)) {
+    CacheGuard guard;
+    CacheEntry &stage = guard.acquire(call.dev, stream).stage;
     size_t need = 0;
     for (size_t s = 0; s < streams.size(); s++) need += (size_t)n * streams[s].elem_bytes * (s ? 2 : 1);
     need += (size_t)n * 4 + 2 * ((size_t)n * (key_bytes_of(key_type) + 4));  // index + the sort's own workspace
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need < free_b / 10 * 9 + stage.bytes)
-      return sort_host_pipelined(o, dev, stage, key_type, ascending, n, streams, stream, stats);
+      return call.done(sort_host_pipelined(o, call.dev, stage, key_type, ascending, n, streams, stream, &call.stats));
     cudaGetLastError();
   }
   // everything else: the whole arrays up, the sort, the whole arrays down
-  return sort_staged(stage, n, streams, nullptr, 0, stream, [&](const std::vector<StreamDesc> &dstreams, const void *) {
-    return sort_device(o, key_type, ascending, n, dstreams, stream, workspace, workspace_bytes, base, stats);
-  });
+  return call.done(sort_staged(call.dev, n, streams, nullptr, 0, stream, sort));
 }
 
 static int check_soa(void *keys, int key_type, int64_t num, int n_payloads, void *const *payloads,
@@ -1197,6 +1219,23 @@ static int check_aos(void *records, int key_type, uint32_t record_bytes, int64_t
   return 0;
 }
 
+// EINVAL unless no output overlaps an input and no two outputs overlap each other (NULL and empty ranges overlap
+// nothing); the calls whose outputs are not written in place check this before any device work
+struct ByteRange { const void *ptr; size_t bytes; };
+static int check_disjoint(const std::vector<ByteRange> &in, const std::vector<ByteRange> &out) {
+  auto overlap = [](const ByteRange &a, const ByteRange &b) {
+    const uintptr_t x = (uintptr_t)a.ptr, y = (uintptr_t)b.ptr;
+    return a.ptr && b.ptr && a.bytes != 0 && b.bytes != 0 && x < y + b.bytes && y < x + a.bytes;
+  };
+  for (size_t i = 0; i < out.size(); i++) {
+    for (const ByteRange &r : in)
+      if (overlap(r, out[i])) return fail(B200SORT_EINVAL, "an output overlaps the input");
+    for (size_t j = 0; j < i; j++)
+      if (overlap(out[j], out[i])) return fail(B200SORT_EINVAL, "two outputs overlap");
+  }
+  return 0;
+}
+
 // the options of the _ex calls' comparison sorter.  CmpSorterInsertionSort: the full sort whatever the threshold.
 // CmpSorterNoSort: buckets of at most cmp_sort_threshold elements may stay unordered (src/radix_sort.hpp:279,
 // src/cmp_sorters.hpp:66-78).
@@ -1220,7 +1259,7 @@ int b200sort_sort_soa_ex(void *keys, int key_type, int64_t num, int ascending, i
   if (int rc = cmp_sorter_opts(cmp_sort_threshold, cmp_sorter, &base)) return rc;
   std::vector<StreamDesc> streams;
   if (int rc = check_soa(keys, key_type, num, n_payloads, payloads, payload_elem_bytes, &streams)) return rc;
-  return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
+  return sort_any(key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base);
 }
 
 int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int64_t num, int ascending,
@@ -1230,7 +1269,7 @@ int b200sort_sort_aos_ex(void *records, int key_type, uint32_t record_bytes, int
   if (int rc = cmp_sorter_opts(cmp_sort_threshold, cmp_sorter, &base)) return rc;
   std::vector<StreamDesc> streams;
   if (int rc = check_aos(records, key_type, record_bytes, num, &streams)) return rc;
-  return sort_any(options(), key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base, &g_last_stats);
+  return sort_any(key_type, ascending != 0, num, streams, stream, workspace, workspace_bytes, base);
 }
 
 int b200sort_sort_soa(void *keys, int key_type, int64_t num, int ascending, int n_payloads, void *const *payloads,

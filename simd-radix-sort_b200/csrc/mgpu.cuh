@@ -934,7 +934,7 @@ struct MgpuSort {
     if (int rc = dev_info(c->dev, &di)) return rc;
     // workspace, laid out for `capacity` records on every rank (so that equal capacities give equal layouts
     // and the local sort finds what the peers wrote where it expects its shadow arrays)
-    g_prof_on = o.profile != 0;
+    start_profile(o);
     stage_bytes = make_stream_set(streams, kb, 16, &ss);
     cfg = pick_tile_cfg(o, kb, stage_bytes, di.smem_optin, num_local);
     tile = kTileCfgs[cfg].threads * kTileCfgs[cfg].ipt;
@@ -1305,8 +1305,12 @@ struct MgpuSort {
       so.start_sel = landing ? 0 : 1;
       so.hint_lead_bits = lead[c->rank];
       so.landing_input = landing;
-      if (recv_total > 0)
+      if (recv_total > 0) {
+        // (the profile lists the local sort alone, without the partition pass: bench.py's multi-GPU roofline averages
+        //  the scatter passes of the local sort)
+        start_profile(o);
         if (int rc = sort_device(o, key_type, ascending, recv_total, streams, stream, nullptr, 0, so, stats)) return rc;
+      }
     } else {
       // all-to-all-v, shadow -> caller arrays
       NCCL_TRY(api.GroupStart());
@@ -1320,8 +1324,10 @@ struct MgpuSort {
       }
       NCCL_TRY(api.GroupEnd());
       trace.mark("exchange");
-      if (recv_total > 1)
+      if (recv_total > 1) {
+        start_profile(o);
         if (int rc = sort_device(o, key_type, ascending, recv_total, streams, stream, nullptr, 0, so, stats)) return rc;
+      }
     }
     trace.mark("local_sort");
     return 0;

@@ -62,34 +62,27 @@ static cudaError_t seg_launch_bin(int kb, int b, const SegSortArgs &a, int sm_co
   return with_kb(kb, [&](auto K) { return launch(PK_SEGMENT, seg_tiny_kernel<decltype(K)::value>, grid, SEG_TINY_THREADS, 0, st, a); });
 }
 
-// The segmented sort of arrays that are all in device memory (the current device), offsets included.  keep_profile:
-// part of a larger call (a top-k), whose profile entries it adds to.
+// The segmented sort of arrays that are all in device memory (the current device), offsets included.
 static int sort_segmented_device(const Options &o, int key_type, bool ascending, int64_t num, int64_t n_segments, const int64_t *offsets,
                                  const std::vector<StreamDesc> &streams, bool soa, cudaStream_t stream, void *caller_workspace,
-                                 size_t workspace_bytes, b200sort_stats *stats, bool keep_profile = false) {
+                                 size_t workspace_bytes, b200sort_stats *stats) {
   const int kb = key_bytes_of(key_type);
-  const uint64_t launches_before = g_launches.load();
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  DevInfo di;
-  if (int rc = dev_info(dev, &di)) return rc;
+  DevSetup su;
+  if (int rc = su.open()) return rc;
   if (((uintptr_t)streams[0].ptr % kb) != 0) return fail(B200SORT_EINVAL, "key array is not aligned to its key type");
   const SegLayout sl = seg_layout(kb, num, n_segments, streams, soa);
-  CacheGuard cache_guard;
-  unsigned char *ws = nullptr;
-  if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, sl.total, cache_guard, &ws)) return rc;
-  start_profile(o, keep_profile);
+  if (int rc = su.workspace(stream, caller_workspace, workspace_bytes, sl.total)) return rc;
 
   // classify (one host wait: the bin counts, the validity flag, the longest segment)
   const int cap_log2 = seg_cap_log2(kb);
-  SegCtrl *ctrl = (SegCtrl *)ws;
+  SegCtrl *ctrl = (SegCtrl *)su.ws;
   CUDA_TRY(cudaMemsetAsync(ctrl, 0, sizeof(SegCtrl), stream));
   SegClassifyArgs ca{};
   ca.offsets = offsets; ca.n_segments = n_segments; ca.num = num; ca.cap = 1u << cap_log2; ca.ctrl = ctrl;
-  for (int b = 0; b < SEG_NBINS; b++) { ca.list[b] = (uint32_t *)(ws + sl.list_off[b]); ca.list_cap[b] = sl.list_cap[b]; }
-  ca.large = (int64_t *)(ws + sl.large_off);
+  for (int b = 0; b < SEG_NBINS; b++) { ca.list[b] = (uint32_t *)(su.ws + sl.list_off[b]); ca.list_cap[b] = sl.list_cap[b]; }
+  ca.large = (int64_t *)(su.ws + sl.large_off);
   ca.large_cap = sl.large_cap;
-  const unsigned cgrid = (unsigned)std::min<int64_t>((n_segments + SEG_CLASSIFY_THREADS - 1) / SEG_CLASSIFY_THREADS, (int64_t)di.sm_count * 8);
+  const unsigned cgrid = (unsigned)std::min<int64_t>((n_segments + SEG_CLASSIFY_THREADS - 1) / SEG_CLASSIFY_THREADS, (int64_t)su.di.sm_count * 8);
   CUDA_TRY(launch(PK_OTHER, seg_classify_kernel, cgrid, SEG_CLASSIFY_THREADS, 0, stream, ca));
   SegCtrl h{};
   CUDA_TRY(cudaMemcpyAsync(&h, ctrl, sizeof h, cudaMemcpyDeviceToHost, stream));
@@ -99,16 +92,15 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
   KeyOrder ko = make_key_order(key_type, ascending);
   std::vector<StreamDesc> sub = streams;
   b200sort_stats inner;
-  DevSortOpts whole;
-  whole.keep_profile = true;  // (the profile of this call lists the segment kernels too)
+  const DevSortOpts whole;
   const bool long_segments = h.max_len > ca.cap;  // (then n_large > 0)
   if (long_segments && kb <= 4) {
     // one sort of (segment index, ordered key) over [offsets[0], offsets[n_segments])
     const int64_t first = h.first, span = h.last - h.first;
     SegCompositeArgs pa{};
     pa.keys = (unsigned char *)streams[0].ptr; pa.key_stride = streams[0].elem_bytes; pa.offsets = offsets; pa.n_segments = n_segments;
-    pa.first = first; pa.span = span; pa.ko = ko; pa.comp = (unsigned long long *)(ws + sl.region_off + sl.comp_off);
-    const unsigned grid = (unsigned)std::min<int64_t>((span + 255) / 256, (int64_t)di.sm_count * 16);
+    pa.first = first; pa.span = span; pa.ko = ko; pa.comp = (unsigned long long *)(su.ws + sl.region_off + sl.comp_off);
+    const unsigned grid = (unsigned)std::min<int64_t>((span + 255) / 256, (int64_t)su.di.sm_count * 16);
     auto pack = [&](auto K, bool unpack) -> cudaError_t {
       constexpr int KB = decltype(K)::value;
       if constexpr (KB <= 4) return launch(PK_OTHER, unpack ? seg_unpack_kernel<KB> : seg_pack_kernel<KB>, grid, 256, 0, stream, pa);
@@ -117,7 +109,7 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
     CUDA_TRY(with_kb(kb, [&](auto K) { return pack(K, false); }));
     std::vector<StreamDesc> cs = {{pa.comp, 8u}};
     for (size_t i = soa ? 1 : 0; i < streams.size(); i++) cs.push_back({(unsigned char *)streams[i].ptr + (size_t)first * streams[i].elem_bytes, streams[i].elem_bytes});
-    if (int rc = sort_device(o, B200SORT_U64, true, span, cs, stream, ws + sl.region_off + sl.sort_off, sl.region_bytes - sl.sort_off,
+    if (int rc = sort_device(o, B200SORT_U64, true, span, cs, stream, su.ws + sl.region_off + sl.sort_off, sl.region_bytes - sl.sort_off,
                              whole, &inner))
       return rc;
     if (soa) CUDA_TRY(with_kb(kb, [&](auto K) { return pack(K, true); }));
@@ -125,11 +117,11 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
     if (long_segments) {
       // 8-byte keys: one sort per long segment (second host wait: their starts and lengths)
       std::vector<int64_t> large(2 * (size_t)h.n_large);
-      CUDA_TRY(cudaMemcpyAsync(large.data(), ws + sl.large_off, large.size() * 8, cudaMemcpyDeviceToHost, stream));
+      CUDA_TRY(cudaMemcpyAsync(large.data(), su.ws + sl.large_off, large.size() * 8, cudaMemcpyDeviceToHost, stream));
       CUDA_TRY(cudaStreamSynchronize(stream));
       for (uint32_t i = 0; i < h.n_large; i++) {
         for (size_t s = 0; s < streams.size(); s++) sub[s].ptr = (unsigned char *)streams[s].ptr + (size_t)large[2 * i] * streams[s].elem_bytes;
-        if (int rc = sort_device(o, key_type, ascending, large[2 * i + 1], sub, stream, ws + sl.region_off, sl.region_bytes, whole, &inner))
+        if (int rc = sort_device(o, key_type, ascending, large[2 * i + 1], sub, stream, su.ws + sl.region_off, sl.region_bytes, whole, &inner))
           return rc;
       }
     }
@@ -138,22 +130,20 @@ static int sort_segmented_device(const Options &o, int key_type, bool ascending,
     sa.ko = ko; sa.offsets = offsets;
     for (int b = 0; b < SEG_NBINS; b++) {
       if (h.count[b] == 0) continue;
-      sa.list = (const uint32_t *)(ws + sl.list_off[b]); sa.count = h.count[b]; sa.ticket = &ctrl->ticket[b];
-      CUDA_TRY(seg_launch_bin(kb, b, sa, di.sm_count, stream));
+      sa.list = (const uint32_t *)(su.ws + sl.list_off[b]); sa.count = h.count[b]; sa.ticket = &ctrl->ticket[b];
+      CUDA_TRY(seg_launch_bin(kb, b, sa, su.di.sm_count, stream));
     }
   }
-  *stats = call_stats(num, streams, kb, launches_before);
-  stats->algo = 3;
+  *stats = su.stats(num, streams, kb, ALGO_SEGMENTED);
   return B200SORT_OK;
 }
 
 // num <= 1: no segment has two records, but invalid offsets are still an error.  The offsets are checked on the
 // host (device offsets are copied there first: the arrays may be empty, so there is nothing to sort on the device).
 static int check_offsets_only(int64_t num, int64_t n_segments, const int64_t *offsets, cudaStream_t stream) {
-  if (int rc = require_device()) return rc;
   Side side;
   int dev = 0;
-  if (int rc = side_of(offsets, &side, &dev)) return rc;
+  if (int rc = place_arrays({}, offsets, nullptr, &side, &dev)) return rc;
   std::vector<int64_t> h;
   const int64_t *v = offsets;
   if (side == SIDE_DEVICE) {
@@ -177,24 +167,15 @@ static int sort_segmented_any(int key_type, bool ascending, int64_t num, int64_t
   if (n_segments == 0) return B200SORT_OK;
   cudaStream_t stream = (cudaStream_t)stream_v;
   if (num <= 1) return check_offsets_only(num, n_segments, offsets, stream);  // (nothing can move)
-  const Options o = options();
-  Side side;
-  int dev = 0;
-  if (int rc = arrays_side(streams, offsets, &side, &dev)) return rc;
-  if (side == SIDE_DEVICE) {
-    DeviceScope scope;
-    if (int rc = scope.enter(dev)) return rc;
-    return sort_segmented_device(o, key_type, ascending, num, n_segments, offsets, streams, soa, stream, workspace, workspace_bytes,
-                                 &g_last_stats);
-  }
+  CallScope call;
+  if (int rc = call.enter(streams, offsets, nullptr)) return rc;
+  auto sort = [&](const std::vector<StreamDesc> &dstreams, const void *doffsets) {
+    return sort_segmented_device(call.o, key_type, ascending, num, n_segments, (const int64_t *)doffsets, dstreams, soa, stream, workspace,
+                                 workspace_bytes, &call.stats);
+  };
+  if (call.side == SIDE_DEVICE) return call.done(sort(streams, offsets));
   // host arrays: the whole arrays and the offsets up, the sort, the arrays down (not when it failed)
-  CUDA_TRY(cudaGetDevice(&dev));
-  CacheGuard cache_guard;
-  return sort_staged(cache_guard.acquire(dev, stream).stage, num, streams, offsets, (size_t)(n_segments + 1) * 8, stream,
-                     [&](const std::vector<StreamDesc> &dstreams, const void *doffsets) {
-                       return sort_segmented_device(o, key_type, ascending, num, n_segments, (const int64_t *)doffsets, dstreams, soa,
-                                                    stream, workspace, workspace_bytes, &g_last_stats);
-                     });
+  return call.done(sort_staged(call.dev, num, streams, offsets, (size_t)(n_segments + 1) * 8, stream, sort));
 }
 
 }  // namespace b200sort

@@ -36,32 +36,26 @@ static int topk_device(const Options &o, int key_type, bool largest, int64_t n_r
                        const std::vector<StreamDesc> &in, const std::vector<StreamDesc> &out, int64_t *out_index, bool soa,
                        cudaStream_t stream, void *caller_workspace, size_t workspace_bytes, b200sort_stats *stats) {
   const int kb = key_bytes_of(key_type);
-  const uint64_t launches_before = g_launches.load();
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  DevInfo di;
-  if (int rc = dev_info(dev, &di)) return rc;
+  DevSetup su;
+  if (int rc = su.open()) return rc;
   const TopkLayout tl = topk_layout(kb, n_rows, row_len, k, soa);
-  CacheGuard cache_guard;
-  unsigned char *ws = nullptr;
-  if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, tl.total, cache_guard, &ws)) return rc;
-  start_profile(o, false);
+  if (int rc = su.workspace(stream, caller_workspace, workspace_bytes, tl.total)) return rc;
 
   // 1. the selection: the k winners of every row, unordered, into (keys, out_index)
-  CUDA_TRY(cudaMemsetAsync(ws, 0, tl.zero_bytes, stream));
+  CUDA_TRY(cudaMemsetAsync(su.ws, 0, tl.zero_bytes, stream));
   TopkArgs a{};
   a.keys = (const unsigned char *)in[0].ptr; a.stride = in[0].elem_bytes; a.n_rows = (uint32_t)n_rows;
   a.row_len = row_len; a.k = k; a.cap = tl.cap; a.chunks_per_row = tl.chunks_per_row;
   a.ko = make_key_order(key_type, !largest);
-  a.rows = (TopkRow *)ws; a.hist = (unsigned long long *)(ws + tl.hist_off); a.ctrl = (TopkCtrl *)(ws + tl.ctrl_off);
-  a.item_row = (uint32_t *)(ws + tl.items_off);
-  for (int b = 0; b < 2; b++) { a.cand_key[b] = ws + tl.cand_key_off[b]; a.cand_pos[b] = (unsigned long long *)(ws + tl.cand_pos_off[b]); }
-  void *sel_keys = soa ? out[0].ptr : (void *)(ws + tl.keys_off);
-  a.out_keys = sel_keys; a.out_index = out_index; a.offsets = (int64_t *)(ws + tl.offsets_off);
-  const unsigned init_grid = (unsigned)std::min<int64_t>((n_rows + 256) / 256, (int64_t)di.sm_count * 8);
+  a.rows = (TopkRow *)su.ws; a.hist = (unsigned long long *)(su.ws + tl.hist_off); a.ctrl = (TopkCtrl *)(su.ws + tl.ctrl_off);
+  a.item_row = (uint32_t *)(su.ws + tl.items_off);
+  for (int b = 0; b < 2; b++) { a.cand_key[b] = su.ws + tl.cand_key_off[b]; a.cand_pos[b] = (unsigned long long *)(su.ws + tl.cand_pos_off[b]); }
+  void *sel_keys = soa ? out[0].ptr : (void *)(su.ws + tl.keys_off);
+  a.out_keys = sel_keys; a.out_index = out_index; a.offsets = (int64_t *)(su.ws + tl.offsets_off);
+  const unsigned init_grid = (unsigned)std::min<int64_t>((n_rows + 256) / 256, (int64_t)su.di.sm_count * 8);
   CUDA_TRY(launch(PK_SELECT, topk_init_kernel, init_grid, 256, 0, stream, a));
-  const unsigned pass_grid = (unsigned)std::min<int64_t>(n_rows * tl.chunks_per_row, (int64_t)di.sm_count * TOPK_PASS_CTAS_PER_SM);
-  const unsigned decide_grid = (unsigned)std::min<int64_t>(n_rows, (int64_t)di.sm_count * 8);
+  const unsigned pass_grid = (unsigned)std::min<int64_t>(n_rows * tl.chunks_per_row, (int64_t)su.di.sm_count * TOPK_PASS_CTAS_PER_SM);
+  const unsigned decide_grid = (unsigned)std::min<int64_t>(n_rows, (int64_t)su.di.sm_count * 8);
   // (key-width + 1 passes and key-width decisions, whatever the keys: rows with nothing left to do exit at once)
   for (int p = 0; p <= kb; p++) {
     a.pass = p;
@@ -75,8 +69,8 @@ static int topk_device(const Options &o, int key_type, bool largest, int64_t n_r
   if (k > 1) {
     const std::vector<StreamDesc> pairs = {{sel_keys, (uint32_t)kb}, {out_index, 8u}};
     b200sort_stats inner;
-    if (int rc = sort_segmented_device(o, key_type, !largest, n_rows * k, n_rows, a.offsets, pairs, true, stream, ws + tl.seg_off,
-                                       tl.total - tl.seg_off, &inner, /*keep_profile=*/true))
+    if (int rc = sort_segmented_device(o, key_type, !largest, n_rows * k, n_rows, a.offsets, pairs, true, stream, su.ws + tl.seg_off,
+                                       tl.total - tl.seg_off, &inner))
       return rc;
   }
 
@@ -90,17 +84,11 @@ static int topk_device(const Options &o, int key_type, bool largest, int64_t n_r
     g.s[g.n_streams++] = {(const unsigned char *)in[s].ptr, (unsigned char *)out[s].ptr, c, eb / c};
   }
   if (g.n_streams > 0) {
-    const unsigned grid = (unsigned)std::min<int64_t>((g.total + 255) / 256, (int64_t)di.sm_count * 16);
+    const unsigned grid = (unsigned)std::min<int64_t>((g.total + 255) / 256, (int64_t)su.di.sm_count * 16);
     CUDA_TRY(launch(PK_SELECT, topk_gather_kernel, grid, 256, 0, stream, g));
   }
-  *stats = call_stats(n_rows * row_len, in, kb, launches_before);
-  stats->algo = 4;
+  *stats = su.stats(n_rows * row_len, in, kb, ALGO_TOPK);
   return B200SORT_OK;
-}
-
-static bool ranges_overlap(const void *a, size_t a_bytes, const void *b, size_t b_bytes) {
-  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
-  return a_bytes != 0 && b_bytes != 0 && x < y + b_bytes && y < x + a_bytes;
 }
 
 // argument checks (all before any device work), then the selection on the arrays' device.  in / out as in topk_device,
@@ -118,29 +106,18 @@ static int topk_any(int key_type, int64_t n_rows, int64_t row_len, int64_t k, bo
   if ((uintptr_t)in[0].ptr % kb != 0 || (uintptr_t)out[0].ptr % kb != 0) return fail(B200SORT_EINVAL, "keys / records are not aligned to their key type");
   if ((uintptr_t)out_index % 8 != 0) return fail(B200SORT_EINVAL, "out_index is not 8-byte aligned");
   const size_t num = (size_t)(n_rows * row_len), sel = (size_t)(n_rows * k);
-  std::vector<std::pair<const void *, size_t>> outs = {{out_index, sel * 8}};
+  std::vector<ByteRange> ins, outs = {{out_index, sel * 8}};
+  for (const StreamDesc &d : in) ins.push_back({d.ptr, num * d.elem_bytes});
   for (const StreamDesc &d : out) outs.push_back({d.ptr, sel * d.elem_bytes});
-  for (const StreamDesc &d : in)
-    for (const auto &w : outs)
-      if (ranges_overlap(d.ptr, num * d.elem_bytes, w.first, w.second)) return fail(B200SORT_EINVAL, "an output overlaps an input");
+  if (int rc = check_disjoint(ins, outs)) return rc;
 
-  // device arrays only, all on one device
-  if (int rc = require_device()) return rc;
   std::vector<StreamDesc> all = in;
   all.insert(all.end(), out.begin(), out.end());
   all.push_back({out_index, 8u});
-  for (const StreamDesc &d : all) {
-    Side sd;
-    if (int rc = side_of(d.ptr, &sd)) return rc;
-    if (sd == SIDE_HOST) return fail(B200SORT_EUNSUPPORTED, "top-k takes device arrays only; an array is in host memory");
-  }
-  Side side;
-  int dev = 0;
-  if (int rc = arrays_side(all, nullptr, &side, &dev)) return rc;
-  DeviceScope scope;
-  if (int rc = scope.enter(dev)) return rc;
-  return topk_device(options(), key_type, largest, n_rows, row_len, k, in, out, out_index, soa, (cudaStream_t)stream_v, workspace,
-                     workspace_bytes, &g_last_stats);
+  CallScope call;
+  if (int rc = call.enter(all, nullptr, "top-k")) return rc;
+  return call.done(topk_device(call.o, key_type, largest, n_rows, row_len, k, in, out, out_index, soa, (cudaStream_t)stream_v, workspace,
+                               workspace_bytes, &call.stats));
 }
 
 // the checks of the three counts: EINVAL unless 0 <= k <= row_len, 0 <= n_rows < 2^31 and n_rows * row_len fits

@@ -1,5 +1,5 @@
-// unique_host.cuh -- host side of unique (b200sort_unique; kernels in unique.cuh).  Included at the end of b200sort.cu,
-// after topk_host.cuh (it uses that file's ranges_overlap).
+// unique_host.cuh -- host side of unique (b200sort_unique; kernels in unique.cuh).  Included at the end of b200sort.cu
+// (it uses that file's internals).
 #pragma once
 
 namespace b200sort {
@@ -32,42 +32,41 @@ static UniqueLayout unique_layout(int kb, int64_t num, bool consecutive, bool wi
   return u;
 }
 
-// unique of device arrays on the current device, num >= 1
+// unique of device arrays on the current device
 static int unique_device(const Options &o, int key_type, int64_t num, bool consecutive, const void *keys, void *out_keys,
                          int64_t *out_counts, int64_t *out_inverse, int64_t *out_num_unique, cudaStream_t stream,
                          void *caller_workspace, size_t workspace_bytes, b200sort_stats *stats) {
   const int kb = key_bytes_of(key_type);
-  const uint64_t launches_before = g_launches.load();
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  DevInfo di;
-  if (int rc = dev_info(dev, &di)) return rc;
+  const std::vector<StreamDesc> in = {{const_cast<void *>(keys), (uint32_t)kb}};
+  DevSetup su;
+  if (num == 0) {  // U = 0 is all there is to write
+    CUDA_TRY(cudaMemsetAsync(out_num_unique, 0, 8, stream));
+    *stats = su.stats(0, in, kb, ALGO_UNIQUE);
+    return B200SORT_OK;
+  }
+  if (int rc = su.open()) return rc;
   const UniqueLayout ul = unique_layout(kb, num, consecutive, out_inverse != nullptr);
-  CacheGuard cache_guard;
-  unsigned char *ws = nullptr;
-  if (int rc = acquire_workspace(dev, stream, caller_workspace, workspace_bytes, ul.total, cache_guard, &ws)) return rc;
-  start_profile(o, false);
-  CUDA_TRY(cudaMemsetAsync(ws, 0, ul.ctrl_bytes, stream));
+  if (int rc = su.workspace(stream, caller_workspace, workspace_bytes, ul.total)) return rc;
+  CUDA_TRY(cudaMemsetAsync(su.ws, 0, ul.ctrl_bytes, stream));
 
   UniqueArgs a{};
   a.keys = (const unsigned char *)keys;
   if (!consecutive) {
     // 1. a copy of the keys (and their positions, for the inverse), sorted by the whole-array sort
-    unsigned char *copy = ws + ul.keys_off, *idx = ws + ul.index_off;
+    unsigned char *copy = su.ws + ul.keys_off, *idx = su.ws + ul.index_off;
     CUDA_TRY(cudaMemcpyAsync(copy, keys, (size_t)num * kb, cudaMemcpyDeviceToDevice, stream));
     std::vector<StreamDesc> sorted = {{copy, (uint32_t)kb}};
     if (ul.index_bytes) {
-      const unsigned grid = (unsigned)std::min<int64_t>((num + 255) / 256, (int64_t)di.sm_count * 8);
+      const unsigned grid = (unsigned)std::min<int64_t>((num + 255) / 256, (int64_t)su.di.sm_count * 8);
       if (ul.index_bytes == 4) CUDA_TRY(launch(PK_UNIQUE, iota_kernel, grid, 256, 0, stream, (uint32_t *)idx, num));
       else CUDA_TRY(launch(PK_UNIQUE, unique_iota64_kernel, grid, 256, 0, stream, (unsigned long long *)idx, num));
       sorted.push_back({idx, ul.index_bytes});
       a.index = idx;
     }
     if (num > 1) {
-      DevSortOpts xo;
-      xo.keep_profile = true;
       b200sort_stats inner;
-      if (int rc = sort_device(o, key_type, true, num, sorted, stream, ws + ul.region_off, ul.total - ul.region_off, xo, &inner))
+      if (int rc = sort_device(o, key_type, true, num, sorted, stream, su.ws + ul.region_off, ul.total - ul.region_off, DevSortOpts(),
+                               &inner))
         return rc;
     }
     a.keys = copy;
@@ -77,20 +76,19 @@ static int unique_device(const Options &o, int key_type, int64_t num, bool conse
   a.num = num; a.n_tiles = ul.n_tiles;
   a.vec = ((uintptr_t)a.keys & 15) == 0 ? 1u : 0u;
   a.out_keys = out_keys; a.out_inverse = out_inverse; a.out_num_unique = out_num_unique;
-  a.start = out_counts ? (int64_t *)(ws + ul.region_off) : nullptr;
-  a.ticket = (uint32_t *)ws; a.status = (uint64_t *)(ws + 256);
+  a.start = out_counts ? (int64_t *)(su.ws + ul.region_off) : nullptr;
+  a.ticket = (uint32_t *)su.ws; a.status = (uint64_t *)(su.ws + 256);
   CUDA_TRY(with_kb(kb, [&](auto K) {
     constexpr int KB = decltype(K)::value;
     auto *k = ul.index_bytes == 4 ? unique_scan_kernel<KB, 4> : ul.index_bytes == 8 ? unique_scan_kernel<KB, 8> : unique_scan_kernel<KB, 0>;
     return launch(PK_UNIQUE, k, (unsigned)ul.n_tiles, UNQ_THREADS, 0, stream, a);
   }));
   if (out_counts) {
-    const unsigned grid = (unsigned)std::min<int64_t>((num + 255) / 256, (int64_t)di.sm_count * 16);
+    const unsigned grid = (unsigned)std::min<int64_t>((num + 255) / 256, (int64_t)su.di.sm_count * 16);
     CUDA_TRY(launch(PK_UNIQUE, unique_counts_kernel, grid, 256, 0, stream, (const int64_t *)a.start, (const int64_t *)out_num_unique,
                     out_counts));
   }
-  *stats = call_stats(num, {{const_cast<void *>(keys), (uint32_t)kb}}, kb, launches_before);
-  stats->algo = 5;
+  *stats = su.stats(num, in, kb, ALGO_UNIQUE);
   return B200SORT_OK;
 }
 
@@ -109,41 +107,17 @@ static int unique_any(int key_type, int64_t num, bool consecutive, const void *k
   if (((uintptr_t)out_counts | (uintptr_t)out_inverse | (uintptr_t)out_num_unique) % 8 != 0)
     return fail(B200SORT_EINVAL, "out_counts, out_inverse and out_num_unique must be 8-byte aligned");
   const size_t n = (size_t)num;
-  const std::pair<const void *, size_t> outs[4] = {{out_keys, n * kb}, {out_counts, n * 8}, {out_inverse, n * 8}, {out_num_unique, 8}};
-  for (int i = 0; i < 4; i++) {
-    if (outs[i].first == nullptr) continue;
-    if (ranges_overlap(keys, n * kb, outs[i].first, outs[i].second)) return fail(B200SORT_EINVAL, "an output overlaps the input");
-    for (int j = 0; j < i; j++)
-      if (outs[j].first && ranges_overlap(outs[j].first, outs[j].second, outs[i].first, outs[i].second))
-        return fail(B200SORT_EINVAL, "two outputs overlap");
-  }
+  if (int rc = check_disjoint({{keys, n * kb}}, {{out_keys, n * kb}, {out_counts, n * 8}, {out_inverse, n * 8}, {out_num_unique, 8}}))
+    return rc;
   if (num == 0 && out_num_unique == nullptr) return B200SORT_OK;
 
-  // device arrays only, all on one device
-  if (int rc = require_device()) return rc;
   std::vector<StreamDesc> all;
   for (const void *p : {keys, (const void *)out_keys, (const void *)out_counts, (const void *)out_inverse, (const void *)out_num_unique})
     if (p != nullptr) all.push_back({const_cast<void *>(p), 1u});
-  for (const StreamDesc &d : all) {
-    Side sd;
-    if (int rc = side_of(d.ptr, &sd)) return rc;
-    if (sd == SIDE_HOST) return fail(B200SORT_EUNSUPPORTED, "unique takes device arrays only; an array is in host memory");
-  }
-  Side side;
-  int dev = 0;
-  if (int rc = arrays_side(all, nullptr, &side, &dev)) return rc;
-  DeviceScope scope;
-  if (int rc = scope.enter(dev)) return rc;
-  const cudaStream_t stream = (cudaStream_t)stream_v;
-  if (num == 0) {
-    const uint64_t launches_before = g_launches.load();
-    CUDA_TRY(cudaMemsetAsync(out_num_unique, 0, 8, stream));
-    g_last_stats = call_stats(0, {{const_cast<void *>(keys), (uint32_t)kb}}, kb, launches_before);
-    g_last_stats.algo = 5;
-    return B200SORT_OK;
-  }
-  return unique_device(options(), key_type, num, consecutive, keys, out_keys, out_counts, out_inverse, out_num_unique, stream,
-                       workspace, workspace_bytes, &g_last_stats);
+  CallScope call;
+  if (int rc = call.enter(all, nullptr, "unique")) return rc;
+  return call.done(unique_device(call.o, key_type, num, consecutive, keys, out_keys, out_counts, out_inverse, out_num_unique,
+                                 (cudaStream_t)stream_v, workspace, workspace_bytes, &call.stats));
 }
 
 }  // namespace b200sort

@@ -51,6 +51,11 @@ def test_argument_errors():
     assert _soa(K, 8, 4, 250, 10, OK, OI, 64, ptrs, (ctypes.c_uint32 * 64)(*([1] * 64)), outs) == -2
     # a NULL output payload
     assert _soa(K, 8, 4, 250, 10, OK, OI, 1, ptrs, (ctypes.c_uint32 * 1)(1), None) == -1
+    # two outputs overlapping each other: the key output inside out_index, an output payload inside the key output
+    assert _soa(K, 8, 4, 250, 10, OI + 8, OI) == -1
+    assert b"two outputs overlap" in L.b200sort_last_error()
+    assert _soa(K, 8, 4, 250, 10, OK, OI, 1, ptrs, (ctypes.c_uint32 * 1)(1), (ctypes.c_void_p * 1)(OK + 4)) == -1
+    assert b"two outputs overlap" in L.b200sort_last_error()
     # AoS record sizes: 24 (not a power of two), 4 for an 8-byte key
     for rb in (24, 4):
         assert L.b200sort_topk_aos(K, 6, rb, 1, 10, 1, 1, OK, OI, None, None, 0) == -3
